@@ -6,6 +6,7 @@ Mpoints/s and frames/s at 1024x768 on 1/2/4/8 B200, % of HBM roofline).
     python bench.py --impl reference ...                   # the reference's own CPU code on the host cores
     python bench.py --config {0..4}                        # another BASELINE.json config (default 2, the metric's)
     python bench.py --scaling weak                         # 4096 frames PER GPU instead of 4096/G (default: strong)
+    python bench.py --dump-outputs DIR                     # also write the last timed step's results to DIR/*.npy
 
 A "step" is one pass of the whole chain (transform -> height-band labels -> per-step reductions -> Stairs
 records on the host) over one batch of synthetic frames that is already resident in HBM. BASELINE.json configs[2]
@@ -27,6 +28,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the tree may be read-only: nothing is cached in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -34,6 +36,9 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 ALGO_BYTES_PER_POINT = 13  # 12 B packed f32 xyz read + 1 B u8 label written (SURVEY.md 8(d))
 NOISY = dict(noise_sigma=0.0025, dropout=0.03, n_holes=3)
 BASE_SEED = 20261017
+DUMP_SEED = 7  # which frames / pixels --dump-outputs samples when the results exceed its budget
+DUMP_MAX_FRAMES = 4096  # per-frame results (steps, plateaus, histograms, frame info) of at most this many frames
+DUMP_LABEL_VALUES = 1 << 21  # labels: at most this many (frame, pixel) values (all dumped arrays stay below 64 MB)
 # BASELINE.json configs (SURVEY.md 8(d)). frames: the batch of the config (global); steps: range of the staircase's
 # step count per frame, (0, 0) = the base scene itself.
 CONFIGS = {
@@ -300,6 +305,42 @@ def parity_block(det, A, cfg, xf, ref, xyz_sample):
             "ok": lab_bad == 0 and hist_bad == 0 and count_bad == 0 and status_bad == 0 and max_err < 1e-4 and not other}
 
 
+def dump_outputs(det, A, out_dir, first, frames, N):
+    """What the timed call hands its caller for each frame (ssd_gpu_get_frame_info / _get_steps / _get_plateaus /
+    _get_histogram / _get_labels), as float64 / float32 .npy files under out_dir. Frames beyond DUMP_MAX_FRAMES and labels
+    beyond DUMP_LABEL_VALUES are a fixed seeded sample (same arguments, same sample); frame_index holds the global frame ids."""
+    rng = np.random.default_rng(DUMP_SEED)
+    sel = np.arange(frames) if frames <= DUMP_MAX_FRAMES else np.sort(rng.choice(frames, DUMP_MAX_FRAMES, replace=False))
+    n = len(sel)
+    info = np.zeros((n, len(A.FrameInfo._fields_)), np.float64)
+    steps = np.zeros((n, A.MAX_STEPS, 9), np.float64)  # height, then the quadrilateral's 4 corners (x, y); zero past n_steps
+    pfields = ("height", "hmin", "hmax", "n_points", "valid", "outlined", "n_in_quad", "quad_status", "mean_z")
+    plats = np.zeros((n, A.MAX_PLATEAUS, len(pfields) + 8), np.float64)  # the fields above, then quad_world; zero past n_plateaus
+    hist = np.zeros((n, A.MAX_BINS), np.float32)  # zero past n_bins
+    for i, f in enumerate(sel):
+        fi = det.frame_info(int(f))
+        info[i] = [getattr(fi, k) for k, _ in A.FrameInfo._fields_]
+        st, _ = det.steps(int(f))
+        for k, (h, q) in enumerate(st):
+            steps[i, k, 0], steps[i, k, 1:] = h, np.asarray(q).ravel()
+        pl, K = det.plateaus(int(f))
+        p = np.ctypeslib.as_array(pl)[:K]
+        plats[i, :K, :len(pfields)] = np.stack([p[k].astype(np.float64) for k in pfields], 1)
+        plats[i, :K, len(pfields):] = p["quad_world"].reshape(K, 8)
+        hg = det.histogram(int(f))
+        hist[i, :len(hg)] = hg
+    n_lab = max(1, min(n, DUMP_LABEL_VALUES // N))
+    lab_frames = sel[np.sort(rng.choice(n, n_lab, replace=False))]
+    pix = np.arange(N) if N <= DUMP_LABEL_VALUES else np.sort(rng.choice(N, DUMP_LABEL_VALUES, replace=False))
+    pix_type = np.float32 if N <= 1 << 24 else np.float64  # float32 holds every pixel index below 2^24 exactly
+    labels = np.stack([det.labels(int(f))[pix] for f in lab_frames]).astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"frame_index": (first + sel).astype(np.float64), "frame_info": info, "steps": steps, "plateaus": plats, "histogram": hist,
+              "labels": labels, "labels_frame_index": (first + lab_frames).astype(np.float64), "labels_pixel_index": pix.astype(pix_type)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def latency_block(S, A, conf, device, reps=60):
     """The reference's real use is one frame per call (detect-stairs.cpp:36-42): per-call latency of one frame through the C ABI,
     device-resident vertices / host vertices / host z16 depth frame (pinned). Median and min of `reps` calls, CUDA events."""
@@ -407,6 +448,8 @@ def run_ours(args):
     barrier_sync()
     wall_ms = (time.perf_counter() - t_wall0) * 1e3
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(det, A, args.dump_outputs, first, frames, N)
     my_ms = sum(dev_ms)
     step_counts = det.n_steps_all(frames)
     n_steps_found = int(step_counts.sum())
@@ -646,7 +689,13 @@ def main():
     ap.add_argument("--parity-frames", type=int, default=16, help="benchmarked frames checked against the reference in the same run (rank 0)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-latency", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0's frames) to DIR/<name>.npy, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

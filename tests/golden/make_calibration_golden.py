@@ -1,7 +1,7 @@
 """Generate tests/golden/calibration/ -- a pair of calibration text files in the reference's own formats
 (calibrationTriangle.cpp:127-146 save(), geometricCalibration.cpp:43-71 savePoints()) and the transformation the
 REFERENCE's GeometricCalibration::load() builds from them (oracle/_ref, reference TUs compiled by path).
-Run in the build container, where /root/reference exists:   python tests/golden/make_calibration_golden.py
+Run with SSD_REFERENCE_DIR set to the original project's sources:   python tests/golden/make_calibration_golden.py
 """
 import ctypes as C
 import json
@@ -51,7 +51,7 @@ def xf_dict(xf):
 
 
 def main():
-    assert H.ref_available(), "needs /root/reference"
+    assert H.ref_available(), "needs SSD_REFERENCE_DIR (the original project's sources)"
     os.makedirs(OUT, exist_ok=True)
     # a camera 1.3 m above the floor looking 48 degrees down sees the three marks of a 2.2 m wide triangle
     sc = S.default_scene(640, 480, cam_height=1.3, cam_pitch_deg=48.0)

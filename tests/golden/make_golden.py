@@ -1,5 +1,5 @@
 """Generate the golden vectors in tests/golden/ from the REFERENCE ITSELF (oracle/_ref: the reference's
-translation units compiled by path, see oracle/Makefile). Run in the build container, where /root/reference exists:
+translation units compiled by path, see oracle/Makefile). Run with SSD_REFERENCE_DIR set to the original project's sources:
 
     python tests/golden/make_golden.py
 
@@ -40,7 +40,7 @@ def scene_fields(sc):
 
 
 def main():
-    assert H.ref_available(), "needs /root/reference"
+    assert H.ref_available(), "needs SSD_REFERENCE_DIR (the original project's sources)"
     for name, (w, h), kw, ridx in CASES:
         cfg = S.default_config(w, h)
         ref = H.load_ref(cfg)

@@ -25,7 +25,7 @@ from test_oracle_golden import load_case  # noqa: E402
 
 
 def main():
-    assert H.ref_available(), "needs /root/reference"
+    assert H.ref_available(), "needs SSD_REFERENCE_DIR (the original project's sources)"
     out = {}
     for i, path in enumerate(sorted(glob.glob(os.path.join(HERE, "*.npz")))):
         z, meta, sc, xf = load_case(path)

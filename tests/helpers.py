@@ -1,9 +1,12 @@
 """Test infrastructure: loaders for the oracle (C restatement), the compiled reference (oracle/_ref)
 and scene helpers. Only tests/, bench.py's CPU legs and __graft_entry__.smoke() use this."""
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 
 import numpy as np
 
@@ -12,7 +15,8 @@ sys.path.insert(0, ROOT)
 from stair_step_detector_b200 import _abi as A  # noqa: E402
 
 ORACLE_DIR = os.path.join(ROOT, "oracle")
-REF_SRC = "/root/reference"
+# the original project's sources (the C++ stair-step-detector); the tests that compare with it skip without them
+REF_SRC = os.environ.get("SSD_REFERENCE_DIR", "")
 _vp = C.c_void_p
 _P = C.POINTER
 
@@ -28,8 +32,18 @@ def ref_tag(cfg):
 
 
 def build_oracle():
-    subprocess.run(["make", "-s", "-C", ORACLE_DIR, "oracle"], check=True)
-    return os.path.join(ORACLE_DIR, "libssd_oracle.so")
+    """oracle/libssd_oracle.so, rebuilt if stale; in a read-only tree a stale library is rebuilt in a temporary directory"""
+    path = os.path.join(ORACLE_DIR, "libssd_oracle.so")
+    if os.access(ORACLE_DIR, os.W_OK):
+        subprocess.run(["make", "-s", "-C", ORACLE_DIR, "oracle"], check=True)
+        return path
+    if subprocess.run(["make", "-s", "-q", "-C", ORACLE_DIR, "oracle"]).returncode == 0:
+        return path
+    tmp = tempfile.mkdtemp(prefix="ssd_oracle_")
+    atexit.register(shutil.rmtree, tmp, True)
+    path = os.path.join(tmp, "libssd_oracle.so")
+    subprocess.run(["make", "-s", "-C", ORACLE_DIR, "oracle", f"ORACLE_LIB={path}"], check=True)
+    return path
 
 
 def load_oracle():
@@ -51,7 +65,7 @@ def load_oracle():
 
 
 def ref_available():
-    return os.path.isdir(REF_SRC)
+    return bool(REF_SRC) and os.path.isdir(REF_SRC)
 
 
 def ref_path(cfg):
@@ -59,10 +73,10 @@ def ref_path(cfg):
 
 
 def build_ref(cfg):
-    """Compile the reference TUs by path for this configuration (needs /root/reference)."""
+    """Compile the reference TUs by path for this configuration (needs SSD_REFERENCE_DIR)."""
     path = ref_path(cfg)
     if ref_available():
-        subprocess.run(["make", "-s", "-C", ORACLE_DIR, "ref", f"W={cfg.width}", f"H={cfg.height}",
+        subprocess.run(["make", "-s", "-C", ORACLE_DIR, "ref", f"REF={REF_SRC}", f"W={cfg.width}", f"H={cfg.height}",
                         f"XMIN={cfg.x_min:g}", f"XMAX={cfg.x_max:g}", f"YMIN={cfg.y_min:g}", f"YMAX={cfg.y_max:g}",
                         f"ZMIN={cfg.z_min:g}", f"ZMAX={cfg.z_max:g}", f"TAG={ref_tag(cfg)}"], check=True)
     return path if os.path.exists(path) else None
@@ -101,6 +115,49 @@ def load_ref(cfg):
 
 def ptr(a):
     return a.ctypes.data_as(_vp)
+
+
+def hexf(v):
+    """a double as exact text (float.hex) for golden JSON files; float.fromhex reads it back"""
+    return float(v).hex()
+
+
+def unhexf(v):
+    return np.array([float.fromhex(x) for x in v]) if isinstance(v, list) else float.fromhex(v)
+
+
+def digest(a):
+    import hashlib
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+_PLATEAU_INTS = ("height", "hmin", "hmax", "n_points", "valid", "outlined", "n_in_quad", "quad_status")
+
+
+def frame_record(r, status_mask):
+    """a FrameResult as JSON: labels as a SHA-256 digest, doubles exact, status with the bits of status_mask only"""
+    info = {k: int(v) for k, v in r.info.items()}
+    info["status"] &= status_mask
+    return dict(labels_sha256=digest(r.labels), hist=[int(v) for v in r.hist], info=info,
+                plateaus=[dict({k: int(p[k]) for k in _PLATEAU_INTS}, quad_world=[hexf(v) for v in p["quad_world"].ravel()], mean_z=hexf(p["mean_z"]))
+                          for p in r.plateaus],
+                steps=[dict(height=hexf(s["height"]), quad=[hexf(v) for v in s["quad"].ravel()]) for s in r.steps])
+
+
+def frame_from_record(d):
+    """frame_record back to a FrameResult (labels None: compare d["labels_sha256"] with digest(labels))"""
+    plats = [dict({k: p[k] for k in _PLATEAU_INTS}, quad_world=unhexf(p["quad_world"]).reshape(4, 2), mean_z=unhexf(p["mean_z"]))
+             for p in d["plateaus"]]
+    steps = [dict(height=unhexf(s["height"]), quad=unhexf(s["quad"]).reshape(4, 2)) for s in d["steps"]]
+    return FrameResult(None, np.array(d["hist"], np.uint32), dict(d["info"]), plats, steps)
+
+
+def compare_with_record(d, o, tol):
+    """compare_results of a stored frame_record against the FrameResult o, labels by digest"""
+    bad = compare_results(frame_from_record(d), o, tol=tol)
+    if digest(o.labels) != d["labels_sha256"]:
+        bad.append("labels differ")
+    return bad
 
 
 class FrameResult:

@@ -72,6 +72,28 @@ def run_frames(S, oracle, cfg, scenes, max_bad=0):
         return out
 
 
+@pytest.mark.parametrize("key", ["frames_random_scenes/320x240", "frames_random_scenes/640x480", "frames_random_scenes/1024x768",
+                                 "frames_hires/2560x1920", "frames_hires/4096x3072"])
+def test_against_the_reference_runs(S, key):
+    """straight against the compiled reference without the oracle in between: the CUDA path on the seeded frames of
+    test_oracle_vs_ref against the reference's results for them (tests/golden/reference_runs.json)"""
+    import test_oracle_vs_ref as R
+    kind, size = key.split("/")
+    w, h = (int(v) for v in size.split("x"))
+    if kind == "frames_hires":
+        _, _, ck, sk, n = next(c for c in R.HIRES_CASES if c[:2] == (w, h))
+        inputs = R.frames_hires_inputs(S, w, h, ck, sk, n)
+    else:
+        inputs = R.frames_random_scenes_inputs(S, w, h, {320: 10, 640: 6, 1024: 3}[w])
+    want = R.stored(key)
+    for i, (cfg, xf, xyz) in enumerate(inputs):
+        with S.Detector(cfg, xf, max_frames=1) as det:
+            det.process_host(xyz[None])
+            g = gpu_result(S, det, 0)
+        assert not H.compare_with_record(want[i], g, tol=TOL), (i, H.compare_with_record(want[i], g, tol=TOL))
+        assert (g.info["status"] & ~R.QUIRKS) == want[i]["info"]["status"], i
+
+
 @pytest.mark.parametrize("w,h", [(1024, 768), (640, 480), (320, 240)])
 def test_clean_frame(S, oracle, w, h):
     cfg = S.default_config(w, h)

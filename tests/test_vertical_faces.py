@@ -1,9 +1,9 @@
 """Vertical faces (risers) from the remainder: SURVEY.md 8(f) row 4, second half. The reference collects the remainder and leaves
 "TODO use remainder to detect vertical faces" (pointcloud.cpp:283-293): there is no reference behaviour, so the checker is the
 oracle's restatement of the DEFINITION in include/ssd_gpu.h (ssd_gpu_riser) -- parity for this row is unpinned by construction --
-cross-checked here against an independent numpy evaluation and against the compiled reference's own label / band output."""
+cross-checked here against an independent numpy evaluation and against the compiled reference's own label / band output
+(live where the compiled reference is available, else its stored output, tests/golden/reference_runs.json)."""
 import ctypes as C
-import os
 
 import numpy as np
 import pytest
@@ -66,19 +66,35 @@ def test_oracle_risers_match_the_definition(S, oracle, w, h):
     assert seen > 0
 
 
-def test_risers_from_the_reference_labels(S, oracle):
-    """the compiled reference's remainder (its labels) and bands give the same risers as the oracle's"""
+def riser_inputs(S):
     cfg = S.default_config(640, 480)
-    if not (os.path.exists(H.ref_path(cfg)) or H.ref_available()):
-        pytest.skip("compiled reference not available")
-    ref = H.load_ref(cfg)
     base = S.default_scene(640, 480, **NOISY)
     xf = S.scene_transform(base)
     for i in range(3):
         sc = S.randomize_scene(base, 4200, i, 3, 8)
-        xyz = S.deproject_host(sc, S.synth_depth_host(sc)).reshape(-1, 3)
-        r = H.ref_process(ref, cfg, xf, xyz)
-        assert same(H.oracle_vertical_faces(oracle, cfg, xf, xyz), H.oracle_vertical_faces(oracle, cfg, xf, xyz, r.labels, r.plateaus))
+        yield cfg, xf, S.deproject_host(sc, S.synth_depth_host(sc)).reshape(-1, 3)
+
+
+def reference_bands(r):
+    """what the riser definition takes from a frame: the labels (as a digest) and the plateaus' height bands"""
+    return dict(labels_sha256=H.digest(r.labels), bands=[[int(p["hmin"]), int(p["hmax"])] for p in r.plateaus])
+
+
+def test_risers_from_the_reference_labels(S, oracle):
+    """the compiled reference's remainder (its labels) and bands give the same risers as the oracle's: live, the risers from
+    the reference's labels and bands are computed; from the stored output, its labels and bands must equal the oracle's"""
+    import test_oracle_vs_ref as R
+    ref = H.load_ref(S.default_config(640, 480))
+    want = None if ref is not None else R.stored("risers_from_the_reference_labels")
+    for i, (cfg, xf, xyz) in enumerate(riser_inputs(S)):
+        mine = H.oracle_vertical_faces(oracle, cfg, xf, xyz)
+        if ref is not None:
+            r = H.ref_process(ref, cfg, xf, xyz)
+            assert same(mine, H.oracle_vertical_faces(oracle, cfg, xf, xyz, r.labels, r.plateaus))
+            continue
+        o = H.oracle_process(oracle, cfg, xf, xyz)
+        assert reference_bands(o) == want[i], i
+        assert same(mine, H.oracle_vertical_faces(oracle, cfg, xf, xyz, o.labels, o.plateaus))
 
 
 def test_no_riser_without_two_plateaus(S, oracle):
