@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SSD_GPU_ABI_VERSION 2
+#define SSD_GPU_ABI_VERSION 3
 
 /* ---- limits ---- */
 #define SSD_GPU_MAX_BINS 253      /* height-histogram bins; bin codes are u8, 253..255 reserved */
@@ -179,6 +179,42 @@ int ssd_gpu_deproject_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const ss
 /* Run every chunk on one stream (no overlap between chunks): with STAGE_TIMING the event brackets are then the kernels' own durations. */
 #define SSD_FLAG_SINGLE_STREAM 0x4
 int ssd_gpu_process_device_ex(ssd_gpu_ctx *ctx, const float *xyz_dev, int n_frames, int flags);
+
+/*
+ * ---- per-frame cameras: frames of many camera mountings (or of a camera whose pose changes) in one batched call ----
+ * A context binds one transform at ssd_gpu_create. A camera table adds any number of others: the camera calls below take the
+ * camera of each frame, and frame i is processed exactly as a context created with camera camera_of_frame[i]'s transform
+ * would process it (labels, histogram, plateaus, steps, overlay, risers: bit for bit). Replaces several Pointcloud instances,
+ * one per camera (pointcloud.cpp:602-606), by one call. The configuration (frame size, measuring range) stays per context.
+ *   xf     CameraToWorld + ToExternalWorld of the camera; checked as ssd_gpu_create checks its own.
+ *   a_inv  WorldToCamera's _aInv (ssd_make_transform_ex): projects the overlay when ssd_gpu_set_overlay has switched it on
+ *          (the a_inv / intrinsics given to ssd_gpu_set_overlay still apply to the plain calls only).
+ *   intr   deprojection of depth-frame input (fx, fy non-zero, depth_unit > 0 for every camera a depth call uses) and the
+ *          overlay's projection; may be all zero for cameras that only see vertex input without overlay.
+ * ssd_gpu_set_cameras replaces the table (n_cameras >= 1, no upper limit; n_cameras == 0 frees it) and leaves the results of the last call
+ * readable. It derives every camera's parameters and, for depth input, its deprojection tables once, on the host and with one
+ * kernel: a call then only uploads camera_of_frame (4 bytes per frame).
+ * camera_of_frame: host array of n_frames indices into the table. Checked before anything is launched: a camera call without a
+ * table returns SSD_E_STATE, an index outside [0, n_cameras) SSD_E_RANGE, a depth call that uses a camera without valid
+ * intrinsics SSD_E_INVALID_ARG; the results of the previous call stay readable. Camera calls run on the default chain only:
+ * SSD_GPU_PATH=records|wordrec|resident (and SSD_GPU_DEPTH_UNFUSED=1 for depth calls) return SSD_E_STATE.
+ * Results are read with the getters above; ssd_gpu_get_stats counts the whole call and reports the largest filter bounds of
+ * the cameras it used. A plain ssd_gpu_process_* call keeps using the context's own transform.
+ */
+typedef struct ssd_gpu_camera
+{
+  ssd_gpu_transform xf;
+  double a_inv[9];
+  ssd_gpu_intrinsics intr;
+} ssd_gpu_camera;
+int ssd_gpu_set_cameras(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, int n_cameras);
+int ssd_gpu_n_cameras(ssd_gpu_ctx *ctx);
+int ssd_gpu_process_cameras_host(ssd_gpu_ctx *ctx, const float *xyz_host, const int32_t *camera_of_frame, int n_frames);
+int ssd_gpu_process_cameras_device(ssd_gpu_ctx *ctx, const float *xyz_dev, const int32_t *camera_of_frame, int n_frames);
+/* flags: SSD_FLAG_STAGE_TIMING / SSD_FLAG_SINGLE_STREAM as for ssd_gpu_process_device_ex */
+int ssd_gpu_process_cameras_device_ex(ssd_gpu_ctx *ctx, const float *xyz_dev, const int32_t *camera_of_frame, int n_frames, int flags);
+int ssd_gpu_process_depth_cameras_host(ssd_gpu_ctx *ctx, const uint16_t *z16_host, const int32_t *camera_of_frame, int n_frames);
+int ssd_gpu_process_depth_cameras_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const int32_t *camera_of_frame, int n_frames);
 
 /* ---- results of the last process call ---- */
 /* Stairs of one frame: out[0..*n) ; replaces the value printed at pointcloud.cpp:624-625. */

@@ -111,6 +111,25 @@ def scene_transform_ex(scene):
     return xf, np.array(a_inv[:])
 
 
+def scene_camera(scene):
+    """The full camera record of a synthetic scene, for Detector.set_cameras: its transform, the camera transformation's
+    _aInv and the depth-stream intrinsics (ssd_gpu_camera)."""
+    xf, a_inv = scene_transform_ex(scene)
+    return make_camera(xf, a_inv, scene_intrinsics(scene))
+
+
+def make_camera(xf, a_inv=None, intrinsics=None):
+    """ssd_gpu_camera from a Transform, the 9 doubles of _aInv (overlay only) and Intrinsics (depth input and overlay; None: zero)."""
+    cam = A.Camera()
+    cam.xf = xf
+    if a_inv is not None:
+        for i, v in enumerate(np.asarray(a_inv, np.float64).ravel()):
+            cam.a_inv[i] = float(v)
+    if intrinsics is not None:
+        cam.intr = intrinsics
+    return cam
+
+
 def inverse3(a):
     """boost::qvm::inverse of a 3x3 (row-major 9 doubles) as Transformation_<3>(rp, rpMapping) computes _aInv."""
     src = (C.c_double * 9)(*[float(v) for v in np.asarray(a, np.float64).ravel()])
@@ -225,6 +244,47 @@ class Detector:
 
     def process_device(self, dev_ptr, n_frames, flags=0):
         self._ck(self._l.ssd_gpu_process_device_ex(self._h, dev_ptr, n_frames, flags), "ssd_gpu_process_device")
+
+    # ---- per-frame cameras ----
+    def set_cameras(self, cameras):
+        """Replace the camera table with a list of A.Camera (scene_camera / make_camera); an empty list frees it."""
+        arr = (A.Camera * max(1, len(cameras)))(*cameras)
+        self._ck(self._l.ssd_gpu_set_cameras(self._h, arr, len(cameras)), "ssd_gpu_set_cameras")
+
+    @property
+    def n_cameras(self):
+        return self._l.ssd_gpu_n_cameras(self._h)
+
+    @staticmethod
+    def _cams(camera_of_frame, n):
+        cams = np.ascontiguousarray(camera_of_frame, np.int32)
+        if cams.size != n:
+            raise ValueError(f"camera_of_frame has {cams.size} entries for {n} frames")
+        return cams
+
+    def process_cameras_host(self, xyz, camera_of_frame):
+        """xyz as for process_host; camera_of_frame: camera table index of each frame."""
+        xyz = np.ascontiguousarray(xyz, np.float32)
+        n = xyz.size // (self.n_points * 3)
+        cams = self._cams(camera_of_frame, n)
+        self._ck(self._l.ssd_gpu_process_cameras_host(self._h, _ptr(xyz), _ptr(cams), n), "ssd_gpu_process_cameras_host")
+        return n
+
+    def process_cameras_device(self, dev_ptr, camera_of_frame, n_frames, flags=0):
+        cams = self._cams(camera_of_frame, n_frames)
+        self._ck(self._l.ssd_gpu_process_cameras_device_ex(self._h, dev_ptr, _ptr(cams), n_frames, flags), "ssd_gpu_process_cameras_device")
+
+    def process_depth_cameras_host(self, depth, camera_of_frame):
+        """depth as for process_depth_host; each frame is deprojected with its camera's intrinsics."""
+        depth = np.ascontiguousarray(depth, np.uint16)
+        n = depth.size // self.n_points
+        cams = self._cams(camera_of_frame, n)
+        self._ck(self._l.ssd_gpu_process_depth_cameras_host(self._h, _ptr(depth), _ptr(cams), n), "ssd_gpu_process_depth_cameras_host")
+        return n
+
+    def process_depth_cameras_device(self, dev_ptr, camera_of_frame, n_frames):
+        cams = self._cams(camera_of_frame, n_frames)
+        self._ck(self._l.ssd_gpu_process_depth_cameras_device(self._h, dev_ptr, _ptr(cams), n_frames), "ssd_gpu_process_depth_cameras_device")
 
     # ---- results ----
     def steps(self, frame):

@@ -50,6 +50,11 @@ class Intrinsics(C.Structure):
                 ("depth_unit", C.c_float), ("reserved", C.c_int32 * 3)]
 
 
+class Camera(C.Structure):
+    """ssd_gpu_camera: one entry of a context's camera table (ssd_gpu_set_cameras)."""
+    _fields_ = [("xf", Transform), ("a_inv", C.c_double * 9), ("intr", Intrinsics)]
+
+
 class Overlay(C.Structure):
     _fields_ = [("px", (C.c_float * 2) * 4)]
 
@@ -113,6 +118,13 @@ PROTOTYPES = {
     "ssd_gpu_process_host": (C.c_int, [_vp, _vp, C.c_int]),
     "ssd_gpu_process_device": (C.c_int, [_vp, _vp, C.c_int]),
     "ssd_gpu_process_device_ex": (C.c_int, [_vp, _vp, C.c_int, C.c_int]),
+    "ssd_gpu_set_cameras": (C.c_int, [_vp, _P(Camera), C.c_int]),
+    "ssd_gpu_n_cameras": (C.c_int, [_vp]),
+    "ssd_gpu_process_cameras_host": (C.c_int, [_vp, _vp, _vp, C.c_int]),
+    "ssd_gpu_process_cameras_device": (C.c_int, [_vp, _vp, _vp, C.c_int]),
+    "ssd_gpu_process_cameras_device_ex": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int]),
+    "ssd_gpu_process_depth_cameras_host": (C.c_int, [_vp, _vp, _vp, C.c_int]),
+    "ssd_gpu_process_depth_cameras_device": (C.c_int, [_vp, _vp, _vp, C.c_int]),
     "ssd_gpu_process_depth_host": (C.c_int, [_vp, _vp, _P(Intrinsics), C.c_int]),
     "ssd_gpu_process_depth_device": (C.c_int, [_vp, _vp, _P(Intrinsics), C.c_int]),
     "ssd_gpu_deproject_device": (C.c_int, [_vp, _vp, _P(Intrinsics), C.c_int, _vp]),

@@ -62,9 +62,9 @@ std::vector<Quadrilateralf_t> Pointcloud::overlay(int frame) const
   return out;
 }
 
-std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, int nFrames, std::vector<unsigned> *status) const
+// overlay / vertical faces / camera table as last requested, once the context exists
+void Pointcloud::applySettings() const
 {
-  ensureContext(frames.width(), frames.height());
   if(_overlay && !_overlayApplied)
   {
     double aInv[9];
@@ -79,6 +79,18 @@ std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, i
       throw std::runtime_error(std::string("ssd_gpu_set_vertical_faces: ") + ssd_gpu_last_error(_ctx));
     _risersApplied = _risers;
   }
+  if(!_camerasApplied)
+  {
+    if(ssd_gpu_set_cameras(_ctx, _cameras.data(), static_cast<int>(_cameras.size())) != SSD_OK)
+      throw std::runtime_error(std::string("ssd_gpu_set_cameras: ") + ssd_gpu_last_error(_ctx));
+    _camerasApplied = true;
+  }
+}
+
+std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, int nFrames, std::vector<unsigned> *status) const
+{
+  ensureContext(frames.width(), frames.height());
+  applySettings();
   int rc;
   if(frames.z16)
     rc = frames.onDevice ? ssd_gpu_process_depth_device(_ctx, frames.z16, &frames.intrinsics, nFrames)
@@ -87,6 +99,49 @@ std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, i
     rc = frames.onDevice ? ssd_gpu_process_device(_ctx, frames.vertices, nFrames) : ssd_gpu_process_host(_ctx, frames.vertices, nFrames);
   if(rc != SSD_OK)
     throw std::runtime_error(std::string("ssd_gpu_process: ") + ssd_gpu_last_error(_ctx));
+  return collect(nFrames, status);
+}
+
+int Pointcloud::addCamera(const GeometricTransformation &trans, const ssd_gpu_intrinsics &intrinsics) const
+{
+  ssd_gpu_camera c{};
+  c.xf = trans.abi();
+  trans.abiInverse(c.a_inv);
+  c.intr = intrinsics;
+  _cameras.push_back(c);
+  _camerasApplied = false;
+  return static_cast<int>(_cameras.size()) - 1;
+}
+
+void Pointcloud::clearCameras() const
+{
+  _cameras.clear();
+  _camerasApplied = false;
+}
+
+std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, int nFrames, const std::vector<int32_t> &cameraOfFrame,
+                                             std::vector<unsigned> *status) const
+{
+  if(nFrames < 0 || cameraOfFrame.size() != static_cast<size_t>(nFrames))
+    throw std::invalid_argument("Pointcloud::processBatch: cameraOfFrame must hold one camera index per frame");
+  ensureContext(frames.width(), frames.height());
+  applySettings();
+  const int32_t *cam = cameraOfFrame.data();
+  int rc;
+  if(frames.z16)
+    rc = frames.onDevice ? ssd_gpu_process_depth_cameras_device(_ctx, frames.z16, cam, nFrames)
+                         : ssd_gpu_process_depth_cameras_host(_ctx, frames.z16, cam, nFrames);
+  else
+    rc = frames.onDevice ? ssd_gpu_process_cameras_device(_ctx, frames.vertices, cam, nFrames)
+                         : ssd_gpu_process_cameras_host(_ctx, frames.vertices, cam, nFrames);
+  if(rc != SSD_OK)
+    throw std::runtime_error(std::string("ssd_gpu_process_cameras: ") + ssd_gpu_last_error(_ctx));
+  return collect(nFrames, status);
+}
+
+// the Stairs of every frame of the last call
+std::vector<Stairs> Pointcloud::collect(int nFrames, std::vector<unsigned> *status) const
+{
   std::vector<Stairs> out(static_cast<size_t>(nFrames));
   if(status)
     status->assign(static_cast<size_t>(nFrames), 0u);

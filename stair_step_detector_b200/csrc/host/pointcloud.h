@@ -1,7 +1,8 @@
 // Host mirror of the reference's pipeline driver (pointcloud.h:32-42, pointcloud.cpp:602-626): same
 // constructor and process() signature. The per-frame chain runs as CUDA kernels behind the C ABI; process()
 // prints the same result line the reference prints. Added on top (the reference only prints):
-// detect() returns the Stairs value, processBatch() runs many independent frames in one call.
+// detect() returns the Stairs value, processBatch() runs many independent frames in one call, also frames of several
+// cameras (addCamera).
 #pragma once
 #include "camera.h"
 #include "configuration.h"
@@ -33,6 +34,16 @@ public:
   Stairs detect(const Camera::DepthFrame &frame) const;
   // nFrames frames stored back to back at frames.vertices
   std::vector<Stairs> processBatch(const Camera::DepthFrame &frames, int nFrames, std::vector<unsigned> *status = nullptr) const;
+  // Per-frame cameras (ssd_gpu_set_cameras): several Pointcloud instances, one per camera mounting, become one Pointcloud and
+  // one call. addCamera registers a camera -- its GeometricTransformation (abi(), abiInverse()) and the intrinsics of its depth
+  // stream (deprojection of z16 frames, overlay) -- and returns its index. processBatch with cameraOfFrame processes frame i as a
+  // Pointcloud built with camera cameraOfFrame[i]'s transformation would (frames.intrinsics is then unused: every z16 frame is
+  // deprojected with its camera's intrinsics).
+  int addCamera(const GeometricTransformation &trans, const ssd_gpu_intrinsics &intrinsics) const;
+  void clearCameras() const;
+  int cameraCount() const { return static_cast<int>(_cameras.size()); }
+  std::vector<Stairs> processBatch(const Camera::DepthFrame &frames, int nFrames, const std::vector<int32_t> &cameraOfFrame,
+                                   std::vector<unsigned> *status = nullptr) const;
   // per-pixel segment labels of frame `frame` of the last call (SSD_LABEL_* codes / plateau index)
   std::vector<uint8_t> labels(int frame = 0) const;
   // drawStairStep (reference pointcloud.cpp:583-597): project the corners of every detected step into the camera image
@@ -48,6 +59,8 @@ public:
 
 private:
   void ensureContext(int width, int height) const;
+  void applySettings() const;
+  std::vector<Stairs> collect(int nFrames, std::vector<unsigned> *status) const;
   const Window &_window;
   const GeometricTransformation &_transformation;
   mutable Configuration _config;
@@ -57,6 +70,8 @@ private:
   mutable bool _overlay = false, _overlayApplied = false;
   mutable bool _risers = false, _risersApplied = false;
   mutable ssd_gpu_intrinsics _overlayIntrinsics{};
+  mutable std::vector<ssd_gpu_camera> _cameras;
+  mutable bool _camerasApplied = true;
 };
 
 } // namespace stairs

@@ -181,6 +181,52 @@ struct OverlayDev
   int enabled, pad;
 };
 
+// Per-frame cameras (ssd_gpu_set_cameras). The kernels of the classic chain take a trailing CAM argument: NoCam (the default)
+// processes every frame with the launch's DevParams, the context's own camera; CamTable takes each frame's parameters from the
+// camera table, derived per camera by derive_params exactly as for a context created with that camera.
+struct NoCam
+{
+};
+struct CamTable
+{
+  const DevParams *params; // n_cameras
+  const OverlayDev *ov;    // n_cameras: drawStairStep projection of each camera (a_inv, intrinsics; enabled = 1)
+  const float *xn, *yn;    // n_cameras x W, n_cameras x H deprojection tables (depth input)
+  const float *unit;       // n_cameras: metres per depth unit
+  const int *cam;          // camera of each frame of the call
+  int frame0;              // first frame of the launch within the call
+};
+
+__device__ __forceinline__ int frame_camera(const CamTable &c, int frame)
+{
+  return __ldg(c.cam + c.frame0 + frame);
+}
+__device__ __forceinline__ const DevParams &frame_params(const DevParams &p, const NoCam &, int)
+{
+  return p;
+}
+// The block copies its frame's table entry into shared memory once; every thread of the block must call this before any
+// thread leaves the kernel.
+__device__ __forceinline__ const DevParams &frame_params(const DevParams &, const CamTable &c, int frame)
+{
+  __shared__ DevParams s_cam_params;
+  static_assert(sizeof(DevParams) % 8 == 0, "DevParams is copied in 8-byte words");
+  const unsigned long long *src = reinterpret_cast<const unsigned long long *>(c.params + frame_camera(c, frame));
+  unsigned long long *dst = reinterpret_cast<unsigned long long *>(&s_cam_params);
+  for(int i = threadIdx.x; i < (int)(sizeof(DevParams) / 8); i += blockDim.x)
+    dst[i] = __ldg(src + i);
+  __syncthreads();
+  return s_cam_params;
+}
+__device__ __forceinline__ const OverlayDev &frame_overlay(const OverlayDev &ov, const NoCam &, int)
+{
+  return ov;
+}
+__device__ __forceinline__ const OverlayDev &frame_overlay(const OverlayDev &ov, const CamTable &c, int frame)
+{
+  return ov.enabled ? c.ov[frame_camera(c, frame)] : ov;
+}
+
 struct P2d
 {
   double x, y;

@@ -13,6 +13,7 @@
 #include <cstring>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #ifndef SSD_PT_ITERS
@@ -89,6 +90,15 @@ struct ssd_gpu_ctx
   int stage_chunks = 0;
   float stage_ms[SSD_GPU_N_STAGES]{};
   int stage_launches[SSD_GPU_N_STAGES]{};
+  // camera table (ssd_gpu_set_cameras): per camera the derived parameters, the overlay projection and the deprojection tables
+  int n_cameras = 0;
+  std::vector<DevParams> cam_dp;         // host copies (filter bounds for ssd_gpu_get_stats)
+  std::vector<unsigned char> cam_depth_ok; // intrinsics admit depth input
+  DevParams *d_cam_dp = nullptr;
+  OverlayDev *d_cam_ov = nullptr;
+  float *d_cam_xn = nullptr, *d_cam_yn = nullptr, *d_cam_unit = nullptr;
+  int *d_cam_of_frame = nullptr;         // max_frames: camera of each frame of the current call
+  double stats_eps0 = 0, stats_eps1 = 0; // filter bounds of the last call (largest over its cameras)
 };
 
 #define CK(call)                                                                                         \
@@ -319,6 +329,21 @@ __global__ void k_deproject_tables(int W, int H, ssd_gpu_intrinsics in, float *_
     yn[i] = __fdiv_rn(__fsub_rn((float)i, in.ppy), in.fy);
 }
 
+// the same tables for every camera of a camera table: grid = (ceil(max(W, H) / 256), min(n_cameras, 65535)), cameras grid-strided
+__global__ void k_deproject_tables_cams(int W, int H, const ssd_gpu_camera *__restrict__ cams, int n_cameras, float *__restrict__ xn,
+                                        float *__restrict__ yn)
+{
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  for(int c = blockIdx.y; c < n_cameras; c += gridDim.y)
+  {
+    const ssd_gpu_intrinsics in = cams[c].intr;
+    if(i < W)
+      xn[(size_t)c * W + i] = __fdiv_rn(__fsub_rn((float)i, in.ppx), in.fx);
+    if(i < H)
+      yn[(size_t)c * H + i] = __fdiv_rn(__fsub_rn((float)i, in.ppy), in.fy);
+  }
+}
+
 // 4 consecutive pixels per thread: one 8-byte load, three 16-byte stores. grid = (ceil(N/4/256), frames). W % 4 == 0.
 __global__ void __launch_bounds__(256) k_deproject(int W, int N, float depth_unit, const float *__restrict__ xn, const float *__restrict__ yn,
                                                    const uint16_t *__restrict__ depth, float *__restrict__ xyz)
@@ -438,13 +463,140 @@ __global__ void k_single_camera_to_world(const __grid_constant__ DevParams p, co
   }
 }
 
+// The classic chain: k_transform_bin -> k_peaks -> k_label_bev -> k_outline -> k_frame_logic -> k_quad_reduce -> k_finalize
+// (+ k_riser_reduce). CAM = NoCam: every frame with the context's own camera; CamTable: each frame with its camera's parameters
+// (camera calls; the word-record variant is never taken there).
+template<class CAM>
+static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const SrcDepth &sd, int frame0, int nf, int *launches, cudaEvent_t *ev,
+                          const CAM cam)
+{
+#define STAGE_EV(i)                         \
+  do                                        \
+  {                                         \
+    if(ev)                                  \
+      CK(cudaEventRecord(ev[i], st));       \
+  } while(0)
+  const DevParams &p = ctx->dp;
+  cudaStream_t st = ctx->stream[s];
+  FrameDev *frames = ctx->d_frames + frame0;
+  unsigned char *labels = ctx->d_labels + (size_t)frame0 * p.N;
+  unsigned *bev = ctx->d_bev + (size_t)s * ctx->chunk_frames * SSD_GPU_MAX_PLATEAUS * ctx->bm_words;
+  const dim3 gpt(p.tiles_per_frame, nf);
+  const int tiles2 = (p.N + SSD_WT_PX * SSD_PT_WARPS - 1) / (SSD_WT_PX * SSD_PT_WARPS);
+  const int bpf = std::max(1, std::min(tiles2, (ctx->pt_blocks_target + nf - 1) / nf));
+  const int bpf_l = ctx->bpf_l_knob > 0 ? std::min(tiles2, ctx->bpf_l_knob) : bpf, bpf_q = ctx->bpf_q_knob > 0 ? std::min(tiles2, ctx->bpf_q_knob) : bpf;
+  const dim3 gpt2l(bpf_l, nf), gpt2q(bpf_q, nf);
+  const bool depth = sv.xyz == nullptr;
+  const float *xyz_dev = sv.xyz;
+  ssd_gpu_overlay *ovl = ctx->d_ovl ? ctx->d_ovl + (size_t)frame0 * SSD_GPU_MAX_STEPS : nullptr;
+  // small batches (the reference's real use is one frame per call): the last block of a frame in k_transform_bin evaluates the
+  // peaks and the last block in k_outline the frame logic -- five launches instead of seven
+  const bool fused = nf <= SSD_FUSE_MAX_FRAMES && !ev;
+  STAGE_EV(0);
+  if(fused)
+  {
+    if(depth)
+      k_transform_bin_depth<SSD_PT_ITERS, true, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, cam);
+    else
+      k_transform_bin<SSD_PT_ITERS, true, CAM><<<gpt, SSD_PT_THREADS, SSD_PT_ITERS * SSD_TB_STAGE_BYTES, st>>>(p, xyz_dev, labels, frames, cam);
+  }
+  else
+  {
+    if(depth)
+      k_transform_bin_depth<SSD_PT_ITERS, false, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, cam);
+    else
+      k_transform_bin<SSD_PT_ITERS, false, CAM><<<gpt, SSD_PT_THREADS, SSD_PT_ITERS * SSD_TB_STAGE_BYTES, st>>>(p, xyz_dev, labels, frames, cam);
+  }
+  STAGE_EV(1);
+  if(!fused)
+    k_peaks<<<nf, 32, 0, st>>>(p, frames, nf);
+  STAGE_EV(2);
+  constexpr bool plain = std::is_same<CAM, NoCam>::value;
+  uint2 *wrec = plain && ctx->wordrec ? ctx->d_wrec + (size_t)s * ctx->chunk_frames * (size_t)(p.N / 4) : nullptr;
+  if constexpr(plain)
+  {
+    if(wrec)
+    {
+      if(depth)
+        k_label_bev<SrcDepth, true><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, wrec);
+      else
+        k_label_bev<SrcVertices, true><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, wrec);
+    }
+  }
+  if(!wrec)
+  {
+    if(depth)
+      k_label_bev<SrcDepth, false, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, nullptr, cam);
+    else
+      k_label_bev<SrcVertices, false, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, nullptr, cam);
+  }
+  STAGE_EV(3);
+  if(fused)
+  {
+    if(ctx->outline_small)
+      k_outline<OutlineSharedSmall, true, CAM><<<dim3(ctx->outline_gridx, nf), SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words, cam);
+    else
+      k_outline<OutlineShared, true, CAM><<<dim3(ctx->outline_gridx, nf), OutlineShared::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words, cam);
+  }
+  else
+  {
+    if(ctx->outline_small)
+      k_outline<OutlineSharedSmall><<<dim3(ctx->outline_gridx, nf), SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
+    else
+      k_outline<OutlineShared><<<dim3(ctx->outline_gridx, nf), OutlineShared::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
+  }
+  STAGE_EV(4);
+  if(!fused)
+    k_frame_logic<CAM><<<nf, 32, 0, st>>>(p, frames, nf, cam);
+  STAGE_EV(5);
+  if constexpr(plain)
+  {
+    if(wrec)
+    {
+      if(depth)
+        k_quad_reduce_rec<SrcDepth><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, wrec);
+      else
+        k_quad_reduce_rec<SrcVertices><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, wrec);
+    }
+  }
+  if(!wrec)
+  {
+    if(depth)
+      k_quad_reduce<SrcDepth, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, cam);
+    else
+      k_quad_reduce<SrcVertices, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, cam);
+  }
+  STAGE_EV(6);
+  if(ctx->outline_small)
+    k_finalize<OutlineSharedSmall, CAM><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words, ctx->smem_cap_words,
+                                                                               ctx->ov, ovl, cam);
+  else
+    k_finalize<OutlineShared, CAM><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words, ctx->smem_cap_words,
+                                                                          ctx->ov, ovl, cam);
+  STAGE_EV(7);
+#undef STAGE_EV
+  *launches += fused ? SSD_GPU_N_STAGES - 2 : SSD_GPU_N_STAGES;
+  if(ctx->risers)
+  {
+    // optional fourth pass: vertical faces from the remainder (labels are final once the chain's label kernel has run)
+    if(depth)
+      k_riser_reduce<SrcDepth, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, cam);
+    else
+      k_riser_reduce<SrcVertices, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, cam);
+    *launches += 1;
+  }
+  CK(cudaGetLastError());
+  return SSD_OK;
+}
+
+
 // ---------------------------------------------------------------------------------------------
 // the launch chain for one chunk of frames on one stream
 // ---------------------------------------------------------------------------------------------
 // xyz_dev: packed vertices of the chunk, or nullptr with z16_dev: the chunk's depth frames, deprojected inside the
-// three point kernels (SrcDepth)
+// three point kernels (SrcDepth). cam: the camera table of a camera call (classic chain only), else nullptr.
 static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uint16_t *z16_dev, float depth_unit, int frame0, int nf, int *launches,
-                        cudaEvent_t *ev)
+                        cudaEvent_t *ev, const CamTable *cam)
 {
 #define STAGE_EV(i)                         \
   do                                        \
@@ -484,6 +636,12 @@ static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uin
     *launches += 1;
   };
 
+  if(cam)
+  {
+    CamTable c = *cam;
+    c.frame0 = frame0;
+    return launch_classic(ctx, s, sv, sd, frame0, nf, launches, ev, c);
+  }
   if(ctx->records)
   {
     // ---- record chain: k_transform_rec -> k_peaks -> k_label_sum -> k_outline -> k_frame_logic -> k_quad_sum -> k_finalize ----
@@ -592,83 +750,8 @@ static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uin
     CK(cudaGetLastError());
     return SSD_OK;
   }
-  // small batches (the reference's real use is one frame per call): the last block of a frame in k_transform_bin evaluates the
-  // peaks and the last block in k_outline the frame logic -- five launches instead of seven
-  const bool fused = nf <= SSD_FUSE_MAX_FRAMES && !ev;
-  STAGE_EV(0);
-  if(fused)
-  {
-    if(depth)
-      k_transform_bin_depth<SSD_PT_ITERS, true><<<gpt, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames);
-    else
-      k_transform_bin<SSD_PT_ITERS, true><<<gpt, SSD_PT_THREADS, SSD_PT_ITERS * SSD_TB_STAGE_BYTES, st>>>(p, xyz_dev, labels, frames);
-  }
-  else
-  {
-    if(depth)
-      k_transform_bin_depth<SSD_PT_ITERS><<<gpt, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames);
-    else
-      k_transform_bin<SSD_PT_ITERS><<<gpt, SSD_PT_THREADS, SSD_PT_ITERS * SSD_TB_STAGE_BYTES, st>>>(p, xyz_dev, labels, frames);
-  }
-  STAGE_EV(1);
-  if(!fused)
-    k_peaks<<<nf, 32, 0, st>>>(p, frames, nf);
-  STAGE_EV(2);
-  uint2 *wrec = ctx->wordrec ? ctx->d_wrec + (size_t)s * ctx->chunk_frames * (size_t)(p.N / 4) : nullptr;
-  if(wrec)
-  {
-    if(depth)
-      k_label_bev<SrcDepth, true><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, wrec);
-    else
-      k_label_bev<SrcVertices, true><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, wrec);
-  }
-  else if(depth)
-    k_label_bev<SrcDepth><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words);
-  else
-    k_label_bev<SrcVertices><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words);
-  STAGE_EV(3);
-  if(fused)
-  {
-    if(ctx->outline_small)
-      k_outline<OutlineSharedSmall, true><<<dim3(ctx->outline_gridx, nf), SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
-    else
-      k_outline<OutlineShared, true><<<dim3(ctx->outline_gridx, nf), OutlineShared::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
-  }
-  else
-  {
-    if(ctx->outline_small)
-      k_outline<OutlineSharedSmall><<<dim3(ctx->outline_gridx, nf), SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
-    else
-      k_outline<OutlineShared><<<dim3(ctx->outline_gridx, nf), OutlineShared::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
-  }
-  STAGE_EV(4);
-  if(!fused)
-    k_frame_logic<<<nf, 32, 0, st>>>(p, frames, nf);
-  STAGE_EV(5);
-  if(wrec)
-  {
-    if(depth)
-      k_quad_reduce_rec<SrcDepth><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, wrec);
-    else
-      k_quad_reduce_rec<SrcVertices><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, wrec);
-  }
-  else if(depth)
-    k_quad_reduce<SrcDepth><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words);
-  else
-    k_quad_reduce<SrcVertices><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words);
-  STAGE_EV(6);
-  if(ctx->outline_small)
-    k_finalize<OutlineSharedSmall><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words, ctx->smem_cap_words, ctx->ov,
-                                                                          ctx->d_ovl ? ctx->d_ovl + (size_t)frame0 * SSD_GPU_MAX_STEPS : nullptr);
-  else
-    k_finalize<OutlineShared><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words, ctx->smem_cap_words, ctx->ov,
-                                                                          ctx->d_ovl ? ctx->d_ovl + (size_t)frame0 * SSD_GPU_MAX_STEPS : nullptr);
-  STAGE_EV(7);
+  return launch_classic(ctx, s, sv, sd, frame0, nf, launches, ev, NoCam());
 #undef STAGE_EV
-  *launches += fused ? SSD_GPU_N_STAGES - 2 : SSD_GPU_N_STAGES;
-  launch_risers();
-  CK(cudaGetLastError());
-  return SSD_OK;
 }
 
 extern "C"
@@ -711,6 +794,12 @@ void ssd_gpu_destroy(ssd_gpu_ctx *ctx)
   cudaFree(ctx->d_img);
   cudaFree(ctx->d_xn);
   cudaFree(ctx->d_yn);
+  cudaFree(ctx->d_cam_dp);
+  cudaFree(ctx->d_cam_ov);
+  cudaFree(ctx->d_cam_xn);
+  cudaFree(ctx->d_cam_yn);
+  cudaFree(ctx->d_cam_unit);
+  cudaFree(ctx->d_cam_of_frame);
   for(int i = 0; i < SSD_MAX_STREAMS; i++)
   {
     cudaFree(ctx->d_stage[i]);
@@ -820,6 +909,8 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
   ctx->ol_dyn_smem = dyn;
   ctx->smem_cap_words = dyn / 4;
   cudaFuncSetAttribute(k_transform_bin<SSD_PT_ITERS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SSD_PT_ITERS * SSD_TB_STAGE_BYTES);
+  cudaFuncSetAttribute(k_transform_bin<SSD_PT_ITERS, true, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, SSD_PT_ITERS * SSD_TB_STAGE_BYTES);
+  cudaFuncSetAttribute(k_transform_bin<SSD_PT_ITERS, false, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, SSD_PT_ITERS * SSD_TB_STAGE_BYTES);
   if(cudaFuncSetAttribute(k_transform_bin<SSD_PT_ITERS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SSD_PT_ITERS * SSD_TB_STAGE_BYTES) != cudaSuccess)
     return bail("cudaFuncSetAttribute(k_transform_bin) failed", SSD_E_CUDA);
   {
@@ -835,6 +926,11 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
       cudaFuncSetAttribute(k_outline<OutlineSharedSmall, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       cudaFuncSetAttribute(k_finalize<OutlineShared>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       cudaFuncSetAttribute(k_finalize<OutlineSharedSmall>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      // the camera-table variants (ssd_gpu_set_cameras) of the kernels with a dynamic work area
+      cudaFuncSetAttribute(k_outline<OutlineShared, true, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      cudaFuncSetAttribute(k_outline<OutlineSharedSmall, true, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      cudaFuncSetAttribute(k_finalize<OutlineShared, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       cudaFuncSetAttribute(k_single_front_edge, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       granted = dyn;
     }
@@ -981,10 +1077,11 @@ static int ensure_deproject_tables(ssd_gpu_ctx *ctx, const ssd_gpu_intrinsics &i
 }
 
 // xyz != nullptr: packed vertices; else z16 depth frames + intrinsics (deprojected chunk by chunk into the vertex staging)
+// cam_of_frame != nullptr: a camera call (validated by check_cameras; the depth tables are the camera table's, intr is unused)
 static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16, const ssd_gpu_intrinsics *intr, bool host_input, int n_frames,
-                        int flags)
+                        int flags, const int32_t *cam_of_frame)
 {
-  if(!ctx || (!xyz && !(z16 && intr)) || n_frames <= 0)
+  if(!ctx || (!xyz && !(z16 && (intr || cam_of_frame))) || n_frames <= 0)
     return fail(ctx, SSD_E_INVALID_ARG, "process: bad argument");
   if(n_frames > ctx->max_frames)
     return fail(ctx, SSD_E_RANGE, "process: n_frames exceeds max_frames of the context");
@@ -1007,7 +1104,7 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
       cf = half;
   }
   const bool depth_input = xyz == nullptr;
-  if(depth_input)
+  if(depth_input && !cam_of_frame)
   {
     const int rc = ensure_deproject_tables(ctx, *intr);
     if(rc)
@@ -1053,6 +1150,25 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
   }
   ctx->n_frames_last = n_frames;
   ctx->flags_last = flags;
+  ctx->stats_eps0 = ctx->dp.E0s;
+  ctx->stats_eps1 = ctx->dp.E1s;
+  CamTable cams{};
+  if(cam_of_frame)
+  {
+    cams.params = ctx->d_cam_dp;
+    cams.ov = ctx->d_cam_ov;
+    cams.xn = ctx->d_cam_xn;
+    cams.yn = ctx->d_cam_yn;
+    cams.unit = ctx->d_cam_unit;
+    cams.cam = ctx->d_cam_of_frame;
+    ctx->stats_eps0 = ctx->stats_eps1 = 0;
+    for(int f = 0; f < n_frames; f++)
+    {
+      const DevParams &d = ctx->cam_dp[cam_of_frame[f]];
+      ctx->stats_eps0 = std::max(ctx->stats_eps0, (double)d.E0s);
+      ctx->stats_eps1 = std::max(ctx->stats_eps1, (double)d.E1s);
+    }
+  }
   // the whole call is ordered after ev_start on stream 0; stream 1 joins via events
   CK(cudaEventRecord(ctx->ev_start, ctx->stream[0]));
   for(int i = 1; i < ctx->n_streams; i++)
@@ -1062,6 +1178,8 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
     CK(cudaEventRecord(ctx->ev_h2d0, ctx->copy_stream));
   // per-frame state: histogram must start at zero
   CK(cudaMemsetAsync(ctx->d_frames, 0, sizeof(FrameDev) * (size_t)n_frames, ctx->stream[0]));
+  if(cam_of_frame)
+    CK(cudaMemcpyAsync(ctx->d_cam_of_frame, cam_of_frame, sizeof(int32_t) * (size_t)n_frames, cudaMemcpyHostToDevice, ctx->stream[0]));
   CK(cudaEventRecord(ctx->ev_chunk_done[0], ctx->stream[0]));
   for(int i = 1; i < ctx->n_streams; i++)
     CK(cudaStreamWaitEvent(ctx->stream[i], ctx->ev_chunk_done[0], 0));
@@ -1102,8 +1220,8 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
         CK(cudaEventRecord(ctx->ev_in_free[s], ctx->stream[s])); // the z16 staging is consumed
     }
     const bool fused = depth_input && !unfused;
-    const int rc = launch_chunk(ctx, s, fused ? nullptr : src, fused ? dsrc : nullptr, fused ? intr->depth_unit : 0.f, f0, nf, &launches,
-                                stage_timing ? &ctx->stage_ev[(size_t)chunk * (SSD_GPU_N_STAGES + 1)] : nullptr);
+    const int rc = launch_chunk(ctx, s, fused ? nullptr : src, fused ? dsrc : nullptr, fused && intr ? intr->depth_unit : 0.f, f0, nf, &launches,
+                                stage_timing ? &ctx->stage_ev[(size_t)chunk * (SSD_GPU_N_STAGES + 1)] : nullptr, cam_of_frame ? &cams : nullptr);
     if(rc)
       return rc;
     if(host_input && (!depth_input || fused))
@@ -1227,9 +1345,9 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
 // unsynchronised and BEV bitmaps half written: the bitmaps are "self-cleaning" only along a complete chain. Bring the context
 // back to a clean state so that the next call starts from zeroed bitmaps and no stale results can be read.
 static int process_common(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16, const ssd_gpu_intrinsics *intr, bool host_input, int n_frames,
-                          int flags)
+                          int flags, const int32_t *cam_of_frame = nullptr)
 {
-  const int rc = process_impl(ctx, xyz, z16, intr, host_input, n_frames, flags);
+  const int rc = process_impl(ctx, xyz, z16, intr, host_input, n_frames, flags, cam_of_frame);
   if(rc != SSD_OK && rc != SSD_E_INVALID_ARG && rc != SSD_E_RANGE && ctx)
   {
     const std::string keep = ctx->err;
@@ -1271,6 +1389,153 @@ int ssd_gpu_process_depth_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, cons
   if(!z16_dev || !intr)
     return fail(ctx, SSD_E_INVALID_ARG, "process_depth: bad argument");
   return process_common(ctx, nullptr, z16_dev, intr, false, n_frames, 0);
+}
+
+// ---- per-frame cameras ----
+static void free_cameras(ssd_gpu_ctx *ctx)
+{
+  for(void *p : { (void *)ctx->d_cam_dp, (void *)ctx->d_cam_ov, (void *)ctx->d_cam_xn, (void *)ctx->d_cam_yn, (void *)ctx->d_cam_unit })
+    cudaFree(p);
+  ctx->d_cam_dp = nullptr;
+  ctx->d_cam_ov = nullptr;
+  ctx->d_cam_xn = ctx->d_cam_yn = ctx->d_cam_unit = nullptr;
+  ctx->cam_dp.clear();
+  ctx->cam_depth_ok.clear();
+  ctx->n_cameras = 0;
+}
+
+int ssd_gpu_set_cameras(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, int n_cameras)
+{
+  if(!ctx || n_cameras < 0 || (n_cameras > 0 && !cams))
+    return fail(ctx, SSD_E_INVALID_ARG, "ssd_gpu_set_cameras: bad argument");
+  // every camera is checked before the table is touched: a rejected table leaves the previous one in place
+  std::vector<DevParams> dp((size_t)n_cameras);
+  std::vector<OverlayDev> ov((size_t)n_cameras);
+  std::vector<float> unit((size_t)n_cameras);
+  std::vector<unsigned char> depth_ok((size_t)n_cameras);
+  for(int c = 0; c < n_cameras; c++)
+  {
+    if(derive_params(ctx->cfg, cams[c].xf, dp[c]))
+      return fail(ctx, SSD_E_INVALID_ARG, "ssd_gpu_set_cameras: camera " + std::to_string(c) + ": transform out of range");
+    const ssd_gpu_intrinsics &in = cams[c].intr;
+    OverlayDev &o = ov[c];
+    memset(&o, 0, sizeof(o));
+    for(int i = 0; i < 9; i++)
+      o.a_inv[i] = cams[c].a_inv[i];
+    o.fx = in.fx;
+    o.fy = in.fy;
+    o.ppx = in.ppx;
+    o.ppy = in.ppy;
+    o.enabled = 1;
+    unit[c] = in.depth_unit;
+    depth_ok[c] = in.fx != 0.f && in.fy != 0.f && in.depth_unit > 0.f; // as ensure_deproject_tables
+  }
+  CK(cudaSetDevice(ctx->device));
+  CK(cudaDeviceSynchronize());
+  free_cameras(ctx);
+  if(n_cameras == 0)
+    return SSD_OK;
+  const DevParams &p = ctx->dp;
+  if(!ctx->d_cam_of_frame)
+    CK(cudaMalloc(&ctx->d_cam_of_frame, sizeof(int32_t) * (size_t)ctx->max_frames));
+  ssd_gpu_camera *d_in = nullptr;
+  CK(cudaMalloc(&ctx->d_cam_dp, sizeof(DevParams) * (size_t)n_cameras));
+  CK(cudaMalloc(&ctx->d_cam_ov, sizeof(OverlayDev) * (size_t)n_cameras));
+  CK(cudaMalloc(&ctx->d_cam_unit, sizeof(float) * (size_t)n_cameras));
+  CK(cudaMalloc(&ctx->d_cam_xn, sizeof(float) * (size_t)n_cameras * p.W));
+  CK(cudaMalloc(&ctx->d_cam_yn, sizeof(float) * (size_t)n_cameras * p.H));
+  CK(cudaMalloc(&d_in, sizeof(ssd_gpu_camera) * (size_t)n_cameras));
+  cudaStream_t st = ctx->stream[0];
+  cudaError_t e = cudaMemcpyAsync(ctx->d_cam_dp, dp.data(), sizeof(DevParams) * (size_t)n_cameras, cudaMemcpyHostToDevice, st);
+  if(e == cudaSuccess)
+    e = cudaMemcpyAsync(ctx->d_cam_ov, ov.data(), sizeof(OverlayDev) * (size_t)n_cameras, cudaMemcpyHostToDevice, st);
+  if(e == cudaSuccess)
+    e = cudaMemcpyAsync(ctx->d_cam_unit, unit.data(), sizeof(float) * (size_t)n_cameras, cudaMemcpyHostToDevice, st);
+  if(e == cudaSuccess)
+    e = cudaMemcpyAsync(d_in, cams, sizeof(ssd_gpu_camera) * (size_t)n_cameras, cudaMemcpyHostToDevice, st);
+  if(e == cudaSuccess)
+  {
+    // (cameras without depth intrinsics get meaningless tables: depth calls never use them)
+    const int n = std::max(p.W, p.H);
+    k_deproject_tables_cams<<<dim3((n + 255) / 256, std::min(n_cameras, 65535)), 256, 0, st>>>(p.W, p.H, d_in, n_cameras, ctx->d_cam_xn, ctx->d_cam_yn);
+    e = cudaGetLastError();
+  }
+  if(e == cudaSuccess)
+    e = cudaStreamSynchronize(st);
+  cudaFree(d_in);
+  if(e != cudaSuccess)
+  {
+    free_cameras(ctx);
+    CK(e);
+  }
+  ctx->cam_dp.swap(dp);
+  ctx->cam_depth_ok.swap(depth_ok);
+  ctx->n_cameras = n_cameras;
+  return SSD_OK;
+}
+
+int ssd_gpu_n_cameras(ssd_gpu_ctx *ctx)
+{
+  return ctx ? ctx->n_cameras : SSD_E_INVALID_ARG;
+}
+
+// Everything a camera call can be refused for, before anything is launched (the previous results stay readable).
+static int check_cameras(ssd_gpu_ctx *ctx, const void *input, const int32_t *cam_of_frame, int n_frames, bool depth)
+{
+  if(!ctx || !input || !cam_of_frame || n_frames <= 0)
+    return fail(ctx, SSD_E_INVALID_ARG, "camera call: bad argument");
+  if(ctx->records || ctx->wordrec || ctx->resident)
+    return fail(ctx, SSD_E_STATE, "camera call: camera tables run on the default (classic) chain only; this context was created with "
+                                  "SSD_GPU_PATH=records|wordrec|resident");
+  if(depth && ctx->depth_unfused)
+    return fail(ctx, SSD_E_STATE, "depth camera call: not available with SSD_GPU_DEPTH_UNFUSED=1 (the fused depth path only)");
+  if(ctx->n_cameras <= 0)
+    return fail(ctx, SSD_E_STATE, "camera call: no camera table (ssd_gpu_set_cameras)");
+  if(n_frames > ctx->max_frames)
+    return fail(ctx, SSD_E_RANGE, "process: n_frames exceeds max_frames of the context");
+  if(depth && ctx->dp.W % 4 != 0)
+    return fail(ctx, SSD_E_INVALID_ARG, "depth input: the frame width must be a multiple of 4");
+  for(int f = 0; f < n_frames; f++)
+  {
+    const int32_t c = cam_of_frame[f];
+    if(c < 0 || c >= ctx->n_cameras)
+      return fail(ctx, SSD_E_RANGE, "camera call: frame " + std::to_string(f) + " names camera " + std::to_string(c) + ", outside [0, " +
+                                      std::to_string(ctx->n_cameras) + ")");
+    if(depth && !ctx->cam_depth_ok[c])
+      return fail(ctx, SSD_E_INVALID_ARG, "depth camera call: camera " + std::to_string(c) + " has no depth intrinsics (fx, fy must be non-zero and "
+                                                                                            "depth_unit positive)");
+  }
+  return SSD_OK;
+}
+
+int ssd_gpu_process_cameras_host(ssd_gpu_ctx *ctx, const float *xyz_host, const int32_t *camera_of_frame, int n_frames)
+{
+  const int rc = check_cameras(ctx, xyz_host, camera_of_frame, n_frames, false);
+  return rc ? rc : process_common(ctx, xyz_host, nullptr, nullptr, true, n_frames, 0, camera_of_frame);
+}
+
+int ssd_gpu_process_cameras_device(ssd_gpu_ctx *ctx, const float *xyz_dev, const int32_t *camera_of_frame, int n_frames)
+{
+  const int rc = check_cameras(ctx, xyz_dev, camera_of_frame, n_frames, false);
+  return rc ? rc : process_common(ctx, xyz_dev, nullptr, nullptr, false, n_frames, 0, camera_of_frame);
+}
+
+int ssd_gpu_process_cameras_device_ex(ssd_gpu_ctx *ctx, const float *xyz_dev, const int32_t *camera_of_frame, int n_frames, int flags)
+{
+  const int rc = check_cameras(ctx, xyz_dev, camera_of_frame, n_frames, false);
+  return rc ? rc : process_common(ctx, xyz_dev, nullptr, nullptr, false, n_frames, flags, camera_of_frame);
+}
+
+int ssd_gpu_process_depth_cameras_host(ssd_gpu_ctx *ctx, const uint16_t *z16_host, const int32_t *camera_of_frame, int n_frames)
+{
+  const int rc = check_cameras(ctx, z16_host, camera_of_frame, n_frames, true);
+  return rc ? rc : process_common(ctx, nullptr, z16_host, nullptr, true, n_frames, 0, camera_of_frame);
+}
+
+int ssd_gpu_process_depth_cameras_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const int32_t *camera_of_frame, int n_frames)
+{
+  const int rc = check_cameras(ctx, z16_dev, camera_of_frame, n_frames, true);
+  return rc ? rc : process_common(ctx, nullptr, z16_dev, nullptr, false, n_frames, 0, camera_of_frame);
 }
 
 int ssd_gpu_deproject_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const ssd_gpu_intrinsics *intr, int n_frames, float *xyz_dev)
@@ -1508,8 +1773,8 @@ int ssd_gpu_get_stats(ssd_gpu_ctx *ctx, ssd_gpu_stats *out)
   out->n_quad_fast = c[1] - c[2];
   out->n_quad_exact = c[2];
   out->n_bev_exact = c[3];
-  out->filter_eps0 = ctx->dp.E0s;
-  out->filter_eps1 = ctx->dp.E1s;
+  out->filter_eps0 = ctx->n_frames_last > 0 ? ctx->stats_eps0 : ctx->dp.E0s;
+  out->filter_eps1 = ctx->n_frames_last > 0 ? ctx->stats_eps1 : ctx->dp.E1s;
   return SSD_OK;
 }
 

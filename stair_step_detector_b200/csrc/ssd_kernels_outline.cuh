@@ -1266,15 +1266,17 @@ __device__ inline void frame_logic_warp(const DevParams &p, FrameDev &F, FrameLo
 #endif
 // FUSE_LOGIC (small batches: latency matters, not occupancy): the last block of a frame to finish runs the frame logic
 // (k_frame_logic) itself -- one launch and one kernel boundary less on the single-frame path.
-template<class OutlineShared, bool FUSE_LOGIC = false>
-__global__ void __launch_bounds__(OutlineShared::THREADS, FUSE_LOGIC ? 1 : (OutlineShared::MINB ? OutlineShared::MINB : SSD_OL_MINB)) k_outline(const __grid_constant__ DevParams p, FrameDev *__restrict__ frames,
-                                                             unsigned *__restrict__ bev, size_t bm_words, size_t smem_cap_words)
+template<class OutlineShared, bool FUSE_LOGIC = false, class CAM = NoCam>
+__global__ void __launch_bounds__(OutlineShared::THREADS, FUSE_LOGIC ? 1 : (OutlineShared::MINB ? OutlineShared::MINB : SSD_OL_MINB)) k_outline(const __grid_constant__ DevParams p0, FrameDev *__restrict__ frames,
+                                                             unsigned *__restrict__ bev, size_t bm_words, size_t smem_cap_words,
+                                                             const CAM cam = CAM())
 {
   extern __shared__ __align__(16) unsigned s_words[];
   __shared__ OutlineShared S;
   __shared__ Band bd;
   __shared__ int s_smem_path;
   const int frame = blockIdx.y, tid = threadIdx.x;
+  const DevParams &p = frame_params(p0, cam, frame);
   FrameDev &F = frames[frame];
   // grid.x blocks per frame walk the frame's outlined plateaus (first_outlined .. n_plateaus-1, k_peaks); grid.x is
   // smaller than SSD_GPU_MAX_PLATEAUS because a frame rarely has more than a handful (ssd_gpu.cu, launch_chain)
@@ -1353,12 +1355,15 @@ __global__ void __launch_bounds__(OutlineShared::THREADS, FUSE_LOGIC ? 1 : (Outl
 // quadrilateral (calcGroundQuadrilateral, :489-512) and one QuadrilateralTest per emitted step.
 // One warp per frame, one lane per plateau.
 // ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(32) k_frame_logic(const __grid_constant__ DevParams p, FrameDev *__restrict__ frames, int n_frames)
+template<class CAM = NoCam>
+__global__ void __launch_bounds__(32) k_frame_logic(const __grid_constant__ DevParams p0, FrameDev *__restrict__ frames, int n_frames,
+                                                    const CAM cam = CAM())
 {
   __shared__ FrameLogicScratch Sc;
   const int f = blockIdx.x;
   if(f >= n_frames)
     return;
+  const DevParams &p = frame_params(p0, cam, f);
   frame_logic_warp(p, frames[f], Sc, threadIdx.x);
 }
 
@@ -1367,17 +1372,19 @@ __global__ void __launch_bounds__(32) k_frame_logic(const __grid_constant__ DevP
 // assembly of detectStairs with ToExternalWorld (:370-383, transformation.cpp:190-194).
 // grid = frames, one block per frame.
 // ---------------------------------------------------------------------------------------------
-template<class OutlineShared>
-__global__ void __launch_bounds__(SSD_OL_THREADS, SSD_OL_MINB) k_finalize(const __grid_constant__ DevParams p, FrameDev *__restrict__ frames,
+template<class OutlineShared, class CAM = NoCam>
+__global__ void __launch_bounds__(SSD_OL_THREADS, SSD_OL_MINB) k_finalize(const __grid_constant__ DevParams p0, FrameDev *__restrict__ frames,
                                                               FrameOut *__restrict__ out, unsigned *__restrict__ bev, size_t bm_words,
-                                                              size_t smem_cap_words, const __grid_constant__ OverlayDev ov,
-                                                              ssd_gpu_overlay *__restrict__ overlay)
+                                                              size_t smem_cap_words, const __grid_constant__ OverlayDev ov0,
+                                                              ssd_gpu_overlay *__restrict__ overlay, const CAM cam = CAM())
 {
   extern __shared__ __align__(16) unsigned s_words[];
   __shared__ OutlineShared S;
   __shared__ Band bd;
   __shared__ int s_smem_path;
   const int frame = blockIdx.x, tid = threadIdx.x;
+  const DevParams &p = frame_params(p0, cam, frame);
+  const OverlayDev &ov = frame_overlay(ov0, cam, frame);
   FrameDev &F = frames[frame];
   FrameOut &O = out[frame];
   const int K = F.n_plateaus, ground = F.ground_index, firstValid = F.first_valid;

@@ -122,6 +122,25 @@ __device__ __forceinline__ FrameD src_frame(const SrcDepth &s, const DevParams &
   f.W = (unsigned)p.W;
   return f;
 }
+// The source of one frame: in camera mode a depth frame is deprojected with its own camera's tables and depth unit.
+template<class SRC>
+__device__ __forceinline__ const SRC &frame_src(const SRC &s, const NoCam &, const DevParams &, int)
+{
+  return s;
+}
+__device__ __forceinline__ SrcVertices frame_src(const SrcVertices &s, const CamTable &, const DevParams &, int)
+{
+  return s;
+}
+__device__ __forceinline__ SrcDepth frame_src(const SrcDepth &s, const CamTable &c, const DevParams &p, int frame)
+{
+  const int cam = frame_camera(c, frame);
+  SrcDepth d = s;
+  d.xn = c.xn + (size_t)cam * p.W;
+  d.yn = c.yn + (size_t)cam * p.H;
+  d.unit = __ldg(c.unit + cam);
+  return d;
+}
 __device__ __forceinline__ void word_zero(WordV &r)
 {
   r.a = r.b = r.c = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -509,9 +528,10 @@ __device__ __forceinline__ void tb_fused_peaks(const DevParams &p, FrameDev &F, 
   }
 }
 
-template<int ITERS, bool FUSE_PEAKS = false>
-__global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin(const __grid_constant__ DevParams p, const float *__restrict__ xyz,
-                                                                   unsigned char *__restrict__ codes, FrameDev *__restrict__ frames)
+template<int ITERS, bool FUSE_PEAKS = false, class CAM = NoCam>
+__global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin(const __grid_constant__ DevParams p0, const float *__restrict__ xyz,
+                                                                   unsigned char *__restrict__ codes, FrameDev *__restrict__ frames,
+                                                                   const CAM cam = CAM())
 {
   extern __shared__ __align__(128) unsigned char s_dyn[]; // ITERS stages of SSD_TB_STAGE_BYTES
   __shared__ __align__(8) unsigned long long s_bar[ITERS];
@@ -519,8 +539,8 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin(const __grid_c
   __shared__ unsigned s_exact;
   const int tid = threadIdx.x;
   const int frame = blockIdx.y;
-  const size_t fbase = (size_t)frame * p.N;
-  const int nquads = p.N >> 2;
+  const size_t fbase = (size_t)frame * p0.N; // (configuration fields: equal in every camera's parameters)
+  const int nquads = p0.N >> 2;
   const int qb = blockIdx.x * (ITERS * SSD_PT_THREADS); // first quad (4 vertices) of the block
   const unsigned stage_sa = (unsigned)__cvta_generic_to_shared(s_dyn);
   const unsigned bar_sa = (unsigned)__cvta_generic_to_shared(s_bar);
@@ -544,6 +564,8 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin(const __grid_c
     }
     s_exact = 0;
   }
+  // camera mode: the frame's parameters are staged while the bulk copies are in flight
+  const DevParams &p = frame_params(p0, cam, frame);
   s_hist[tid] = 0; // SSD_PT_THREADS == SSD_BINS_PAD
   __syncthreads();
 
@@ -585,14 +607,17 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin(const __grid_c
 // deprojected vertices live in registers only. No staging: the loads are 8 bytes per lane (256 B per warp, coalesced) and
 // all ITERS words of a thread are requested before the first is consumed. Not HBM-bound (3 B/point): issue-bound.
 // ---------------------------------------------------------------------------------------------
-template<int ITERS, bool FUSE_PEAKS = false>
-__global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_depth(const __grid_constant__ DevParams p, const SrcDepth src,
-                                                                         unsigned char *__restrict__ codes, FrameDev *__restrict__ frames)
+template<int ITERS, bool FUSE_PEAKS = false, class CAM = NoCam>
+__global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_depth(const __grid_constant__ DevParams p0, const SrcDepth src0,
+                                                                         unsigned char *__restrict__ codes, FrameDev *__restrict__ frames,
+                                                                         const CAM cam = CAM())
 {
   __shared__ unsigned s_hist[SSD_BINS_PAD];
   __shared__ unsigned s_exact;
   const int tid = threadIdx.x;
   const int frame = blockIdx.y;
+  const DevParams &p = frame_params(p0, cam, frame);
+  const auto &src = frame_src(src0, cam, p, frame);
   const size_t fbase = (size_t)frame * p.N;
   const int nquads = p.N >> 2;
   const int q0 = blockIdx.x * (ITERS * SSD_PT_THREADS) + tid;
@@ -755,14 +780,17 @@ __device__ __forceinline__ uint2 word_rec_pack(bool eligible, int xlo, int ylo, 
   return make_uint2(lo, zsum | (count << 25));
 }
 
-template<class SRC, bool REC = false>
-__global__ void __launch_bounds__(SSD_PT_THREADS, SSD_LB_MINB) k_label_bev(const __grid_constant__ DevParams p, const SRC src,
+template<class SRC, bool REC = false, class CAM = NoCam>
+__global__ void __launch_bounds__(SSD_PT_THREADS, SSD_LB_MINB) k_label_bev(const __grid_constant__ DevParams p0, const SRC src0,
                                                                unsigned char *__restrict__ labels, FrameDev *__restrict__ frames,
-                                                               unsigned *__restrict__ bev, size_t bm_words, uint2 *__restrict__ wrec = nullptr)
+                                                               unsigned *__restrict__ bev, size_t bm_words, uint2 *__restrict__ wrec = nullptr,
+                                                               const CAM cam = CAM())
 {
   __shared__ LabelBevShared S;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int frame = blockIdx.y;
+  const DevParams &p = frame_params(p0, cam, frame);
+  const auto &src = frame_src(src0, cam, p, frame);
   FrameDev &F = frames[frame];
   const size_t fbase = (size_t)frame * p.N;
   unsigned *lab32 = reinterpret_cast<unsigned *>(labels + fbase);
@@ -1354,14 +1382,16 @@ __device__ __forceinline__ void qr_epilogue(QuadReduceShared &S, QrWarp &W, Fram
 #ifndef SSD_QR_MINB
 #define SSD_QR_MINB 4
 #endif
-template<class SRC>
-__global__ void __launch_bounds__(SSD_PT_THREADS, SSD_QR_MINB) k_quad_reduce(const __grid_constant__ DevParams p, const SRC src,
+template<class SRC, class CAM = NoCam>
+__global__ void __launch_bounds__(SSD_PT_THREADS, SSD_QR_MINB) k_quad_reduce(const __grid_constant__ DevParams p0, const SRC src0,
                                                                  const unsigned char *__restrict__ labels, FrameDev *__restrict__ frames,
-                                                                 unsigned *__restrict__ bev, size_t bm_words)
+                                                                 unsigned *__restrict__ bev, size_t bm_words, const CAM cam = CAM())
 {
   __shared__ QuadReduceShared S;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int frame = blockIdx.y;
+  const DevParams &p = frame_params(p0, cam, frame);
+  const auto &src = frame_src(src0, cam, p, frame);
   FrameDev &F = frames[frame];
   const unsigned amask = F.quad_amask;
   if(amask == 0u)
@@ -1623,13 +1653,16 @@ __device__ __forceinline__ void riser_flush(RiserShared &S, RiserSeg &g)
   g.xmax = g.ymax = -1;
 }
 
-template<class SRC>
-__global__ void __launch_bounds__(SSD_PT_THREADS) k_riser_reduce(const __grid_constant__ DevParams p, const SRC src,
-                                                                 const unsigned char *__restrict__ labels, FrameDev *__restrict__ frames)
+template<class SRC, class CAM = NoCam>
+__global__ void __launch_bounds__(SSD_PT_THREADS) k_riser_reduce(const __grid_constant__ DevParams p0, const SRC src0,
+                                                                 const unsigned char *__restrict__ labels, FrameDev *__restrict__ frames,
+                                                                 const CAM cam = CAM())
 {
   __shared__ RiserShared S;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int frame = blockIdx.y;
+  const DevParams &p = frame_params(p0, cam, frame);
+  const auto &src = frame_src(src0, cam, p, frame);
   FrameDev &F = frames[frame];
   const int K = F.n_plateaus;
   if(K < 2)
