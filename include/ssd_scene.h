@@ -1,6 +1,6 @@
 /*
  * ssd_scene.h -- synthetic input source for tests and benchmarks: procedurally generated staircases seen by a pin-hole
- * L515-like depth camera (SURVEY.md 8(d) configs). It stands in for the stubbed RealSense capture
+ * L515-like depth camera (optionally with a Brown-Conrady lens) (SURVEY.md 8(d) configs). It stands in for the stubbed RealSense capture
  * (Camera::waitForFrames, camera.cpp:27-60) and for rs2::pointcloud::calculate on the host (pointcloud.cpp:138).
  * NOT part of the product: it lives in its own library (stair_step_detector_b200/lib/libssd_scene.so) so that nothing
  * that only generates input or runs the CPU reference has to load the product library libssd_gpu.so.
@@ -38,6 +38,8 @@ typedef struct ssd_scene
   int32_t rotate180;           /* camera mounted upside down (README "descending stairs") */
   int32_t randomize_camera;    /* ssd_scene_randomize also jitters the camera pose (needs a per-frame calibration) */
   uint64_t seed;
+  int32_t distortion_model;    /* lens (ssd_gpu_distortion, include/ssd_gpu.h): SSD_DISTORTION_NONE = the pin-hole camera */
+  float coeffs[5];             /* k1, k2, p1, p2, k3: pixel (u, v) is cast along its deprojected ray */
 } ssd_scene;
 
 void ssd_scene_default(ssd_scene *s, int32_t width, int32_t height);

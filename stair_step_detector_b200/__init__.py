@@ -170,6 +170,23 @@ def scene_intrinsics(scene):
     return k
 
 
+def scene_distortion(scene):
+    """The lens of a synthetic scene (A.Distortion): its distortion_model and coeffs."""
+    return make_distortion(scene.distortion_model, scene.coeffs[:])
+
+
+def make_distortion(model, coeffs=(0.0, 0.0, 0.0, 0.0, 0.0)):
+    """ssd_gpu_distortion from an rs2 model value (A.DISTORTION_*) and the five coefficients [k1, k2, p1, p2, k3]."""
+    coeffs = [float(c) for c in coeffs]
+    if len(coeffs) != 5:
+        raise ValueError(f"a lens has 5 coefficients, got {len(coeffs)}")
+    d = A.Distortion()
+    d.model = int(model)
+    for i, c in enumerate(coeffs):
+        d.coeffs[i] = c
+    return d
+
+
 def serialize(steps):
     """Stairs::serialize (reference stairs.cpp:55-70) of a list of (height, 4x2 quad)."""
     arr = (Step * max(1, len(steps)))()
@@ -246,10 +263,25 @@ class Detector:
         self._ck(self._l.ssd_gpu_process_device_ex(self._h, dev_ptr, n_frames, flags), "ssd_gpu_process_device")
 
     # ---- per-frame cameras ----
-    def set_cameras(self, cameras):
-        """Replace the camera table with a list of A.Camera (scene_camera / make_camera); an empty list frees it."""
+    def set_cameras(self, cameras, distortions=None):
+        """Replace the camera table with a list of A.Camera (scene_camera / make_camera); an empty list frees it.
+        distortions: one A.Distortion per camera (make_distortion / scene_distortion), or None for pin-hole lenses."""
         arr = (A.Camera * max(1, len(cameras)))(*cameras)
-        self._ck(self._l.ssd_gpu_set_cameras(self._h, arr, len(cameras)), "ssd_gpu_set_cameras")
+        if distortions is None:
+            self._ck(self._l.ssd_gpu_set_cameras(self._h, arr, len(cameras)), "ssd_gpu_set_cameras")
+            return
+        if len(distortions) != len(cameras):
+            raise ValueError(f"{len(distortions)} distortions for {len(cameras)} cameras")
+        dist = (A.Distortion * max(1, len(distortions)))(*distortions)
+        self._ck(self._l.ssd_gpu_set_cameras_ex(self._h, arr, dist, len(cameras)), "ssd_gpu_set_cameras_ex")
+
+    def set_distortion(self, distortion):
+        """Lens of the plain calls (depth input, deproject_device, overlay); None switches it off (pin-hole)."""
+        self._ck(self._l.ssd_gpu_set_distortion(self._h, None if distortion is None else C.byref(distortion)), "ssd_gpu_set_distortion")
+
+    @property
+    def n_ray_tables(self):
+        return self._l.ssd_gpu_n_ray_tables(self._h)
 
     @property
     def n_cameras(self):

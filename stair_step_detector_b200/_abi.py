@@ -25,6 +25,14 @@ STATUS_TOO_MANY_PLATEAUS = 0x10
 STATUS_BEV_OOB = 0x20
 STATUS_HMIN_WRAP = 0x40
 
+# lens models (rs2_distortion values); 1, 3 and 5 are rejected
+DISTORTION_NONE = 0
+DISTORTION_MODIFIED_BROWN_CONRADY = 1
+DISTORTION_INVERSE_BROWN_CONRADY = 2
+DISTORTION_FTHETA = 3
+DISTORTION_BROWN_CONRADY = 4
+DISTORTION_KANNALA_BRANDT4 = 5
+
 FLAG_STAGE_TIMING = 0x2
 FLAG_SINGLE_STREAM = 0x4
 N_STAGES = 7
@@ -53,6 +61,11 @@ class Intrinsics(C.Structure):
 class Camera(C.Structure):
     """ssd_gpu_camera: one entry of a context's camera table (ssd_gpu_set_cameras)."""
     _fields_ = [("xf", Transform), ("a_inv", C.c_double * 9), ("intr", Intrinsics)]
+
+
+class Distortion(C.Structure):
+    """ssd_gpu_distortion: rs2_intrinsics.model and .coeffs [k1, k2, p1, p2, k3]."""
+    _fields_ = [("model", C.c_int32), ("coeffs", C.c_float * 5)]
 
 
 class Overlay(C.Structure):
@@ -101,7 +114,7 @@ class Scene(C.Structure):
                 ("first_riser_y", C.c_float), ("x_center", C.c_float), ("top_landing", C.c_float),
                 ("noise_sigma", C.c_float), ("dropout", C.c_float),
                 ("n_holes", C.c_int32), ("n_occluders", C.c_int32), ("rotate180", C.c_int32), ("randomize_camera", C.c_int32),
-                ("seed", C.c_uint64)]
+                ("seed", C.c_uint64), ("distortion_model", C.c_int32), ("coeffs", C.c_float * 5)]
 
 
 _P = C.POINTER
@@ -120,6 +133,9 @@ PROTOTYPES = {
     "ssd_gpu_process_device_ex": (C.c_int, [_vp, _vp, C.c_int, C.c_int]),
     "ssd_gpu_set_cameras": (C.c_int, [_vp, _P(Camera), C.c_int]),
     "ssd_gpu_n_cameras": (C.c_int, [_vp]),
+    "ssd_gpu_set_distortion": (C.c_int, [_vp, _P(Distortion)]),
+    "ssd_gpu_set_cameras_ex": (C.c_int, [_vp, _P(Camera), _P(Distortion), C.c_int]),
+    "ssd_gpu_n_ray_tables": (C.c_int, [_vp]),
     "ssd_gpu_process_cameras_host": (C.c_int, [_vp, _vp, _vp, C.c_int]),
     "ssd_gpu_process_cameras_device": (C.c_int, [_vp, _vp, _vp, C.c_int]),
     "ssd_gpu_process_cameras_device_ex": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int]),

@@ -21,6 +21,7 @@ public:
     const float *vertices = nullptr; // width*height*3 floats, row-major pixel order, invalid pixel = (0,0,0)
     const uint16_t *z16 = nullptr;   // width*height depth counts, 0 = invalid
     ssd_gpu_intrinsics intrinsics{}; // of the depth stream (used with z16)
+    ssd_gpu_distortion distortion{}; // lens of the depth stream (rs2_intrinsics.model / coeffs; used with z16); zero: pin-hole
     int w = 0, h = 0;
     bool onDevice = false;
 
@@ -28,6 +29,11 @@ public:
     DepthFrame(const float *xyz, int width, int height, bool deviceMemory = false) : vertices(xyz), w(width), h(height), onDevice(deviceMemory) {}
     DepthFrame(const uint16_t *depth, const ssd_gpu_intrinsics &intr, int width, int height, bool deviceMemory = false)
     : z16(depth), intrinsics(intr), w(width), h(height), onDevice(deviceMemory)
+    {
+    }
+    DepthFrame(const uint16_t *depth, const ssd_gpu_intrinsics &intr, const ssd_gpu_distortion &lens, int width, int height,
+               bool deviceMemory = false)
+    : z16(depth), intrinsics(intr), distortion(lens), w(width), h(height), onDevice(deviceMemory)
     {
     }
     int width() const { return w; }

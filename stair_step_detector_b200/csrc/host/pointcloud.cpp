@@ -3,6 +3,7 @@
 #include "pointcloud.h"
 #include "transformation.h"
 #include "window.h"
+#include <cstring>
 #include <iostream>
 #include <stdexcept>
 
@@ -41,7 +42,13 @@ void Pointcloud::ensureContext(int width, int height) const
 
 void Pointcloud::enableOverlay(const ssd_gpu_intrinsics &intrinsics) const
 {
+  enableOverlay(intrinsics, ssd_gpu_distortion{});
+}
+
+void Pointcloud::enableOverlay(const ssd_gpu_intrinsics &intrinsics, const ssd_gpu_distortion &distortion) const
+{
   _overlayIntrinsics = intrinsics;
+  _overlayDistortion = distortion;
   _overlay = true;
   _overlayApplied = false;
   _risersApplied = false;
@@ -81,8 +88,8 @@ void Pointcloud::applySettings() const
   }
   if(!_camerasApplied)
   {
-    if(ssd_gpu_set_cameras(_ctx, _cameras.data(), static_cast<int>(_cameras.size())) != SSD_OK)
-      throw std::runtime_error(std::string("ssd_gpu_set_cameras: ") + ssd_gpu_last_error(_ctx));
+    if(ssd_gpu_set_cameras_ex(_ctx, _cameras.data(), _cameraDistortions.data(), static_cast<int>(_cameras.size())) != SSD_OK)
+      throw std::runtime_error(std::string("ssd_gpu_set_cameras_ex: ") + ssd_gpu_last_error(_ctx));
     _camerasApplied = true;
   }
 }
@@ -91,6 +98,14 @@ std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, i
 {
   ensureContext(frames.width(), frames.height());
   applySettings();
+  // the lens of the plain call: the frame's for z16 frames, the overlay's for vertex frames (set only when it changes)
+  const ssd_gpu_distortion &lens = frames.z16 ? frames.distortion : _overlayDistortion;
+  if(memcmp(&lens, &_lensApplied, sizeof(lens)) != 0)
+  {
+    if(ssd_gpu_set_distortion(_ctx, &lens) != SSD_OK)
+      throw std::runtime_error(std::string("ssd_gpu_set_distortion: ") + ssd_gpu_last_error(_ctx));
+    _lensApplied = lens;
+  }
   int rc;
   if(frames.z16)
     rc = frames.onDevice ? ssd_gpu_process_depth_device(_ctx, frames.z16, &frames.intrinsics, nFrames)
@@ -104,11 +119,17 @@ std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, i
 
 int Pointcloud::addCamera(const GeometricTransformation &trans, const ssd_gpu_intrinsics &intrinsics) const
 {
+  return addCamera(trans, intrinsics, ssd_gpu_distortion{});
+}
+
+int Pointcloud::addCamera(const GeometricTransformation &trans, const ssd_gpu_intrinsics &intrinsics, const ssd_gpu_distortion &distortion) const
+{
   ssd_gpu_camera c{};
   c.xf = trans.abi();
   trans.abiInverse(c.a_inv);
   c.intr = intrinsics;
   _cameras.push_back(c);
+  _cameraDistortions.push_back(distortion);
   _camerasApplied = false;
   return static_cast<int>(_cameras.size()) - 1;
 }
@@ -116,6 +137,7 @@ int Pointcloud::addCamera(const GeometricTransformation &trans, const ssd_gpu_in
 void Pointcloud::clearCameras() const
 {
   _cameras.clear();
+  _cameraDistortions.clear();
   _camerasApplied = false;
 }
 

@@ -40,6 +40,8 @@ public:
   // Pointcloud built with camera cameraOfFrame[i]'s transformation would (frames.intrinsics is then unused: every z16 frame is
   // deprojected with its camera's intrinsics).
   int addCamera(const GeometricTransformation &trans, const ssd_gpu_intrinsics &intrinsics) const;
+  // the same for a camera with lens distortion (ssd_gpu_set_cameras_ex): its z16 frames and its overlay go through the lens
+  int addCamera(const GeometricTransformation &trans, const ssd_gpu_intrinsics &intrinsics, const ssd_gpu_distortion &distortion) const;
   void clearCameras() const;
   int cameraCount() const { return static_cast<int>(_cameras.size()); }
   std::vector<Stairs> processBatch(const Camera::DepthFrame &frames, int nFrames, const std::vector<int32_t> &cameraOfFrame,
@@ -50,6 +52,9 @@ public:
   // (WorldToCamera, then DepthFrame::project with these depth-stream intrinsics). The quadrilaterals the reference
   // hands to drawQuadrilateral are then available per frame after process()/processBatch().
   void enableOverlay(const ssd_gpu_intrinsics &intrinsics) const;
+  // ... through a lens (ssd_gpu_set_distortion). The overlay of z16 frames uses the lens of the frame (DepthFrame::distortion),
+  // the overlay of vertex frames this one.
+  void enableOverlay(const ssd_gpu_intrinsics &intrinsics, const ssd_gpu_distortion &distortion) const;
   std::vector<Quadrilateralf_t> overlay(int frame = 0) const;
   // vertical faces (risers) from the remainder points -- the reference stops at "TODO use remainder to detect vertical faces"
   // (pointcloud.cpp:293); definition: include/ssd_gpu.h, ssd_gpu_riser. One more pass over the points when enabled.
@@ -70,7 +75,9 @@ private:
   mutable bool _overlay = false, _overlayApplied = false;
   mutable bool _risers = false, _risersApplied = false;
   mutable ssd_gpu_intrinsics _overlayIntrinsics{};
+  mutable ssd_gpu_distortion _overlayDistortion{}, _lensApplied{};
   mutable std::vector<ssd_gpu_camera> _cameras;
+  mutable std::vector<ssd_gpu_distortion> _cameraDistortions;
   mutable bool _camerasApplied = true;
 };
 

@@ -12,6 +12,7 @@
 #define SSD_SCENE_MODEL_H_
 
 #include "../../../include/ssd_scene.h"
+#include "../ssd_lens.h"
 #include <math.h>
 
 #ifdef __CUDACC__
@@ -93,6 +94,18 @@ SSD_HD void ssd_scene_default_hd(ssd_scene *s, int32_t width, int32_t height)
   s->rotate180 = 0;
   s->randomize_camera = 0;
   s->seed = 12345;
+  s->distortion_model = SSD_DISTORTION_NONE;
+  for(int i = 0; i < 5; i++)
+    s->coeffs[i] = 0.f;
+}
+
+SSD_HD ssd_gpu_distortion ssd_scene_lens(const ssd_scene *s)
+{
+  ssd_gpu_distortion d;
+  d.model = s->distortion_model;
+  for(int i = 0; i < 5; i++)
+    d.coeffs[i] = s->coeffs[i];
+  return d;
 }
 
 // frame `index` of a batch: geometry drawn from the distributions of SURVEY.md 8(d) config 3
@@ -210,7 +223,9 @@ SSD_HD uint16_t ssd_scene_depth(const ssd_scene *s, const ssd_scene_rt *rt, int 
   if(s->dropout > 0.f && ssd_u01(ph) < s->dropout)
     return 0;
 
-  const float dx = ((float)u - s->ppx) / s->fx, dy = ((float)v - s->ppy) / s->fy;
+  float dx = ((float)u - s->ppx) / s->fx, dy = ((float)v - s->ppy) / s->fy;
+  const ssd_gpu_distortion lens = ssd_scene_lens(s);
+  ssd_lens_deproject(&lens, dx, dy, &dx, &dy); // the ray of pixel (u, v) at z = 1 (the identity for the pin-hole)
   const float D[3] = { dx * rt->xc[0] + dy * rt->yc[0] + rt->zc[0], dx * rt->xc[1] + dy * rt->yc[1] + rt->zc[1],
                        dx * rt->xc[2] + dy * rt->yc[2] + rt->zc[2] };
   const float O[3] = { rt->ox, rt->oy, rt->oz };
@@ -331,19 +346,23 @@ SSD_HD uint16_t ssd_scene_depth(const ssd_scene *s, const ssd_scene_rt *rt, int 
   return (uint16_t)counts;
 }
 
-// z16 count -> vertex; single-rounded f32 operations in this order (the stubbed SDK deprojection)
+// z16 count -> vertex; single-rounded f32 operations in this order (the stubbed SDK deprojection), the scene's lens applied to
+// the normalised coordinates (include/ssd_gpu.h, ssd_gpu_distortion)
 SSD_HD void ssd_deproject_pixel(const ssd_scene *s, int u, int v, uint16_t d, float out[3])
 {
+  const ssd_gpu_distortion lens = ssd_scene_lens(s);
 #ifdef __CUDA_ARCH__
-  const float xn = __fdiv_rn(__fsub_rn((float)u, s->ppx), s->fx);
-  const float yn = __fdiv_rn(__fsub_rn((float)v, s->ppy), s->fy);
+  float xn = __fdiv_rn(__fsub_rn((float)u, s->ppx), s->fx);
+  float yn = __fdiv_rn(__fsub_rn((float)v, s->ppy), s->fy);
+  ssd_lens_deproject(&lens, xn, yn, &xn, &yn);
   const float z = __fmul_rn((float)d, s->depth_unit);
   out[0] = __fmul_rn(z, xn);
   out[1] = __fmul_rn(z, yn);
   out[2] = z;
 #else
-  const float xn = ((float)u - s->ppx) / s->fx;
-  const float yn = ((float)v - s->ppy) / s->fy;
+  float xn = ((float)u - s->ppx) / s->fx;
+  float yn = ((float)v - s->ppy) / s->fy;
+  ssd_lens_deproject(&lens, xn, yn, &xn, &yn);
   const float z = (float)d * s->depth_unit;
   out[0] = z * xn;
   out[1] = z * yn;

@@ -5,6 +5,7 @@
 // Every formula cites the reference file:line whose arithmetic (operation order) it reproduces.
 #pragma once
 #include "../../include/ssd_gpu.h"
+#include "ssd_lens.h"
 #include <cstdint>
 #include <cuda_runtime.h>
 
@@ -225,6 +226,40 @@ __device__ __forceinline__ const OverlayDev &frame_overlay(const OverlayDev &ov,
 __device__ __forceinline__ const OverlayDev &frame_overlay(const OverlayDev &ov, const CamTable &c, int frame)
 {
   return ov.enabled ? c.ov[frame_camera(c, frame)] : ov;
+}
+// The overlay through a distorted lens (k_finalize only): LensCam<NoCam> / LensCam<CamTable> behave as their BASE and add the lens
+// of the plain overlay (lens[0]) or of each camera (lens[camera]). NoCam and CamTable project through the pin-hole.
+template<class BASE>
+struct LensCam
+{
+  BASE base;
+  const ssd_gpu_distortion *lens;
+};
+template<class BASE>
+__device__ __forceinline__ const DevParams &frame_params(const DevParams &p, const LensCam<BASE> &c, int frame)
+{
+  return frame_params(p, c.base, frame);
+}
+template<class BASE>
+__device__ __forceinline__ const OverlayDev &frame_overlay(const OverlayDev &ov, const LensCam<BASE> &c, int frame)
+{
+  return frame_overlay(ov, c.base, frame);
+}
+template<class CAM>
+__device__ __forceinline__ void overlay_lens(const CAM &, int, float x, float y, float &xd, float &yd)
+{
+  xd = x;
+  yd = y;
+}
+__device__ __forceinline__ void overlay_lens(const LensCam<NoCam> &c, int, float x, float y, float &xd, float &yd)
+{
+  const ssd_gpu_distortion d = c.lens[0];
+  ssd_lens_project(&d, x, y, &xd, &yd);
+}
+__device__ __forceinline__ void overlay_lens(const LensCam<CamTable> &c, int frame, float x, float y, float &xd, float &yd)
+{
+  const ssd_gpu_distortion d = c.lens[frame_camera(c.base, frame)];
+  ssd_lens_project(&d, x, y, &xd, &yd);
 }
 
 struct P2d

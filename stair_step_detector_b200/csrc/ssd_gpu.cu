@@ -98,6 +98,17 @@ struct ssd_gpu_ctx
   OverlayDev *d_cam_ov = nullptr;
   float *d_cam_xn = nullptr, *d_cam_yn = nullptr, *d_cam_unit = nullptr;
   int *d_cam_of_frame = nullptr;         // max_frames: camera of each frame of the current call
+  // lenses (ssd_gpu_set_distortion / ssd_gpu_set_cameras_ex): one per-pixel ray table per distinct distorted lens
+  ssd_gpu_distortion lens{};             // lens of the plain calls (model NONE: pin-hole)
+  ssd_gpu_distortion *d_lens = nullptr;  // ... its device copy (overlay)
+  float2 *d_ray = nullptr;               // ray table of the plain calls' lens, built for ray_intr
+  ssd_gpu_intrinsics ray_intr{};
+  bool ray_valid = false;
+  std::vector<float2 *> cam_rays;        // distinct ray tables of the camera table (only when one of its cameras is distorted)
+  std::vector<unsigned char> cam_distorted;
+  bool cams_distorted = false;           // some camera of the table has a distorted lens
+  const float2 **d_cam_ray = nullptr;    // n_cameras: ray table of each camera
+  ssd_gpu_distortion *d_cam_lens = nullptr; // n_cameras
   double stats_eps0 = 0, stats_eps1 = 0; // filter bounds of the last call (largest over its cameras)
 };
 
@@ -364,6 +375,42 @@ __global__ void __launch_bounds__(256) k_deproject(int W, int N, float depth_uni
   dst[2] = make_float4(z2, __fmul_rn(z3, x4.w), __fmul_rn(z3, y), z3);
 }
 
+// Ray table of a lens (include/ssd_gpu.h, ssd_gpu_distortion): pixel (u, v) -> (x, y) of its ray at z = 1, x0 and y0 computed as
+// k_deproject_tables computes xn[u], yn[v] (so a pin-hole lens's table holds exactly those values), then the model's deprojection.
+// *bad is set when a ray is not finite (P^-1 diverged). grid-stride over the W*H pixels.
+__global__ void k_lens_rays(int W, int H, ssd_gpu_intrinsics in, ssd_gpu_distortion d, float2 *__restrict__ ray, unsigned *__restrict__ bad)
+{
+  const size_t N = (size_t)W * H;
+  for(size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (size_t)gridDim.x * blockDim.x)
+  {
+    const int v = (int)(i / W), u = (int)(i - (size_t)v * W);
+    const float x0 = __fdiv_rn(__fsub_rn((float)u, in.ppx), in.fx), y0 = __fdiv_rn(__fsub_rn((float)v, in.ppy), in.fy);
+    float x, y;
+    ssd_lens_deproject(&d, x0, y0, &x, &y);
+    ray[i] = make_float2(x, y);
+    if(!isfinite(x) || !isfinite(y))
+      *bad = 1u;
+  }
+}
+
+// k_deproject with a ray table: 4 consecutive pixels per thread. grid = (ceil(N/4/256), frames).
+__global__ void __launch_bounds__(256) k_deproject_lens(int N, float depth_unit, const float2 *__restrict__ ray, const uint16_t *__restrict__ depth,
+                                                        float *__restrict__ xyz)
+{
+  const int q = blockIdx.x * blockDim.x + threadIdx.x;
+  if(q * 4 >= N)
+    return;
+  const size_t fbase = (size_t)blockIdx.y * N;
+  const uint2 d = __ldg(reinterpret_cast<const uint2 *>(depth + fbase) + q);
+  const float4 r01 = __ldg(reinterpret_cast<const float4 *>(ray) + (size_t)q * 2), r23 = __ldg(reinterpret_cast<const float4 *>(ray) + (size_t)q * 2 + 1);
+  const float z0 = __fmul_rn((float)(d.x & 0xffffu), depth_unit), z1 = __fmul_rn((float)(d.x >> 16), depth_unit);
+  const float z2 = __fmul_rn((float)(d.y & 0xffffu), depth_unit), z3 = __fmul_rn((float)(d.y >> 16), depth_unit);
+  float4 *dst = reinterpret_cast<float4 *>(xyz + (fbase + (size_t)q * 4) * 3);
+  dst[0] = make_float4(__fmul_rn(z0, r01.x), __fmul_rn(z0, r01.y), z0, __fmul_rn(z1, r01.z));
+  dst[1] = make_float4(__fmul_rn(z1, r01.w), z1, __fmul_rn(z2, r23.x), __fmul_rn(z2, r23.y));
+  dst[2] = make_float4(z2, __fmul_rn(z3, r23.z), __fmul_rn(z3, r23.w), z3);
+}
+
 // ---------------------------------------------------------------------------------------------
 // single-stage kernels behind ssd_gpu_detect_outline / _front_edge / _points_in_quad / _camera_to_world: the host classes
 // Segmentation, QuadrilateralTest and CameraToWorld call them (same device functions as the chain)
@@ -466,9 +513,11 @@ __global__ void k_single_camera_to_world(const __grid_constant__ DevParams p, co
 // The classic chain: k_transform_bin -> k_peaks -> k_label_bev -> k_outline -> k_frame_logic -> k_quad_reduce -> k_finalize
 // (+ k_riser_reduce). CAM = NoCam: every frame with the context's own camera; CamTable: each frame with its camera's parameters
 // (camera calls; the word-record variant is never taken there).
+// sl: the chunk's z16 frames through ray tables (a call with a distorted lens), else nullptr. ov_lens: the lenses the overlay
+// projects through (LensCam), else nullptr.
 template<class CAM>
-static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const SrcDepth &sd, int frame0, int nf, int *launches, cudaEvent_t *ev,
-                          const CAM cam)
+static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const SrcDepth &sd, const SrcLens *sl, int frame0, int nf, int *launches,
+                          cudaEvent_t *ev, const CAM cam, const ssd_gpu_distortion *ov_lens)
 {
 #define STAGE_EV(i)                         \
   do                                        \
@@ -495,14 +544,18 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   STAGE_EV(0);
   if(fused)
   {
-    if(depth)
+    if(sl)
+      k_transform_bin_lens<SSD_PT_ITERS, true, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, cam);
+    else if(depth)
       k_transform_bin_depth<SSD_PT_ITERS, true, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, cam);
     else
       k_transform_bin<SSD_PT_ITERS, true, CAM><<<gpt, SSD_PT_THREADS, SSD_PT_ITERS * SSD_TB_STAGE_BYTES, st>>>(p, xyz_dev, labels, frames, cam);
   }
   else
   {
-    if(depth)
+    if(sl)
+      k_transform_bin_lens<SSD_PT_ITERS, false, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, cam);
+    else if(depth)
       k_transform_bin_depth<SSD_PT_ITERS, false, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, cam);
     else
       k_transform_bin<SSD_PT_ITERS, false, CAM><<<gpt, SSD_PT_THREADS, SSD_PT_ITERS * SSD_TB_STAGE_BYTES, st>>>(p, xyz_dev, labels, frames, cam);
@@ -525,7 +578,9 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   }
   if(!wrec)
   {
-    if(depth)
+    if(sl)
+      k_label_bev<SrcLens, false, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, nullptr, cam);
+    else if(depth)
       k_label_bev<SrcDepth, false, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, nullptr, cam);
     else
       k_label_bev<SrcVertices, false, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, nullptr, cam);
@@ -561,13 +616,25 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   }
   if(!wrec)
   {
-    if(depth)
+    if(sl)
+      k_quad_reduce<SrcLens, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, cam);
+    else if(depth)
       k_quad_reduce<SrcDepth, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, cam);
     else
       k_quad_reduce<SrcVertices, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, cam);
   }
   STAGE_EV(6);
-  if(ctx->outline_small)
+  if(ov_lens)
+  {
+    const LensCam<CAM> lc = { cam, ov_lens };
+    if(ctx->outline_small)
+      k_finalize<OutlineSharedSmall, LensCam<CAM>><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words,
+                                                                                             ctx->smem_cap_words, ctx->ov, ovl, lc);
+    else
+      k_finalize<OutlineShared, LensCam<CAM>><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words,
+                                                                                        ctx->smem_cap_words, ctx->ov, ovl, lc);
+  }
+  else if(ctx->outline_small)
     k_finalize<OutlineSharedSmall, CAM><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words, ctx->smem_cap_words,
                                                                                ctx->ov, ovl, cam);
   else
@@ -579,7 +646,9 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   if(ctx->risers)
   {
     // optional fourth pass: vertical faces from the remainder (labels are final once the chain's label kernel has run)
-    if(depth)
+    if(sl)
+      k_riser_reduce<SrcLens, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, cam);
+    else if(depth)
       k_riser_reduce<SrcDepth, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, cam);
     else
       k_riser_reduce<SrcVertices, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, cam);
@@ -595,8 +664,9 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
 // ---------------------------------------------------------------------------------------------
 // xyz_dev: packed vertices of the chunk, or nullptr with z16_dev: the chunk's depth frames, deprojected inside the
 // three point kernels (SrcDepth). cam: the camera table of a camera call (classic chain only), else nullptr.
+// sl: the call's lens source (its z16 member is set here), else nullptr; ov_lens: see launch_classic.
 static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uint16_t *z16_dev, float depth_unit, int frame0, int nf, int *launches,
-                        cudaEvent_t *ev, const CamTable *cam)
+                        cudaEvent_t *ev, const CamTable *cam, const SrcLens *sl, const ssd_gpu_distortion *ov_lens)
 {
 #define STAGE_EV(i)                         \
   do                                        \
@@ -636,11 +706,17 @@ static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uin
     *launches += 1;
   };
 
+  SrcLens sll;
+  if(sl)
+  {
+    sll = *sl;
+    sll.z16 = z16_dev;
+  }
   if(cam)
   {
     CamTable c = *cam;
     c.frame0 = frame0;
-    return launch_classic(ctx, s, sv, sd, frame0, nf, launches, ev, c);
+    return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, launches, ev, c, ov_lens);
   }
   if(ctx->records)
   {
@@ -750,7 +826,7 @@ static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uin
     CK(cudaGetLastError());
     return SSD_OK;
   }
-  return launch_classic(ctx, s, sv, sd, frame0, nf, launches, ev, NoCam());
+  return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, launches, ev, NoCam(), ov_lens);
 #undef STAGE_EV
 }
 
@@ -800,6 +876,12 @@ void ssd_gpu_destroy(ssd_gpu_ctx *ctx)
   cudaFree(ctx->d_cam_yn);
   cudaFree(ctx->d_cam_unit);
   cudaFree(ctx->d_cam_of_frame);
+  for(float2 *t : ctx->cam_rays)
+    cudaFree(t);
+  cudaFree(ctx->d_cam_ray);
+  cudaFree(ctx->d_cam_lens);
+  cudaFree(ctx->d_ray);
+  cudaFree(ctx->d_lens);
   for(int i = 0; i < SSD_MAX_STREAMS; i++)
   {
     cudaFree(ctx->d_stage[i]);
@@ -931,6 +1013,11 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
       cudaFuncSetAttribute(k_outline<OutlineSharedSmall, true, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       cudaFuncSetAttribute(k_finalize<OutlineShared, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      // the overlay through a distorted lens (ssd_gpu_set_distortion / ssd_gpu_set_cameras_ex)
+      cudaFuncSetAttribute(k_finalize<OutlineShared, LensCam<NoCam>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, LensCam<NoCam>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      cudaFuncSetAttribute(k_finalize<OutlineShared, LensCam<CamTable>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, LensCam<CamTable>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       cudaFuncSetAttribute(k_single_front_edge, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       granted = dyn;
     }
@@ -1051,6 +1138,45 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
   return SSD_OK;
 }
 
+// The ray table of lens d with intrinsics in into ray (N entries), on stream 0, synchronously. SSD_E_INVALID_ARG when a ray is
+// not finite: the lens does not admit this frame.
+static int build_ray_table(ssd_gpu_ctx *ctx, const ssd_gpu_intrinsics &in, const ssd_gpu_distortion &d, float2 *ray)
+{
+  const DevParams &p = ctx->dp;
+  unsigned *d_bad = nullptr;
+  CK(cudaMalloc(&d_bad, sizeof(unsigned)));
+  unsigned bad = 0;
+  cudaStream_t st = ctx->stream[0];
+  cudaError_t e = cudaMemsetAsync(d_bad, 0, sizeof(unsigned), st);
+  if(e == cudaSuccess)
+  {
+    k_lens_rays<<<(int)std::min<size_t>(((size_t)p.N + 255) / 256, 4096), 256, 0, st>>>(p.W, p.H, in, d, ray, d_bad);
+    e = cudaGetLastError();
+  }
+  if(e == cudaSuccess)
+    e = cudaMemcpyAsync(&bad, d_bad, sizeof(unsigned), cudaMemcpyDeviceToHost, st);
+  if(e == cudaSuccess)
+    e = cudaStreamSynchronize(st); // every stream reads the table
+  cudaFree(d_bad);
+  CK(e);
+  if(bad)
+    return fail(ctx, SSD_E_INVALID_ARG, "lens distortion: the deprojection is not finite at some pixel of the frame (the lens model diverges there)");
+  return SSD_OK;
+}
+
+static int check_distortion(ssd_gpu_ctx *ctx, const ssd_gpu_distortion &d, const std::string &who)
+{
+  static const char *const names[] = { "NONE", "MODIFIED_BROWN_CONRADY", "INVERSE_BROWN_CONRADY", "FTHETA", "BROWN_CONRADY", "KANNALA_BRANDT4" };
+  if(d.model != SSD_DISTORTION_NONE && d.model != SSD_DISTORTION_INVERSE_BROWN_CONRADY && d.model != SSD_DISTORTION_BROWN_CONRADY)
+    return fail(ctx, SSD_E_INVALID_ARG, who + ": distortion model " + std::to_string(d.model) +
+                                            (d.model >= 0 && d.model <= 5 ? std::string(" (") + names[d.model] + ")" : std::string()) +
+                                            " is not supported (NONE, INVERSE_BROWN_CONRADY and BROWN_CONRADY are)");
+  for(int i = 0; i < 5; i++)
+    if(!std::isfinite(d.coeffs[i]))
+      return fail(ctx, SSD_E_INVALID_ARG, who + ": distortion coefficient " + std::to_string(i) + " is not finite");
+  return SSD_OK;
+}
+
 // (re)build the deprojection tables when the intrinsics change
 static int ensure_deproject_tables(ssd_gpu_ctx *ctx, const ssd_gpu_intrinsics &in)
 {
@@ -1072,6 +1198,20 @@ static int ensure_deproject_tables(ssd_gpu_ctx *ctx, const ssd_gpu_intrinsics &i
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(ctx->stream[0])); // every stream reads the tables
     ctx->intr = in;
+  }
+  if(ssd_lens_is_pinhole(&ctx->lens))
+    return SSD_OK;
+  // a distorted lens: its ray table, rebuilt when the intrinsics change (ssd_gpu_set_distortion invalidates it)
+  if(!ctx->ray_valid || memcmp(&ctx->ray_intr, &in, sizeof(float) * 4) != 0)
+  {
+    if(!ctx->d_ray)
+      CK(cudaMalloc(&ctx->d_ray, sizeof(float2) * (size_t)p.N));
+    ctx->ray_valid = false;
+    const int rc = build_ray_table(ctx, in, ctx->lens, ctx->d_ray);
+    if(rc)
+      return rc;
+    ctx->ray_intr = in;
+    ctx->ray_valid = true;
   }
   return SSD_OK;
 }
@@ -1104,11 +1244,32 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
       cf = half;
   }
   const bool depth_input = xyz == nullptr;
+  // a distorted lens: depth frames read their rays from ray tables (SrcLens), the overlay projects through the lens (LensCam)
+  const bool plain_lens = !cam_of_frame && !ssd_lens_is_pinhole(&ctx->lens);
+  SrcLens sl{};
+  bool use_lens = false;
+  const ssd_gpu_distortion *ov_lens = nullptr;
+  if(cam_of_frame)
+  {
+    for(int f = 0; f < n_frames && depth_input && ctx->cams_distorted && !use_lens; f++)
+      use_lens = ctx->cam_distorted[cam_of_frame[f]] != 0;
+    sl.cam_ray = ctx->d_cam_ray;
+    if(ctx->cams_distorted && ctx->ov.enabled)
+      ov_lens = ctx->d_cam_lens;
+  }
+  else if(plain_lens)
+  {
+    use_lens = depth_input;
+    if(ctx->ov.enabled)
+      ov_lens = ctx->d_lens;
+  }
   if(depth_input && !cam_of_frame)
   {
     const int rc = ensure_deproject_tables(ctx, *intr);
     if(rc)
       return rc;
+    sl.ray = ctx->d_ray;
+    sl.unit = intr->depth_unit;
   }
   // depth frames are deprojected inside the point kernels (SrcDepth): no vertex array is ever written.
   const bool unfused = ctx->depth_unfused; // A/B switch (SSD_GPU_DEPTH_UNFUSED, read in ssd_gpu_create)
@@ -1213,7 +1374,10 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
     {
       // A/B path (SSD_GPU_DEPTH_UNFUSED=1): materialise the vertices, then the vertex kernels
       // (the vertex staging of stream s is free: the chunk that used it last ran on this very stream)
-      k_deproject<<<dim3((p.N / 4 + 255) / 256, nf), 256, 0, ctx->stream[s]>>>(p.W, p.N, intr->depth_unit, ctx->d_xn, ctx->d_yn, dsrc, ctx->d_stage[s]);
+      if(use_lens)
+        k_deproject_lens<<<dim3((p.N / 4 + 255) / 256, nf), 256, 0, ctx->stream[s]>>>(p.N, intr->depth_unit, ctx->d_ray, dsrc, ctx->d_stage[s]);
+      else
+        k_deproject<<<dim3((p.N / 4 + 255) / 256, nf), 256, 0, ctx->stream[s]>>>(p.W, p.N, intr->depth_unit, ctx->d_xn, ctx->d_yn, dsrc, ctx->d_stage[s]);
       launches++;
       src = ctx->d_stage[s];
       if(host_input)
@@ -1221,7 +1385,8 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
     }
     const bool fused = depth_input && !unfused;
     const int rc = launch_chunk(ctx, s, fused ? nullptr : src, fused ? dsrc : nullptr, fused && intr ? intr->depth_unit : 0.f, f0, nf, &launches,
-                                stage_timing ? &ctx->stage_ev[(size_t)chunk * (SSD_GPU_N_STAGES + 1)] : nullptr, cam_of_frame ? &cams : nullptr);
+                                stage_timing ? &ctx->stage_ev[(size_t)chunk * (SSD_GPU_N_STAGES + 1)] : nullptr, cam_of_frame ? &cams : nullptr,
+                                fused && use_lens ? &sl : nullptr, ov_lens);
     if(rc)
       return rc;
     if(host_input && (!depth_input || fused))
@@ -1347,6 +1512,10 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
 static int process_common(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16, const ssd_gpu_intrinsics *intr, bool host_input, int n_frames,
                           int flags, const int32_t *cam_of_frame = nullptr)
 {
+  // refused before anything is launched: the results of the previous call stay readable
+  if(ctx && !cam_of_frame && !ssd_lens_is_pinhole(&ctx->lens) && (ctx->records || ctx->wordrec || ctx->resident) && (!xyz || ctx->ov.enabled))
+    return fail(ctx, SSD_E_STATE, "lens distortion runs on the default (classic) chain only; this context was created with "
+                                  "SSD_GPU_PATH=records|wordrec|resident");
   const int rc = process_impl(ctx, xyz, z16, intr, host_input, n_frames, flags, cam_of_frame);
   if(rc != SSD_OK && rc != SSD_E_INVALID_ARG && rc != SSD_E_RANGE && ctx)
   {
@@ -1394,8 +1563,16 @@ int ssd_gpu_process_depth_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, cons
 // ---- per-frame cameras ----
 static void free_cameras(ssd_gpu_ctx *ctx)
 {
-  for(void *p : { (void *)ctx->d_cam_dp, (void *)ctx->d_cam_ov, (void *)ctx->d_cam_xn, (void *)ctx->d_cam_yn, (void *)ctx->d_cam_unit })
+  for(void *p : { (void *)ctx->d_cam_dp, (void *)ctx->d_cam_ov, (void *)ctx->d_cam_xn, (void *)ctx->d_cam_yn, (void *)ctx->d_cam_unit,
+                  (void *)ctx->d_cam_ray, (void *)ctx->d_cam_lens })
     cudaFree(p);
+  for(float2 *t : ctx->cam_rays)
+    cudaFree(t);
+  ctx->cam_rays.clear();
+  ctx->cam_distorted.clear();
+  ctx->cams_distorted = false;
+  ctx->d_cam_ray = nullptr;
+  ctx->d_cam_lens = nullptr;
   ctx->d_cam_dp = nullptr;
   ctx->d_cam_ov = nullptr;
   ctx->d_cam_xn = ctx->d_cam_yn = ctx->d_cam_unit = nullptr;
@@ -1404,10 +1581,76 @@ static void free_cameras(ssd_gpu_ctx *ctx)
   ctx->n_cameras = 0;
 }
 
+// The ray tables of a camera table with at least one distorted lens: one per distinct lens (the intrinsics' fx, fy, ppx, ppy and the
+// distortion, compared bitwise; a pin-hole camera's lens is model NONE), built and checked before the table is replaced. Cameras
+// without depth intrinsics get none. On failure every table built here is freed.
+struct CamLensKey
+{
+  float in[4];
+  ssd_gpu_distortion d;
+};
+static int build_camera_rays(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, const std::vector<ssd_gpu_distortion> &lens,
+                             const std::vector<unsigned char> &depth_ok, std::vector<float2 *> &tables, std::vector<const float2 *> &of_camera)
+{
+  std::vector<CamLensKey> keys;
+  of_camera.assign(lens.size(), nullptr);
+  for(size_t c = 0; c < lens.size(); c++)
+  {
+    if(!depth_ok[c])
+      continue;
+    CamLensKey k;
+    memset(&k, 0, sizeof(k));
+    memcpy(k.in, &cams[c].intr, sizeof(k.in));
+    if(!ssd_lens_is_pinhole(&lens[c]))
+      k.d = lens[c];
+    size_t t = 0;
+    while(t < keys.size() && memcmp(&keys[t], &k, sizeof(k)) != 0)
+      t++;
+    if(t == keys.size())
+    {
+      float2 *ray = nullptr;
+      cudaError_t e = cudaMalloc(&ray, sizeof(float2) * (size_t)ctx->dp.N);
+      if(e != cudaSuccess)
+      {
+        ctx->err = std::string("cudaMalloc (ray table): ") + cudaGetErrorString(e);
+        return SSD_E_CUDA;
+      }
+      tables.push_back(ray);
+      keys.push_back(k);
+      const int rc = build_ray_table(ctx, cams[c].intr, k.d, ray);
+      if(rc)
+      {
+        if(rc == SSD_E_INVALID_ARG)
+          ctx->err = "ssd_gpu_set_cameras_ex: camera " + std::to_string(c) + ": " + ctx->err;
+        return rc;
+      }
+    }
+    of_camera[c] = tables[t];
+  }
+  return SSD_OK;
+}
+
 int ssd_gpu_set_cameras(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, int n_cameras)
+{
+  return ssd_gpu_set_cameras_ex(ctx, cams, nullptr, n_cameras);
+}
+
+int ssd_gpu_set_cameras_ex(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, const ssd_gpu_distortion *dist, int n_cameras)
 {
   if(!ctx || n_cameras < 0 || (n_cameras > 0 && !cams))
     return fail(ctx, SSD_E_INVALID_ARG, "ssd_gpu_set_cameras: bad argument");
+  std::vector<ssd_gpu_distortion> lens((size_t)n_cameras);
+  std::vector<unsigned char> distorted((size_t)n_cameras, 0);
+  bool any_distorted = false;
+  for(int c = 0; c < n_cameras && dist; c++)
+  {
+    const int rc = check_distortion(ctx, dist[c], "ssd_gpu_set_cameras_ex: camera " + std::to_string(c));
+    if(rc)
+      return rc;
+    lens[c] = dist[c];
+    distorted[c] = !ssd_lens_is_pinhole(&dist[c]);
+    any_distorted = any_distorted || distorted[c];
+  }
   // every camera is checked before the table is touched: a rejected table leaves the previous one in place
   std::vector<DevParams> dp((size_t)n_cameras);
   std::vector<OverlayDev> ov((size_t)n_cameras);
@@ -1432,7 +1675,21 @@ int ssd_gpu_set_cameras(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, int n_came
   }
   CK(cudaSetDevice(ctx->device));
   CK(cudaDeviceSynchronize());
+  // the ray tables are built (and the lenses checked) before the previous table is freed
+  std::vector<float2 *> rays;
+  std::vector<const float2 *> ray_of_camera;
+  if(any_distorted)
+  {
+    const int rc = build_camera_rays(ctx, cams, lens, depth_ok, rays, ray_of_camera);
+    if(rc)
+    {
+      for(float2 *t : rays)
+        cudaFree(t);
+      return rc;
+    }
+  }
   free_cameras(ctx);
+  ctx->cam_rays.swap(rays);
   if(n_cameras == 0)
     return SSD_OK;
   const DevParams &p = ctx->dp;
@@ -1445,6 +1702,8 @@ int ssd_gpu_set_cameras(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, int n_came
   CK(cudaMalloc(&ctx->d_cam_xn, sizeof(float) * (size_t)n_cameras * p.W));
   CK(cudaMalloc(&ctx->d_cam_yn, sizeof(float) * (size_t)n_cameras * p.H));
   CK(cudaMalloc(&d_in, sizeof(ssd_gpu_camera) * (size_t)n_cameras));
+  CK(cudaMalloc(&ctx->d_cam_lens, sizeof(ssd_gpu_distortion) * (size_t)n_cameras));
+  CK(cudaMalloc(&ctx->d_cam_ray, sizeof(float2 *) * (size_t)n_cameras));
   cudaStream_t st = ctx->stream[0];
   cudaError_t e = cudaMemcpyAsync(ctx->d_cam_dp, dp.data(), sizeof(DevParams) * (size_t)n_cameras, cudaMemcpyHostToDevice, st);
   if(e == cudaSuccess)
@@ -1453,6 +1712,10 @@ int ssd_gpu_set_cameras(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, int n_came
     e = cudaMemcpyAsync(ctx->d_cam_unit, unit.data(), sizeof(float) * (size_t)n_cameras, cudaMemcpyHostToDevice, st);
   if(e == cudaSuccess)
     e = cudaMemcpyAsync(d_in, cams, sizeof(ssd_gpu_camera) * (size_t)n_cameras, cudaMemcpyHostToDevice, st);
+  if(e == cudaSuccess)
+    e = cudaMemcpyAsync(ctx->d_cam_lens, lens.data(), sizeof(ssd_gpu_distortion) * (size_t)n_cameras, cudaMemcpyHostToDevice, st);
+  if(e == cudaSuccess && any_distorted)
+    e = cudaMemcpyAsync(ctx->d_cam_ray, ray_of_camera.data(), sizeof(float2 *) * (size_t)n_cameras, cudaMemcpyHostToDevice, st);
   if(e == cudaSuccess)
   {
     // (cameras without depth intrinsics get meaningless tables: depth calls never use them)
@@ -1470,8 +1733,43 @@ int ssd_gpu_set_cameras(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, int n_came
   }
   ctx->cam_dp.swap(dp);
   ctx->cam_depth_ok.swap(depth_ok);
+  ctx->cam_distorted.swap(distorted);
+  ctx->cams_distorted = any_distorted;
   ctx->n_cameras = n_cameras;
   return SSD_OK;
+}
+
+int ssd_gpu_set_distortion(ssd_gpu_ctx *ctx, const ssd_gpu_distortion *d)
+{
+  if(!ctx)
+    return SSD_E_INVALID_ARG;
+  ssd_gpu_distortion nd{};
+  if(d)
+  {
+    const int rc = check_distortion(ctx, *d, "ssd_gpu_set_distortion");
+    if(rc)
+      return rc;
+    nd = *d;
+  }
+  if(!ssd_lens_is_pinhole(&nd))
+  {
+    CK(cudaSetDevice(ctx->device));
+    if(!ctx->d_lens)
+      CK(cudaMalloc(&ctx->d_lens, sizeof(ssd_gpu_distortion)));
+    CK(cudaDeviceSynchronize()); // no call in flight reads the lens or the ray table
+    CK(cudaMemcpy(ctx->d_lens, &nd, sizeof(nd), cudaMemcpyHostToDevice));
+  }
+  if(memcmp(&nd, &ctx->lens, sizeof(nd)) != 0)
+    ctx->ray_valid = false; // rebuilt for the next depth call's intrinsics
+  ctx->lens = nd;
+  return SSD_OK;
+}
+
+int ssd_gpu_n_ray_tables(ssd_gpu_ctx *ctx)
+{
+  if(!ctx)
+    return SSD_E_INVALID_ARG;
+  return (int)ctx->cam_rays.size() + (ctx->ray_valid && !ssd_lens_is_pinhole(&ctx->lens) ? 1 : 0);
 }
 
 int ssd_gpu_n_cameras(ssd_gpu_ctx *ctx)
@@ -1547,9 +1845,16 @@ int ssd_gpu_deproject_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const ss
   if(rc)
     return rc;
   const DevParams &p = ctx->dp;
+  const bool lens = !ssd_lens_is_pinhole(&ctx->lens);
   for(int f0 = 0; f0 < n_frames; f0 += 32768)
   {
     const int nf = std::min(32768, n_frames - f0);
+    if(lens)
+    {
+      k_deproject_lens<<<dim3((p.N / 4 + 255) / 256, nf), 256, 0, ctx->stream[0]>>>(p.N, intr->depth_unit, ctx->d_ray, z16_dev + (size_t)f0 * p.N,
+                                                                                  xyz_dev + (size_t)f0 * p.N * 3);
+      continue;
+    }
     k_deproject<<<dim3((p.N / 4 + 255) / 256, nf), 256, 0, ctx->stream[0]>>>(p.W, p.N, intr->depth_unit, ctx->d_xn, ctx->d_yn, z16_dev + (size_t)f0 * p.N,
                                                                             xyz_dev + (size_t)f0 * p.N * 3);
   }

@@ -1512,7 +1512,8 @@ __global__ void __launch_bounds__(SSD_OL_THREADS, SSD_OL_MINB) k_finalize(const 
         const float X = (float)((ov.a_inv[0] * dx + ov.a_inv[1] * dy) + ov.a_inv[2] * dz);
         const float Y = (float)((ov.a_inv[3] * dx + ov.a_inv[4] * dy) + ov.a_inv[5] * dz);
         const float Z = (float)((ov.a_inv[6] * dx + ov.a_inv[7] * dy) + ov.a_inv[8] * dz);
-        const float x = __fdiv_rn(X, Z), y = __fdiv_rn(Y, Z);
+        float x, y;
+        overlay_lens(cam, frame, __fdiv_rn(X, Z), __fdiv_rn(Y, Z), x, y);
         Q[s].px[c][0] = __fadd_rn(__fmul_rn(x, ov.fx), ov.ppx);
         Q[s].px[c][1] = __fadd_rn(__fmul_rn(y, ov.fy), ov.ppy);
       }

@@ -69,9 +69,30 @@ struct SrcDepth
   float unit;                  // metres per depth unit
   unsigned long long wmagic;   // ceil(2^40 / W): row of pixel i = (i * wmagic) >> 40, exact for i * W < 2^40
 };
+// SrcLens: z16 frames of a camera with a distorted lens (ssd_gpu_set_distortion). Its ray (x, y) depends on u and v, so it is
+// read per pixel from the lens's ray table (k_lens_rays): 2 B of depth + 8 B of ray per point, the table shared by every frame
+// of the lens and L2-resident at the usual frame sizes. Then X = z * x, Y = z * y as for SrcDepth.
+struct SrcLens
+{
+  const uint16_t *z16;              // n_frames x N
+  const float2 *ray;                // N rays of the lens (plain calls)
+  const float2 *const *cam_ray;     // camera calls: the ray table of each camera (a pin-hole camera's holds (xn[u], yn[v]))
+  float unit;
+};
 struct FrameV
 {
   const float4 *f4;
+};
+struct FrameL
+{
+  const uint2 *d2;    // four z16 pixels per element
+  const float4 *r4;   // two rays per element
+  float unit;
+};
+struct WordL
+{
+  uint2 d;
+  float4 r01, r23;
 };
 struct FrameD
 {
@@ -105,6 +126,66 @@ struct SrcTraits<SrcDepth>
   typedef FrameD Frame;
   typedef WordD Word;
 };
+template<>
+struct SrcTraits<SrcLens>
+{
+  typedef FrameL Frame;
+  typedef WordL Word;
+};
+__device__ __forceinline__ FrameL src_frame(const SrcLens &s, const DevParams &, size_t fbase)
+{
+  FrameL f;
+  f.d2 = reinterpret_cast<const uint2 *>(s.z16 + fbase);
+  f.r4 = reinterpret_cast<const float4 *>(s.ray);
+  f.unit = s.unit;
+  return f;
+}
+__device__ __forceinline__ SrcLens frame_src(const SrcLens &s, const CamTable &c, const DevParams &, int frame)
+{
+  const int cam = frame_camera(c, frame);
+  SrcLens d = s;
+  d.ray = s.cam_ray[cam];
+  d.unit = __ldg(c.unit + cam);
+  return d;
+}
+__device__ __forceinline__ void word_zero(WordL &r)
+{
+  r.d = make_uint2(0u, 0u);
+  r.r01 = r.r23 = make_float4(0.f, 0.f, 0.f, 0.f);
+}
+__device__ __forceinline__ void word_load(const FrameL &f, unsigned w, WordL &r)
+{
+  r.d = __ldg(f.d2 + w);
+  r.r01 = __ldg(f.r4 + (size_t)w * 2);
+  r.r23 = __ldg(f.r4 + (size_t)w * 2 + 1);
+}
+__device__ __forceinline__ void word_unpack(const FrameL &f, const WordL &r, float vx[4], float vy[4], float vz[4])
+{
+  vz[0] = __fmul_rn((float)(r.d.x & 0xffffu), f.unit);
+  vz[1] = __fmul_rn((float)(r.d.x >> 16), f.unit);
+  vz[2] = __fmul_rn((float)(r.d.y & 0xffffu), f.unit);
+  vz[3] = __fmul_rn((float)(r.d.y >> 16), f.unit);
+  const float rx[4] = { r.r01.x, r.r01.z, r.r23.x, r.r23.z }, ry[4] = { r.r01.y, r.r01.w, r.r23.y, r.r23.w };
+#pragma unroll
+  for(int j = 0; j < 4; j++)
+  {
+    vx[j] = __fmul_rn(vz[j], rx[j]);
+    vy[j] = __fmul_rn(vz[j], ry[j]);
+  }
+}
+__device__ __forceinline__ void word_prefetch_l2(const FrameL &f, unsigned w)
+{
+  asm volatile("prefetch.global.L2 [%0];" ::"l"(f.d2 + w));
+  asm volatile("prefetch.global.L2 [%0];" ::"l"(f.r4 + (size_t)w * 2)); // the word's 32 bytes of rays: one sector
+}
+__device__ __forceinline__ void point_load(const FrameL &f, unsigned pt, float &x, float &y, float &z)
+{
+  const unsigned d = __ldg(reinterpret_cast<const unsigned short *>(f.d2) + pt);
+  const float2 r = __ldg(reinterpret_cast<const float2 *>(f.r4) + pt);
+  z = __fmul_rn((float)d, f.unit);
+  x = __fmul_rn(z, r.x);
+  y = __fmul_rn(z, r.y);
+}
 __device__ __forceinline__ FrameV src_frame(const SrcVertices &s, const DevParams &p, size_t fbase)
 {
   FrameV f;
@@ -623,6 +704,60 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_depth(const __
   const int q0 = blockIdx.x * (ITERS * SSD_PT_THREADS) + tid;
   const FrameD F = src_frame(src, p, fbase);
   WordD w[ITERS];
+#pragma unroll
+  for(int it = 0; it < ITERS; it++)
+  {
+    word_zero(w[it]);
+    if(q0 + it * SSD_PT_THREADS < nquads)
+      word_load(F, (unsigned)(q0 + it * SSD_PT_THREADS), w[it]);
+  }
+  s_hist[tid] = 0; // SSD_PT_THREADS == SSD_BINS_PAD
+  if(tid == 0)
+    s_exact = 0;
+  __syncthreads();
+  unsigned *dst = reinterpret_cast<unsigned *>(codes + fbase) + q0;
+  unsigned exact = 0;
+#pragma unroll
+  for(int it = 0; it < ITERS; it++)
+    if(q0 + it * SSD_PT_THREADS < nquads)
+    {
+      float vx[4], vy[4], vz[4];
+      word_unpack(F, w[it], vx, vy, vz);
+      tb_word(p, vx, vy, vz, dst + it * SSD_PT_THREADS, s_hist, exact);
+    }
+  if(exact)
+    atomicAdd(&s_exact, exact);
+  __syncthreads();
+  const unsigned sum = s_hist[tid];
+  if(sum)
+    atomicAdd(&frames[frame].hist[tid], sum);
+  if(tid == 0 && s_exact)
+    atomicAdd(&frames[frame].n_exact_bin, s_exact);
+  if(FUSE_PEAKS)
+  {
+    __shared__ PeaksScratch K;
+    __shared__ unsigned s_last;
+    tb_fused_peaks(p, frames[frame], K, s_last, tid);
+  }
+}
+// k_transform_bin_lens: the same pass on z16 frames of a distorted lens (SrcLens), 10 bytes per point in (2 of depth, 8 of ray
+// from the L2-resident table). A copy of k_transform_bin_depth's body: that kernel's code stays as it was.
+template<int ITERS, bool FUSE_PEAKS = false, class CAM = NoCam>
+__global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_lens(const __grid_constant__ DevParams p0, const SrcLens src0,
+                                                                        unsigned char *__restrict__ codes, FrameDev *__restrict__ frames,
+                                                                        const CAM cam = CAM())
+{
+  __shared__ unsigned s_hist[SSD_BINS_PAD];
+  __shared__ unsigned s_exact;
+  const int tid = threadIdx.x;
+  const int frame = blockIdx.y;
+  const DevParams &p = frame_params(p0, cam, frame);
+  const auto &src = frame_src(src0, cam, p, frame);
+  const size_t fbase = (size_t)frame * p.N;
+  const int nquads = p.N >> 2;
+  const int q0 = blockIdx.x * (ITERS * SSD_PT_THREADS) + tid;
+  const FrameL F = src_frame(src, p, fbase);
+  WordL w[ITERS];
 #pragma unroll
   for(int it = 0; it < ITERS; it++)
   {
