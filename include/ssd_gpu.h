@@ -196,8 +196,7 @@ int ssd_gpu_process_device_ex(ssd_gpu_ctx *ctx, const float *xyz_dev, int n_fram
  * kernel: a call then only uploads camera_of_frame (4 bytes per frame).
  * camera_of_frame: host array of n_frames indices into the table. Checked before anything is launched: a camera call without a
  * table returns SSD_E_STATE, an index outside [0, n_cameras) SSD_E_RANGE, a depth call that uses a camera without valid
- * intrinsics SSD_E_INVALID_ARG; the results of the previous call stay readable. Camera calls run on the default chain only:
- * SSD_GPU_PATH=records|wordrec|resident (and SSD_GPU_DEPTH_UNFUSED=1 for depth calls) return SSD_E_STATE.
+ * intrinsics SSD_E_INVALID_ARG; the results of the previous call stay readable.
  * Results are read with the getters above; ssd_gpu_get_stats counts the whole call and reports the largest filter bounds of
  * the cameras it used. A plain ssd_gpu_process_* call keeps using the context's own transform.
  */
@@ -245,8 +244,7 @@ int ssd_gpu_process_depth_cameras_device(ssd_gpu_ctx *ctx, const uint16_t *z16_d
  *
  * ssd_gpu_set_distortion: the lens of the plain calls (ssd_gpu_process_depth_host/_device, ssd_gpu_deproject_device and the
  * plain overlay of ssd_gpu_set_overlay); NULL or SSD_DISTORTION_NONE switches it off. Vertex input is already deprojected:
- * there only the overlay uses it. A depth call with a distorted lens on SSD_GPU_PATH=records|wordrec|resident returns
- * SSD_E_STATE; SSD_GPU_DEPTH_UNFUSED=1 deprojects with the kernel of ssd_gpu_deproject_device.
+ * there only the overlay uses it.
  * ssd_gpu_set_cameras_ex: ssd_gpu_set_cameras with one lens per camera (dist: n_cameras entries, NULL = all pin-hole); the lens
  * applies to the camera's depth frames and overlay. ssd_gpu_set_cameras(c, n) is ssd_gpu_set_cameras_ex(c, NULL, n). A rejected
  * lens or table leaves the previous one and the previous results in place.

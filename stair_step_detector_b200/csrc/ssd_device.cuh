@@ -59,15 +59,6 @@ struct DevParams
   unsigned long long axy2[3], bxy2, auv2[3], buv2;
   // {sa[j], sa[3+j]}, {sb[0], sb[1]}: the x and y rows of the range-scaled transform (point_code_scaled)
   unsigned long long sxy2[3], sbxy2;
-  // record chain / resident-frame path. Per-point record: ix | iy << rec_bx | (bin code & 1) << (rec_bx + rec_by) | d << (32 - rec_zbits), d = the point's
-  // height offset from the centre of its bin in units of 2^-rec_zshift m (rec_mf = height_interval * 2^rec_zshift,
-  // |d| <= rec_mf / 2 < 2^(rec_zbits - 1)); iy == H marks a pixel the f32 chain could not decide. rec_zbits == 0: the
-  // frame size does not admit the path.
-  int rec_bx, rec_by, rec_zbits, rec_zshift;
-  float rec_mf;
-  int gs_steps;            // 128-point steps per frame
-  // k_quad_sum: world rectangle of a BEV pixel box in single precision (x = ix * gs_xw + gs_x0, y = gs_y0 - iy * gs_yw)
-  float gs_xw, gs_x0, gs_yw, gs_y0, gs_margin, pad4;
 };
 
 struct SegmentDev
@@ -123,11 +114,7 @@ struct PlateauDev
   double quad_px[4][2];
   double quad_world[4][2];
   double mean_z;
-  unsigned long long sum_fix; // sum of z_fix_u() over the points inside the quadrilateral that were tested one by one
-  // ... and of the points taken in as whole 32-pixel summaries (k_quad_sum): height offsets, bin codes, how many
-  long long sum_d;
-  unsigned long long sum_c;
-  unsigned n_sum, pad_s;
+  unsigned long long sum_fix; // sum of z_fix_u() over the points inside the quadrilateral
   int row_min, row_max;       // BEV rows touched by this plateau's bitmap
   int front_valid;
   int pad;
@@ -148,7 +135,6 @@ struct FrameDev
   unsigned hist[SSD_BINS_PAD];
   unsigned short lut16[SSD_BINS_PAD]; // bin code -> segment label | 0x100 if that label gets a BEV image (k_peaks)
   unsigned quad_amask;                // labels k_quad_reduce reduces: ground + valid plateaus with a usable test (k_frame_logic)
-  unsigned ready;                     // k_frame_stream: plateau records and lut16 are written (the frame barrier's flag)
   unsigned tb_done, ol_done;          // fused small-batch chain: blocks of k_transform_bin / k_outline that have finished this frame
   QuadFilterDev qf[SSD_GPU_MAX_PLATEAUS]; // f32 image of each step's QuadrilateralTest (k_frame_logic)
   unsigned status;

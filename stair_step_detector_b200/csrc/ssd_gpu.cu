@@ -3,17 +3,13 @@
 #include "ssd_device.cuh"
 #include "ssd_kernels_points.cuh"
 #include "ssd_kernels_outline.cuh"
-#include "ssd_kernels_stream.cuh"
-#include "ssd_kernels_records.cuh"
 
 #include <algorithm>
 #include <cmath>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <string>
-#include <type_traits>
 #include <vector>
 
 #ifndef SSD_PT_ITERS
@@ -45,9 +41,9 @@ struct ssd_gpu_ctx
   int n_streams = 2;
   cudaStream_t stream[SSD_MAX_STREAMS]{};
   cudaStream_t copy_stream{};
-  // knobs, read once in ssd_gpu_create (DESIGN.md): blocks per frame of the point kernels, small-batch split, depth A/B path
+  // knobs, read once in ssd_gpu_create (DESIGN.md): blocks per frame of the point kernels, small-batch split
   int bpf_l_knob = 0, bpf_q_knob = 0;
-  bool no_split_small = false, depth_unfused = false;
+  bool no_split_small = false;
   cudaEvent_t ev_start{}, ev_stop{}, ev_h2d0{}, ev_h2d1{};
   cudaEvent_t ev_in_ready[SSD_MAX_STREAMS]{}, ev_in_free[SSD_MAX_STREAMS]{}, ev_chunk_done[SSD_MAX_STREAMS]{};
   FrameDev *d_frames = nullptr;   // max_frames
@@ -57,27 +53,11 @@ struct ssd_gpu_ctx
   ssd_gpu_overlay *d_ovl = nullptr, *h_ovl = nullptr; // max_frames * SSD_GPU_MAX_STEPS, allocated by ssd_gpu_set_overlay
   unsigned char *d_labels = nullptr; // max_frames * N
   unsigned *d_bev = nullptr; // 2 x chunk_frames * MAX_PLATEAUS * bm_words (per stream)
-  float *d_stage[SSD_MAX_STREAMS]{};            // vertex staging (host input / deprojected depth)
-  int stage_frames[SSD_MAX_STREAMS]{};          // ... and its capacity in frames
+  float *d_stage[SSD_MAX_STREAMS]{};            // vertex staging of the host-input calls (host_chunk_frames)
   uint16_t *d_depth[SSD_MAX_STREAMS]{};         // z16 staging of the host depth-frame path
   float *d_xn = nullptr, *d_yn = nullptr;       // deprojection tables: (u - ppx) / fx per column, (v - ppy) / fy per row
   ssd_gpu_intrinsics intr{};                    // intrinsics the tables were built for
-  // resident-frame path (ssd_kernels_stream.cuh): one persistent kernel per chunk instead of the three point passes
-  bool resident = false;
-  bool records = false;           // record chain (ssd_kernels_records.cuh): the default where the frame size admits it
-  uint4 *d_rec4 = nullptr;        // n_streams x chunk_frames x N/4 x {4 records}
-  // word-record chain (SSD_GPU_PATH=wordrec, experimental): k_label_bev<SRC, true> leaves 8 bytes per 4-pixel word of the
-  // outlined plateaus, k_quad_reduce_rec takes the words that lie inside their step's quadrilateral from those
-  bool wordrec = false;
   bool risers = false;            // ssd_gpu_set_vertical_faces: k_riser_reduce after the chain
-  uint2 *d_wrec = nullptr;        // n_streams x chunk_frames x N/4
-  int fs_grid = 0, fs_d_raw = 4, fs_d_rec = 0, fs_lag_frames = 8;
-  GroupSum *d_sums = nullptr;     // n_streams x chunk_frames x N/32 summaries
-  unsigned *d_done = nullptr;     // n_streams x chunk_frames frame counters (self-resetting)
-  unsigned char *d_recs = nullptr; // record ring of k_frame_stream (one kernel at a time uses it): grid x 16 warps x fs_d_rec slots, L2-resident
-  unsigned long long *d_prof = nullptr; // SSD_GPU_FS_PROF=1: cycle counters of k_frame_stream
-  cudaEvent_t ev_fs{};            // the persistent kernels of consecutive chunks never overlap (each wants every SM)
-  bool fs_pending = false;
   int pt_blocks_target = 0;       // blocks per launch of the tile-looping point kernels
   int n_frames_last = 0;
   int flags_last = 0;
@@ -290,33 +270,6 @@ static int derive_params(const ssd_gpu_config &c, const ssd_gpu_transform &t, De
     d.sbxy2 = f2_pack_bits(d.sb[0], d.sb[1]);
     d.buv2 = f2_pack_bits(d.bu, d.bv);
   }
-  {
-    // resident-frame path: record layout and the summary -> world-rectangle map (ssd_kernels_stream.cuh)
-    int bx = 1, by = 1;
-    while((1 << bx) < c.width)
-      bx++;
-    while((1 << by) < c.height + 1)
-      by++;
-    const int zbits = std::min(12, 32 - bx - by - 1); // (one bit: parity of the bin code)
-    d.rec_bx = bx;
-    d.rec_by = by;
-    d.rec_zbits = 0;
-    d.gs_steps = d.N / SSD_FS_STEP_PX;
-    if(zbits >= 10 && d.N % SSD_FS_STEP_PX == 0 && c.width <= 0xfffe && c.height <= 0xfffe)
-    {
-      int sh = 0;
-      while(sh < 24 && 0.5 * std::ldexp(c.height_interval, sh + 1) + 1.0 < std::ldexp(1.0, zbits - 1) - 1.0)
-        sh++;
-      d.rec_zbits = zbits;
-      d.rec_zshift = sh;
-      d.rec_mf = (float)std::ldexp(1.0 / d.hir, sh);
-    }
-    d.gs_xw = (float)d.x_to_world;
-    d.gs_x0 = (float)c.x_min;
-    d.gs_yw = (float)d.y_to_world;
-    d.gs_y0 = (float)c.y_max;
-    d.gs_margin = (float)(16.0 / 16777216.0 * (std::fabs(c.x_min) + std::fabs(c.x_max) + std::fabs(c.y_min) + std::fabs(c.y_max) + 1.0) + 1e-7);
-  }
   if(d.n_bins < 3 || d.n_bins > SSD_GPU_MAX_BINS)
     return SSD_E_RANGE;
   if(d.N % 16 != 0)
@@ -512,7 +465,7 @@ __global__ void k_single_camera_to_world(const __grid_constant__ DevParams p, co
 
 // The classic chain: k_transform_bin -> k_peaks -> k_label_bev -> k_outline -> k_frame_logic -> k_quad_reduce -> k_finalize
 // (+ k_riser_reduce). CAM = NoCam: every frame with the context's own camera; CamTable: each frame with its camera's parameters
-// (camera calls; the word-record variant is never taken there).
+// (camera calls).
 // sl: the chunk's z16 frames through ray tables (a call with a distorted lens), else nullptr. ov_lens: the lenses the overlay
 // projects through (LensCam), else nullptr.
 template<class CAM>
@@ -531,7 +484,8 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   unsigned char *labels = ctx->d_labels + (size_t)frame0 * p.N;
   unsigned *bev = ctx->d_bev + (size_t)s * ctx->chunk_frames * SSD_GPU_MAX_PLATEAUS * ctx->bm_words;
   const dim3 gpt(p.tiles_per_frame, nf);
-  const int tiles2 = (p.N + SSD_WT_PX * SSD_PT_WARPS - 1) / (SSD_WT_PX * SSD_PT_WARPS);
+  // k_label_bev / k_quad_reduce: each block loops over tiles of its frame; enough blocks for ~6 waves of the GPU
+  const int tiles2 = (p.N + SSD_WT_PX * SSD_PT_WARPS - 1) / (SSD_WT_PX * SSD_PT_WARPS); // at least one warp-tile per warp
   const int bpf = std::max(1, std::min(tiles2, (ctx->pt_blocks_target + nf - 1) / nf));
   const int bpf_l = ctx->bpf_l_knob > 0 ? std::min(tiles2, ctx->bpf_l_knob) : bpf, bpf_q = ctx->bpf_q_knob > 0 ? std::min(tiles2, ctx->bpf_q_knob) : bpf;
   const dim3 gpt2l(bpf_l, nf), gpt2q(bpf_q, nf);
@@ -564,27 +518,12 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   if(!fused)
     k_peaks<<<nf, 32, 0, st>>>(p, frames, nf);
   STAGE_EV(2);
-  constexpr bool plain = std::is_same<CAM, NoCam>::value;
-  uint2 *wrec = plain && ctx->wordrec ? ctx->d_wrec + (size_t)s * ctx->chunk_frames * (size_t)(p.N / 4) : nullptr;
-  if constexpr(plain)
-  {
-    if(wrec)
-    {
-      if(depth)
-        k_label_bev<SrcDepth, true><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, wrec);
-      else
-        k_label_bev<SrcVertices, true><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, wrec);
-    }
-  }
-  if(!wrec)
-  {
-    if(sl)
-      k_label_bev<SrcLens, false, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, nullptr, cam);
-    else if(depth)
-      k_label_bev<SrcDepth, false, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, nullptr, cam);
-    else
-      k_label_bev<SrcVertices, false, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, nullptr, cam);
-  }
+  if(sl)
+    k_label_bev<SrcLens, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, cam);
+  else if(depth)
+    k_label_bev<SrcDepth, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, cam);
+  else
+    k_label_bev<SrcVertices, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, cam);
   STAGE_EV(3);
   if(fused)
   {
@@ -604,25 +543,12 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   if(!fused)
     k_frame_logic<CAM><<<nf, 32, 0, st>>>(p, frames, nf, cam);
   STAGE_EV(5);
-  if constexpr(plain)
-  {
-    if(wrec)
-    {
-      if(depth)
-        k_quad_reduce_rec<SrcDepth><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, wrec);
-      else
-        k_quad_reduce_rec<SrcVertices><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, wrec);
-    }
-  }
-  if(!wrec)
-  {
-    if(sl)
-      k_quad_reduce<SrcLens, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, cam);
-    else if(depth)
-      k_quad_reduce<SrcDepth, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, cam);
-    else
-      k_quad_reduce<SrcVertices, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, cam);
-  }
+  if(sl)
+    k_quad_reduce<SrcLens, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, cam);
+  else if(depth)
+    k_quad_reduce<SrcDepth, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, cam);
+  else
+    k_quad_reduce<SrcVertices, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, cam);
   STAGE_EV(6);
   if(ov_lens)
   {
@@ -663,29 +589,12 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
 // the launch chain for one chunk of frames on one stream
 // ---------------------------------------------------------------------------------------------
 // xyz_dev: packed vertices of the chunk, or nullptr with z16_dev: the chunk's depth frames, deprojected inside the
-// three point kernels (SrcDepth). cam: the camera table of a camera call (classic chain only), else nullptr.
+// three point kernels (SrcDepth). cam: the camera table of a camera call, else nullptr.
 // sl: the call's lens source (its z16 member is set here), else nullptr; ov_lens: see launch_classic.
 static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uint16_t *z16_dev, float depth_unit, int frame0, int nf, int *launches,
                         cudaEvent_t *ev, const CamTable *cam, const SrcLens *sl, const ssd_gpu_distortion *ov_lens)
 {
-#define STAGE_EV(i)                         \
-  do                                        \
-  {                                         \
-    if(ev)                                  \
-      CK(cudaEventRecord(ev[i], st));       \
-  } while(0)
   const DevParams &p = ctx->dp;
-  cudaStream_t st = ctx->stream[s];
-  FrameDev *frames = ctx->d_frames + frame0;
-  unsigned char *labels = ctx->d_labels + (size_t)frame0 * p.N;
-  unsigned *bev = ctx->d_bev + (size_t)s * ctx->chunk_frames * SSD_GPU_MAX_PLATEAUS * ctx->bm_words;
-  const dim3 gpt(p.tiles_per_frame, nf);
-  // k_label_bev / k_quad_reduce: each block loops over tiles of its frame; enough blocks for ~6 waves of the GPU
-  const int tiles2 = (p.N + SSD_WT_PX * SSD_PT_WARPS - 1) / (SSD_WT_PX * SSD_PT_WARPS); // at least one warp-tile per warp
-  const int bpf = std::max(1, std::min(tiles2, (ctx->pt_blocks_target + nf - 1) / nf));
-  const int bpf_l = ctx->bpf_l_knob > 0 ? std::min(tiles2, ctx->bpf_l_knob) : bpf, bpf_q = ctx->bpf_q_knob > 0 ? std::min(tiles2, ctx->bpf_q_knob) : bpf;
-  const dim3 gpt2l(bpf_l, nf), gpt2q(bpf_q, nf);
-  const bool depth = xyz_dev == nullptr;
   SrcVertices sv;
   sv.xyz = xyz_dev;
   SrcDepth sd;
@@ -694,18 +603,6 @@ static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uin
   sd.yn = ctx->d_yn;
   sd.unit = depth_unit;
   sd.wmagic = (((unsigned long long)1 << 40) + (unsigned long long)p.W - 1) / (unsigned long long)p.W;
-  // optional fourth pass: vertical faces from the remainder (labels are final once the chain's label kernel has run)
-  auto launch_risers = [&]()
-  {
-    if(!ctx->risers)
-      return;
-    if(depth)
-      k_riser_reduce<SrcDepth><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames);
-    else
-      k_riser_reduce<SrcVertices><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames);
-    *launches += 1;
-  };
-
   SrcLens sll;
   if(sl)
   {
@@ -718,116 +615,7 @@ static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uin
     c.frame0 = frame0;
     return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, launches, ev, c, ov_lens);
   }
-  if(ctx->records)
-  {
-    // ---- record chain: k_transform_rec -> k_peaks -> k_label_sum -> k_outline -> k_frame_logic -> k_quad_sum -> k_finalize ----
-    uint4 *recs = ctx->d_rec4 + (size_t)s * ctx->chunk_frames * (size_t)(p.N / 4);
-    STAGE_EV(0);
-    if(depth)
-      k_transform_rec_depth<SSD_PT_ITERS><<<gpt, SSD_PT_THREADS, 0, st>>>(p, sd, labels, recs, frames);
-    else
-      k_transform_rec<SSD_PT_ITERS><<<gpt, SSD_PT_THREADS, SSD_PT_ITERS * SSD_TB_STAGE_BYTES, st>>>(p, xyz_dev, labels, recs, frames);
-    STAGE_EV(1);
-    k_peaks<<<nf, 32, 0, st>>>(p, frames, nf);
-    STAGE_EV(2);
-    if(depth)
-      k_label_rec<SrcDepth><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sd, labels, recs, frames, bev, ctx->bm_words);
-    else
-      k_label_rec<SrcVertices><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sv, labels, recs, frames, bev, ctx->bm_words);
-    STAGE_EV(3);
-    if(ctx->outline_small)
-      k_outline<OutlineSharedSmall><<<dim3(ctx->outline_gridx, nf), SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
-    else
-      k_outline<OutlineShared><<<dim3(ctx->outline_gridx, nf), OutlineShared::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
-    STAGE_EV(4);
-    k_frame_logic<<<nf, 32, 0, st>>>(p, frames, nf);
-    STAGE_EV(5);
-    if(depth)
-      k_quad_rec<SrcDepth><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, recs);
-    else
-      k_quad_rec<SrcVertices><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, recs);
-    STAGE_EV(6);
-    if(ctx->outline_small)
-      k_finalize<OutlineSharedSmall><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words, ctx->smem_cap_words, ctx->ov,
-                                                                            ctx->d_ovl ? ctx->d_ovl + (size_t)frame0 * SSD_GPU_MAX_STEPS : nullptr);
-    else
-      k_finalize<OutlineShared><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words, ctx->smem_cap_words, ctx->ov,
-                                                                            ctx->d_ovl ? ctx->d_ovl + (size_t)frame0 * SSD_GPU_MAX_STEPS : nullptr);
-    STAGE_EV(7);
-    *launches += SSD_GPU_N_STAGES;
-    launch_risers();
-    CK(cudaGetLastError());
-    return SSD_OK;
-  }
-  if(ctx->resident)
-  {
-    // ---- resident-frame chain: k_frame_stream -> k_outline -> k_frame_logic -> k_quad_sum -> k_finalize ----
-    FsParams a;
-    a.n_frames = nf;
-    a.d_raw = ctx->fs_d_raw;
-    a.d_rec = ctx->fs_d_rec;
-    a.flags = 0;
-    a.done = ctx->d_done + (size_t)s * ctx->chunk_frames;
-    a.sums = ctx->d_sums + (size_t)s * ctx->chunk_frames * (size_t)(p.N / 32);
-    a.recs = ctx->d_recs;
-    a.prof = ctx->d_prof;
-    a.prof_warp_off = FS_PROF_HDR + (size_t)FS_PROF_PER_FRAME * ctx->chunk_frames;
-    if(ctx->d_prof)
-    {
-      std::vector<unsigned long long> init(FS_PROF_HDR + (size_t)FS_PROF_PER_FRAME * ctx->chunk_frames + (size_t)8 * ctx->fs_grid * SSD_FS_WARPS, 0ull);
-      for(int f = 0; f < ctx->chunk_frames; f++)
-        init[FS_PROF_HDR + (size_t)f * FS_PROF_PER_FRAME + 0] = init[FS_PROF_HDR + (size_t)f * FS_PROF_PER_FRAME + 3] = ~0ull;
-      CK(cudaStreamSynchronize(st));
-      CK(cudaMemcpy(ctx->d_prof, init.data(), init.size() * 8, cudaMemcpyHostToDevice));
-    }
-    size_t bmw = ctx->bm_words;
-    DevParams pp = p;
-    if(ctx->fs_pending)
-      CK(cudaStreamWaitEvent(st, ctx->ev_fs, 0));
-    STAGE_EV(0);
-    if(depth)
-    {
-      void *args[] = { &pp, &sd, &a, &labels, &frames, &bev, &bmw };
-      CK(cudaLaunchCooperativeKernel((const void *)k_frame_stream<SrcDepth>, dim3(ctx->fs_grid), dim3(SSD_FS_THREADS), args,
-                                     fs_smem_bytes(FsSrc<SrcDepth>::STEP_BYTES, a.d_raw, a.d_rec), st));
-    }
-    else
-    {
-      void *args[] = { &pp, &sv, &a, &labels, &frames, &bev, &bmw };
-      CK(cudaLaunchCooperativeKernel((const void *)k_frame_stream<SrcVertices>, dim3(ctx->fs_grid), dim3(SSD_FS_THREADS), args,
-                                     fs_smem_bytes(FsSrc<SrcVertices>::STEP_BYTES, a.d_raw, a.d_rec), st));
-    }
-    CK(cudaEventRecord(ctx->ev_fs, st));
-    ctx->fs_pending = true;
-    STAGE_EV(1);
-    STAGE_EV(2);
-    STAGE_EV(3);
-    if(ctx->outline_small)
-      k_outline<OutlineSharedSmall><<<dim3(ctx->outline_gridx, nf), SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
-    else
-      k_outline<OutlineShared><<<dim3(ctx->outline_gridx, nf), OutlineShared::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
-    STAGE_EV(4);
-    k_frame_logic<<<nf, 32, 0, st>>>(p, frames, nf);
-    STAGE_EV(5);
-    if(depth)
-      k_quad_sum<SrcDepth><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, a.sums, nullptr);
-    else
-      k_quad_sum<SrcVertices><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, a.sums, nullptr);
-    STAGE_EV(6);
-    if(ctx->outline_small)
-      k_finalize<OutlineSharedSmall><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words, ctx->smem_cap_words, ctx->ov,
-                                                                            ctx->d_ovl ? ctx->d_ovl + (size_t)frame0 * SSD_GPU_MAX_STEPS : nullptr);
-    else
-      k_finalize<OutlineShared><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words, ctx->smem_cap_words, ctx->ov,
-                                                                            ctx->d_ovl ? ctx->d_ovl + (size_t)frame0 * SSD_GPU_MAX_STEPS : nullptr);
-    STAGE_EV(7);
-    *launches += 5;
-    launch_risers();
-    CK(cudaGetLastError());
-    return SSD_OK;
-  }
   return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, launches, ev, NoCam(), ov_lens);
-#undef STAGE_EV
 }
 
 extern "C"
@@ -859,14 +647,6 @@ void ssd_gpu_destroy(ssd_gpu_ctx *ctx)
   cudaFreeHost(ctx->h_ovl);
   cudaFree(ctx->d_labels);
   cudaFree(ctx->d_bev);
-  cudaFree(ctx->d_sums);
-  cudaFree(ctx->d_done);
-  cudaFree(ctx->d_recs);
-  cudaFree(ctx->d_rec4);
-  cudaFree(ctx->d_wrec);
-  cudaFree(ctx->d_prof);
-  if(ctx->ev_fs)
-    cudaEventDestroy(ctx->ev_fs);
   cudaFree(ctx->d_img);
   cudaFree(ctx->d_xn);
   cudaFree(ctx->d_yn);
@@ -1039,8 +819,6 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
     ctx->bpf_q_knob = std::max(0, atoi(e));
   if(const char *e = getenv("SSD_GPU_NO_SPLIT_SMALL"))
     ctx->no_split_small = atoi(e) != 0;
-  if(const char *e = getenv("SSD_GPU_DEPTH_UNFUSED"))
-    ctx->depth_unfused = atoi(e) != 0;
   for(int i = 0; i < ctx->n_streams; i++)
   {
     CKC(cudaStreamCreateWithFlags(&ctx->stream[i], cudaStreamNonBlocking));
@@ -1060,75 +838,6 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
   const size_t bev_bytes = (size_t)ctx->n_streams * ctx->chunk_frames * SSD_GPU_MAX_PLATEAUS * ctx->bm_words * 4;
   CKC(cudaMalloc(&ctx->d_bev, bev_bytes));
   CKC(cudaMemset(ctx->d_bev, 0, bev_bytes)); // bitmaps are self-cleaning afterwards
-  {
-    // Resident-frame path: used when a frame's records fit the shared memory of the GPU with room for the frame barrier's
-    // latency (every warp must hold all its steps of one frame, plus what it works ahead). SSD_GPU_PATH=classic|resident.
-    const char *pe = getenv("SSD_GPU_PATH");
-    const bool want = pe && !strcmp(pe, "resident"); // experimental: measured slower than the record chain (DESIGN.md)
-    // word-record chain (experimental: measured slower than the classic chain, DESIGN.md): box coordinates are 12 bits each
-    if(pe && !strcmp(pe, "wordrec") && dp.W <= 4096 && dp.H <= 4096)
-    {
-      ctx->wordrec = true;
-      CKC(cudaMalloc(&ctx->d_wrec, (size_t)ctx->n_streams * ctx->chunk_frames * (size_t)(dp.N / 4) * sizeof(uint2)));
-    }
-    if(pe && !strcmp(pe, "wordrec") && !ctx->wordrec)
-      return bail("SSD_GPU_PATH=wordrec: the frame size does not admit the word-record chain", SSD_E_RANGE);
-    if(pe && !strcmp(pe, "records") && dp.rec_zbits > 0) // experimental: measured slower than the classic chain (DESIGN.md)
-    {
-      ctx->records = true;
-      CKC(cudaMalloc(&ctx->d_rec4, (size_t)ctx->n_streams * ctx->chunk_frames * (size_t)(dp.N / 4) * sizeof(uint4)));
-      if(cudaFuncSetAttribute(k_transform_rec<SSD_PT_ITERS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SSD_PT_ITERS * SSD_TB_STAGE_BYTES) != cudaSuccess)
-        return bail("cudaFuncSetAttribute(k_transform_rec) failed", SSD_E_CUDA);
-    }
-    if(pe && !strcmp(pe, "records") && !ctx->records)
-      return bail("SSD_GPU_PATH=records: the frame size does not admit the record chain", SSD_E_RANGE);
-    int sms = 148, coop = 0;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-    cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device);
-    if(const char *e = getenv("SSD_GPU_FS_RAW"))
-      ctx->fs_d_raw = std::max(2, atoi(e));
-    if(const char *e = getenv("SSD_GPU_FS_REC"))
-      ctx->fs_d_rec = std::max(2, atoi(e));
-    int grid = sms;
-    if(const char *e = getenv("SSD_GPU_FS_CTAS"))
-      grid = std::max(1, std::min(sms, atoi(e)));
-    if(want && coop && dp.rec_zbits > 0 && dp.gs_steps % SSD_FS_SUB == 0 && dp.gs_steps / SSD_FS_SUB >= 64)
-    {
-      // record ring: fs_lag_frames frames of a warp's steps (phase 2 may trail phase 1 by that much: the frame barrier's
-      // latency and the skew between the CTAs disappear in it); ~3.9 MB per frame at 1024x768, re-used before L2 evicts it
-      if(const char *e = getenv("SSD_GPU_FS_LAG"))
-        ctx->fs_lag_frames = std::max(1, std::min(SSD_FS_NB - 3, atoi(e)));
-      const long long S = dp.gs_steps / SSD_FS_SUB, TW = (long long)grid * SSD_FS_WARPS;
-      const int per_warp = (int)((S + TW - 1) / TW);
-      if(!ctx->fs_d_rec)
-        ctx->fs_d_rec = (int)((ctx->fs_lag_frames * S + TW - 1) / TW) + 2;
-      ctx->fs_d_rec = std::max(ctx->fs_d_rec, per_warp + 2);
-      const size_t sm_v = fs_smem_bytes(FsSrc<SrcVertices>::STEP_BYTES, ctx->fs_d_raw, ctx->fs_d_rec);
-      const size_t sm_d = fs_smem_bytes(FsSrc<SrcDepth>::STEP_BYTES, ctx->fs_d_raw, ctx->fs_d_rec);
-      int occ = 0;
-      if(sm_v <= (size_t)max_optin &&
-         cudaFuncSetAttribute(k_frame_stream<SrcVertices>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_v) == cudaSuccess &&
-         cudaFuncSetAttribute(k_frame_stream<SrcDepth>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm_d) == cudaSuccess &&
-         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_frame_stream<SrcVertices>, SSD_FS_THREADS, sm_v) == cudaSuccess && occ >= 1)
-      {
-        ctx->resident = true;
-        ctx->fs_grid = grid;
-        const size_t n_sums = (size_t)ctx->n_streams * ctx->chunk_frames * (size_t)(dp.N / 32);
-        CKC(cudaMalloc(&ctx->d_sums, n_sums * sizeof(GroupSum)));
-        CKC(cudaMalloc(&ctx->d_done, (size_t)ctx->n_streams * ctx->chunk_frames * sizeof(unsigned)));
-        CKC(cudaMalloc(&ctx->d_recs, (size_t)grid * SSD_FS_WARPS * ctx->fs_d_rec * SSD_FS_REC_BYTES * SSD_FS_SUB));
-        CKC(cudaMemset(ctx->d_done, 0, (size_t)ctx->n_streams * ctx->chunk_frames * sizeof(unsigned)));
-        CKC(cudaEventCreateWithFlags(&ctx->ev_fs, cudaEventDisableTiming));
-        if(getenv("SSD_GPU_FS_PROF"))
-        {
-          CKC(cudaMalloc(&ctx->d_prof, 8 * (FS_PROF_HDR + (size_t)FS_PROF_PER_FRAME * ctx->chunk_frames + (size_t)8 * grid * SSD_FS_WARPS)));
-        }
-      }
-      cudaGetLastError();
-    }
-    if(pe && !strcmp(pe, "resident") && !ctx->resident)
-      return bail("SSD_GPU_PATH=resident: the frame size does not admit the resident-frame path", SSD_E_RANGE);
-  }
   CKC(cudaMemset(ctx->d_frames, 0, sizeof(FrameDev) * (size_t)max_frames));
   CKC(cudaMemset(ctx->d_out, 0, sizeof(FrameOut) * (size_t)max_frames));
   memset(ctx->h_out, 0, sizeof(FrameOut) * (size_t)max_frames);
@@ -1272,27 +981,13 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
     sl.unit = intr->depth_unit;
   }
   // depth frames are deprojected inside the point kernels (SrcDepth): no vertex array is ever written.
-  const bool unfused = ctx->depth_unfused; // A/B switch (SSD_GPU_DEPTH_UNFUSED, read in ssd_gpu_create)
-  if(host_input || depth_input)
+  if(host_input)
     for(int i = 0; i < ctx->n_streams; i++)
     {
-      if(depth_input && !unfused)
-      {
-        if(host_input && !ctx->d_depth[i])
-          CK(cudaMalloc(&ctx->d_depth[i], (size_t)ctx->host_chunk_frames * p.N * sizeof(uint16_t)));
-        continue;
-      }
-      if(ctx->stage_frames[i] < cf) // grows once when a device-depth call follows host-input calls
-      {
-        CK(cudaDeviceSynchronize());
-        if(ctx->d_stage[i])
-          CK(cudaFree(ctx->d_stage[i]));
-        ctx->d_stage[i] = nullptr;
-        CK(cudaMalloc(&ctx->d_stage[i], (size_t)cf * frame_floats * sizeof(float)));
-        ctx->stage_frames[i] = cf;
-      }
-      if(depth_input && host_input && !ctx->d_depth[i])
+      if(depth_input && !ctx->d_depth[i])
         CK(cudaMalloc(&ctx->d_depth[i], (size_t)ctx->host_chunk_frames * p.N * sizeof(uint16_t)));
+      if(!depth_input && !ctx->d_stage[i])
+        CK(cudaMalloc(&ctx->d_stage[i], (size_t)ctx->host_chunk_frames * frame_floats * sizeof(float)));
     }
 
   int launches = 0;
@@ -1370,26 +1065,12 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
       CK(cudaEventRecord(ctx->ev_in_ready[s], ctx->copy_stream));
       CK(cudaStreamWaitEvent(ctx->stream[s], ctx->ev_in_ready[s], 0));
     }
-    if(depth_input && unfused)
-    {
-      // A/B path (SSD_GPU_DEPTH_UNFUSED=1): materialise the vertices, then the vertex kernels
-      // (the vertex staging of stream s is free: the chunk that used it last ran on this very stream)
-      if(use_lens)
-        k_deproject_lens<<<dim3((p.N / 4 + 255) / 256, nf), 256, 0, ctx->stream[s]>>>(p.N, intr->depth_unit, ctx->d_ray, dsrc, ctx->d_stage[s]);
-      else
-        k_deproject<<<dim3((p.N / 4 + 255) / 256, nf), 256, 0, ctx->stream[s]>>>(p.W, p.N, intr->depth_unit, ctx->d_xn, ctx->d_yn, dsrc, ctx->d_stage[s]);
-      launches++;
-      src = ctx->d_stage[s];
-      if(host_input)
-        CK(cudaEventRecord(ctx->ev_in_free[s], ctx->stream[s])); // the z16 staging is consumed
-    }
-    const bool fused = depth_input && !unfused;
-    const int rc = launch_chunk(ctx, s, fused ? nullptr : src, fused ? dsrc : nullptr, fused && intr ? intr->depth_unit : 0.f, f0, nf, &launches,
+    const int rc = launch_chunk(ctx, s, src, dsrc, depth_input && intr ? intr->depth_unit : 0.f, f0, nf, &launches,
                                 stage_timing ? &ctx->stage_ev[(size_t)chunk * (SSD_GPU_N_STAGES + 1)] : nullptr, cam_of_frame ? &cams : nullptr,
-                                fused && use_lens ? &sl : nullptr, ov_lens);
+                                use_lens ? &sl : nullptr, ov_lens);
     if(rc)
       return rc;
-    if(host_input && (!depth_input || fused))
+    if(host_input)
       CK(cudaEventRecord(ctx->ev_in_free[s], ctx->stream[s])); // all three passes have read the staging
   }
   if(host_input)
@@ -1406,73 +1087,6 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
   CK(cudaEventRecord(ctx->ev_stop, ctx->stream[0]));
   CK(cudaEventSynchronize(ctx->ev_stop));
   CK(cudaGetLastError());
-  if(ctx->d_prof)
-  {
-    // (profiling runs use one chunk per call: the buffer is reset before every launch)
-    const int nf = std::min(n_frames, ctx->chunk_frames);
-    const size_t woff = FS_PROF_HDR + (size_t)FS_PROF_PER_FRAME * ctx->chunk_frames;
-    std::vector<unsigned long long> h(woff + (size_t)8 * ctx->fs_grid * SSD_FS_WARPS);
-    CK(cudaMemcpy(h.data(), ctx->d_prof, h.size() * 8, cudaMemcpyDeviceToHost));
-    const double w = h[5] ? (double)h[5] : 1.0;
-    fprintf(stderr, "[fs prof] warps %llu  per warp: total %.0f cyc, phase1 %.0f, phase2 %.0f, TMA wait %.0f, idle loops %.1f (input done %.1f, ring full %.1f, other %.1f; mean lag %.2f frames), polls %.1f\n",
-            h[5], h[2] / w, h[0] / w, h[1] / w, h[6] / w, h[3] / w, h[7] / w, h[8] / w, h[9] / w, h[3] ? (double)h[10] / (double)h[3] : 0.0, h[4] / w);
-    fprintf(stderr, "[fs prof] per warp: busy iterations %.0f cyc, idle iterations %.0f cyc; section TMA issue %.0f, sections prefetch+poll issue %.0f\n", h[11] / w, h[12] / w, h[13] / w, h[14] / w);
-    double skew = 0, own = 0, peaks = 0, detect = 0, p2span = 0, period = 0;
-    int cnt = 0;
-    for(int f = 16; f + 16 < nf; f++)
-    {
-      const unsigned long long *q = &h[FS_PROF_HDR + (size_t)f * FS_PROF_PER_FRAME];
-      skew += (double)(q[5] - q[0]);
-      own += (double)q[1] - (double)q[5];
-      peaks += (double)(q[2] - q[1]);
-      detect += (double)q[3] - (double)q[2];
-      p2span += (double)(q[4] - q[3]);
-      period += (double)(q[5 + FS_PROF_PER_FRAME] - q[5]);
-      cnt++;
-    }
-    if(n_frames >= 64)
-    {
-      // per CTA: sums over its warps
-      double best_idle = 1e30, worst_idle = -1;
-      int bi = -1, wi = -1;
-      std::vector<double> ci(ctx->fs_grid, 0.0);
-      for(int c = 0; c < ctx->fs_grid; c++)
-      {
-        for(int q = 0; q < SSD_FS_WARPS; q++)
-          ci[c] += (double)h[woff + ((size_t)c * SSD_FS_WARPS + q) * 8 + 3];
-        if(ci[c] < best_idle)
-          best_idle = ci[c], bi = c;
-        if(ci[c] > worst_idle)
-          worst_idle = ci[c], wi = c;
-      }
-      for(int c : { bi, wi })
-      {
-        double s8[8] = { 0 };
-        for(int q = 0; q < SSD_FS_WARPS; q++)
-          for(int i = 0; i < 8; i++)
-            s8[i] += (double)h[woff + ((size_t)c * SSD_FS_WARPS + q) * 8 + i] / SSD_FS_WARPS;
-        fprintf(stderr, "[fs prof] CTA %d (%s idle): per warp p1 %.0f p2 %.0f tma %.0f idle loops %.0f (ring %.0f) total %.0f leave %.0f peaks %.0f\n", c,
-                c == bi ? "least" : "most", s8[0], s8[1], s8[2], s8[3], s8[5], s8[4], s8[6], s8[7]);
-      }
-      {
-        double mn = 1e30, mx = 0, sm = 0;
-        const int nw = ctx->fs_grid * SSD_FS_WARPS;
-        for(int q = 0; q < nw; q++)
-        {
-          const double v = (double)h[woff + (size_t)q * 8 + 0] + (double)h[woff + (size_t)q * 8 + 1];
-          mn = std::min(mn, v), mx = std::max(mx, v), sm += v;
-        }
-        fprintf(stderr, "[fs prof] phase1+phase2 cycles per warp: min %.0f mean %.0f max %.0f\n", mn, sm / nw, mx);
-      }
-      int n_low = 0;
-      for(int c = 0; c < ctx->fs_grid; c++)
-        n_low += ci[c] < 0.25 * worst_idle;
-      fprintf(stderr, "[fs prof] CTAs with less than a quarter of the worst CTA's idle loops: %d of %d\n", n_low, ctx->fs_grid);
-    }
-    if(cnt)
-      fprintf(stderr, "[fs prof] per frame (ns): first -> last CTA delivered %.0f, -> owner saw it complete %.0f, -> LUT published %.0f, -> first phase-2 step %.0f, phase-2 span %.0f, period %.0f\n",
-              skew / cnt, own / cnt, peaks / cnt, detect / cnt, p2span / cnt, period / cnt);
-  }
   float ms = 0;
   CK(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
   ctx->timing.total_ms = ms;
@@ -1512,10 +1126,6 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
 static int process_common(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16, const ssd_gpu_intrinsics *intr, bool host_input, int n_frames,
                           int flags, const int32_t *cam_of_frame = nullptr)
 {
-  // refused before anything is launched: the results of the previous call stay readable
-  if(ctx && !cam_of_frame && !ssd_lens_is_pinhole(&ctx->lens) && (ctx->records || ctx->wordrec || ctx->resident) && (!xyz || ctx->ov.enabled))
-    return fail(ctx, SSD_E_STATE, "lens distortion runs on the default (classic) chain only; this context was created with "
-                                  "SSD_GPU_PATH=records|wordrec|resident");
   const int rc = process_impl(ctx, xyz, z16, intr, host_input, n_frames, flags, cam_of_frame);
   if(rc != SSD_OK && rc != SSD_E_INVALID_ARG && rc != SSD_E_RANGE && ctx)
   {
@@ -1524,7 +1134,6 @@ static int process_common(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z1
     cudaGetLastError();
     if(ctx->d_bev)
       cudaMemset(ctx->d_bev, 0, (size_t)ctx->n_streams * ctx->chunk_frames * SSD_GPU_MAX_PLATEAUS * ctx->bm_words * 4);
-    ctx->fs_pending = false;
     ctx->n_frames_last = 0;
     ctx->err = keep;
   }
@@ -1782,11 +1391,6 @@ static int check_cameras(ssd_gpu_ctx *ctx, const void *input, const int32_t *cam
 {
   if(!ctx || !input || !cam_of_frame || n_frames <= 0)
     return fail(ctx, SSD_E_INVALID_ARG, "camera call: bad argument");
-  if(ctx->records || ctx->wordrec || ctx->resident)
-    return fail(ctx, SSD_E_STATE, "camera call: camera tables run on the default (classic) chain only; this context was created with "
-                                  "SSD_GPU_PATH=records|wordrec|resident");
-  if(depth && ctx->depth_unfused)
-    return fail(ctx, SSD_E_STATE, "depth camera call: not available with SSD_GPU_DEPTH_UNFUSED=1 (the fused depth path only)");
   if(ctx->n_cameras <= 0)
     return fail(ctx, SSD_E_STATE, "camera call: no camera table (ssd_gpu_set_cameras)");
   if(n_frames > ctx->max_frames)

@@ -1424,13 +1424,10 @@ __global__ void __launch_bounds__(SSD_OL_THREADS, SSD_OL_MINB) k_finalize(const 
       PlateauDev &P = F.plat[i];
       if(P.valid && P.quad_status == 0)
       {
-        // calcAverageZ (:574-581). Points tested one by one: z_fix_u sums; points taken in as whole summaries (k_quad_sum):
-        // z = z_min + (code + 0.5 + d / rec_mf) / hir, summed as integers. Both sums are order independent.
-        const double n_pp = (double)(P.n_in_quad - P.n_sum);
-        double zs = ((double)P.sum_fix - n_pp * (double)SSD_ZFIX_BIAS) / (double)(1u << p.zshift);
-        if(P.n_sum)
-          zs += (double)P.n_sum * (p.z_min + 0.5 / p.hir) + (double)P.sum_c / p.hir + (double)P.sum_d / (double)(1u << p.rec_zshift);
-        P.mean_z = zs / (double)P.n_in_quad;
+        // calcAverageZ (:574-581) from the z_fix_u sum, which is order independent
+        const double n_pp = (double)P.n_in_quad;
+        const double zs = ((double)P.sum_fix - n_pp * (double)SSD_ZFIX_BIAS) / (double)(1u << p.zshift);
+        P.mean_z = zs / n_pp;
       }
     }
     if(groundStep)

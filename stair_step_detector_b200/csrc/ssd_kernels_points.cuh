@@ -335,7 +335,6 @@ __device__ __forceinline__ unsigned peaks_bit_at(const unsigned (&w)[8], int r, 
 }
 
 // K: scratch in shared memory, private to the calling warp for the duration of the call. h0, h1: bins 8 lane .. 8 lane + 7.
-// lut_flags: OR-ed into every lut16 entry (SSD_LUT_VALID for the resident-frame path's polling).
 __device__ inline void peaks_warp(const DevParams &p, FrameDev &F, PeaksScratch &K, const uint4 h0, const uint4 h1, int lane)
 {
   {
@@ -477,9 +476,6 @@ __device__ inline void peaks_warp(const DevParams &p, FrameDev &F, PeaksScratch 
     P.quad_status = -1;
     P.mean_z = 0;
     P.sum_fix = 0;
-    P.sum_d = 0;
-    P.sum_c = 0;
-    P.n_sum = 0;
     P.row_min = 0x7fffffff;
     P.row_max = -1;
     P.front_valid = 0;
@@ -905,21 +901,10 @@ __device__ __forceinline__ void label_bev_exact_point(const DevParams &p, float 
 #ifndef SSD_LB_MINB
 #define SSD_LB_MINB 4
 #endif
-// REC: every 4-pixel word with points of outlined plateaus also leaves an 8-byte word record for k_quad_reduce_rec (word_rec_*):
-// the box of its BEV pixels and the fixed-point z sum of those points, so that pass 3 takes a word that lies inside its step's
-// quadrilateral without reading its vertices again.
-#define SSD_WREC_ELIGIBLE 0x40000000u // one label, every pixel certain, box at most 8 x 8 pixels
-__device__ __forceinline__ uint2 word_rec_pack(bool eligible, int xlo, int ylo, int xhi, int yhi, unsigned zsum, unsigned count)
-{
-  const unsigned lo = eligible ? ((unsigned)xlo | ((unsigned)ylo << 12) | ((unsigned)(xhi - xlo) << 24) | ((unsigned)(yhi - ylo) << 27) | SSD_WREC_ELIGIBLE) : 0u;
-  return make_uint2(lo, zsum | (count << 25));
-}
-
-template<class SRC, bool REC = false, class CAM = NoCam>
+template<class SRC, class CAM = NoCam>
 __global__ void __launch_bounds__(SSD_PT_THREADS, SSD_LB_MINB) k_label_bev(const __grid_constant__ DevParams p0, const SRC src0,
                                                                unsigned char *__restrict__ labels, FrameDev *__restrict__ frames,
-                                                               unsigned *__restrict__ bev, size_t bm_words, uint2 *__restrict__ wrec = nullptr,
-                                                               const CAM cam = CAM())
+                                                               unsigned *__restrict__ bev, size_t bm_words, const CAM cam = CAM())
 {
   __shared__ LabelBevShared S;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1029,7 +1014,7 @@ __global__ void __launch_bounds__(SSD_PT_THREADS, SSD_LB_MINB) k_label_bev(const
       const unsigned l0 = (lab >> (8 * (__ffs(m4 | 16u) - 1) & 31)) & 0xffu;
       const unsigned bytes = ((m4 * 0x00204081u) & 0x01010101u) * 0xffu;
       const bool uniform = ((lab ^ (l0 * 0x01010101u)) & bytes) == 0u;
-      int ylo = 0x7fffffff, yhi = -1, xlo = 0x7fffffff, xhi = -1;
+      int ylo = 0x7fffffff, yhi = -1;
       if(uniform)
       {
         // word index of the plateau's bitmap within the stream's BEV buffer: 32-bit (the buffer holds < 2^32 words, see
@@ -1043,11 +1028,6 @@ __global__ void __launch_bounds__(SSD_PT_THREADS, SSD_LB_MINB) k_label_bev(const
             atomicOr(bev + (lidx + (unsigned)iy[j] * wpr + ((unsigned)ix[j] >> 5)), 1u << (ix[j] & 31));
             ylo = min(ylo, iy[j]);
             yhi = max(yhi, iy[j]);
-            if(REC)
-            {
-              xlo = min(xlo, ix[j]);
-              xhi = max(xhi, ix[j]);
-            }
           }
         if(yhi >= 0)
         {
@@ -1085,15 +1065,6 @@ __global__ void __launch_bounds__(SSD_PT_THREADS, SSD_LB_MINB) k_label_bev(const
         for(int j = 0; j < 4; j++)
           if((bad >> j) & 1u)
             defer_push(S.L, warp, ((e >> 4) << 2) | (unsigned)j);
-      }
-      if(REC && e)
-      {
-        unsigned zs = 0;
-#pragma unroll
-        for(int j = 0; j < 4; j++)
-          zs += z_fix_u(p, vx[j], vy[j], vz[j]) & (0u - ((m4 >> j) & 1u));
-        const bool eligible = uniform && bad == 0u && yhi >= 0 && xhi - xlo < 8 && yhi - ylo < 8;
-        wrec[(size_t)frame * (size_t)nquads + wbase + (e >> 4)] = word_rec_pack(eligible, xlo, ylo, xhi, yhi, zs, (unsigned)__popc(m4));
       }
       e = e1;
       wc = wn;
@@ -1218,7 +1189,7 @@ __device__ __forceinline__ void quad_reduce_exact_point(const DevParams &p, floa
 #define SSD_DEF_MID 0x2000u     // deferred point between inner and reject box: f32 image of the test first
 #define SSD_DEF_GENERIC 0x4000u // deferred point of a word with mixed labels: not yet checked against amask
 
-// state a warp of k_quad_reduce / k_quad_sum carries across its warp-tiles
+// state a warp of k_quad_reduce carries across its warp-tiles
 struct QrWarp
 {
   unsigned seg_l, seg_n, n_def, n_mid;
@@ -1443,7 +1414,7 @@ __device__ __forceinline__ void qr_dense(const DevParams &p, const FRAME &FR, Qu
   qr_seg_combine(S, W, lane);
 }
 
-// the frame's filter tables and the block's accumulators (k_quad_reduce / k_quad_sum)
+// the frame's filter tables and the block's accumulators (k_quad_reduce)
 __device__ __forceinline__ void qr_init(QuadReduceShared &S, const FrameDev &F, unsigned amask, int tid)
 {
     // the frame's filter tables: one coalesced copy, independent of anything else
@@ -1476,7 +1447,7 @@ __device__ __forceinline__ void qr_init(QuadReduceShared &S, const FrameDev &F, 
     }
 }
 
-// end of k_quad_reduce / k_quad_sum: the warps' leftovers into the block's accumulators, the block's into the frame's
+// end of k_quad_reduce: the warps' leftovers into the block's accumulators, the block's into the frame's
 __device__ __forceinline__ void qr_epilogue(QuadReduceShared &S, QrWarp &W, FrameDev &F, int ground, int tid, int lane)
 {
   unsigned n_def = W.n_def;
@@ -1583,163 +1554,6 @@ __global__ void __launch_bounds__(SSD_PT_THREADS, SSD_QR_MINB) k_quad_reduce(con
     qr_dense<SRC>(p, FR, S, W, F, amask, ground, gbev, wbase, n, warp, lane);
     __syncwarp();
   }
-  qr_epilogue(S, W, F, ground, tid, lane);
-}
-
-
-// ---------------------------------------------------------------------------------------------
-// k_quad_reduce_rec: k_quad_reduce for the chain whose k_label_bev<SRC, true> left word records. A 4-pixel word whose plateau
-// points share one label of a valid (non-ground) step and whose record is eligible is decided as a whole: the world
-// rectangle that every point with a BEV pixel in the record's box lies in -- centre (cx, cy), half extents widened by the
-// rounding margins -- goes through the step's verified inner box and, failing that, through the f32 image of the reference's
-// test (quadfilter_eval with the half extent as the position uncertainty: "certainly inside" then holds for every point of the
-// rectangle). Such a word adds the record's z sum and count; its 48 bytes of vertices are not read. Everything else -- ground
-// words (they also feed the ground's BEV image), words with mixed labels or an uncertain pixel, words the quadrilateral's
-// edges come near -- is re-compacted and takes the dense pass of k_quad_reduce (qr_dense) unchanged, so both chains produce
-// the same integer sums and counts.
-// ---------------------------------------------------------------------------------------------
-template<class SRC>
-__global__ void __launch_bounds__(SSD_PT_THREADS, SSD_QR_MINB) k_quad_reduce_rec(const __grid_constant__ DevParams p, const SRC src,
-                                                                     const unsigned char *__restrict__ labels, FrameDev *__restrict__ frames,
-                                                                     unsigned *__restrict__ bev, size_t bm_words, const uint2 *__restrict__ wrec)
-{
-  __shared__ QuadReduceShared S;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int frame = blockIdx.y;
-  FrameDev &F = frames[frame];
-  const unsigned amask = F.quad_amask;
-  if(amask == 0u)
-    return; // no valid plateau: nothing is emitted (pointcloud.cpp:434)
-  const int ground = F.ground_index;
-  const unsigned wmask = ground >= 0 ? amask & ~(1u << ground) : amask; // steps whose words can be taken whole
-  const size_t fbase = (size_t)frame * p.N;
-  const unsigned *lab32 = reinterpret_cast<const unsigned *>(labels + fbase);
-  unsigned *gbev = ground >= 0 ? bev + ((size_t)frame * SSD_GPU_MAX_PLATEAUS + ground) * bm_words : nullptr;
-  const int nquads = p.N >> 2;
-  const uint2 *frec = wrec + (size_t)frame * (size_t)nquads;
-  int wt, wt_end, wt_stride;
-  warp_tile_range((p.N + SSD_WT_PX - 1) / SSD_WT_PX, warp, wt, wt_end, wt_stride);
-
-  qr_init(S, F, amask, tid);
-  __syncthreads();
-
-  unsigned short *act = S.L.act[warp];
-  unsigned *labs = S.L.lab[warp];
-  QrWarp W = { 0xffu, 0u, 0u, 0u, 0ull, 0x7fffffff, -1 };
-  const typename SrcTraits<SRC>::Frame FR = src_frame(src, p, fbase);
-  const unsigned lt = (1u << lane) - 1u;
-
-  for(; wt < wt_end; wt += wt_stride)
-  {
-    const unsigned wbase = (unsigned)wt * (SSD_WT_PX / 4); // first word of the warp-tile within the frame
-    // ---- phase A: compaction of the words holding plateau labels (bit 7 of a label byte clear <=> label < 128) ----
-    unsigned n = 0;
-    unsigned labw[SSD_WT_WORDS];
-#pragma unroll
-    for(int it = 0; it < SSD_WT_WORDS; it++)
-    {
-      const int q = wt * (SSD_WT_PX / 4) + it * 32 + lane;
-      labw[it] = q < nquads ? __ldg(lab32 + q) : 0xffffffffu;
-    }
-    if(wt + wt_stride < wt_end)
-      asm volatile("prefetch.global.L2 [%0];" ::"l"(lab32 + (size_t)(wt + wt_stride) * (SSD_WT_PX / 4) + lane * 8));
-#pragma unroll
-    for(int it = 0; it < SSD_WT_WORDS; it++)
-    {
-      const unsigned lw = labw[it];
-      const unsigned am4 = (((~lw >> 7) & 0x01010101u) * 0x10204080u) >> 28; // bit j <-> byte j < 128
-      if(__any_sync(0xffffffffu, am4 != 0u))
-      {
-        if(am4)
-          labs[it * 32 + lane] = lw;
-        n = compact_append(act, n, am4, it, lane);
-      }
-    }
-    if(n == 0)
-      continue;
-    __syncwarp();
-
-    // ---- phase B': whole words from their records; the rest is re-compacted in place (writes trail the reads) ----
-    unsigned n2 = 0;
-    for(unsigned s0 = 0; s0 < n; s0 += 32)
-    {
-      const unsigned i0 = s0 + lane;
-      const unsigned e = i0 < n ? act[i0] : 0u;
-      bool dense = false;
-      if(e)
-      {
-        const unsigned m4 = e & 15u;
-        const unsigned lw = labs[e >> 4];
-        const unsigned l0 = (lw >> (8 * (__ffs(m4) - 1))) & 0xffu;
-        const unsigned bytes = ((m4 * 0x00204081u) & 0x01010101u) * 0xffu;
-        const bool uniform = ((lw ^ (l0 * 0x01010101u)) & bytes) == 0u;
-        if(!uniform)
-          dense = true;
-        else if(l0 < SSD_GPU_MAX_PLATEAUS && ((amask >> l0) & 1u))
-        {
-          dense = true;
-          if((wmask >> l0) & 1u)
-          {
-            const uint2 r = __ldg(frec + wbase + (e >> 4));
-            if(r.x & SSD_WREC_ELIGIBLE)
-            {
-              // centre and half extents of the pixel box [x0, x0 + w] x [y0, y0 + h] in pixels, then in metres
-              const float hw = 0.5f * (float)(((r.x >> 24) & 7u) + 1u), hh = 0.5f * (float)(((r.x >> 27) & 7u) + 1u);
-              const float cx = fmaf((float)(r.x & 0xfffu) + hw, p.gs_xw, p.gs_x0);
-              const float cy = fmaf(-((float)((r.x >> 12) & 0xfffu) + hh), p.gs_yw, p.gs_y0);
-              const float eb = fmaxf(hw * p.gs_xw, hh * p.gs_yw) + p.gs_margin;
-              const float4 ib = S.fast[l0].ibe;
-              bool whole = fabsf(cx - ib.x) < ib.z - eb && fabsf(cy - ib.y) < ib.w - eb;
-              if(!whole)
-              {
-                bool unc;
-                const bool in = quadfilter_eval(S.qf[l0], cx, cy, eb + p.epsc, unc);
-                whole = in && !unc;
-              }
-              if(whole)
-              {
-                dense = false;
-                if(l0 != W.seg_l)
-                {
-                  if(W.seg_n)
-                    seg_flush(S, W.seg_l, W.seg_sum, W.seg_n);
-                  W.seg_l = l0;
-                  W.seg_sum = 0;
-                  W.seg_n = 0;
-                }
-                W.seg_sum += r.y & 0x1ffffffu;
-                W.seg_n += r.y >> 25;
-              }
-            }
-          }
-        }
-      }
-      const unsigned b = __ballot_sync(0xffffffffu, dense);
-      __syncwarp();
-#ifdef SSD_WREC_DEBUG
-      {
-        // debug build: words taken whole / words sent to the dense pass, in the counters the stats call reports as n_bev_exact / n_quad_exact
-        const unsigned bw = __ballot_sync(0xffffffffu, e != 0u && !dense);
-        if(lane == 0)
-        {
-          atomicAdd(&F.n_def_bev, (unsigned)__popc(bw));
-          atomicAdd(&F.n_def_quad, (unsigned)__popc(b));
-        }
-      }
-#endif
-      if(dense)
-      {
-        act[n2 + __popc(b & lt)] = (unsigned short)e;
-        word_prefetch_l2(FR, wbase + (e >> 4));
-      }
-      n2 += __popc(b);
-    }
-    __syncwarp();
-    if(n2)
-      qr_dense<SRC>(p, FR, S, W, F, amask, ground, gbev, wbase, n2, warp, lane);
-    __syncwarp();
-  }
-  qr_seg_combine(S, W, lane);
   qr_epilogue(S, W, F, ground, tid, lane);
 }
 

@@ -288,7 +288,8 @@ def test_lens_z16_4096x3072(S, name):
 
 @gpu
 @pytest.mark.parametrize("name", ["BC", "IBC"])
-def test_deproject_device_and_unfused_route(S, name, monkeypatch):
+def test_deproject_device(S, name):
+    """ssd_gpu_deproject_device through a lens: bit for bit the host deprojection"""
     w, h, n = 640, 480, 3
     base, depth, xyz = lens_frames(S, w, h, LENSES[name], n, 5)
     cfg = S.default_config(w, h)
@@ -302,15 +303,8 @@ def test_deproject_device_and_unfused_route(S, name, monkeypatch):
         got = np.empty_like(xyz)
         det.d2h(got, d_xyz)
         assert got.tobytes() == xyz.tobytes()
-        det.process_host(xyz)
-        want = [exact(gpu_result(S, det, f)) for f in range(n)]
         det.free(d_z16)
         det.free(d_xyz)
-    monkeypatch.setenv("SSD_GPU_DEPTH_UNFUSED", "1")
-    with S.Detector(cfg, xf, max_frames=n) as det:
-        det.set_distortion(dist)
-        det.process_depth_host(depth, intr)
-        assert [exact(gpu_result(S, det, f)) for f in range(n)] == want
 
 
 @gpu
@@ -489,25 +483,6 @@ def test_errors_leave_results_and_table_in_place(S):
         # the camera table still works after the rejections
         det.process_depth_cameras_host(depth, np.zeros(n, np.int32))
         unchanged()
-
-
-@gpu
-def test_experimental_chain_rejects_a_distorted_depth_call(S, monkeypatch):
-    w, h, n = 640, 480, 2
-    base, depth, xyz = lens_frames(S, w, h, BC, n, 23)
-    cfg = S.default_config(w, h)
-    xf = S.scene_transform(base)
-    intr = S.scene_intrinsics(base)
-    monkeypatch.setenv("SSD_GPU_PATH", "records")
-    with S.Detector(cfg, xf, max_frames=n) as det:
-        det.process_host(xyz)
-        want = [exact(gpu_result(S, det, f)) for f in range(n)]
-        det.set_distortion(S.scene_distortion(base))
-        with pytest.raises(S.SsdError, match=r"\(-5\)"):
-            det.process_depth_host(depth, intr)
-        assert [exact(gpu_result(S, det, f)) for f in range(n)] == want
-        det.process_host(xyz)  # vertex input without overlay does not use the lens
-        assert [exact(gpu_result(S, det, f)) for f in range(n)] == want
 
 
 @gpu

@@ -1,5 +1,5 @@
 """GPU: directed tests of the reference's degenerate behaviours that parity requires reproducing (SURVEY.md 5 / 8(a) notes):
-hand-built vertex frames that force each SSD_STATUS_* bit, GPU (all three chains) against the C oracle and -- where it
+hand-built vertex frames that force each SSD_STATUS_* bit, GPU (fused and seven-launch chain) against the C oracle and -- where it
 survives the input -- the compiled reference (oracle/_ref). Every test asserts that the bit is actually set.
 
 The frames are built in WORLD coordinates and pushed through an affine camera-to-world map that is the identity (or a pure
@@ -52,23 +52,31 @@ def shifted(xf):
     return xf
 
 
-def run_paths(S, cfg, xf, xyz, monkeypatch):
-    """the frame through the classic chain and the two experimental ones"""
+def run_paths(S, cfg, xf, xyz):
+    """the frame through both forms of the chain: a one-frame host call takes the fused small-batch form (the peaks in
+    k_transform_bin, the frame logic in k_outline); stage timing selects the seven-launch form with k_peaks and k_frame_logic
+    at any batch size"""
+    import test_gpu_parity as T
     res = {}
-    for path in ("classic", "records", "resident"):
-        monkeypatch.setenv("SSD_GPU_PATH", path)
-        with S.Detector(cfg, xf, max_frames=1) as det:
-            det.process_host(xyz[None])
-            import test_gpu_parity as T
-            res[path] = T.gpu_result(S, det, 0)
-    monkeypatch.delenv("SSD_GPU_PATH")
+    with S.Detector(cfg, xf, max_frames=1) as det:
+        det.process_host(xyz[None])
+        assert det.timing().n_launches == 5
+        res["fused"] = T.gpu_result(S, det, 0)
+        d = det.malloc(xyz.nbytes)
+        try:
+            det.h2d(d, xyz)
+            det.process_device(d, 1, A.FLAG_STAGE_TIMING)
+            assert det.timing().n_launches == 7
+            res["seven-launch"] = T.gpu_result(S, det, 0)
+        finally:
+            det.free(d)
     return res
 
 
-def check(S, oracle, cfg, xf, xyz, monkeypatch, bit, ref_too=True, ref_mask=0):
+def check(S, oracle, cfg, xf, xyz, bit, ref_too=True, ref_mask=0):
     o = H.oracle_process(oracle, cfg, xf, xyz)
     assert o.info["status"] & bit, hex(o.info["status"])
-    for path, g in run_paths(S, cfg, xf, xyz, monkeypatch).items():
+    for path, g in run_paths(S, cfg, xf, xyz).items():
         assert g.info["status"] == o.info["status"], (path, hex(g.info["status"]), hex(o.info["status"]))
         bad = H.compare_results(o, g, tol=TOL)
         assert not bad, (path, bad)
@@ -81,7 +89,7 @@ def check(S, oracle, cfg, xf, xyz, monkeypatch, bit, ref_too=True, ref_mask=0):
     return o
 
 
-def test_hmin_wrap_empties_every_plateau(S, oracle, monkeypatch):
+def test_hmin_wrap_empties_every_plateau(S, oracle):
     """SSD_STATUS_HMIN_WRAP: a peak at bin 1 with hist[0] > hist[2] -- heightMin - 1 wraps as uint16 (pointcloud.cpp:324), every
     remaining point falls into the remainder and that plateau and all later ones come out empty."""
     rng = np.random.default_rng(11)
@@ -89,22 +97,22 @@ def test_hmin_wrap_empties_every_plateau(S, oracle, monkeypatch):
     parts = [slab(rng, 1500, -0.4, 0.4, 0.2, 0.6, -0.095), slab(rng, 4000, -0.4, 0.4, 0.2, 0.6, -0.085),  # bins 0 and 1
              slab(rng, 6000, -0.4, 0.4, 0.7, 1.1, 0.305)]                                               # a regular plateau above
     xyz = frame_of(parts)
-    o = check(S, oracle, cfg, shifted(identity_xf()), xyz, monkeypatch, A.STATUS_HMIN_WRAP, ref_mask=A.STATUS_HMIN_WRAP)
+    o = check(S, oracle, cfg, shifted(identity_xf()), xyz, A.STATUS_HMIN_WRAP, ref_mask=A.STATUS_HMIN_WRAP)
     assert o.info["n_plateaus"] == 2 and all(p["n_points"] == 0 for p in o.plateaus)
     assert not (o.labels < 32).any()
 
 
-def test_more_peaks_than_plateau_slots(S, oracle, monkeypatch):
+def test_more_peaks_than_plateau_slots(S, oracle):
     """SSD_STATUS_TOO_MANY_PLATEAUS: 35 histogram peaks; the ABI keeps the first 32 (the reference has no limit: not compared)."""
     rng = np.random.default_rng(12)
     cfg = S.default_config(W, HH)
     parts = [slab(rng, 2100, -0.5, 0.5, 0.2, 1.2, -0.1 + (1 + 3 * k + 0.5) * 0.01) for k in range(35)]
     xyz = frame_of(parts)
-    o = check(S, oracle, cfg, shifted(identity_xf()), xyz, monkeypatch, A.STATUS_TOO_MANY_PLATEAUS, ref_too=False)
+    o = check(S, oracle, cfg, shifted(identity_xf()), xyz, A.STATUS_TOO_MANY_PLATEAUS, ref_too=False)
     assert o.info["n_plateaus"] == 32
 
 
-def test_ground_without_points_in_its_quadrilateral(S, oracle, monkeypatch):
+def test_ground_without_points_in_its_quadrilateral(S, oracle):
     """SSD_STATUS_INVALID_FRONT_EDGE: the ground plateau exists, but none of its points lies between y_min and the first step's
     front edge: calcGround finds no front edge and returns the all-zero quadrilateral, which is still emitted as a step
     (pointcloud.cpp:546, 442)."""
@@ -113,11 +121,11 @@ def test_ground_without_points_in_its_quadrilateral(S, oracle, monkeypatch):
     parts = [slab(rng, 9000, -0.45, 0.45, 1.0, 1.25, 0.004),   # ground only BEHIND the step
              slab(rng, 30000, -0.45, 0.45, 0.45, 0.75, 0.185)]  # one step
     xyz = frame_of(parts)
-    o = check(S, oracle, cfg, shifted(identity_xf()), xyz, monkeypatch, A.STATUS_INVALID_FRONT_EDGE, ref_mask=A.STATUS_INVALID_FRONT_EDGE)
+    o = check(S, oracle, cfg, shifted(identity_xf()), xyz, A.STATUS_INVALID_FRONT_EDGE, ref_mask=A.STATUS_INVALID_FRONT_EDGE)
     assert o.info["n_steps"] == 2 and o.steps[0]["height"] == 0.0 and not o.steps[0]["quad"].any()
 
 
-def test_bev_pixel_past_the_image(S, oracle, monkeypatch):
+def test_bev_pixel_past_the_image(S, oracle):
     """SSD_STATUS_BEV_OOB: Projection2D::worldToImage has no bounds check (pointcloud.cpp:81, 468). A world y one double-ulp
     above y_min is inside the measuring range, but (y_max - y) * yToImage rounds up to H: the reference writes past the end of
     the image (undefined behaviour there: not run); the ABI drops the pixel and raises the bit. World y = a11 * y_camera with
@@ -142,7 +150,7 @@ def test_bev_pixel_past_the_image(S, oracle, monkeypatch):
     o = H.oracle_process(oracle, cfg, xf, xyz)
     assert o.info["status"] & A.STATUS_BEV_OOB, hex(o.info["status"])
     assert o.info["n_steps"] >= 2
-    for path, g in run_paths(S, cfg, xf, xyz, monkeypatch).items():
+    for path, g in run_paths(S, cfg, xf, xyz).items():
         assert g.info["status"] == o.info["status"], (path, hex(g.info["status"]), hex(o.info["status"]))
         assert not H.compare_results(o, g, tol=TOL), path
 
@@ -163,20 +171,6 @@ def test_two_contexts_of_different_sizes_alternate(S, oracle):
                 big.process_host(big_xyz[None])
                 assert not H.compare_results(H.oracle_process(oracle, big_cfg, big_xf, big_xyz), T.gpu_result(S, big, 0), tol=TOL)
                 assert not H.compare_results(H.oracle_process(oracle, small_cfg, small_xf, small_xyz), T.gpu_result(S, small, 0), tol=TOL)
-
-
-@pytest.mark.parametrize("path", ["wordrec", "records", "resident"])
-def test_experimental_chains_match_the_oracle(S, oracle, monkeypatch, path):
-    """the word-record chain, the record chain and the resident-frame chain (SSD_GPU_PATH, DESIGN.md): same results as the oracle on a random batch"""
-    monkeypatch.setenv("SSD_GPU_PATH", path)
-    import test_gpu_parity as T
-    cfg = S.default_config(1024, 768)
-    base = S.default_scene(1024, 768, **T.NOISY)
-    scenes = [S.randomize_scene(base, 777, i, 3, 8) for i in range(6)]
-    T.run_frames(S, oracle, cfg, scenes)
-    cfg = S.default_config(640, 480)
-    base = S.default_scene(640, 480, rotate180=1, n_occluders=2, **T.NOISY)
-    T.run_frames(S, oracle, cfg, [S.randomize_scene(base, 778, i, 3, 8) for i in range(4)])
 
 
 def test_misaligned_device_input_is_refused(S):

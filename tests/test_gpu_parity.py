@@ -149,11 +149,10 @@ def test_empty_and_garbage_frames(S, oracle):
 
 
 @pytest.mark.parametrize("w,h", [(640, 480), (1024, 768)])
-def test_depth_frame_input(S, oracle, monkeypatch, w, h):
+def test_depth_frame_input(S, oracle, w, h):
     """The z16 depth-frame entry points (what the reference's process() receives): on-device deprojection is bit-identical
     to the host's, and host / device depth input -- deprojected inside the three point kernels, no vertex array in
-    memory -- give exactly the results of the vertex path, which is checked against the oracle. The unfused A/B path
-    (separate deprojection kernel) must agree too."""
+    memory -- give exactly the results of the vertex path, which is checked against the oracle."""
     cfg = S.default_config(w, h)
     base = S.default_scene(w, h, **NOISY)
     scenes = [S.randomize_scene(base, 77, i, 3, 6) for i in range(5)]
@@ -181,9 +180,8 @@ def test_depth_frame_input(S, oracle, monkeypatch, w, h):
         for f in range(n):
             o = H.oracle_process(oracle, cfg, xf, xyz[f])
             assert not H.compare_results(o, gpu_result(S, det, f), tol=TOL), f
-        for run in ("host", "device", "device-unfused", "host-unfused"):
-            monkeypatch.setenv("SSD_GPU_DEPTH_UNFUSED", "1" if run.endswith("unfused") else "0")
-            if run.startswith("host"):
+        for run in ("host", "device"):
+            if run == "host":
                 det.process_depth_host(depth, k)
             else:
                 det.process_depth_device(d_depth, k, n)

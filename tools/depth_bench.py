@@ -1,5 +1,5 @@
-"""GPU box: device-resident z16 depth frames through the chain, deprojection inside the point kernels (SrcDepth) against the
-A/B path with a separate deprojection kernel and a vertex array (SSD_GPU_DEPTH_UNFUSED=1), next to the packed-vertex input.
+"""GPU box: device-resident z16 depth frames through the chain, deprojection inside the point kernels (SrcDepth), next to the
+packed-vertex input.
     python tools/depth_bench.py --frames 2048"""
 import argparse, json, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -42,7 +42,4 @@ def run(name, fn, flags_fn=None):
 
 run("packed vertices (12 B/point)", lambda: det.process_device(d_xyz, args.frames),
     lambda: det.process_device(d_xyz, args.frames, flags=A.FLAG_STAGE_TIMING | A.FLAG_SINGLE_STREAM))
-os.environ["SSD_GPU_DEPTH_UNFUSED"] = "0"
 run("z16 depth (2 B/point), deprojected inside the point kernels", lambda: det.process_depth_device(d_depth, intr, args.frames))
-os.environ["SSD_GPU_DEPTH_UNFUSED"] = "1"
-run("z16 depth, separate deprojection kernel + vertex array (A/B)", lambda: det.process_depth_device(d_depth, intr, args.frames))

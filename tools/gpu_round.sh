@@ -1,6 +1,6 @@
 #!/bin/bash
 # One GPU-box session. Usage (repo root, under gpurun):  bash tools/gpu_round.sh <tag> [steps...]
-#   steps: test bench sweep launches ncu paths configs reference latency   (default: test bench sweep launches ncu)
+#   steps: test bench sweep launches ncu configs reference latency   (default: test bench sweep launches ncu)
 TAG=${1:-r01}; shift
 STEPS=${@:-test bench sweep launches ncu}
 OUT=gpurun_out/$TAG
@@ -15,7 +15,6 @@ launches) echo "== ncu launches"; timeout 600 ncu --metrics gpu__time_duration.s
    python bench.py --steps 2 --warmup 3 --frames 512 --e2e-frames 16 --no-cpu-baseline --no-latency --parity-frames 0 > $OUT/bench_under_ncu.log 2>&1; grep -c k_ $OUT/launches.csv;;
 ncu) echo "== ncu full"; timeout 900 ncu --set full --clock-control none --import-source on -k "regex:${NCU_KERNELS:-k_transform_bin|k_label_bev|k_quad_reduce|k_outline}" -s ${NCU_SKIP:-8} -c ${NCU_COUNT:-4} \
    -o $OUT/prof python bench.py --steps 1 --warmup 3 --frames 512 --e2e-frames 16 --no-cpu-baseline --no-latency --parity-frames 0 > $OUT/ncu_full.log 2>&1; tail -3 $OUT/ncu_full.log | cut -c1-300;;
-paths) echo "== experimental chains"; for pth in ${PATHS:-wordrec classic records resident}; do SSD_GPU_PATH=$pth timeout 300 python tools/sweep.py --frames 2048 --chunks 1024 --reps 3 --warm 2 2>&1 | tail -1 | sed "s/^/{\"path\": \"$pth\", \"run\": /; s/$/}/"; done | tee $OUT/paths.jsonl;;
 configs) echo "== configs"; for c in 0 1 3 4; do timeout 600 python bench.py --config $c --steps 5 --warmup 3 --no-cpu-baseline > $OUT/bench_config$c.json 2> $OUT/bench_config$c.err; tail -c 300 $OUT/bench_config$c.json; echo; done;;
 reference) echo "== reference arm"; timeout 600 python bench.py --impl reference --steps 3 --warmup 1 > $OUT/bench_reference.json 2> $OUT/bench_reference.err; tail -c 400 $OUT/bench_reference.json;;
 latency) echo "== latency"; (python tools/latency.py; python tools/latency.py --w 640 --h 480) | tee $OUT/latency.jsonl;;

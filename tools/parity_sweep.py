@@ -63,6 +63,6 @@ while done < args.frames:
             bad += 1
             print("MISMATCH group", done // B, "frame", f, kw, flush=True)
     done += B
-print(json.dumps({"path": os.environ.get("SSD_GPU_PATH", "classic"), "tol_m": args.tol, "frames": done, "mismatches": bad, "size": [W, Hh], "seconds": round(time.time() - t0, 1),
+print(json.dumps({"tol_m": args.tol, "frames": done, "mismatches": bad, "size": [W, Hh], "seconds": round(time.time() - t0, 1),
                   "overlay": {"values": ov_n, "bit_identical": ov_exact, "max_abs_diff_px": ov_max}}))
 sys.exit(1 if bad else 0)

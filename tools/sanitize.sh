@@ -29,14 +29,6 @@ with S.Detector(cfg, xf, max_frames=len(scenes)) as det:
     assert ris == [det.vertical_faces(f) for f in range(len(scenes))]
 for f in range(len(scenes)):
     assert ris[f] == helpers.oracle_vertical_faces(orc, cfg, xf, xyz[f].reshape(-1, 3))
-import os
-os.environ["SSD_GPU_PATH"] = "wordrec"  # k_label_bev<.., true> / k_quad_reduce_rec
-with S.Detector(cfg, xf, max_frames=len(scenes)) as det:
-    det.process_host(xyz)
-    w = [det.steps(f)[0] for f in range(len(scenes))]
-del os.environ["SSD_GPU_PATH"]
-for f in range(len(scenes)):
-    assert len(w[f]) == len(a[f]) and all(h0 == h1 and np.array_equal(q0, q1) for (h0, q0), (h1, q1) in zip(w[f], a[f]))
 for f in range(len(scenes)):
     o = helpers.oracle_process(orc, cfg, xf, xyz[f])
     assert np.array_equal(labels[f], o.labels) and len(a[f]) == len(o.steps) == len(b[f])
