@@ -98,7 +98,9 @@ __device__ inline void band_stage(const DevParams &p, unsigned *sm, const Band &
 {
   const unsigned wpr = (unsigned)p.wpr;
   const unsigned total = (unsigned)bd.nb * wpr;
-  const unsigned magic = 0xffffffffu / wpr + 1u; // row = (i * magic) >> 32, exact for i * wpr < 2^32
+  // row = (i * magic) >> 32, exact for i * wpr < 2^32. One word per row (W <= 32) would need magic = 2^32, which wraps
+  // to 0 in 32 bits: there the row is i itself.
+  const unsigned magic = 0xffffffffu / wpr + 1u;
   unsigned *src = g + (size_t)bd.b0 * wpr;
   for(unsigned base = (unsigned)tid; base < total; base += (unsigned)nthreads * 8u)
   {
@@ -117,7 +119,8 @@ __device__ inline void band_stage(const DevParams &p, unsigned *sm, const Band &
       {
         if(v[k])
           src[i] = 0u;
-        sm[i + __umulhi(i, magic) * (unsigned)(bd.rs - (int)wpr)] = v[k]; // row stride rs: r * rs + (i - r * wpr)
+        const unsigned r = wpr == 1u ? i : __umulhi(i, magic);
+        sm[i + r * (unsigned)(bd.rs - (int)wpr)] = v[k]; // row stride rs: r * rs + (i - r * wpr)
       }
     }
   }
