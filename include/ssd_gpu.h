@@ -267,6 +267,39 @@ int ssd_gpu_set_cameras_ex(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, const s
  * lens is a pin-hole: then no call reads a ray table. */
 int ssd_gpu_n_ray_tables(ssd_gpu_ctx *ctx);
 
+/*
+ * ---- frame groups: one stair detection from the combined points of several cameras or frames ----
+ * A call takes n_groups groups of consecutive frames; group g has group_frames[g] members, 1 <= group_frames[g] <=
+ * SSD_GPU_MAX_GROUP_FRAMES. Every frame has a camera index (camera_of_frame, as in the camera calls); a camera table is required.
+ *  - Points: member i's vertices go through camera camera_of_frame[i]'s CameraToWorld, as given or deprojected from z16 with that
+ *    camera's intrinsics and lens, with the per-point arithmetic of the camera calls. From there on the group is one point cloud:
+ *    the union of its members' points.
+ *  - Chain: range filter, height index, histogram, peaks, plateau bands, BEV images, outlines, ground / first-valid logic, ground
+ *    quadrilateral, points in quadrilateral, mean z and the risers' remainder run once per group, over the union, with the
+ *    context's configuration. min_peak_points stays absolute, as in the reference (pointcloud.cpp:251): a caller who fuses k views
+ *    may raise it in the configuration; the library does not scale it.
+ *  - External world: the group's steps go through the ToExternalWorld of the camera of the group's first member.
+ *  - Overlay: when it is on, every member frame gets the group's steps projected into its own camera (a_inv, intrinsics, lens).
+ *  - Labels: each member frame's pixels get labels as in the other calls; plateau indices are the group's.
+ *  - Getters stay frame-indexed: for any member frame, ssd_gpu_get_steps, _get_frame_info, _get_plateaus, _get_histogram and
+ *    _get_vertical_faces return its group's record (frame_info.n_nonzero and n_in_range are the group's totals); _get_labels and
+ *    _get_overlay return the frame's own data. ssd_gpu_get_stats counts the whole call.
+ *  - A group of one frame gives, bit for bit, what the camera call gives for that frame.
+ * Every argument is checked before anything is launched; a rejected call leaves the previous results readable: no camera table
+ * SSD_E_STATE; a camera index outside the table, or more frames in all than max_frames, SSD_E_RANGE; n_groups < 1, a NULL array or a
+ * group size outside [1, SSD_GPU_MAX_GROUP_FRAMES] SSD_E_INVALID_ARG; a depth call that uses a camera without valid intrinsics
+ * SSD_E_INVALID_ARG; misaligned input as in the other calls. flags: SSD_FLAG_STAGE_TIMING, SSD_FLAG_SINGLE_STREAM.
+ */
+#define SSD_GPU_MAX_GROUP_FRAMES 32
+int ssd_gpu_process_groups_host(ssd_gpu_ctx *ctx, const float *xyz_host, const int32_t *camera_of_frame, const int32_t *group_frames,
+                                int n_groups);
+int ssd_gpu_process_groups_device(ssd_gpu_ctx *ctx, const float *xyz_dev, const int32_t *camera_of_frame, const int32_t *group_frames,
+                                  int n_groups, int flags);
+int ssd_gpu_process_depth_groups_host(ssd_gpu_ctx *ctx, const uint16_t *z16_host, const int32_t *camera_of_frame, const int32_t *group_frames,
+                                      int n_groups);
+int ssd_gpu_process_depth_groups_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const int32_t *camera_of_frame, const int32_t *group_frames,
+                                        int n_groups, int flags);
+
 /* ---- results of the last process call ---- */
 /* Stairs of one frame: out[0..*n) ; replaces the value printed at pointcloud.cpp:624-625. */
 int ssd_gpu_get_steps(ssd_gpu_ctx *ctx, int frame, ssd_gpu_step *out, int cap, int *n, uint32_t *status);

@@ -318,6 +318,44 @@ class Detector:
         cams = self._cams(camera_of_frame, n_frames)
         self._ck(self._l.ssd_gpu_process_depth_cameras_device(self._h, dev_ptr, _ptr(cams), n_frames), "ssd_gpu_process_depth_cameras_device")
 
+    # ---- frame groups: one detection from the union of several frames' points (include/ssd_gpu.h) ----
+    @staticmethod
+    def _groups(group_frames, n_frames=None):
+        g = np.ascontiguousarray(group_frames, np.int32)
+        if n_frames is not None and int(g.sum()) != n_frames:
+            raise ValueError(f"group_frames add up to {int(g.sum())} frames, the input holds {n_frames}")
+        return g
+
+    def process_groups_host(self, xyz, camera_of_frame, group_frames):
+        """xyz as for process_host; camera_of_frame: camera table index of each frame; group_frames: members of each group
+        (consecutive frames). Returns the number of frames."""
+        xyz = np.ascontiguousarray(xyz, np.float32)
+        n = xyz.size // (self.n_points * 3)
+        cams = self._cams(camera_of_frame, n)
+        g = self._groups(group_frames, n)
+        self._ck(self._l.ssd_gpu_process_groups_host(self._h, _ptr(xyz), _ptr(cams), _ptr(g), g.size), "ssd_gpu_process_groups_host")
+        return n
+
+    def process_groups_device(self, dev_ptr, camera_of_frame, group_frames, flags=0):
+        g = self._groups(group_frames)
+        cams = self._cams(camera_of_frame, int(g.sum()))
+        self._ck(self._l.ssd_gpu_process_groups_device(self._h, dev_ptr, _ptr(cams), _ptr(g), g.size, flags), "ssd_gpu_process_groups_device")
+
+    def process_depth_groups_host(self, depth, camera_of_frame, group_frames):
+        """depth as for process_depth_host; each frame is deprojected with its camera's intrinsics and lens."""
+        depth = np.ascontiguousarray(depth, np.uint16)
+        n = depth.size // self.n_points
+        cams = self._cams(camera_of_frame, n)
+        g = self._groups(group_frames, n)
+        self._ck(self._l.ssd_gpu_process_depth_groups_host(self._h, _ptr(depth), _ptr(cams), _ptr(g), g.size), "ssd_gpu_process_depth_groups_host")
+        return n
+
+    def process_depth_groups_device(self, dev_ptr, camera_of_frame, group_frames, flags=0):
+        g = self._groups(group_frames)
+        cams = self._cams(camera_of_frame, int(g.sum()))
+        self._ck(self._l.ssd_gpu_process_depth_groups_device(self._h, dev_ptr, _ptr(cams), _ptr(g), g.size, flags),
+                 "ssd_gpu_process_depth_groups_device")
+
     # ---- results ----
     def steps(self, frame):
         out = (Step * A.MAX_STEPS)()

@@ -10,6 +10,7 @@ import os
 MAX_BINS = 253
 MAX_PLATEAUS = 32
 MAX_STEPS = 32
+MAX_GROUP_FRAMES = 32  # members of one frame group (ssd_gpu_process_groups_*)
 LABEL_REMAINDER = 253
 LABEL_OUT_OF_RANGE = 254
 LABEL_INVALID = 255
@@ -141,6 +142,10 @@ PROTOTYPES = {
     "ssd_gpu_process_cameras_device_ex": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int]),
     "ssd_gpu_process_depth_cameras_host": (C.c_int, [_vp, _vp, _vp, C.c_int]),
     "ssd_gpu_process_depth_cameras_device": (C.c_int, [_vp, _vp, _vp, C.c_int]),
+    "ssd_gpu_process_groups_host": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int]),
+    "ssd_gpu_process_groups_device": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int]),
+    "ssd_gpu_process_depth_groups_host": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int]),
+    "ssd_gpu_process_depth_groups_device": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int]),
     "ssd_gpu_process_depth_host": (C.c_int, [_vp, _vp, _P(Intrinsics), C.c_int]),
     "ssd_gpu_process_depth_device": (C.c_int, [_vp, _vp, _P(Intrinsics), C.c_int]),
     "ssd_gpu_deproject_device": (C.c_int, [_vp, _vp, _P(Intrinsics), C.c_int, _vp]),

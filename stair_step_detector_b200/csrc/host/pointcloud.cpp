@@ -161,6 +161,47 @@ std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, i
   return collect(nFrames, status);
 }
 
+std::vector<Stairs> Pointcloud::processGroups(const Camera::DepthFrame &frames, int nFrames, const std::vector<int32_t> &cameraOfFrame,
+                                              const std::vector<int32_t> &groupFrames, std::vector<unsigned> *status) const
+{
+  if(nFrames < 0 || cameraOfFrame.size() != static_cast<size_t>(nFrames))
+    throw std::invalid_argument("Pointcloud::processGroups: cameraOfFrame must hold one camera index per frame");
+  long long total = 0;
+  for(int32_t k : groupFrames)
+    total += k;
+  if(total != nFrames)
+    throw std::invalid_argument("Pointcloud::processGroups: groupFrames must add up to nFrames");
+  ensureContext(frames.width(), frames.height());
+  applySettings();
+  const int32_t *cam = cameraOfFrame.data(), *grp = groupFrames.data();
+  const int nGroups = static_cast<int>(groupFrames.size());
+  int rc;
+  if(frames.z16)
+    rc = frames.onDevice ? ssd_gpu_process_depth_groups_device(_ctx, frames.z16, cam, grp, nGroups, 0)
+                         : ssd_gpu_process_depth_groups_host(_ctx, frames.z16, cam, grp, nGroups);
+  else
+    rc = frames.onDevice ? ssd_gpu_process_groups_device(_ctx, frames.vertices, cam, grp, nGroups, 0)
+                         : ssd_gpu_process_groups_host(_ctx, frames.vertices, cam, grp, nGroups);
+  if(rc != SSD_OK)
+    throw std::runtime_error(std::string("ssd_gpu_process_groups: ") + ssd_gpu_last_error(_ctx));
+  // every member frame reads its group's result: keep the first member's
+  const std::vector<Stairs> all = collect(nFrames, nullptr);
+  std::vector<Stairs> out;
+  if(status)
+    status->clear();
+  for(int g = 0, f = 0; g < nGroups; f += grp[g], g++)
+  {
+    out.push_back(all[static_cast<size_t>(f)]);
+    if(status)
+    {
+      uint32_t st = 0;
+      ssd_gpu_get_steps(_ctx, f, nullptr, 0, nullptr, &st);
+      status->push_back(st);
+    }
+  }
+  return out;
+}
+
 // the Stairs of every frame of the last call
 std::vector<Stairs> Pointcloud::collect(int nFrames, std::vector<unsigned> *status) const
 {

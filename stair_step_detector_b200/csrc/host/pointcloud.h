@@ -46,6 +46,11 @@ public:
   int cameraCount() const { return static_cast<int>(_cameras.size()); }
   std::vector<Stairs> processBatch(const Camera::DepthFrame &frames, int nFrames, const std::vector<int32_t> &cameraOfFrame,
                                    std::vector<unsigned> *status = nullptr) const;
+  // Frame groups (ssd_gpu_process_groups_*): groupFrames[g] consecutive frames form group g, and each group is detected once from
+  // the union of its members' points, every frame through its camera cameraOfFrame[i]. Returns one Stairs per group (in the
+  // external world of the group's first member's camera); status: one per group.
+  std::vector<Stairs> processGroups(const Camera::DepthFrame &frames, int nFrames, const std::vector<int32_t> &cameraOfFrame,
+                                    const std::vector<int32_t> &groupFrames, std::vector<unsigned> *status = nullptr) const;
   // per-pixel segment labels of frame `frame` of the last call (SSD_LABEL_* codes / plateau index)
   std::vector<uint8_t> labels(int frame = 0) const;
   // drawStairStep (reference pointcloud.cpp:583-597): project the corners of every detected step into the camera image

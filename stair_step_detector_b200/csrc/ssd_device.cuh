@@ -213,6 +213,74 @@ __device__ __forceinline__ const OverlayDev &frame_overlay(const OverlayDev &ov,
 {
   return ov.enabled ? c.ov[frame_camera(c, frame)] : ov;
 }
+
+// Frame groups (ssd_gpu_process_groups_*): the member frames of a group are one point cloud. The point kernels keep one block row
+// per member frame and take its camera from cams, as CamTable does, but accumulate into the group's frame state (FrameDev, BEV
+// slots): frame_slot. The per-group kernels run one block per group; group_params gives them the parameters of the group's first
+// member's camera with epsc raised to the largest of the group's cameras, so the quadrilateral filters k_frame_logic builds hold
+// for the points of every member.
+struct GroupTable
+{
+  CamTable cams;        // camera of every frame of the call (cams.frame0: first frame of the launch)
+  const int *group;     // frames of the call: index of the frame's group within the call
+  const int2 *members;  // groups of the call: first frame (index within the call), number of members
+  const float *epsc;    // groups of the call: the largest epsc of the members' cameras
+  int group0;           // first group of the launch within the call
+};
+__device__ __forceinline__ int frame_slot(const NoCam &, int frame)
+{
+  return frame;
+}
+__device__ __forceinline__ int frame_slot(const CamTable &, int frame)
+{
+  return frame;
+}
+__device__ __forceinline__ int frame_slot(const GroupTable &g, int frame)
+{
+  return __ldg(g.group + g.cams.frame0 + frame) - g.group0;
+}
+__device__ __forceinline__ const DevParams &frame_params(const DevParams &p, const GroupTable &g, int frame)
+{
+  return frame_params(p, g.cams, frame);
+}
+// first member (index within the call) and member count of the launch's group slot g
+__device__ __forceinline__ int2 group_members(const GroupTable &c, int g)
+{
+  return c.members[c.group0 + g];
+}
+template<class CAM>
+__device__ __forceinline__ const DevParams &group_params(const DevParams &p, const CAM &c, int g)
+{
+  return frame_params(p, c, g);
+}
+__device__ __forceinline__ const DevParams &group_params(const DevParams &, const GroupTable &c, int g)
+{
+  __shared__ DevParams s_group_params;
+  const int2 m = group_members(c, g);
+  const unsigned long long *src = reinterpret_cast<const unsigned long long *>(c.cams.params + __ldg(c.cams.cam + m.x));
+  unsigned long long *dst = reinterpret_cast<unsigned long long *>(&s_group_params);
+  for(int i = threadIdx.x; i < (int)(sizeof(DevParams) / 8); i += blockDim.x)
+    dst[i] = __ldg(src + i);
+  __syncthreads();
+  if(threadIdx.x == 0)
+    s_group_params.epsc = __ldg(c.epsc + c.group0 + g);
+  __syncthreads();
+  return s_group_params;
+}
+// points of a group's frames beyond one frame's (k_peaks counts n_nonzero / n_in_range from one frame's N)
+template<class CAM>
+__device__ __forceinline__ unsigned group_extra_points(const CAM &, int, unsigned)
+{
+  return 0u;
+}
+__device__ __forceinline__ unsigned group_extra_points(const GroupTable &c, int g, unsigned N)
+{
+  return (unsigned)(group_members(c, g).y - 1) * N;
+}
+__device__ __forceinline__ const OverlayDev &frame_overlay(const OverlayDev &ov, const GroupTable &, int)
+{
+  return ov; // (only its `enabled` is read: k_finalize projects through each member's own camera)
+}
 // The overlay through a distorted lens (k_finalize only): LensCam<NoCam> / LensCam<CamTable> behave as their BASE and add the lens
 // of the plain overlay (lens[0]) or of each camera (lens[camera]). NoCam and CamTable project through the pin-hole.
 template<class BASE>
@@ -230,6 +298,16 @@ template<class BASE>
 __device__ __forceinline__ const OverlayDev &frame_overlay(const OverlayDev &ov, const LensCam<BASE> &c, int frame)
 {
   return frame_overlay(ov, c.base, frame);
+}
+template<class BASE>
+__device__ __forceinline__ const DevParams &group_params(const DevParams &p, const LensCam<BASE> &c, int g)
+{
+  return group_params(p, c.base, g);
+}
+template<class BASE>
+__device__ __forceinline__ unsigned group_extra_points(const LensCam<BASE> &c, int g, unsigned N)
+{
+  return group_extra_points(c.base, g, N);
 }
 template<class CAM>
 __device__ __forceinline__ void overlay_lens(const CAM &, int, float x, float y, float &xd, float &yd)

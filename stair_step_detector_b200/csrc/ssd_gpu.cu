@@ -10,6 +10,7 @@
 #include <cstring>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #ifndef SSD_PT_ITERS
@@ -90,7 +91,25 @@ struct ssd_gpu_ctx
   const float2 **d_cam_ray = nullptr;    // n_cameras: ray table of each camera
   ssd_gpu_distortion *d_cam_lens = nullptr; // n_cameras
   double stats_eps0 = 0, stats_eps1 = 0; // filter bounds of the last call (largest over its cameras)
+  // frame groups (ssd_gpu_process_groups_*): per frame its group, per group its first frame, member count and largest epsc
+  int *d_grp_of_frame = nullptr;         // max_frames
+  int2 *d_grp_members = nullptr;         // max_frames
+  float *d_grp_epsc = nullptr;           // max_frames
+  std::vector<int> grp_of_frame;         // host copy of the last call's (empty after a call without groups)
+  std::vector<int2> grp_members;
+  std::vector<float> grp_epsc;
+  int stage_frames = 0;                  // frames the host-input staging buffers hold (host_chunk_frames, more for a larger group)
 };
+
+// the result record (FrameDev / FrameOut) of a frame of the last call: its group's in a group call
+static int frame_record(const ssd_gpu_ctx *ctx, int frame)
+{
+  return ctx->grp_of_frame.empty() ? frame : ctx->grp_of_frame[frame];
+}
+static int n_records_last(const ssd_gpu_ctx *ctx)
+{
+  return ctx->grp_of_frame.empty() || ctx->n_frames_last <= 0 ? ctx->n_frames_last : (int)ctx->grp_members.size();
+}
 
 #define CK(call)                                                                                         \
   do                                                                                                     \
@@ -465,12 +484,13 @@ __global__ void k_single_camera_to_world(const __grid_constant__ DevParams p, co
 
 // The classic chain: k_transform_bin -> k_peaks -> k_label_bev -> k_outline -> k_frame_logic -> k_quad_reduce -> k_finalize
 // (+ k_riser_reduce). CAM = NoCam: every frame with the context's own camera; CamTable: each frame with its camera's parameters
-// (camera calls).
+// (camera calls); GroupTable: as CamTable, with the frames of each group accumulated into one record (group calls).
+// Records (FrameDev, FrameOut, BEV slots): rec0 is the launch's first within the call, nr their number (frames, or groups).
 // sl: the chunk's z16 frames through ray tables (a call with a distorted lens), else nullptr. ov_lens: the lenses the overlay
 // projects through (LensCam), else nullptr.
 template<class CAM>
-static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const SrcDepth &sd, const SrcLens *sl, int frame0, int nf, int *launches,
-                          cudaEvent_t *ev, const CAM cam, const ssd_gpu_distortion *ov_lens)
+static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const SrcDepth &sd, const SrcLens *sl, int frame0, int nf, int rec0,
+                          int nr, int *launches, cudaEvent_t *ev, const CAM cam, const ssd_gpu_distortion *ov_lens)
 {
 #define STAGE_EV(i)                         \
   do                                        \
@@ -480,7 +500,8 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   } while(0)
   const DevParams &p = ctx->dp;
   cudaStream_t st = ctx->stream[s];
-  FrameDev *frames = ctx->d_frames + frame0;
+  constexpr bool grouped = std::is_same<CAM, GroupTable>::value;
+  FrameDev *frames = ctx->d_frames + rec0;
   unsigned char *labels = ctx->d_labels + (size_t)frame0 * p.N;
   unsigned *bev = ctx->d_bev + (size_t)s * ctx->chunk_frames * SSD_GPU_MAX_PLATEAUS * ctx->bm_words;
   const dim3 gpt(p.tiles_per_frame, nf);
@@ -493,12 +514,15 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   const float *xyz_dev = sv.xyz;
   ssd_gpu_overlay *ovl = ctx->d_ovl ? ctx->d_ovl + (size_t)frame0 * SSD_GPU_MAX_STEPS : nullptr;
   // small batches (the reference's real use is one frame per call): the last block of a frame in k_transform_bin evaluates the
-  // peaks and the last block in k_outline the frame logic -- five launches instead of seven
-  const bool fused = nf <= SSD_FUSE_MAX_FRAMES && !ev;
+  // peaks and the last block in k_outline the frame logic -- five launches instead of seven. Group calls take the seven
+  // (their blocks do not count a frame's completion).
+  const bool fused = !grouped && nf <= SSD_FUSE_MAX_FRAMES && !ev;
   STAGE_EV(0);
   if(fused)
   {
-    if(sl)
+    if constexpr(grouped)
+      ;
+    else if(sl)
       k_transform_bin_lens<SSD_PT_ITERS, true, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, cam);
     else if(depth)
       k_transform_bin_depth<SSD_PT_ITERS, true, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, cam);
@@ -516,7 +540,7 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   }
   STAGE_EV(1);
   if(!fused)
-    k_peaks<<<nf, 32, 0, st>>>(p, frames, nf);
+    k_peaks<<<nr, 32, 0, st>>>(p, frames, nr);
   STAGE_EV(2);
   if(sl)
     k_label_bev<SrcLens, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, cam);
@@ -527,7 +551,9 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   STAGE_EV(3);
   if(fused)
   {
-    if(ctx->outline_small)
+    if constexpr(grouped)
+      ;
+    else if(ctx->outline_small)
       k_outline<OutlineSharedSmall, true, CAM><<<dim3(ctx->outline_gridx, nf), SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words, cam);
     else
       k_outline<OutlineShared, true, CAM><<<dim3(ctx->outline_gridx, nf), OutlineShared::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words, cam);
@@ -535,13 +561,13 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   else
   {
     if(ctx->outline_small)
-      k_outline<OutlineSharedSmall><<<dim3(ctx->outline_gridx, nf), SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
+      k_outline<OutlineSharedSmall><<<dim3(ctx->outline_gridx, nr), SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
     else
-      k_outline<OutlineShared><<<dim3(ctx->outline_gridx, nf), OutlineShared::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
+      k_outline<OutlineShared><<<dim3(ctx->outline_gridx, nr), OutlineShared::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
   }
   STAGE_EV(4);
   if(!fused)
-    k_frame_logic<CAM><<<nf, 32, 0, st>>>(p, frames, nf, cam);
+    k_frame_logic<CAM><<<nr, 32, 0, st>>>(p, frames, nr, cam);
   STAGE_EV(5);
   if(sl)
     k_quad_reduce<SrcLens, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, cam);
@@ -554,17 +580,17 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   {
     const LensCam<CAM> lc = { cam, ov_lens };
     if(ctx->outline_small)
-      k_finalize<OutlineSharedSmall, LensCam<CAM>><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words,
+      k_finalize<OutlineSharedSmall, LensCam<CAM>><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words,
                                                                                              ctx->smem_cap_words, ctx->ov, ovl, lc);
     else
-      k_finalize<OutlineShared, LensCam<CAM>><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words,
+      k_finalize<OutlineShared, LensCam<CAM>><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words,
                                                                                         ctx->smem_cap_words, ctx->ov, ovl, lc);
   }
   else if(ctx->outline_small)
-    k_finalize<OutlineSharedSmall, CAM><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words, ctx->smem_cap_words,
+    k_finalize<OutlineSharedSmall, CAM><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words, ctx->smem_cap_words,
                                                                                ctx->ov, ovl, cam);
   else
-    k_finalize<OutlineShared, CAM><<<nf, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + frame0, bev, ctx->bm_words, ctx->smem_cap_words,
+    k_finalize<OutlineShared, CAM><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words, ctx->smem_cap_words,
                                                                           ctx->ov, ovl, cam);
   STAGE_EV(7);
 #undef STAGE_EV
@@ -589,10 +615,12 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
 // the launch chain for one chunk of frames on one stream
 // ---------------------------------------------------------------------------------------------
 // xyz_dev: packed vertices of the chunk, or nullptr with z16_dev: the chunk's depth frames, deprojected inside the
-// three point kernels (SrcDepth). cam: the camera table of a camera call, else nullptr.
+// three point kernels (SrcDepth). cam: the camera table of a camera call, else nullptr. grp: the group tables of a group call (its
+// cams are *cam), else nullptr; the chunk then holds the whole groups rec0 .. rec0 + nr - 1.
 // sl: the call's lens source (its z16 member is set here), else nullptr; ov_lens: see launch_classic.
-static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uint16_t *z16_dev, float depth_unit, int frame0, int nf, int *launches,
-                        cudaEvent_t *ev, const CamTable *cam, const SrcLens *sl, const ssd_gpu_distortion *ov_lens)
+static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uint16_t *z16_dev, float depth_unit, int frame0, int nf, int rec0,
+                        int nr, int *launches, cudaEvent_t *ev, const CamTable *cam, const GroupTable *grp, const SrcLens *sl,
+                        const ssd_gpu_distortion *ov_lens)
 {
   const DevParams &p = ctx->dp;
   SrcVertices sv;
@@ -609,13 +637,21 @@ static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uin
     sll = *sl;
     sll.z16 = z16_dev;
   }
+  if(grp)
+  {
+    GroupTable g = *grp;
+    g.cams = *cam;
+    g.cams.frame0 = frame0;
+    g.group0 = rec0;
+    return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, rec0, nr, launches, ev, g, ov_lens);
+  }
   if(cam)
   {
     CamTable c = *cam;
     c.frame0 = frame0;
-    return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, launches, ev, c, ov_lens);
+    return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, frame0, nf, launches, ev, c, ov_lens);
   }
-  return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, launches, ev, NoCam(), ov_lens);
+  return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, frame0, nf, launches, ev, NoCam(), ov_lens);
 }
 
 extern "C"
@@ -656,6 +692,9 @@ void ssd_gpu_destroy(ssd_gpu_ctx *ctx)
   cudaFree(ctx->d_cam_yn);
   cudaFree(ctx->d_cam_unit);
   cudaFree(ctx->d_cam_of_frame);
+  cudaFree(ctx->d_grp_of_frame);
+  cudaFree(ctx->d_grp_members);
+  cudaFree(ctx->d_grp_epsc);
   for(float2 *t : ctx->cam_rays)
     cudaFree(t);
   cudaFree(ctx->d_cam_ray);
@@ -739,6 +778,7 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
     if(const char *e = getenv("SSD_GPU_HOST_CHUNK_FRAMES"))
       hc = atoi(e);
     ctx->host_chunk_frames = std::max(1, std::min(hc, cf));
+    ctx->stage_frames = ctx->host_chunk_frames;
   }
 
   {
@@ -773,6 +813,7 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
   cudaFuncSetAttribute(k_transform_bin<SSD_PT_ITERS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SSD_PT_ITERS * SSD_TB_STAGE_BYTES);
   cudaFuncSetAttribute(k_transform_bin<SSD_PT_ITERS, true, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, SSD_PT_ITERS * SSD_TB_STAGE_BYTES);
   cudaFuncSetAttribute(k_transform_bin<SSD_PT_ITERS, false, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, SSD_PT_ITERS * SSD_TB_STAGE_BYTES);
+  cudaFuncSetAttribute(k_transform_bin<SSD_PT_ITERS, false, GroupTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, SSD_PT_ITERS * SSD_TB_STAGE_BYTES);
   if(cudaFuncSetAttribute(k_transform_bin<SSD_PT_ITERS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SSD_PT_ITERS * SSD_TB_STAGE_BYTES) != cudaSuccess)
     return bail("cudaFuncSetAttribute(k_transform_bin) failed", SSD_E_CUDA);
   {
@@ -798,6 +839,11 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
       cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, LensCam<NoCam>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       cudaFuncSetAttribute(k_finalize<OutlineShared, LensCam<CamTable>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, LensCam<CamTable>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      // frame groups (ssd_gpu_process_groups_*)
+      cudaFuncSetAttribute(k_finalize<OutlineShared, GroupTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, GroupTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      cudaFuncSetAttribute(k_finalize<OutlineShared, LensCam<GroupTable>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, LensCam<GroupTable>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       cudaFuncSetAttribute(k_single_front_edge, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       granted = dyn;
     }
@@ -927,8 +973,9 @@ static int ensure_deproject_tables(ssd_gpu_ctx *ctx, const ssd_gpu_intrinsics &i
 
 // xyz != nullptr: packed vertices; else z16 depth frames + intrinsics (deprojected chunk by chunk into the vertex staging)
 // cam_of_frame != nullptr: a camera call (validated by check_cameras; the depth tables are the camera table's, intr is unused)
+// group_frames != nullptr: a group call of n_groups groups (validated by check_groups; a camera call as well)
 static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16, const ssd_gpu_intrinsics *intr, bool host_input, int n_frames,
-                        int flags, const int32_t *cam_of_frame)
+                        int flags, const int32_t *cam_of_frame, const int32_t *group_frames, int n_groups)
 {
   if(!ctx || (!xyz && !(z16 && (intr || cam_of_frame))) || n_frames <= 0)
     return fail(ctx, SSD_E_INVALID_ARG, "process: bad argument");
@@ -980,19 +1027,60 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
     sl.ray = ctx->d_ray;
     sl.unit = intr->depth_unit;
   }
+  // chunks {first frame, frames, first record, records}: cf frames each, or in a group call whole groups up to cf frames (a group
+  // larger than cf is a chunk of its own)
+  struct Chunk
+  {
+    int f0, nf, r0, nr;
+  };
+  std::vector<Chunk> chunks;
+  int max_nf = 0;
+  if(group_frames)
+  {
+    for(int g = 0, f = 0; g < n_groups; f += group_frames[g], g++)
+    {
+      if(chunks.empty() || chunks.back().nf + group_frames[g] > cf)
+        chunks.push_back({ f, 0, g, 0 });
+      chunks.back().nf += group_frames[g];
+      chunks.back().nr++;
+      max_nf = std::max(max_nf, chunks.back().nf);
+    }
+  }
+  else
+    for(int f0 = 0; f0 < n_frames; f0 += cf)
+    {
+      const int nf = std::min(cf, n_frames - f0);
+      chunks.push_back({ f0, nf, f0, nf });
+      max_nf = std::max(max_nf, nf);
+    }
+  const int n_records = group_frames ? n_groups : n_frames;
   // depth frames are deprojected inside the point kernels (SrcDepth): no vertex array is ever written.
   if(host_input)
+  {
+    if(max_nf > ctx->stage_frames)
+    {
+      // a group larger than the host chunk: the staging buffers grow to hold it (no call is in flight between calls)
+      for(int i = 0; i < SSD_MAX_STREAMS; i++)
+      {
+        CK(cudaFree(ctx->d_stage[i]));
+        CK(cudaFree(ctx->d_depth[i]));
+        ctx->d_stage[i] = nullptr;
+        ctx->d_depth[i] = nullptr;
+      }
+      ctx->stage_frames = max_nf;
+    }
     for(int i = 0; i < ctx->n_streams; i++)
     {
       if(depth_input && !ctx->d_depth[i])
-        CK(cudaMalloc(&ctx->d_depth[i], (size_t)ctx->host_chunk_frames * p.N * sizeof(uint16_t)));
+        CK(cudaMalloc(&ctx->d_depth[i], (size_t)ctx->stage_frames * p.N * sizeof(uint16_t)));
       if(!depth_input && !ctx->d_stage[i])
-        CK(cudaMalloc(&ctx->d_stage[i], (size_t)ctx->host_chunk_frames * frame_floats * sizeof(float)));
+        CK(cudaMalloc(&ctx->d_stage[i], (size_t)ctx->stage_frames * frame_floats * sizeof(float)));
     }
+  }
 
   int launches = 0;
   const bool stage_timing = (flags & SSD_FLAG_STAGE_TIMING) != 0;
-  const int n_chunks = (n_frames + cf - 1) / cf;
+  const int n_chunks = (int)chunks.size();
   if(stage_timing && ctx->stage_chunks < n_chunks)
   {
     const size_t want = (size_t)n_chunks * (SSD_GPU_N_STAGES + 1);
@@ -1006,6 +1094,9 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
   }
   ctx->n_frames_last = n_frames;
   ctx->flags_last = flags;
+  ctx->grp_of_frame.clear();
+  ctx->grp_members.clear();
+  ctx->grp_epsc.clear();
   ctx->stats_eps0 = ctx->dp.E0s;
   ctx->stats_eps1 = ctx->dp.E1s;
   CamTable cams{};
@@ -1025,6 +1116,31 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
       ctx->stats_eps1 = std::max(ctx->stats_eps1, (double)d.E1s);
     }
   }
+  GroupTable grp{};
+  if(group_frames)
+  {
+    if(!ctx->d_grp_of_frame)
+    {
+      CK(cudaMalloc(&ctx->d_grp_of_frame, sizeof(int) * (size_t)ctx->max_frames));
+      CK(cudaMalloc(&ctx->d_grp_members, sizeof(int2) * (size_t)ctx->max_frames));
+      CK(cudaMalloc(&ctx->d_grp_epsc, sizeof(float) * (size_t)ctx->max_frames));
+    }
+    // the quadrilateral filters of a group decide the points of all its cameras: the largest of their bounds
+    for(int g = 0, f = 0; g < n_groups; f += group_frames[g], g++)
+    {
+      float e = 0.f;
+      for(int i = 0; i < group_frames[g]; i++)
+      {
+        ctx->grp_of_frame.push_back(g);
+        e = std::max(e, ctx->cam_dp[cam_of_frame[f + i]].epsc); // (an infinite bound stays infinite: every decision is exact)
+      }
+      ctx->grp_members.push_back(make_int2(f, group_frames[g]));
+      ctx->grp_epsc.push_back(e);
+    }
+    grp.group = ctx->d_grp_of_frame;
+    grp.members = ctx->d_grp_members;
+    grp.epsc = ctx->d_grp_epsc;
+  }
   // the whole call is ordered after ev_start on stream 0; stream 1 joins via events
   CK(cudaEventRecord(ctx->ev_start, ctx->stream[0]));
   for(int i = 1; i < ctx->n_streams; i++)
@@ -1033,17 +1149,22 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
   if(host_input)
     CK(cudaEventRecord(ctx->ev_h2d0, ctx->copy_stream));
   // per-frame state: histogram must start at zero
-  CK(cudaMemsetAsync(ctx->d_frames, 0, sizeof(FrameDev) * (size_t)n_frames, ctx->stream[0]));
+  CK(cudaMemsetAsync(ctx->d_frames, 0, sizeof(FrameDev) * (size_t)n_records, ctx->stream[0]));
   if(cam_of_frame)
     CK(cudaMemcpyAsync(ctx->d_cam_of_frame, cam_of_frame, sizeof(int32_t) * (size_t)n_frames, cudaMemcpyHostToDevice, ctx->stream[0]));
+  if(group_frames)
+  {
+    CK(cudaMemcpyAsync(ctx->d_grp_of_frame, ctx->grp_of_frame.data(), sizeof(int) * (size_t)n_frames, cudaMemcpyHostToDevice, ctx->stream[0]));
+    CK(cudaMemcpyAsync(ctx->d_grp_members, ctx->grp_members.data(), sizeof(int2) * (size_t)n_groups, cudaMemcpyHostToDevice, ctx->stream[0]));
+    CK(cudaMemcpyAsync(ctx->d_grp_epsc, ctx->grp_epsc.data(), sizeof(float) * (size_t)n_groups, cudaMemcpyHostToDevice, ctx->stream[0]));
+  }
   CK(cudaEventRecord(ctx->ev_chunk_done[0], ctx->stream[0]));
   for(int i = 1; i < ctx->n_streams; i++)
     CK(cudaStreamWaitEvent(ctx->stream[i], ctx->ev_chunk_done[0], 0));
 
-  int chunk = 0;
-  for(int f0 = 0; f0 < n_frames; f0 += cf, chunk++)
+  for(int chunk = 0; chunk < n_chunks; chunk++)
   {
-    const int nf = std::min(cf, n_frames - f0);
+    const int f0 = chunks[chunk].f0, nf = chunks[chunk].nf;
     const int s = (flags & SSD_FLAG_SINGLE_STREAM) ? 0 : chunk % ctx->n_streams;
     const float *src = depth_input ? nullptr : xyz + (size_t)f0 * frame_floats;
     const uint16_t *dsrc = depth_input ? z16 + (size_t)f0 * p.N : nullptr;
@@ -1065,9 +1186,9 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
       CK(cudaEventRecord(ctx->ev_in_ready[s], ctx->copy_stream));
       CK(cudaStreamWaitEvent(ctx->stream[s], ctx->ev_in_ready[s], 0));
     }
-    const int rc = launch_chunk(ctx, s, src, dsrc, depth_input && intr ? intr->depth_unit : 0.f, f0, nf, &launches,
-                                stage_timing ? &ctx->stage_ev[(size_t)chunk * (SSD_GPU_N_STAGES + 1)] : nullptr, cam_of_frame ? &cams : nullptr,
-                                use_lens ? &sl : nullptr, ov_lens);
+    const int rc = launch_chunk(ctx, s, src, dsrc, depth_input && intr ? intr->depth_unit : 0.f, f0, nf, chunks[chunk].r0, chunks[chunk].nr,
+                                &launches, stage_timing ? &ctx->stage_ev[(size_t)chunk * (SSD_GPU_N_STAGES + 1)] : nullptr,
+                                cam_of_frame ? &cams : nullptr, group_frames ? &grp : nullptr, use_lens ? &sl : nullptr, ov_lens);
     if(rc)
       return rc;
     if(host_input)
@@ -1081,7 +1202,7 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
     CK(cudaEventRecord(ctx->ev_chunk_done[i], ctx->stream[i]));
     CK(cudaStreamWaitEvent(ctx->stream[0], ctx->ev_chunk_done[i], 0));
   }
-  CK(cudaMemcpyAsync(ctx->h_out, ctx->d_out, sizeof(FrameOut) * (size_t)n_frames, cudaMemcpyDeviceToHost, ctx->stream[0]));
+  CK(cudaMemcpyAsync(ctx->h_out, ctx->d_out, sizeof(FrameOut) * (size_t)n_records, cudaMemcpyDeviceToHost, ctx->stream[0]));
   if(ctx->ov.enabled)
     CK(cudaMemcpyAsync(ctx->h_ovl, ctx->d_ovl, sizeof(ssd_gpu_overlay) * SSD_GPU_MAX_STEPS * (size_t)n_frames, cudaMemcpyDeviceToHost, ctx->stream[0]));
   CK(cudaEventRecord(ctx->ev_stop, ctx->stream[0]));
@@ -1124,9 +1245,9 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
 // unsynchronised and BEV bitmaps half written: the bitmaps are "self-cleaning" only along a complete chain. Bring the context
 // back to a clean state so that the next call starts from zeroed bitmaps and no stale results can be read.
 static int process_common(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16, const ssd_gpu_intrinsics *intr, bool host_input, int n_frames,
-                          int flags, const int32_t *cam_of_frame = nullptr)
+                          int flags, const int32_t *cam_of_frame = nullptr, const int32_t *group_frames = nullptr, int n_groups = 0)
 {
-  const int rc = process_impl(ctx, xyz, z16, intr, host_input, n_frames, flags, cam_of_frame);
+  const int rc = process_impl(ctx, xyz, z16, intr, host_input, n_frames, flags, cam_of_frame, group_frames, n_groups);
   if(rc != SSD_OK && rc != SSD_E_INVALID_ARG && rc != SSD_E_RANGE && ctx)
   {
     const std::string keep = ctx->err;
@@ -1440,6 +1561,60 @@ int ssd_gpu_process_depth_cameras_device(ssd_gpu_ctx *ctx, const uint16_t *z16_d
   return rc ? rc : process_common(ctx, nullptr, z16_dev, nullptr, false, n_frames, 0, camera_of_frame);
 }
 
+// Everything a group call can be refused for, before anything is launched (the previous results stay readable). *n_frames: the
+// call's frames.
+static int check_groups(ssd_gpu_ctx *ctx, const void *input, const int32_t *cam_of_frame, const int32_t *group_frames, int n_groups, bool depth,
+                        int *n_frames)
+{
+  if(!ctx || !input || !cam_of_frame || !group_frames || n_groups < 1)
+    return fail(ctx, SSD_E_INVALID_ARG, "group call: bad argument");
+  long long total = 0;
+  for(int g = 0; g < n_groups; g++)
+  {
+    if(group_frames[g] < 1 || group_frames[g] > SSD_GPU_MAX_GROUP_FRAMES)
+      return fail(ctx, SSD_E_INVALID_ARG, "group call: group " + std::to_string(g) + " has " + std::to_string(group_frames[g]) +
+                                              " frames, outside [1, " + std::to_string(SSD_GPU_MAX_GROUP_FRAMES) + "]");
+    total += group_frames[g];
+  }
+  if(ctx->n_cameras <= 0)
+    return fail(ctx, SSD_E_STATE, "group call: no camera table (ssd_gpu_set_cameras)");
+  if(total > ctx->max_frames)
+    return fail(ctx, SSD_E_RANGE, "group call: the groups hold " + std::to_string(total) + " frames, more than max_frames of the context");
+  *n_frames = (int)total;
+  return check_cameras(ctx, input, cam_of_frame, (int)total, depth);
+}
+
+int ssd_gpu_process_groups_host(ssd_gpu_ctx *ctx, const float *xyz_host, const int32_t *camera_of_frame, const int32_t *group_frames, int n_groups)
+{
+  int n = 0;
+  const int rc = check_groups(ctx, xyz_host, camera_of_frame, group_frames, n_groups, false, &n);
+  return rc ? rc : process_common(ctx, xyz_host, nullptr, nullptr, true, n, 0, camera_of_frame, group_frames, n_groups);
+}
+
+int ssd_gpu_process_groups_device(ssd_gpu_ctx *ctx, const float *xyz_dev, const int32_t *camera_of_frame, const int32_t *group_frames, int n_groups,
+                                  int flags)
+{
+  int n = 0;
+  const int rc = check_groups(ctx, xyz_dev, camera_of_frame, group_frames, n_groups, false, &n);
+  return rc ? rc : process_common(ctx, xyz_dev, nullptr, nullptr, false, n, flags, camera_of_frame, group_frames, n_groups);
+}
+
+int ssd_gpu_process_depth_groups_host(ssd_gpu_ctx *ctx, const uint16_t *z16_host, const int32_t *camera_of_frame, const int32_t *group_frames,
+                                      int n_groups)
+{
+  int n = 0;
+  const int rc = check_groups(ctx, z16_host, camera_of_frame, group_frames, n_groups, true, &n);
+  return rc ? rc : process_common(ctx, nullptr, z16_host, nullptr, true, n, 0, camera_of_frame, group_frames, n_groups);
+}
+
+int ssd_gpu_process_depth_groups_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const int32_t *camera_of_frame, const int32_t *group_frames,
+                                        int n_groups, int flags)
+{
+  int n = 0;
+  const int rc = check_groups(ctx, z16_dev, camera_of_frame, group_frames, n_groups, true, &n);
+  return rc ? rc : process_common(ctx, nullptr, z16_dev, nullptr, false, n, flags, camera_of_frame, group_frames, n_groups);
+}
+
 int ssd_gpu_deproject_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const ssd_gpu_intrinsics *intr, int n_frames, float *xyz_dev)
 {
   if(!ctx || !z16_dev || !intr || !xyz_dev || n_frames <= 0)
@@ -1483,7 +1658,7 @@ int ssd_gpu_get_steps(ssd_gpu_ctx *ctx, int frame, ssd_gpu_step *out, int cap, i
   const int rc = check_frame(ctx, frame);
   if(rc)
     return rc;
-  const FrameOut &o = ctx->h_out[frame];
+  const FrameOut &o = ctx->h_out[frame_record(ctx, frame)];
   if(n)
     *n = o.info.n_steps;
   if(status)
@@ -1532,7 +1707,7 @@ int ssd_gpu_get_overlay(ssd_gpu_ctx *ctx, int frame, ssd_gpu_overlay *out, int c
     return rc;
   if(!ctx->ov.enabled || !ctx->h_ovl)
     return fail(ctx, SSD_E_STATE, "ssd_gpu_get_overlay: overlay not enabled (ssd_gpu_set_overlay)");
-  const int ns = ctx->h_out[frame].info.n_steps;
+  const int ns = ctx->h_out[frame_record(ctx, frame)].info.n_steps;
   if(n)
     *n = ns;
   if(out)
@@ -1558,11 +1733,12 @@ int ssd_gpu_get_vertical_faces(ssd_gpu_ctx *ctx, int frame, ssd_gpu_riser *out, 
   if(!ctx->risers)
     return fail(ctx, SSD_E_STATE, "ssd_gpu_get_vertical_faces: not enabled (ssd_gpu_set_vertical_faces)");
   CK(cudaSetDevice(ctx->device));
+  const int r = frame_record(ctx, frame);
   std::vector<PlateauDev> pl(SSD_GPU_MAX_PLATEAUS);
   std::vector<RiserDev> rs(SSD_GPU_MAX_PLATEAUS);
-  CK(cudaMemcpy(pl.data(), ctx->d_frames[frame].plat, sizeof(PlateauDev) * SSD_GPU_MAX_PLATEAUS, cudaMemcpyDeviceToHost));
-  CK(cudaMemcpy(rs.data(), ctx->d_frames[frame].ris, sizeof(RiserDev) * SSD_GPU_MAX_PLATEAUS, cudaMemcpyDeviceToHost));
-  const int K = ctx->h_out[frame].info.n_plateaus;
+  CK(cudaMemcpy(pl.data(), ctx->d_frames[r].plat, sizeof(PlateauDev) * SSD_GPU_MAX_PLATEAUS, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(rs.data(), ctx->d_frames[r].ris, sizeof(RiserDev) * SSD_GPU_MAX_PLATEAUS, cudaMemcpyDeviceToHost));
+  const int K = ctx->h_out[r].info.n_plateaus;
   const int R = K > 1 ? K - 1 : 0;
   if(n)
     *n = R;
@@ -1596,7 +1772,7 @@ int ssd_gpu_get_frame_info(ssd_gpu_ctx *ctx, int frame, ssd_gpu_frame_info *out)
     return rc;
   if(!out)
     return SSD_E_INVALID_ARG;
-  *out = ctx->h_out[frame].info;
+  *out = ctx->h_out[frame_record(ctx, frame)].info;
   return SSD_OK;
 }
 
@@ -1606,9 +1782,10 @@ int ssd_gpu_get_plateaus(ssd_gpu_ctx *ctx, int frame, ssd_gpu_plateau *out, int 
   if(rc)
     return rc;
   CK(cudaSetDevice(ctx->device));
+  const int r = frame_record(ctx, frame);
   std::vector<PlateauDev> tmp(SSD_GPU_MAX_PLATEAUS);
-  CK(cudaMemcpy(tmp.data(), ctx->d_frames[frame].plat, sizeof(PlateauDev) * SSD_GPU_MAX_PLATEAUS, cudaMemcpyDeviceToHost));
-  const int K = ctx->h_out[frame].info.n_plateaus;
+  CK(cudaMemcpy(tmp.data(), ctx->d_frames[r].plat, sizeof(PlateauDev) * SSD_GPU_MAX_PLATEAUS, cudaMemcpyDeviceToHost));
+  const int K = ctx->h_out[r].info.n_plateaus;
   if(n)
     *n = K;
   for(int k = 0; k < K && k < cap && out; k++)
@@ -1648,7 +1825,7 @@ int ssd_gpu_get_histogram(ssd_gpu_ctx *ctx, int frame, uint32_t *out, int cap, i
     return rc;
   CK(cudaSetDevice(ctx->device));
   uint32_t tmp[SSD_BINS_PAD];
-  CK(cudaMemcpy(tmp, ctx->d_frames[frame].hist, sizeof(tmp), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(tmp, ctx->d_frames[frame_record(ctx, frame)].hist, sizeof(tmp), cudaMemcpyDeviceToHost));
   if(n_bins)
     *n_bins = ctx->dp.n_bins;
   for(int i = 0; i < ctx->dp.n_bins && i < cap && out; i++)
@@ -1669,7 +1846,7 @@ int ssd_gpu_get_stats(ssd_gpu_ctx *ctx, ssd_gpu_stats *out)
   if(!ctx || !out)
     return SSD_E_INVALID_ARG;
   uint64_t c[4] = { 0, 0, 0, 0 };
-  for(int f = 0; f < ctx->n_frames_last; f++)
+  for(int f = 0; f < n_records_last(ctx); f++)
   {
     const FrameOut &o = ctx->h_out[f];
     c[0] += o.n_exact_bin;

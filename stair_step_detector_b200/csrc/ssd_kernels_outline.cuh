@@ -8,6 +8,7 @@
 // the global bitmap is zeroed behind the read so it is clean for the next batch.
 #pragma once
 #include "ssd_device.cuh"
+#include <type_traits>
 #ifdef SSD_OL_PROF
 #include <cstdio>
 #endif
@@ -1366,8 +1367,74 @@ __global__ void __launch_bounds__(32) k_frame_logic(const __grid_constant__ DevP
   const int f = blockIdx.x;
   if(f >= n_frames)
     return;
-  const DevParams &p = frame_params(p0, cam, f);
+  const DevParams &p = group_params(p0, cam, f);
   frame_logic_warp(p, frames[f], Sc, threadIdx.x);
+}
+
+// the lenses of a group call's overlay (LensCam<GroupTable>), or none (pin-hole)
+__device__ __forceinline__ const ssd_gpu_distortion *group_lens(const GroupTable &)
+{
+  return nullptr;
+}
+__device__ __forceinline__ const ssd_gpu_distortion *group_lens(const LensCam<GroupTable> &c)
+{
+  return c.lens;
+}
+// A group's steps into the overlay of every member frame, each through its own camera (b, a_inv, intrinsics, lens).
+template<class GCAM>
+__device__ __forceinline__ void group_overlay(const GroupTable &g, const GCAM &cam, int slot, const double (*sq)[4][3], int nSteps,
+                                              ssd_gpu_overlay *__restrict__ overlay)
+{
+  const int2 m = group_members(g, slot);
+  for(int i = 0; i < m.y; i++)
+  {
+    const int frame = m.x + i - g.cams.frame0; // within the launch
+    const int c = frame_camera(g.cams, frame);
+    double b[3];
+    for(int j = 0; j < 3; j++)
+      b[j] = g.cams.params[c].b[j];
+    const OverlayDev &ov = g.cams.ov[c];
+    ssd_gpu_overlay *Q = overlay + (size_t)frame * SSD_GPU_MAX_STEPS;
+    for(int s = 0; s < nSteps; s++)
+      for(int k = 0; k < 4; k++)
+      {
+        const double dx = sq[s][k][0] - b[0], dy = sq[s][k][1] - b[1], dz = sq[s][k][2] - b[2];
+        const float X = (float)((ov.a_inv[0] * dx + ov.a_inv[1] * dy) + ov.a_inv[2] * dz);
+        const float Y = (float)((ov.a_inv[3] * dx + ov.a_inv[4] * dy) + ov.a_inv[5] * dz);
+        const float Z = (float)((ov.a_inv[6] * dx + ov.a_inv[7] * dy) + ov.a_inv[8] * dz);
+        float x = __fdiv_rn(X, Z), y = __fdiv_rn(Y, Z);
+        if constexpr(!std::is_same<GCAM, GroupTable>::value)
+        {
+          const ssd_gpu_distortion d = group_lens(cam)[c];
+          float xd, yd;
+          ssd_lens_project(&d, x, y, &xd, &yd);
+          x = xd;
+          y = yd;
+        }
+        Q[s].px[k][0] = __fadd_rn(__fmul_rn(x, ov.fx), ov.ppx);
+        Q[s].px[k][1] = __fadd_rn(__fmul_rn(y, ov.fy), ov.ppy);
+      }
+  }
+}
+template<class CAM>
+struct IsGroupCam : std::false_type
+{
+};
+template<>
+struct IsGroupCam<GroupTable> : std::true_type
+{
+};
+template<>
+struct IsGroupCam<LensCam<GroupTable>> : std::true_type
+{
+};
+__device__ __forceinline__ const GroupTable &group_table(const GroupTable &c)
+{
+  return c;
+}
+__device__ __forceinline__ const GroupTable &group_table(const LensCam<GroupTable> &c)
+{
+  return c.base;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1386,7 +1453,7 @@ __global__ void __launch_bounds__(SSD_OL_THREADS, SSD_OL_MINB) k_finalize(const 
   __shared__ Band bd;
   __shared__ int s_smem_path;
   const int frame = blockIdx.x, tid = threadIdx.x;
-  const DevParams &p = frame_params(p0, cam, frame);
+  const DevParams &p = group_params(p0, cam, frame);
   const OverlayDev &ov = frame_overlay(ov0, cam, frame);
   FrameDev &F = frames[frame];
   FrameOut &O = out[frame];
@@ -1501,7 +1568,12 @@ __global__ void __launch_bounds__(SSD_OL_THREADS, SSD_OL_MINB) k_finalize(const 
     }
     O.steps[s].height = p.ext_z + sq[s][0][2];
   }
-  if(ov.enabled)
+  if constexpr(IsGroupCam<CAM>::value)
+  {
+    if(ov.enabled)
+      group_overlay(group_table(cam), cam, frame, sq, nSteps, overlay);
+  }
+  else if(ov.enabled)
   {
     // drawStairStep (pointcloud.cpp:588-597): quadriWorld -> worldToCamera -> DepthFrame::project
     ssd_gpu_overlay *Q = overlay + (size_t)frame * SSD_GPU_MAX_STEPS;
@@ -1526,8 +1598,8 @@ __global__ void __launch_bounds__(SSD_OL_THREADS, SSD_OL_MINB) k_finalize(const 
   O.info.ground_index = ground;
   O.info.first_valid_index = firstValid;
   O.info.n_steps = nSteps;
-  O.info.n_nonzero = F.n_nonzero;
-  O.info.n_in_range = F.n_in_range;
+  O.info.n_nonzero = F.n_nonzero + group_extra_points(cam, frame, (unsigned)p.N);
+  O.info.n_in_range = F.n_in_range + group_extra_points(cam, frame, (unsigned)p.N);
   O.n_exact_bin = F.n_exact_bin;
   {
     // points tested against a quadrilateral: every point of the ground and of the valid plateaus (k_quad_reduce)

@@ -222,6 +222,11 @@ __device__ __forceinline__ SrcDepth frame_src(const SrcDepth &s, const CamTable 
   d.unit = __ldg(c.unit + cam);
   return d;
 }
+template<class SRC>
+__device__ __forceinline__ SRC frame_src(const SRC &s, const GroupTable &g, const DevParams &p, int frame)
+{
+  return frame_src(s, g.cams, p, frame);
+}
 __device__ __forceinline__ void word_zero(WordV &r)
 {
   r.a = r.b = r.c = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -668,14 +673,14 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin(const __grid_c
   __syncthreads();
   const unsigned sum = s_hist[tid];
   if(sum)
-    atomicAdd(&frames[frame].hist[tid], sum);
+    atomicAdd(&frames[frame_slot(cam, frame)].hist[tid], sum);
   if(tid == 0 && s_exact)
-    atomicAdd(&frames[frame].n_exact_bin, s_exact);
+    atomicAdd(&frames[frame_slot(cam, frame)].n_exact_bin, s_exact);
   if(FUSE_PEAKS)
   {
     __shared__ PeaksScratch K;
     __shared__ unsigned s_last;
-    tb_fused_peaks(p, frames[frame], K, s_last, tid);
+    tb_fused_peaks(p, frames[frame_slot(cam, frame)], K, s_last, tid);
   }
 }
 
@@ -726,14 +731,14 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_depth(const __
   __syncthreads();
   const unsigned sum = s_hist[tid];
   if(sum)
-    atomicAdd(&frames[frame].hist[tid], sum);
+    atomicAdd(&frames[frame_slot(cam, frame)].hist[tid], sum);
   if(tid == 0 && s_exact)
-    atomicAdd(&frames[frame].n_exact_bin, s_exact);
+    atomicAdd(&frames[frame_slot(cam, frame)].n_exact_bin, s_exact);
   if(FUSE_PEAKS)
   {
     __shared__ PeaksScratch K;
     __shared__ unsigned s_last;
-    tb_fused_peaks(p, frames[frame], K, s_last, tid);
+    tb_fused_peaks(p, frames[frame_slot(cam, frame)], K, s_last, tid);
   }
 }
 // k_transform_bin_lens: the same pass on z16 frames of a distorted lens (SrcLens), 10 bytes per point in (2 of depth, 8 of ray
@@ -780,14 +785,14 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_lens(const __g
   __syncthreads();
   const unsigned sum = s_hist[tid];
   if(sum)
-    atomicAdd(&frames[frame].hist[tid], sum);
+    atomicAdd(&frames[frame_slot(cam, frame)].hist[tid], sum);
   if(tid == 0 && s_exact)
-    atomicAdd(&frames[frame].n_exact_bin, s_exact);
+    atomicAdd(&frames[frame_slot(cam, frame)].n_exact_bin, s_exact);
   if(FUSE_PEAKS)
   {
     __shared__ PeaksScratch K;
     __shared__ unsigned s_last;
-    tb_fused_peaks(p, frames[frame], K, s_last, tid);
+    tb_fused_peaks(p, frames[frame_slot(cam, frame)], K, s_last, tid);
   }
 }
 
@@ -911,10 +916,11 @@ __global__ void __launch_bounds__(SSD_PT_THREADS, SSD_LB_MINB) k_label_bev(const
   const int frame = blockIdx.y;
   const DevParams &p = frame_params(p0, cam, frame);
   const auto &src = frame_src(src0, cam, p, frame);
-  FrameDev &F = frames[frame];
+  FrameDev &F = frames[frame_slot(cam, frame)];
   const size_t fbase = (size_t)frame * p.N;
   unsigned *lab32 = reinterpret_cast<unsigned *>(labels + fbase);
-  unsigned *fbev = bev + (size_t)frame * SSD_GPU_MAX_PLATEAUS * bm_words;
+  const int slot = frame_slot(cam, frame);
+  unsigned *fbev = bev + (size_t)slot * SSD_GPU_MAX_PLATEAUS * bm_words;
   const typename SrcTraits<SRC>::Frame FR = src_frame(src, p, fbase);
   const int nquads = p.N >> 2;
   int wt, wt_end, wt_stride;
@@ -1019,7 +1025,7 @@ __global__ void __launch_bounds__(SSD_PT_THREADS, SSD_LB_MINB) k_label_bev(const
       {
         // word index of the plateau's bitmap within the stream's BEV buffer: 32-bit (the buffer holds < 2^32 words, see
         // ssd_gpu_create), so a reduction's address is one widening multiply-add on the kernel's base pointer
-        unsigned lidx = ((unsigned)frame * SSD_GPU_MAX_PLATEAUS + l0) * bmw;
+        unsigned lidx = ((unsigned)slot * SSD_GPU_MAX_PLATEAUS + l0) * bmw;
         asm volatile("" : "+r"(lidx)); // keep it in a register: the compiler otherwise recomputes it inside every predicated reduction
 #pragma unroll
         for(int j = 0; j < 4; j++)
@@ -1498,14 +1504,14 @@ __global__ void __launch_bounds__(SSD_PT_THREADS, SSD_QR_MINB) k_quad_reduce(con
   const int frame = blockIdx.y;
   const DevParams &p = frame_params(p0, cam, frame);
   const auto &src = frame_src(src0, cam, p, frame);
-  FrameDev &F = frames[frame];
+  FrameDev &F = frames[frame_slot(cam, frame)];
   const unsigned amask = F.quad_amask;
   if(amask == 0u)
     return; // no valid plateau: nothing is emitted (pointcloud.cpp:434)
   const int ground = F.ground_index;
   const size_t fbase = (size_t)frame * p.N;
   const unsigned *lab32 = reinterpret_cast<const unsigned *>(labels + fbase);
-  unsigned *gbev = ground >= 0 ? bev + ((size_t)frame * SSD_GPU_MAX_PLATEAUS + ground) * bm_words : nullptr;
+  unsigned *gbev = ground >= 0 ? bev + ((size_t)frame_slot(cam, frame) * SSD_GPU_MAX_PLATEAUS + ground) * bm_words : nullptr;
   const int nquads = p.N >> 2;
   int wt, wt_end, wt_stride;
   warp_tile_range((p.N + SSD_WT_PX - 1) / SSD_WT_PX, warp, wt, wt_end, wt_stride);
@@ -1612,7 +1618,7 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_riser_reduce(const __grid_co
   const int frame = blockIdx.y;
   const DevParams &p = frame_params(p0, cam, frame);
   const auto &src = frame_src(src0, cam, p, frame);
-  FrameDev &F = frames[frame];
+  FrameDev &F = frames[frame_slot(cam, frame)];
   const int K = F.n_plateaus;
   if(K < 2)
     return;
