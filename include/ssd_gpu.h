@@ -356,6 +356,32 @@ typedef struct ssd_gpu_riser
 int ssd_gpu_set_vertical_faces(ssd_gpu_ctx *ctx, int enable);
 /* out[0..min(*n, cap)): *n = max(0, n_plateaus - 1) risers of the frame, ascending. */
 int ssd_gpu_get_vertical_faces(ssd_gpu_ctx *ctx, int frame, ssd_gpu_riser *out, int cap, int *n);
+/*
+ * Step labels: which pixels each step stands on. For frame f of the last call, step_labels[f][i] (u8 per pixel, row-major
+ * like the segment labels) is
+ *   s (0 <= s < n_steps) when pixel i's point is one of the points whose z step s of ssd_gpu_get_steps(f) averages: the set
+ *     StairsDetector::getPointsInQuadrilateral (pointcloud.cpp:560-572) returns for that step and calcAverageZ (:574-581)
+ *     averages, decided on the exact double-precision world point (CameraToWorld, QuadrilateralTest::isPointWithin). For a
+ *     plateau step (calcStairStep, :549-558) the points of that plateau inside its quadrilateral; for the ground step
+ *     (calcGround, :528-547) the points of the ground plateau inside the ground quadrilateral (calcGroundQuadrilateral) --
+ *     also when the front edge is invalid and the step is the all-zero one (SSD_STATUS_INVALID_FRONT_EDGE): the reference
+ *     computes the set either way, and the status bit says that the step's corners are not usable;
+ *   SSD_STEP_LABEL_NONE for every other pixel: frames without steps, plateaus dropped as SSD_STATUS_DEGENERATE_QUAD, the
+ *     points of a plateau outside its quadrilateral, invalid, out-of-range and remainder pixels.
+ * So count(step_labels == s) is n_in_quad of the step's plateau, step_labels == s implies that the pixel's segment label is
+ * that plateau, and a step with SSD_STATUS_EMPTY_MEAN has no pixels. In group calls each member frame's step labels index its
+ * group's steps, its pixels tested through its own camera (as its segment labels index the group's plateaus).
+ * Off until enabled; enable != 0 applies to the following ssd_gpu_process_* calls (every entry point) and allocates
+ * max_frames * width*height bytes (SSD_E_NOMEM, and the option stays off, when that fails); enable == 0 frees them. The
+ * getters return SSD_E_STATE when the option is off or the last call ran without it, SSD_E_RANGE for a frame outside the
+ * last call. With the option off nothing changes: the same kernels, launches and results.
+ */
+#define SSD_STEP_LABEL_NONE 255u
+int ssd_gpu_set_step_labels(ssd_gpu_ctx *ctx, int enable);
+/* device -> host copy of frame's width*height step labels */
+int ssd_gpu_get_step_labels(ssd_gpu_ctx *ctx, int frame, uint8_t *out_host);
+/* Device pointer to the step labels of the last call (n_frames * width*height bytes). */
+int ssd_gpu_step_labels_device_ptr(ssd_gpu_ctx *ctx, const uint8_t **out);
 /* Per-pixel segment labels (device -> host copy of width*height bytes). */
 int ssd_gpu_get_labels(ssd_gpu_ctx *ctx, int frame, uint8_t *out_host);
 /* Height histogram, HeightsHistogram::calcHist (pointcloud.cpp:194-204). */

@@ -391,6 +391,23 @@ class Detector:
         self._ck(self._l.ssd_gpu_get_vertical_faces(self._h, frame, out, A.MAX_PLATEAUS, C.byref(n)), "ssd_gpu_get_vertical_faces")
         return [{f: getattr(r, f) for f, _ in A.Riser._fields_ if f != "pad"} for r in out[:n.value]]
 
+    def set_step_labels(self, enable=True):
+        """Step labels (include/ssd_gpu.h: ssd_gpu_set_step_labels): per pixel the step of steps(frame) whose height its point
+        is averaged into, or STEP_LABEL_NONE (255). Applies to the following process calls; allocates max_frames frames of bytes."""
+        self._ck(self._l.ssd_gpu_set_step_labels(self._h, 1 if enable else 0), "ssd_gpu_set_step_labels")
+
+    def step_labels(self, frame):
+        """(n_points,) uint8 step labels of the frame, row-major like labels(frame)."""
+        out = np.empty(self.n_points, np.uint8)
+        self._ck(self._l.ssd_gpu_get_step_labels(self._h, frame, _ptr(out)), "ssd_gpu_get_step_labels")
+        return out
+
+    def step_labels_device_ptr(self):
+        """Device address of the last call's step labels (n_frames * n_points bytes, frame-major)."""
+        p = C.c_void_p()
+        self._ck(self._l.ssd_gpu_step_labels_device_ptr(self._h, C.byref(p)), "ssd_gpu_step_labels_device_ptr")
+        return p.value
+
     def n_steps_all(self, n_frames):
         out = np.empty(n_frames, np.int32)
         n = C.c_int()

@@ -14,6 +14,7 @@ MAX_GROUP_FRAMES = 32  # members of one frame group (ssd_gpu_process_groups_*)
 LABEL_REMAINDER = 253
 LABEL_OUT_OF_RANGE = 254
 LABEL_INVALID = 255
+STEP_LABEL_NONE = 255  # step labels: pixel on no step (ssd_gpu_set_step_labels)
 
 OK = 0
 E_INVALID_ARG, E_CUDA, E_NOMEM, E_RANGE, E_STATE = -1, -2, -3, -4, -5
@@ -154,6 +155,9 @@ PROTOTYPES = {
     "ssd_gpu_get_overlay": (C.c_int, [_vp, C.c_int, _P(Overlay), C.c_int, _P(C.c_int)]),
     "ssd_gpu_set_vertical_faces": (C.c_int, [_vp, C.c_int]),
     "ssd_gpu_get_vertical_faces": (C.c_int, [_vp, C.c_int, _P(Riser), C.c_int, _P(C.c_int)]),
+    "ssd_gpu_set_step_labels": (C.c_int, [_vp, C.c_int]),
+    "ssd_gpu_get_step_labels": (C.c_int, [_vp, C.c_int, _vp]),
+    "ssd_gpu_step_labels_device_ptr": (C.c_int, [_vp, _P(_vp)]),
     "ssd_gpu_get_frame_info": (C.c_int, [_vp, C.c_int, _P(FrameInfo)]),
     "ssd_gpu_get_plateaus": (C.c_int, [_vp, C.c_int, _P(Plateau), C.c_int, _P(C.c_int)]),
     "ssd_gpu_get_labels": (C.c_int, [_vp, C.c_int, _vp]),

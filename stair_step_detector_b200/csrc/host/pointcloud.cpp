@@ -69,7 +69,7 @@ std::vector<Quadrilateralf_t> Pointcloud::overlay(int frame) const
   return out;
 }
 
-// overlay / vertical faces / camera table as last requested, once the context exists
+// overlay / vertical faces / step labels / camera table as last requested, once the context exists
 void Pointcloud::applySettings() const
 {
   if(_overlay && !_overlayApplied)
@@ -85,6 +85,12 @@ void Pointcloud::applySettings() const
     if(ssd_gpu_set_vertical_faces(_ctx, _risers ? 1 : 0) != SSD_OK)
       throw std::runtime_error(std::string("ssd_gpu_set_vertical_faces: ") + ssd_gpu_last_error(_ctx));
     _risersApplied = _risers;
+  }
+  if(_stepLabels != _stepLabelsApplied)
+  {
+    if(ssd_gpu_set_step_labels(_ctx, _stepLabels ? 1 : 0) != SSD_OK)
+      throw std::runtime_error(std::string("ssd_gpu_set_step_labels: ") + ssd_gpu_last_error(_ctx));
+    _stepLabelsApplied = _stepLabels;
   }
   if(!_camerasApplied)
   {
@@ -255,6 +261,21 @@ std::vector<ssd_gpu_riser> Pointcloud::verticalFaces(int frame) const
   if(ssd_gpu_get_vertical_faces(_ctx, frame, r, SSD_GPU_MAX_PLATEAUS, &n) != SSD_OK)
     throw std::runtime_error(std::string("ssd_gpu_get_vertical_faces: ") + ssd_gpu_last_error(_ctx));
   return std::vector<ssd_gpu_riser>(r, r + n);
+}
+
+void Pointcloud::enableStepLabels(bool enable) const
+{
+  _stepLabels = enable;
+}
+
+std::vector<uint8_t> Pointcloud::stepLabels(int frame) const
+{
+  if(!_ctx)
+    throw std::logic_error("Pointcloud::stepLabels before any frame was processed");
+  std::vector<uint8_t> l(static_cast<size_t>(_config.streams.depth.width) * _config.streams.depth.height);
+  if(ssd_gpu_get_step_labels(_ctx, frame, l.data()) != SSD_OK)
+    throw std::runtime_error(std::string("ssd_gpu_get_step_labels: ") + ssd_gpu_last_error(_ctx));
+  return l;
 }
 
 std::vector<uint8_t> Pointcloud::labels(int frame) const

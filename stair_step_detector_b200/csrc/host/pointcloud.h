@@ -65,6 +65,10 @@ public:
   // (pointcloud.cpp:293); definition: include/ssd_gpu.h, ssd_gpu_riser. One more pass over the points when enabled.
   void enableVerticalFaces(bool enable = true) const;
   std::vector<ssd_gpu_riser> verticalFaces(int frame = 0) const;
+  // step labels: per pixel the index of the step whose height its point is averaged into (getPointsInQuadrilateral,
+  // pointcloud.cpp:560-572), SSD_STEP_LABEL_NONE elsewhere; definition: include/ssd_gpu.h, ssd_gpu_set_step_labels
+  void enableStepLabels(bool enable = true) const;
+  std::vector<uint8_t> stepLabels(int frame = 0) const;
   ssd_gpu_ctx *context() const { return _ctx; }
 
 private:
@@ -79,6 +83,7 @@ private:
   mutable bool _explicitConfig = false;
   mutable bool _overlay = false, _overlayApplied = false;
   mutable bool _risers = false, _risersApplied = false;
+  mutable bool _stepLabels = false, _stepLabelsApplied = false;
   mutable ssd_gpu_intrinsics _overlayIntrinsics{};
   mutable ssd_gpu_distortion _overlayDistortion{}, _lensApplied{};
   mutable std::vector<ssd_gpu_camera> _cameras;

@@ -59,6 +59,9 @@ struct ssd_gpu_ctx
   float *d_xn = nullptr, *d_yn = nullptr;       // deprojection tables: (u - ppx) / fx per column, (v - ppy) / fy per row
   ssd_gpu_intrinsics intr{};                    // intrinsics the tables were built for
   bool risers = false;            // ssd_gpu_set_vertical_faces: k_riser_reduce after the chain
+  unsigned char *d_step_labels = nullptr; // max_frames * N, allocated by ssd_gpu_set_step_labels
+  bool step_labels = false;       // ssd_gpu_set_step_labels: k_quad_reduce's STEPS variant writes d_step_labels
+  bool step_labels_last = false;  // the last accepted process call wrote them
   int pt_blocks_target = 0;       // blocks per launch of the tile-looping point kernels
   int n_frames_last = 0;
   int flags_last = 0;
@@ -569,12 +572,26 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   if(!fused)
     k_frame_logic<CAM><<<nr, 32, 0, st>>>(p, frames, nr, cam);
   STAGE_EV(5);
-  if(sl)
-    k_quad_reduce<SrcLens, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, cam);
-  else if(depth)
-    k_quad_reduce<SrcDepth, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, cam);
+  const auto quad_reduce = [&](auto so) {
+    constexpr bool STEPS = std::is_same<decltype(so), StepLabelsOut<true>>::value;
+    if(sl)
+      k_quad_reduce<SrcLens, CAM, STEPS><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, cam, so);
+    else if(depth)
+      k_quad_reduce<SrcDepth, CAM, STEPS><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, cam, so);
+    else
+      k_quad_reduce<SrcVertices, CAM, STEPS><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, cam, so);
+  };
+  if(ctx->step_labels)
+  {
+    // step labels: the chunk's slice starts as SSD_STEP_LABEL_NONE (words without counted points, labels outside quad_amask and
+    // frames without steps are never written by k_quad_reduce). The memset is part of the quad_reduce stage's time and is not
+    // counted in timing.n_launches (a copy-engine / driver fill, not one of the chain's kernels).
+    unsigned char *steps = ctx->d_step_labels + (size_t)frame0 * p.N;
+    CK(cudaMemsetAsync(steps, SSD_STEP_LABEL_NONE, (size_t)nf * p.N, st));
+    quad_reduce(StepLabelsOut<true>{ steps });
+  }
   else
-    k_quad_reduce<SrcVertices, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, cam);
+    quad_reduce(StepLabelsOut<false>());
   STAGE_EV(6);
   if(ov_lens)
   {
@@ -682,6 +699,7 @@ void ssd_gpu_destroy(ssd_gpu_ctx *ctx)
   cudaFree(ctx->d_ovl);
   cudaFreeHost(ctx->h_ovl);
   cudaFree(ctx->d_labels);
+  cudaFree(ctx->d_step_labels);
   cudaFree(ctx->d_bev);
   cudaFree(ctx->d_img);
   cudaFree(ctx->d_xn);
@@ -1094,6 +1112,7 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
   }
   ctx->n_frames_last = n_frames;
   ctx->flags_last = flags;
+  ctx->step_labels_last = ctx->step_labels;
   ctx->grp_of_frame.clear();
   ctx->grp_members.clear();
   ctx->grp_epsc.clear();
@@ -1256,6 +1275,7 @@ static int process_common(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z1
     if(ctx->d_bev)
       cudaMemset(ctx->d_bev, 0, (size_t)ctx->n_streams * ctx->chunk_frames * SSD_GPU_MAX_PLATEAUS * ctx->bm_words * 4);
     ctx->n_frames_last = 0;
+    ctx->step_labels_last = false;
     ctx->err = keep;
   }
   return rc;
@@ -1762,6 +1782,72 @@ int ssd_gpu_get_vertical_faces(ssd_gpu_ctx *ctx, int frame, ssd_gpu_riser *out, 
     }
     out[k] = o;
   }
+  return SSD_OK;
+}
+
+int ssd_gpu_set_step_labels(ssd_gpu_ctx *ctx, int enable)
+{
+  if(!ctx)
+    return SSD_E_INVALID_ARG;
+  CK(cudaSetDevice(ctx->device));
+  if((enable != 0) != ctx->step_labels)
+    ctx->step_labels_last = false; // the map of an earlier call is not kept across a switch
+  if(!enable)
+  {
+    // the pointer and the flag are cleared whatever the free returns: a failed free must not leave a pointer to free again
+    const cudaError_t e = cudaFree(ctx->d_step_labels);
+    ctx->d_step_labels = nullptr;
+    ctx->step_labels = false;
+    if(e != cudaSuccess)
+      return fail(ctx, SSD_E_CUDA, std::string("ssd_gpu_set_step_labels: ") + cudaGetErrorString(e));
+    return SSD_OK;
+  }
+  if(!ctx->d_step_labels)
+  {
+    const cudaError_t e = cudaMalloc(&ctx->d_step_labels, (size_t)ctx->max_frames * ctx->dp.N);
+    if(e != cudaSuccess)
+    {
+      cudaGetLastError(); // clear the sticky allocation error: the context stays usable
+      ctx->d_step_labels = nullptr;
+      ctx->step_labels = false;
+      return fail(ctx, SSD_E_NOMEM, std::string("ssd_gpu_set_step_labels: ") + cudaGetErrorString(e));
+    }
+  }
+  ctx->step_labels = true;
+  return SSD_OK;
+}
+
+// the step labels of the last call: SSD_E_STATE unless that call ran with them, they are still enabled and the call's results are
+// readable (a failed call, or a setting that invalidates earlier results, sets n_frames_last to 0)
+static int check_step_labels(ssd_gpu_ctx *ctx, const char *fn)
+{
+  if(!ctx->step_labels || !ctx->step_labels_last || ctx->n_frames_last <= 0)
+    return fail(ctx, SSD_E_STATE, std::string(fn) + ": not enabled for the last call (ssd_gpu_set_step_labels)");
+  return SSD_OK;
+}
+
+int ssd_gpu_get_step_labels(ssd_gpu_ctx *ctx, int frame, uint8_t *out_host)
+{
+  int rc = check_frame(ctx, frame);
+  if(rc)
+    return rc;
+  if(!out_host)
+    return SSD_E_INVALID_ARG;
+  if((rc = check_step_labels(ctx, "ssd_gpu_get_step_labels")))
+    return rc;
+  CK(cudaSetDevice(ctx->device));
+  CK(cudaMemcpy(out_host, ctx->d_step_labels + (size_t)frame * ctx->dp.N, (size_t)ctx->dp.N, cudaMemcpyDeviceToHost));
+  return SSD_OK;
+}
+
+int ssd_gpu_step_labels_device_ptr(ssd_gpu_ctx *ctx, const uint8_t **out)
+{
+  if(!ctx || !out)
+    return SSD_E_INVALID_ARG;
+  const int rc = check_step_labels(ctx, "ssd_gpu_step_labels_device_ptr");
+  if(rc)
+    return rc;
+  *out = ctx->d_step_labels;
   return SSD_OK;
 }
 

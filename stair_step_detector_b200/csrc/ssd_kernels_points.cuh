@@ -1164,9 +1164,21 @@ __device__ __forceinline__ void seg_flush(QuadReduceShared &S, unsigned l, unsig
   atomicAdd(&S.cnt[l], n);
 }
 
-// one point of the compacted exact pass: the reference's own double-precision test
+// Step code of plateau l in the step labels (include/ssd_gpu.h: ssd_gpu_set_step_labels). k_finalize emits the ground first
+// (ground_index < first_outlined <= first_valid, k_peaks) and then the valid plateaus in ascending order, each exactly when
+// its bit of quad_amask (k_frame_logic: emitted and a usable quadrilateral) is set; quad_amask is 0 when nothing is emitted.
+// So the step of plateau l is the number of quad_amask bits below l.
+__device__ __forceinline__ unsigned step_code(unsigned amask, unsigned l)
+{
+  return (unsigned)__popc(amask & ((1u << l) - 1u));
+}
+
+// one point of the compacted exact pass: the reference's own double-precision test. STEPS: the point's step code goes to
+// *step when it is counted (a step-label byte of the frame; nullptr without step labels).
+template<bool STEPS = false>
 __device__ __forceinline__ void quad_reduce_exact_point(const DevParams &p, float fx, float fy, float fz, unsigned l, bool bevonly, const FrameDev &F,
-                                                        unsigned amask, int ground, unsigned *__restrict__ gbev, QuadReduceShared &S)
+                                                        unsigned amask, int ground, unsigned *__restrict__ gbev, QuadReduceShared &S,
+                                                        unsigned char *step = nullptr)
 {
   if(l >= SSD_GPU_MAX_PLATEAUS || !((amask >> l) & 1u))
     return;
@@ -1177,6 +1189,8 @@ __device__ __forceinline__ void quad_reduce_exact_point(const DevParams &p, floa
     if(!quadtest_within(F.plat[l].qt, wx, wy))
       return;
     seg_flush(S, l, z_fix_u(p, fx, fy, fz), 1u);
+    if constexpr(STEPS)
+      *step = (unsigned char)step_code(amask, l);
   }
   if((int)l == ground)
   {
@@ -1221,10 +1235,14 @@ __device__ __forceinline__ void qr_seg_combine(QuadReduceShared &S, QrWarp &W, i
 
 // The dense part of one warp-tile: phase B over the n compacted words of the warp's list (S.L.act / S.L.lab), the exact
 // pass over the deferred points, the queued ground BEV pixels, and the warp's segmented reduce. wbase: first 4-point word
-// of the warp-tile within the frame.
-template<class SRC, class FRAME>
+// of the warp-tile within the frame. STEPS: every counted point also writes its step code into steps (the frame's step
+// labels, cleared to SSD_STEP_LABEL_NONE before the launch) -- at the three places a point is counted: a uniform word's
+// inner-box points (one 32-bit store per word), the deferred points the f32 image of the test settles as inside, and the
+// exact pass. A word's store precedes the byte stores of its deferred points (the __syncwarp before the exact pass).
+template<class SRC, bool STEPS = false, class FRAME>
 __device__ __forceinline__ void qr_dense(const DevParams &p, const FRAME &FR, QuadReduceShared &S, QrWarp &W, const FrameDev &F, unsigned amask, int ground,
-                                         unsigned *__restrict__ gbev, unsigned wbase, unsigned n, int warp, int lane)
+                                         unsigned *__restrict__ gbev, unsigned wbase, unsigned n, int warp, int lane,
+                                         unsigned char *__restrict__ steps = nullptr)
 {
   unsigned short *act = S.L.act[warp];
   unsigned *labs = S.L.lab[warp];
@@ -1283,6 +1301,14 @@ __device__ __forceinline__ void qr_dense(const DevParams &p, const FRAME &FR, Qu
         zs += z_fix_u(p, vx[j], vy[j], vz[j]) & (unsigned)inm[j];
         cnt -= inm[j];
       }
+      if constexpr(STEPS)
+        if(cnt)
+        {
+          // the word's step labels: the step code in the bytes of its inner-box points, SSD_STEP_LABEL_NONE elsewhere (its
+          // deferred points are settled below). Word index < N / 4 < 2^32.
+          const unsigned inb = ((unsigned)inm[0] & 0xffu) | ((unsigned)inm[1] & 0xff00u) | ((unsigned)inm[2] & 0xff0000u) | ((unsigned)inm[3] & 0xff000000u);
+          reinterpret_cast<unsigned *>(steps)[wbase + (e >> 4)] = ((step_code(amask, l0) * 0x01010101u) & inb) | ~inb;
+        }
       // between the inner box and the reject box (a few percent of the points, but in most warp steps): deferred to
       // the dense pass at the end of the warp-tile, which evaluates the f32 image of the full test one point per lane
       if((midm[0] | midm[1] | midm[2] | midm[3]) < 0)
@@ -1370,11 +1396,13 @@ __device__ __forceinline__ void qr_dense(const DevParams &p, const FRAME &FR, Qu
             }
             seg_sum += z_fix_u(p, fx, fy, fz);
             seg_n++;
+            if constexpr(STEPS)
+              steps[(wbase + w) * 4u + j] = (unsigned char)step_code(amask, l); // pixel index < N < 2^32
           }
         }
       }
       if(exact)
-        quad_reduce_exact_point(p, fx, fy, fz, l, bevonly, F, amask, ground, gbev, S);
+        quad_reduce_exact_point<STEPS>(p, fx, fy, fz, l, bevonly, F, amask, ground, gbev, S, STEPS ? steps + ((wbase + w) * 4u + j) : nullptr);
     }
     __syncwarp();
     n_def += nd;
@@ -1494,10 +1522,23 @@ __device__ __forceinline__ void qr_epilogue(QuadReduceShared &S, QrWarp &W, Fram
 #ifndef SSD_QR_MINB
 #define SSD_QR_MINB 4
 #endif
-template<class SRC, class CAM = NoCam>
+// k_quad_reduce's step-label output: a pointer in the STEPS variant only, so the other variants' parameters stay as they are
+template<bool STEPS>
+struct StepLabelsOut
+{
+};
+template<>
+struct StepLabelsOut<true>
+{
+  unsigned char *p;
+};
+// STEPS (ssd_gpu_set_step_labels): the variant that also writes the step labels; steps holds them for the launch's frames
+// (frame-major like labels, cleared to SSD_STEP_LABEL_NONE before the launch: pixels no counted point reaches keep it).
+template<class SRC, class CAM = NoCam, bool STEPS = false>
 __global__ void __launch_bounds__(SSD_PT_THREADS, SSD_QR_MINB) k_quad_reduce(const __grid_constant__ DevParams p0, const SRC src0,
                                                                  const unsigned char *__restrict__ labels, FrameDev *__restrict__ frames,
-                                                                 unsigned *__restrict__ bev, size_t bm_words, const CAM cam = CAM())
+                                                                 unsigned *__restrict__ bev, size_t bm_words, const CAM cam = CAM(),
+                                                                 StepLabelsOut<STEPS> steps_out = StepLabelsOut<STEPS>())
 {
   __shared__ QuadReduceShared S;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1557,7 +1598,10 @@ __global__ void __launch_bounds__(SSD_PT_THREADS, SSD_QR_MINB) k_quad_reduce(con
       continue;
     __syncwarp();
 
-    qr_dense<SRC>(p, FR, S, W, F, amask, ground, gbev, wbase, n, warp, lane);
+    if constexpr(STEPS)
+      qr_dense<SRC, true>(p, FR, S, W, F, amask, ground, gbev, wbase, n, warp, lane, steps_out.p + fbase);
+    else
+      qr_dense<SRC>(p, FR, S, W, F, amask, ground, gbev, wbase, n, warp, lane);
     __syncwarp();
   }
   qr_epilogue(S, W, F, ground, tid, lane);
