@@ -548,6 +548,36 @@ __host__ __device__ __forceinline__ double hypot_cr(double x, double y)
   return h + r / (2.0 * h);
 }
 
+// glibc's hypot (2.35 and later, the generic double version without FMA that x86-64 builds select) for the integer line
+// coefficients of the line fits: |x| <= 5109 and |y| <= 9349, so x*x + y*y is exact and no scaling branch applies. It is not
+// correctly rounded: it corrects the square root by (t1 + t2) / (2 h), which moves about 0.6 % of the results by one ulp. The
+// line fit selects on residual / hypot, so two pairs with equal a*a + b*b can tie under the correctly rounded value and not under
+// glibc's; the device must see glibc's value. tools/hypot_glibc_check.cu compares this function with the host's libm over the
+// whole operand domain.
+__host__ __device__ __forceinline__ double hypot_glibc_int(double x, double y)
+{
+  x = fabs(x);
+  y = fabs(y);
+  const double ax = x < y ? y : x, ay = x < y ? x : y;
+  if(ay == 0.0)
+    return ax;
+  double h = sqrt(ax * ax + ay * ay), t1, t2;
+  if(h <= 2.0 * ay)
+  {
+    const double delta = h - ay;
+    t1 = ax * (2.0 * delta - ax);
+    t2 = (delta - 2.0 * (ax - ay)) * delta;
+  }
+  else
+  {
+    const double delta = h - ax;
+    t1 = 2.0 * delta * (ax - 2.0 * ay);
+    t2 = (4.0 * delta - ay) * ay + delta * delta;
+  }
+  h -= (t1 + t2) / (2.0 * h);
+  return h;
+}
+
 // ---- lines (types.h:117-163, segmentation.cpp:321-401) ----
 __device__ __forceinline__ LineId linei_from(P2id p, P2id q)
 {

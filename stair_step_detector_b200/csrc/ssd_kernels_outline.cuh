@@ -285,7 +285,7 @@ __device__ inline bool pair_abandoned(const P2id *pts, int n, int pi, int qi, Li
     return false;
   const int m = n - 2;
   const int cnt = m > 4 ? (m - 1) / 2 : 1;
-  const double Bf = bound * ((double)(size_t)cnt * sqrt((double)((long long)l.a * l.a + (long long)l.b * l.b))) * (1.0 + 1e-12);
+  const double Bf = bound * ((double)(size_t)cnt * hypot_glibc_int(l.a, l.b)) * (1.0 + 1e-12);
   if(!(Bf < 4e18))
     return false;
   const long long B = (long long)Bf + 1;
@@ -366,7 +366,7 @@ __device__ inline double pair_residual(const P2id *pts, int n, int pi, int qi, L
     int hi = -1, lo = 0;
     if(bound < 1e300)
     {
-      const double Bf = bound * ((double)(size_t)cnt * sqrt((double)((long long)l.a * l.a + (long long)l.b * l.b))) * (1.0 + 1e-12);
+      const double Bf = bound * ((double)(size_t)cnt * hypot_glibc_int(l.a, l.b)) * (1.0 + 1e-12);
       if(Bf < 4e18)
       {
         const long long B = (long long)Bf + 1;
@@ -466,9 +466,9 @@ __device__ inline double pair_residual(const P2id *pts, int n, int pi, int qi, L
     sum += (long long)(cnt - below) * lo;
   }
   // the reference sums into int (segmentation.cpp:434); keep its wrap-around semantics.
-  // hypot of two ints: a*a+b*b is exact in double, so the IEEE square root is the correctly rounded hypot.
+  // glibc's hypot, not the correctly rounded one: equal a*a+b*b with different glibc roundings must not tie (hypot_glibc_int)
   const int isum = (int)sum;
-  const double h = sqrt((double)((long long)l.a * l.a + (long long)l.b * l.b));
+  const double h = hypot_glibc_int(l.a, l.b);
   return isum / ((double)(size_t)cnt * h); // :442
 }
 
