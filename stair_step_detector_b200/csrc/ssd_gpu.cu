@@ -485,15 +485,30 @@ __global__ void k_single_camera_to_world(const __grid_constant__ DevParams p, co
   }
 }
 
+// Pass 1 (k_transform_bin): packed vertices through the kernel's bulk-copy staging, z16 frames (SrcDepth, SrcLens) from registers
+template<bool FUSE, class CAM>
+static void launch_transform_bin(const dim3 &grid, cudaStream_t st, const DevParams &p, const SrcVertices &src, unsigned char *labels,
+                                 FrameDev *frames, const CAM &cam)
+{
+  k_transform_bin<SSD_PT_ITERS, FUSE, CAM><<<grid, SSD_PT_THREADS, SSD_PT_ITERS * SSD_TB_STAGE_BYTES, st>>>(p, src.xyz, labels, frames, cam);
+}
+template<bool FUSE, class SRC, class CAM>
+static void launch_transform_bin(const dim3 &grid, cudaStream_t st, const DevParams &p, const SRC &src, unsigned char *labels, FrameDev *frames,
+                                 const CAM &cam)
+{
+  k_transform_bin_z16<SSD_PT_ITERS, FUSE, SRC, CAM><<<grid, SSD_PT_THREADS, 0, st>>>(p, src, labels, frames, cam);
+}
+
 // The classic chain: k_transform_bin -> k_peaks -> k_label_bev -> k_outline -> k_frame_logic -> k_quad_reduce -> k_finalize
-// (+ k_riser_reduce). CAM = NoCam: every frame with the context's own camera; CamTable: each frame with its camera's parameters
-// (camera calls); GroupTable: as CamTable, with the frames of each group accumulated into one record (group calls).
+// (+ k_riser_reduce), for one chunk of frames on stream s. SRC: where the points come from (SrcVertices, SrcDepth, SrcLens), its
+// input pointer the chunk's. CAM = NoCam: every frame with the context's own camera; CamTable: each frame with its camera's
+// parameters (camera calls); GroupTable: as CamTable, with the frames of each group accumulated into one record (group calls).
+// OL: the outline work area of the frame size (OutlineSharedSmall, OutlineShared).
 // Records (FrameDev, FrameOut, BEV slots): rec0 is the launch's first within the call, nr their number (frames, or groups).
-// sl: the chunk's z16 frames through ray tables (a call with a distorted lens), else nullptr. ov_lens: the lenses the overlay
-// projects through (LensCam), else nullptr.
-template<class CAM>
-static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const SrcDepth &sd, const SrcLens *sl, int frame0, int nf, int rec0,
-                          int nr, int *launches, cudaEvent_t *ev, const CAM cam, const ssd_gpu_distortion *ov_lens)
+// ov_lens: the lenses the overlay projects through (LensCam), else nullptr.
+template<class OL, class SRC, class CAM>
+static int launch_classic(ssd_gpu_ctx *ctx, int s, const SRC &src, int frame0, int nf, int rec0, int nr, int *launches, cudaEvent_t *ev,
+                          const CAM &cam, const ssd_gpu_distortion *ov_lens)
 {
 #define STAGE_EV(i)                         \
   do                                        \
@@ -503,7 +518,6 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   } while(0)
   const DevParams &p = ctx->dp;
   cudaStream_t st = ctx->stream[s];
-  constexpr bool grouped = std::is_same<CAM, GroupTable>::value;
   FrameDev *frames = ctx->d_frames + rec0;
   unsigned char *labels = ctx->d_labels + (size_t)frame0 * p.N;
   unsigned *bev = ctx->d_bev + (size_t)s * ctx->chunk_frames * SSD_GPU_MAX_PLATEAUS * ctx->bm_words;
@@ -513,73 +527,35 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   const int bpf = std::max(1, std::min(tiles2, (ctx->pt_blocks_target + nf - 1) / nf));
   const int bpf_l = ctx->bpf_l_knob > 0 ? std::min(tiles2, ctx->bpf_l_knob) : bpf, bpf_q = ctx->bpf_q_knob > 0 ? std::min(tiles2, ctx->bpf_q_knob) : bpf;
   const dim3 gpt2l(bpf_l, nf), gpt2q(bpf_q, nf);
-  const bool depth = sv.xyz == nullptr;
-  const float *xyz_dev = sv.xyz;
   ssd_gpu_overlay *ovl = ctx->d_ovl ? ctx->d_ovl + (size_t)frame0 * SSD_GPU_MAX_STEPS : nullptr;
   // small batches (the reference's real use is one frame per call): the last block of a frame in k_transform_bin evaluates the
   // peaks and the last block in k_outline the frame logic -- five launches instead of seven. Group calls take the seven
   // (their blocks do not count a frame's completion).
-  const bool fused = !grouped && nf <= SSD_FUSE_MAX_FRAMES && !ev;
+  constexpr bool FUSABLE = !IsGroupCam<CAM>::value;
+  const bool fused = FUSABLE && nf <= SSD_FUSE_MAX_FRAMES && !ev;
   STAGE_EV(0);
-  if(fused)
-  {
-    if constexpr(grouped)
-      ;
-    else if(sl)
-      k_transform_bin_lens<SSD_PT_ITERS, true, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, cam);
-    else if(depth)
-      k_transform_bin_depth<SSD_PT_ITERS, true, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, cam);
-    else
-      k_transform_bin<SSD_PT_ITERS, true, CAM><<<gpt, SSD_PT_THREADS, SSD_PT_ITERS * SSD_TB_STAGE_BYTES, st>>>(p, xyz_dev, labels, frames, cam);
-  }
-  else
-  {
-    if(sl)
-      k_transform_bin_lens<SSD_PT_ITERS, false, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, cam);
-    else if(depth)
-      k_transform_bin_depth<SSD_PT_ITERS, false, CAM><<<gpt, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, cam);
-    else
-      k_transform_bin<SSD_PT_ITERS, false, CAM><<<gpt, SSD_PT_THREADS, SSD_PT_ITERS * SSD_TB_STAGE_BYTES, st>>>(p, xyz_dev, labels, frames, cam);
-  }
+  if(!fused)
+    launch_transform_bin<false>(gpt, st, p, src, labels, frames, cam);
+  else if constexpr(FUSABLE)
+    launch_transform_bin<true>(gpt, st, p, src, labels, frames, cam);
   STAGE_EV(1);
   if(!fused)
     k_peaks<<<nr, 32, 0, st>>>(p, frames, nr);
   STAGE_EV(2);
-  if(sl)
-    k_label_bev<SrcLens, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, cam);
-  else if(depth)
-    k_label_bev<SrcDepth, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, cam);
-  else
-    k_label_bev<SrcVertices, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, cam);
+  k_label_bev<SRC, CAM><<<gpt2l, SSD_PT_THREADS, 0, st>>>(p, src, labels, frames, bev, ctx->bm_words, cam);
   STAGE_EV(3);
-  if(fused)
-  {
-    if constexpr(grouped)
-      ;
-    else if(ctx->outline_small)
-      k_outline<OutlineSharedSmall, true, CAM><<<dim3(ctx->outline_gridx, nf), SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words, cam);
-    else
-      k_outline<OutlineShared, true, CAM><<<dim3(ctx->outline_gridx, nf), OutlineShared::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words, cam);
-  }
-  else
-  {
-    if(ctx->outline_small)
-      k_outline<OutlineSharedSmall><<<dim3(ctx->outline_gridx, nr), SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
-    else
-      k_outline<OutlineShared><<<dim3(ctx->outline_gridx, nr), OutlineShared::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
-  }
+  // the unfused k_outline reads configuration fields only: one kernel for every camera type
+  if(!fused)
+    k_outline<OL><<<dim3(ctx->outline_gridx, nr), OL::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words);
+  else if constexpr(FUSABLE)
+    k_outline<OL, true, CAM><<<dim3(ctx->outline_gridx, nf), OL::THREADS, ctx->ol_dyn_smem, st>>>(p, frames, bev, ctx->bm_words, ctx->smem_cap_words, cam);
   STAGE_EV(4);
   if(!fused)
     k_frame_logic<CAM><<<nr, 32, 0, st>>>(p, frames, nr, cam);
   STAGE_EV(5);
   const auto quad_reduce = [&](auto so) {
     constexpr bool STEPS = std::is_same<decltype(so), StepLabelsOut<true>>::value;
-    if(sl)
-      k_quad_reduce<SrcLens, CAM, STEPS><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, bev, ctx->bm_words, cam, so);
-    else if(depth)
-      k_quad_reduce<SrcDepth, CAM, STEPS><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, bev, ctx->bm_words, cam, so);
-    else
-      k_quad_reduce<SrcVertices, CAM, STEPS><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, bev, ctx->bm_words, cam, so);
+    k_quad_reduce<SRC, CAM, STEPS><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, src, labels, frames, bev, ctx->bm_words, cam, so);
   };
   if(ctx->step_labels)
   {
@@ -593,82 +569,70 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SrcVertices &sv, const 
   else
     quad_reduce(StepLabelsOut<false>());
   STAGE_EV(6);
+  // k_finalize runs SSD_OL_THREADS on either work area
   if(ov_lens)
-  {
-    const LensCam<CAM> lc = { cam, ov_lens };
-    if(ctx->outline_small)
-      k_finalize<OutlineSharedSmall, LensCam<CAM>><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words,
-                                                                                             ctx->smem_cap_words, ctx->ov, ovl, lc);
-    else
-      k_finalize<OutlineShared, LensCam<CAM>><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words,
-                                                                                        ctx->smem_cap_words, ctx->ov, ovl, lc);
-  }
-  else if(ctx->outline_small)
-    k_finalize<OutlineSharedSmall, CAM><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words, ctx->smem_cap_words,
-                                                                               ctx->ov, ovl, cam);
+    k_finalize<OL, LensCam<CAM>><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words, ctx->smem_cap_words,
+                                                                              ctx->ov, ovl, LensCam<CAM>{ cam, ov_lens });
   else
-    k_finalize<OutlineShared, CAM><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words, ctx->smem_cap_words,
-                                                                          ctx->ov, ovl, cam);
+    k_finalize<OL, CAM><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words, ctx->smem_cap_words, ctx->ov,
+                                                                     ovl, cam);
   STAGE_EV(7);
 #undef STAGE_EV
   *launches += fused ? SSD_GPU_N_STAGES - 2 : SSD_GPU_N_STAGES;
   if(ctx->risers)
   {
     // optional fourth pass: vertical faces from the remainder (labels are final once the chain's label kernel has run)
-    if(sl)
-      k_riser_reduce<SrcLens, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, *sl, labels, frames, cam);
-    else if(depth)
-      k_riser_reduce<SrcDepth, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sd, labels, frames, cam);
-    else
-      k_riser_reduce<SrcVertices, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, sv, labels, frames, cam);
+    k_riser_reduce<SRC, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, src, labels, frames, cam);
     *launches += 1;
   }
   CK(cudaGetLastError());
   return SSD_OK;
 }
 
-
-// ---------------------------------------------------------------------------------------------
-// the launch chain for one chunk of frames on one stream
-// ---------------------------------------------------------------------------------------------
-// xyz_dev: packed vertices of the chunk, or nullptr with z16_dev: the chunk's depth frames, deprojected inside the
-// three point kernels (SrcDepth). cam: the camera table of a camera call, else nullptr. grp: the group tables of a group call (its
-// cams are *cam), else nullptr; the chunk then holds the whole groups rec0 .. rec0 + nr - 1.
-// sl: the call's lens source (its z16 member is set here), else nullptr; ov_lens: see launch_classic.
-static int launch_chunk(ssd_gpu_ctx *ctx, int s, const float *xyz_dev, const uint16_t *z16_dev, float depth_unit, int frame0, int nf, int rec0,
-                        int nr, int *launches, cudaEvent_t *ev, const CamTable *cam, const GroupTable *grp, const SrcLens *sl,
-                        const ssd_gpu_distortion *ov_lens)
+// A chunk's source and camera: the call's, with the chunk's input (the caller's frames or the staging buffer they were copied to)
+// and, in camera and group calls, its first frame and first group.
+static SrcVertices chunk_src(SrcVertices s, const void *in)
 {
-  const DevParams &p = ctx->dp;
-  SrcVertices sv;
-  sv.xyz = xyz_dev;
-  SrcDepth sd;
-  sd.z16 = z16_dev;
-  sd.xn = ctx->d_xn;
-  sd.yn = ctx->d_yn;
-  sd.unit = depth_unit;
-  sd.wmagic = (((unsigned long long)1 << 40) + (unsigned long long)p.W - 1) / (unsigned long long)p.W;
-  SrcLens sll;
-  if(sl)
+  s.xyz = static_cast<const float *>(in);
+  return s;
+}
+template<class SRC>
+static SRC chunk_src(SRC s, const void *in)
+{
+  s.z16 = static_cast<const uint16_t *>(in);
+  return s;
+}
+static NoCam chunk_cam(NoCam c, int, int)
+{
+  return c;
+}
+static CamTable chunk_cam(CamTable c, int frame0, int)
+{
+  c.frame0 = frame0;
+  return c;
+}
+static GroupTable chunk_cam(GroupTable g, int frame0, int rec0)
+{
+  g.cams.frame0 = frame0;
+  g.group0 = rec0;
+  return g;
+}
+
+// The dynamic work area of the outline kernels a chain of camera type CAM launches with a dynamic band (launch_classic): the fused
+// k_outline (not in group calls) and k_finalize with and without the overlay's lens, on both work areas.
+template<class CAM>
+static void allow_outline_smem(int dyn)
+{
+  const auto allow = [dyn](auto kernel) { cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn); };
+  if constexpr(!IsGroupCam<CAM>::value)
   {
-    sll = *sl;
-    sll.z16 = z16_dev;
+    allow(k_outline<OutlineSharedSmall, true, CAM>);
+    allow(k_outline<OutlineShared, true, CAM>);
   }
-  if(grp)
-  {
-    GroupTable g = *grp;
-    g.cams = *cam;
-    g.cams.frame0 = frame0;
-    g.group0 = rec0;
-    return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, rec0, nr, launches, ev, g, ov_lens);
-  }
-  if(cam)
-  {
-    CamTable c = *cam;
-    c.frame0 = frame0;
-    return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, frame0, nf, launches, ev, c, ov_lens);
-  }
-  return launch_classic(ctx, s, sv, sd, sl ? &sll : nullptr, frame0, nf, frame0, nf, launches, ev, NoCam(), ov_lens);
+  allow(k_finalize<OutlineSharedSmall, CAM>);
+  allow(k_finalize<OutlineShared, CAM>);
+  allow(k_finalize<OutlineSharedSmall, LensCam<CAM>>);
+  allow(k_finalize<OutlineShared, LensCam<CAM>>);
 }
 
 extern "C"
@@ -843,25 +807,9 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
     {
       cudaFuncSetAttribute(k_outline<OutlineShared>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       cudaFuncSetAttribute(k_outline<OutlineSharedSmall>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_outline<OutlineShared, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_outline<OutlineSharedSmall, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_finalize<OutlineShared>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_finalize<OutlineSharedSmall>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      // the camera-table variants (ssd_gpu_set_cameras) of the kernels with a dynamic work area
-      cudaFuncSetAttribute(k_outline<OutlineShared, true, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_outline<OutlineSharedSmall, true, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_finalize<OutlineShared, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, CamTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      // the overlay through a distorted lens (ssd_gpu_set_distortion / ssd_gpu_set_cameras_ex)
-      cudaFuncSetAttribute(k_finalize<OutlineShared, LensCam<NoCam>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, LensCam<NoCam>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_finalize<OutlineShared, LensCam<CamTable>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, LensCam<CamTable>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      // frame groups (ssd_gpu_process_groups_*)
-      cudaFuncSetAttribute(k_finalize<OutlineShared, GroupTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, GroupTable>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_finalize<OutlineShared, LensCam<GroupTable>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-      cudaFuncSetAttribute(k_finalize<OutlineSharedSmall, LensCam<GroupTable>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+      allow_outline_smem<NoCam>((int)dyn);
+      allow_outline_smem<CamTable>((int)dyn);
+      allow_outline_smem<GroupTable>((int)dyn);
       cudaFuncSetAttribute(k_single_front_edge, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
       granted = dyn;
     }
@@ -1156,6 +1104,7 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
       ctx->grp_members.push_back(make_int2(f, group_frames[g]));
       ctx->grp_epsc.push_back(e);
     }
+    grp.cams = cams;
     grp.group = ctx->d_grp_of_frame;
     grp.members = ctx->d_grp_members;
     grp.epsc = ctx->d_grp_epsc;
@@ -1181,38 +1130,64 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
   for(int i = 1; i < ctx->n_streams; i++)
     CK(cudaStreamWaitEvent(ctx->stream[i], ctx->ev_chunk_done[0], 0));
 
-  for(int chunk = 0; chunk < n_chunks; chunk++)
-  {
-    const int f0 = chunks[chunk].f0, nf = chunks[chunk].nf;
-    const int s = (flags & SSD_FLAG_SINGLE_STREAM) ? 0 : chunk % ctx->n_streams;
-    const float *src = depth_input ? nullptr : xyz + (size_t)f0 * frame_floats;
-    const uint16_t *dsrc = depth_input ? z16 + (size_t)f0 * p.N : nullptr;
-    if(host_input)
+  // the chunk loop for the call's one source and camera type
+  const auto run_chunks = [&](const auto &src, const auto &cam) -> int {
+    for(int chunk = 0; chunk < n_chunks; chunk++)
     {
-      // staging buffer s may be overwritten once the chunk that last used it has consumed it
-      if(chunk >= ((flags & SSD_FLAG_SINGLE_STREAM) ? 1 : ctx->n_streams))
-        CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_in_free[s], 0));
-      if(depth_input)
+      const int f0 = chunks[chunk].f0, nf = chunks[chunk].nf;
+      const int s = (flags & SSD_FLAG_SINGLE_STREAM) ? 0 : chunk % ctx->n_streams;
+      const void *in = depth_input ? (const void *)(z16 + (size_t)f0 * p.N) : (const void *)(xyz + (size_t)f0 * frame_floats);
+      if(host_input)
       {
-        CK(cudaMemcpyAsync(ctx->d_depth[s], dsrc, (size_t)nf * p.N * sizeof(uint16_t), cudaMemcpyHostToDevice, ctx->copy_stream));
-        dsrc = ctx->d_depth[s];
+        // staging buffer s may be overwritten once the chunk that last used it has consumed it
+        if(chunk >= ((flags & SSD_FLAG_SINGLE_STREAM) ? 1 : ctx->n_streams))
+          CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_in_free[s], 0));
+        if(depth_input)
+        {
+          CK(cudaMemcpyAsync(ctx->d_depth[s], in, (size_t)nf * p.N * sizeof(uint16_t), cudaMemcpyHostToDevice, ctx->copy_stream));
+          in = ctx->d_depth[s];
+        }
+        else
+        {
+          CK(cudaMemcpyAsync(ctx->d_stage[s], in, (size_t)nf * frame_floats * sizeof(float), cudaMemcpyHostToDevice, ctx->copy_stream));
+          in = ctx->d_stage[s];
+        }
+        CK(cudaEventRecord(ctx->ev_in_ready[s], ctx->copy_stream));
+        CK(cudaStreamWaitEvent(ctx->stream[s], ctx->ev_in_ready[s], 0));
       }
-      else
-      {
-        CK(cudaMemcpyAsync(ctx->d_stage[s], src, (size_t)nf * frame_floats * sizeof(float), cudaMemcpyHostToDevice, ctx->copy_stream));
-        src = ctx->d_stage[s];
-      }
-      CK(cudaEventRecord(ctx->ev_in_ready[s], ctx->copy_stream));
-      CK(cudaStreamWaitEvent(ctx->stream[s], ctx->ev_in_ready[s], 0));
+      const auto csrc = chunk_src(src, in);
+      const auto ccam = chunk_cam(cam, f0, chunks[chunk].r0);
+      cudaEvent_t *ev = stage_timing ? &ctx->stage_ev[(size_t)chunk * (SSD_GPU_N_STAGES + 1)] : nullptr;
+      const int rc = ctx->outline_small
+                       ? launch_classic<OutlineSharedSmall>(ctx, s, csrc, f0, nf, chunks[chunk].r0, chunks[chunk].nr, &launches, ev, ccam, ov_lens)
+                       : launch_classic<OutlineShared>(ctx, s, csrc, f0, nf, chunks[chunk].r0, chunks[chunk].nr, &launches, ev, ccam, ov_lens);
+      if(rc)
+        return rc;
+      if(host_input)
+        CK(cudaEventRecord(ctx->ev_in_free[s], ctx->stream[s])); // all three passes have read the staging
     }
-    const int rc = launch_chunk(ctx, s, src, dsrc, depth_input && intr ? intr->depth_unit : 0.f, f0, nf, chunks[chunk].r0, chunks[chunk].nr,
-                                &launches, stage_timing ? &ctx->stage_ev[(size_t)chunk * (SSD_GPU_N_STAGES + 1)] : nullptr,
-                                cam_of_frame ? &cams : nullptr, group_frames ? &grp : nullptr, use_lens ? &sl : nullptr, ov_lens);
-    if(rc)
-      return rc;
-    if(host_input)
-      CK(cudaEventRecord(ctx->ev_in_free[s], ctx->stream[s])); // all three passes have read the staging
+    return SSD_OK;
+  };
+  const auto run_source = [&](const auto &src) -> int {
+    if(group_frames)
+      return run_chunks(src, grp);
+    if(cam_of_frame)
+      return run_chunks(src, cams);
+    return run_chunks(src, NoCam());
+  };
+  int rc;
+  if(!depth_input)
+    rc = run_source(SrcVertices{ xyz });
+  else if(use_lens)
+    rc = run_source(sl);
+  else
+  {
+    // depth frames are deprojected inside the point kernels with the pin-hole tables (a camera call's per camera)
+    const unsigned long long wmagic = (((unsigned long long)1 << 40) + (unsigned long long)p.W - 1) / (unsigned long long)p.W;
+    rc = run_source(SrcDepth{ z16, ctx->d_xn, ctx->d_yn, intr ? intr->depth_unit : 0.f, wmagic });
   }
+  if(rc)
+    return rc;
   if(host_input)
     CK(cudaEventRecord(ctx->ev_h2d1, ctx->copy_stream));
   // join stream 1 into stream 0, then bring the compact results home

@@ -685,12 +685,13 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin(const __grid_c
 }
 
 // ---------------------------------------------------------------------------------------------
-// k_transform_bin_depth: the same pass on a z16 depth frame (SrcDepth): 2 bytes per point come in, 1 goes out, the
-// deprojected vertices live in registers only. No staging: the loads are 8 bytes per lane (256 B per warp, coalesced) and
-// all ITERS words of a thread are requested before the first is consumed. Not HBM-bound (3 B/point): issue-bound.
+// k_transform_bin_z16: the same pass on z16 depth frames, SRC = SrcDepth (pin-hole tables) or SrcLens (ray table of a distorted
+// lens: 10 bytes per point in, 2 of depth and 8 of L2-resident ray): 2 bytes per point come in, 1 goes out, the deprojected
+// vertices live in registers only. No staging: the loads are 8 bytes per lane (256 B per warp, coalesced) and all ITERS words
+// of a thread are requested before the first is consumed. Not HBM-bound (3 B/point with SrcDepth): issue-bound.
 // ---------------------------------------------------------------------------------------------
-template<int ITERS, bool FUSE_PEAKS = false, class CAM = NoCam>
-__global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_depth(const __grid_constant__ DevParams p0, const SrcDepth src0,
+template<int ITERS, bool FUSE_PEAKS, class SRC, class CAM>
+__global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_z16(const __grid_constant__ DevParams p0, const SRC src0,
                                                                          unsigned char *__restrict__ codes, FrameDev *__restrict__ frames,
                                                                          const CAM cam = CAM())
 {
@@ -703,8 +704,8 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_depth(const __
   const size_t fbase = (size_t)frame * p.N;
   const int nquads = p.N >> 2;
   const int q0 = blockIdx.x * (ITERS * SSD_PT_THREADS) + tid;
-  const FrameD F = src_frame(src, p, fbase);
-  WordD w[ITERS];
+  const typename SrcTraits<SRC>::Frame F = src_frame(src, p, fbase);
+  typename SrcTraits<SRC>::Word w[ITERS];
 #pragma unroll
   for(int it = 0; it < ITERS; it++)
   {
@@ -741,61 +742,6 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_depth(const __
     tb_fused_peaks(p, frames[frame_slot(cam, frame)], K, s_last, tid);
   }
 }
-// k_transform_bin_lens: the same pass on z16 frames of a distorted lens (SrcLens), 10 bytes per point in (2 of depth, 8 of ray
-// from the L2-resident table). A copy of k_transform_bin_depth's body: that kernel's code stays as it was.
-template<int ITERS, bool FUSE_PEAKS = false, class CAM = NoCam>
-__global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_lens(const __grid_constant__ DevParams p0, const SrcLens src0,
-                                                                        unsigned char *__restrict__ codes, FrameDev *__restrict__ frames,
-                                                                        const CAM cam = CAM())
-{
-  __shared__ unsigned s_hist[SSD_BINS_PAD];
-  __shared__ unsigned s_exact;
-  const int tid = threadIdx.x;
-  const int frame = blockIdx.y;
-  const DevParams &p = frame_params(p0, cam, frame);
-  const auto &src = frame_src(src0, cam, p, frame);
-  const size_t fbase = (size_t)frame * p.N;
-  const int nquads = p.N >> 2;
-  const int q0 = blockIdx.x * (ITERS * SSD_PT_THREADS) + tid;
-  const FrameL F = src_frame(src, p, fbase);
-  WordL w[ITERS];
-#pragma unroll
-  for(int it = 0; it < ITERS; it++)
-  {
-    word_zero(w[it]);
-    if(q0 + it * SSD_PT_THREADS < nquads)
-      word_load(F, (unsigned)(q0 + it * SSD_PT_THREADS), w[it]);
-  }
-  s_hist[tid] = 0; // SSD_PT_THREADS == SSD_BINS_PAD
-  if(tid == 0)
-    s_exact = 0;
-  __syncthreads();
-  unsigned *dst = reinterpret_cast<unsigned *>(codes + fbase) + q0;
-  unsigned exact = 0;
-#pragma unroll
-  for(int it = 0; it < ITERS; it++)
-    if(q0 + it * SSD_PT_THREADS < nquads)
-    {
-      float vx[4], vy[4], vz[4];
-      word_unpack(F, w[it], vx, vy, vz);
-      tb_word(p, vx, vy, vz, dst + it * SSD_PT_THREADS, s_hist, exact);
-    }
-  if(exact)
-    atomicAdd(&s_exact, exact);
-  __syncthreads();
-  const unsigned sum = s_hist[tid];
-  if(sum)
-    atomicAdd(&frames[frame_slot(cam, frame)].hist[tid], sum);
-  if(tid == 0 && s_exact)
-    atomicAdd(&frames[frame_slot(cam, frame)].n_exact_bin, s_exact);
-  if(FUSE_PEAKS)
-  {
-    __shared__ PeaksScratch K;
-    __shared__ unsigned s_last;
-    tb_fused_peaks(p, frames[frame_slot(cam, frame)], K, s_last, tid);
-  }
-}
-
 // ---------------------------------------------------------------------------------------------
 // k_peaks: HeightsHistogram::findPeaks/filterPeaks (pointcloud.cpp:214-256), the plateau bands of
 // PlateausExtraction::extractPlateauPoints (:300-335) folded into a bin->label LUT, and the ground /
