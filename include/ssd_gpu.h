@@ -382,6 +382,55 @@ int ssd_gpu_set_step_labels(ssd_gpu_ctx *ctx, int enable);
 int ssd_gpu_get_step_labels(ssd_gpu_ctx *ctx, int frame, uint8_t *out_host);
 /* Device pointer to the step labels of the last call (n_frames * width*height bytes). */
 int ssd_gpu_step_labels_device_ptr(ssd_gpu_ctx *ctx, const uint8_t **out);
+/*
+ * Step surfaces: what the point set behind each step's height looks like -- a level tread, a ramp, a tread with something on
+ * it, or a floor seen through a tilted calibration. For step s of frame f of the last call, the points are the pixels with
+ * step_labels == s (in a group call: of every member frame of the group), each taken as its exact double-precision world
+ * point (wx, wy, wz) through the frame's own camera (CameraToWorld, as ssd_gpu_camera_to_world). Definition (restated in
+ * tests/native/oracle_step_surfaces.c: ssd_oracle_step_surfaces):
+ *   fixed point: X = (int64)((wx - x_min) * 65536), Y = (int64)((wy - y_min) * 65536), Z = (int64)((wz - z_min) * 65536) with
+ *     the configuration's range bounds (>= 0: the points are in range);
+ *   exact integer moments n, Sx, Sy, Sz, Sxx, Sxy, Syy, Sxz, Syz, Szz (Sxy = sum X*Y, ...) and Zmin, Zmax: independent of the
+ *     order the points are visited in;
+ *   on the host, in double without FMA contraction, each integer below converted to double once:
+ *     cxx = n*Sxx - Sx*Sx, cxy = n*Sxy - Sx*Sy, cyy = n*Syy - Sy*Sy, cxz = n*Sxz - Sx*Sz, cyz = n*Syz - Sy*Sz,
+ *       czz = n*Szz - Sz*Sz (exact in signed 128-bit arithmetic, then converted);
+ *     det = cxx*cyy - cxy*cxy; fit_valid = n >= 3 && det > 0;
+ *     a = (cxz*cyy - cyz*cxy) / det, b = (cyz*cxx - cxz*cxy) / det: the least-squares plane z = a x + b y + c through the
+ *       centroid;
+ *     rms_dz = sqrt(max(czz - a*cxz - b*cyz, 0)) / n / 65536 metres (RMS vertical residual: flatness);
+ *     tilt_deg = atan(sqrt(a*a + b*b)) * (180 / M_PI);
+ *     a, b, tilt_deg and rms_dz are 0 when fit_valid is 0;
+ *   reported in the external world of ssd_gpu_step, through the ToExternalWorld the step's corners went through (plain calls:
+ *   the context's; camera calls: the frame's camera's; group calls: the group's first member's camera's), in k_finalize's
+ *   operation order: xm = x_min + (double)Sx / (double)n / 65536 (ym, zm likewise),
+ *     centroid = ((ext_a[0]*xm + ext_a[1]*ym) + ext_b[0], (ext_a[2]*xm + ext_a[3]*ym) + ext_b[1], ext_z + zm),
+ *     gradient = (ext_a[0]*a + ext_a[1]*b, ext_a[2]*a + ext_a[3]*b) (for a rotation: dz/dx, dz/dy in the rotated axes),
+ *     z_lo = ext_z + (z_min + (double)Zmin / 65536), z_hi likewise with Zmax.
+ * n == 0 (a step with SSD_STATUS_EMPTY_MEAN) gives an all-zero record. The ground step with an invalid front edge still gets
+ * the surface of the pixels its step labels mark. n_points = n_in_quad of the step's plateau.
+ * The option only reports: it changes no step, label or other result. It reads the step labels, so enabling it while step
+ * labels are off, and switching step labels off while it is on, return SSD_E_STATE. Enabling allocates
+ * max_frames * SSD_GPU_MAX_STEPS moment records (SSD_E_NOMEM, and the option stays off, when that fails) and returns SSD_E_RANGE
+ * for a configuration with a range (x_max - x_min, y_max - y_min or z_max - z_min) of 65536 m or more, for which X, Y or Z
+ * could reach 2^32 (the bound under which the moments are exact); enable == 0 frees them. The pass runs after the chain of
+ * every ssd_gpu_process_* call and is counted in timing.n_launches. The getter returns SSD_E_STATE when the option is off,
+ * the last call ran without it or its results are no longer readable (a failed call, a single-stage entry point), SSD_E_RANGE
+ * for a frame outside the last call. Results are fixed when the call runs: replacing the camera table afterwards changes none.
+ */
+typedef struct ssd_gpu_step_surface
+{
+  uint32_t n_points;    /* points of the step: count(step_labels == s) over the frame / group */
+  int32_t fit_valid;    /* n >= 3 && det > 0 */
+  double centroid[3];   /* metres, external world */
+  double gradient[2];   /* dz/dx, dz/dy of the fitted plane, external axes */
+  double tilt_deg;      /* angle of the plane from level, degrees */
+  double rms_dz;        /* RMS vertical residual about the plane, metres */
+  double z_lo, z_hi;    /* z extent of the points, metres, external world */
+} ssd_gpu_step_surface; /* 80 bytes */
+int ssd_gpu_set_step_surfaces(ssd_gpu_ctx *ctx, int enable);
+/* out[0..min(*n, cap)): *n = n_steps of the frame, in the order of ssd_gpu_get_steps. */
+int ssd_gpu_get_step_surfaces(ssd_gpu_ctx *ctx, int frame, ssd_gpu_step_surface *out, int cap, int *n);
 /* Per-pixel segment labels (device -> host copy of width*height bytes). */
 int ssd_gpu_get_labels(ssd_gpu_ctx *ctx, int frame, uint8_t *out_host);
 /* Height histogram, HeightsHistogram::calcHist (pointcloud.cpp:194-204). */

@@ -408,6 +408,19 @@ class Detector:
         self._ck(self._l.ssd_gpu_step_labels_device_ptr(self._h, C.byref(p)), "ssd_gpu_step_labels_device_ptr")
         return p.value
 
+    def set_step_surfaces(self, enable=True):
+        """Step surfaces (include/ssd_gpu.h: ssd_gpu_set_step_surfaces): least-squares plane, tilt, flatness and z extent of the
+        points each step is measured from. Needs the step labels on; one more pass over the points of the following calls."""
+        self._ck(self._l.ssd_gpu_set_step_surfaces(self._h, 1 if enable else 0), "ssd_gpu_set_step_surfaces")
+
+    def step_surfaces(self, frame):
+        """list of dicts, one per step of steps(frame), in the same order"""
+        out = (A.StepSurface * A.MAX_STEPS)()
+        n = C.c_int()
+        self._ck(self._l.ssd_gpu_get_step_surfaces(self._h, frame, out, A.MAX_STEPS, C.byref(n)), "ssd_gpu_get_step_surfaces")
+        return [{f: (tuple(getattr(r, f)) if f in ("centroid", "gradient") else getattr(r, f)) for f, _ in A.StepSurface._fields_}
+                for r in out[:n.value]]
+
     def n_steps_all(self, n_frames):
         out = np.empty(n_frames, np.int32)
         n = C.c_int()

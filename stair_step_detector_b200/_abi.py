@@ -80,6 +80,11 @@ class Riser(C.Structure):
                 ("x_mean", C.c_double), ("y_mean", C.c_double), ("z_bottom", C.c_double), ("z_top", C.c_double)]
 
 
+class StepSurface(C.Structure):
+    _fields_ = [("n_points", C.c_uint32), ("fit_valid", C.c_int32), ("centroid", C.c_double * 3), ("gradient", C.c_double * 2),
+                ("tilt_deg", C.c_double), ("rms_dz", C.c_double), ("z_lo", C.c_double), ("z_hi", C.c_double)]
+
+
 class Step(C.Structure):
     _fields_ = [("height", C.c_double), ("quad", (C.c_double * 2) * 4)]
 
@@ -158,6 +163,8 @@ PROTOTYPES = {
     "ssd_gpu_set_step_labels": (C.c_int, [_vp, C.c_int]),
     "ssd_gpu_get_step_labels": (C.c_int, [_vp, C.c_int, _vp]),
     "ssd_gpu_step_labels_device_ptr": (C.c_int, [_vp, _P(_vp)]),
+    "ssd_gpu_set_step_surfaces": (C.c_int, [_vp, C.c_int]),
+    "ssd_gpu_get_step_surfaces": (C.c_int, [_vp, C.c_int, _P(StepSurface), C.c_int, _P(C.c_int)]),
     "ssd_gpu_get_frame_info": (C.c_int, [_vp, C.c_int, _P(FrameInfo)]),
     "ssd_gpu_get_plateaus": (C.c_int, [_vp, C.c_int, _P(Plateau), C.c_int, _P(C.c_int)]),
     "ssd_gpu_get_labels": (C.c_int, [_vp, C.c_int, _vp]),

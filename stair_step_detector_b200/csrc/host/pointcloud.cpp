@@ -69,7 +69,8 @@ std::vector<Quadrilateralf_t> Pointcloud::overlay(int frame) const
   return out;
 }
 
-// overlay / vertical faces / step labels / camera table as last requested, once the context exists
+// overlay / vertical faces / step labels / step surfaces / camera table as last requested, once the context exists (the surfaces
+// read the step labels: they go off before the labels and on after them)
 void Pointcloud::applySettings() const
 {
   if(_overlay && !_overlayApplied)
@@ -86,11 +87,23 @@ void Pointcloud::applySettings() const
       throw std::runtime_error(std::string("ssd_gpu_set_vertical_faces: ") + ssd_gpu_last_error(_ctx));
     _risersApplied = _risers;
   }
+  if(!_stepSurfaces && _stepSurfacesApplied)
+  {
+    if(ssd_gpu_set_step_surfaces(_ctx, 0) != SSD_OK)
+      throw std::runtime_error(std::string("ssd_gpu_set_step_surfaces: ") + ssd_gpu_last_error(_ctx));
+    _stepSurfacesApplied = false;
+  }
   if(_stepLabels != _stepLabelsApplied)
   {
     if(ssd_gpu_set_step_labels(_ctx, _stepLabels ? 1 : 0) != SSD_OK)
       throw std::runtime_error(std::string("ssd_gpu_set_step_labels: ") + ssd_gpu_last_error(_ctx));
     _stepLabelsApplied = _stepLabels;
+  }
+  if(_stepSurfaces && !_stepSurfacesApplied)
+  {
+    if(ssd_gpu_set_step_surfaces(_ctx, 1) != SSD_OK)
+      throw std::runtime_error(std::string("ssd_gpu_set_step_surfaces: ") + ssd_gpu_last_error(_ctx));
+    _stepSurfacesApplied = true;
   }
   if(!_camerasApplied)
   {
@@ -276,6 +289,24 @@ std::vector<uint8_t> Pointcloud::stepLabels(int frame) const
   if(ssd_gpu_get_step_labels(_ctx, frame, l.data()) != SSD_OK)
     throw std::runtime_error(std::string("ssd_gpu_get_step_labels: ") + ssd_gpu_last_error(_ctx));
   return l;
+}
+
+void Pointcloud::enableStepSurfaces(bool enable) const
+{
+  _stepSurfaces = enable;
+  if(enable)
+    _stepLabels = true;
+}
+
+std::vector<ssd_gpu_step_surface> Pointcloud::stepSurfaces(int frame) const
+{
+  if(!_ctx)
+    throw std::logic_error("Pointcloud::stepSurfaces before any frame was processed");
+  ssd_gpu_step_surface s[SSD_GPU_MAX_STEPS];
+  int n = 0;
+  if(ssd_gpu_get_step_surfaces(_ctx, frame, s, SSD_GPU_MAX_STEPS, &n) != SSD_OK)
+    throw std::runtime_error(std::string("ssd_gpu_get_step_surfaces: ") + ssd_gpu_last_error(_ctx));
+  return std::vector<ssd_gpu_step_surface>(s, s + n);
 }
 
 std::vector<uint8_t> Pointcloud::labels(int frame) const

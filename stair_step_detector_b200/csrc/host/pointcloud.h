@@ -69,6 +69,10 @@ public:
   // pointcloud.cpp:560-572), SSD_STEP_LABEL_NONE elsewhere; definition: include/ssd_gpu.h, ssd_gpu_set_step_labels
   void enableStepLabels(bool enable = true) const;
   std::vector<uint8_t> stepLabels(int frame = 0) const;
+  // step surfaces: least-squares plane, tilt, flatness and z extent of the points each step is measured from; definition:
+  // include/ssd_gpu.h, ssd_gpu_set_step_surfaces. Enabling them also enables the step labels they are computed from.
+  void enableStepSurfaces(bool enable = true) const;
+  std::vector<ssd_gpu_step_surface> stepSurfaces(int frame = 0) const;
   ssd_gpu_ctx *context() const { return _ctx; }
 
 private:
@@ -84,6 +88,7 @@ private:
   mutable bool _overlay = false, _overlayApplied = false;
   mutable bool _risers = false, _risersApplied = false;
   mutable bool _stepLabels = false, _stepLabelsApplied = false;
+  mutable bool _stepSurfaces = false, _stepSurfacesApplied = false;
   mutable ssd_gpu_intrinsics _overlayIntrinsics{};
   mutable ssd_gpu_distortion _overlayDistortion{}, _lensApplied{};
   mutable std::vector<ssd_gpu_camera> _cameras;

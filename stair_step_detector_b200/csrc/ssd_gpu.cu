@@ -22,6 +22,12 @@
 
 static thread_local std::string g_create_error;
 
+// ToExternalWorld of one result record (ssd_gpu_get_step_surfaces), taken when the call runs
+struct SurfaceXf
+{
+  double ext_a[4], ext_b[2], ext_z;
+};
+
 struct ssd_gpu_ctx
 {
   int device = 0;
@@ -62,6 +68,10 @@ struct ssd_gpu_ctx
   unsigned char *d_step_labels = nullptr; // max_frames * N, allocated by ssd_gpu_set_step_labels
   bool step_labels = false;       // ssd_gpu_set_step_labels: k_quad_reduce's STEPS variant writes d_step_labels
   bool step_labels_last = false;  // the last accepted process call wrote them
+  SurfaceDev *d_surf = nullptr;   // max_frames * SSD_GPU_MAX_STEPS, allocated by ssd_gpu_set_step_surfaces
+  bool surfaces = false;          // ssd_gpu_set_step_surfaces: k_step_surface after the chain
+  bool surfaces_last = false;     // the last accepted process call ran it
+  std::vector<SurfaceXf> surf_xf; // per record of the last call: the ToExternalWorld its surfaces are reported through
   int pt_blocks_target = 0;       // blocks per launch of the tile-looping point kernels
   int n_frames_last = 0;
   int flags_last = 0;
@@ -585,6 +595,15 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SRC &src, int frame0, i
     k_riser_reduce<SRC, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, src, labels, frames, cam);
     *launches += 1;
   }
+  if(ctx->surfaces)
+  {
+    // optional pass: step surfaces from the step labels k_quad_reduce wrote. The memset clears the chunk's records (not counted in
+    // timing.n_launches, like the step labels' memset).
+    SurfaceDev *surf = ctx->d_surf + (size_t)rec0 * SSD_GPU_MAX_STEPS;
+    CK(cudaMemsetAsync(surf, 0, sizeof(SurfaceDev) * SSD_GPU_MAX_STEPS * (size_t)nr, st));
+    k_step_surface<SRC, CAM><<<gpt2q, SSD_PT_THREADS, 0, st>>>(p, src, ctx->d_step_labels + (size_t)frame0 * p.N, frames, surf, cam);
+    *launches += 1;
+  }
   CK(cudaGetLastError());
   return SSD_OK;
 }
@@ -664,6 +683,7 @@ void ssd_gpu_destroy(ssd_gpu_ctx *ctx)
   cudaFreeHost(ctx->h_ovl);
   cudaFree(ctx->d_labels);
   cudaFree(ctx->d_step_labels);
+  cudaFree(ctx->d_surf);
   cudaFree(ctx->d_bev);
   cudaFree(ctx->d_img);
   cudaFree(ctx->d_xn);
@@ -1061,6 +1081,7 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
   ctx->n_frames_last = n_frames;
   ctx->flags_last = flags;
   ctx->step_labels_last = ctx->step_labels;
+  ctx->surfaces_last = ctx->surfaces;
   ctx->grp_of_frame.clear();
   ctx->grp_members.clear();
   ctx->grp_epsc.clear();
@@ -1108,6 +1129,19 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
     grp.group = ctx->d_grp_of_frame;
     grp.members = ctx->d_grp_members;
     grp.epsc = ctx->d_grp_epsc;
+  }
+  if(ctx->surfaces)
+  {
+    // each record's ToExternalWorld as k_finalize uses it: the context's, the frame's camera's, the group's first member's
+    ctx->surf_xf.resize((size_t)n_records);
+    for(int r = 0; r < n_records; r++)
+    {
+      const DevParams &d = !cam_of_frame ? ctx->dp : ctx->cam_dp[cam_of_frame[group_frames ? ctx->grp_members[r].x : r]];
+      SurfaceXf &x = ctx->surf_xf[r];
+      memcpy(x.ext_a, d.ext_a, sizeof(x.ext_a));
+      memcpy(x.ext_b, d.ext_b, sizeof(x.ext_b));
+      x.ext_z = d.ext_z;
+    }
   }
   // the whole call is ordered after ev_start on stream 0; stream 1 joins via events
   CK(cudaEventRecord(ctx->ev_start, ctx->stream[0]));
@@ -1251,6 +1285,7 @@ static int process_common(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z1
       cudaMemset(ctx->d_bev, 0, (size_t)ctx->n_streams * ctx->chunk_frames * SSD_GPU_MAX_PLATEAUS * ctx->bm_words * 4);
     ctx->n_frames_last = 0;
     ctx->step_labels_last = false;
+    ctx->surfaces_last = false;
     ctx->err = keep;
   }
   return rc;
@@ -1764,6 +1799,8 @@ int ssd_gpu_set_step_labels(ssd_gpu_ctx *ctx, int enable)
 {
   if(!ctx)
     return SSD_E_INVALID_ARG;
+  if(!enable && ctx->surfaces)
+    return fail(ctx, SSD_E_STATE, "ssd_gpu_set_step_labels: step surfaces are on and read the step labels (ssd_gpu_set_step_surfaces)");
   CK(cudaSetDevice(ctx->device));
   if((enable != 0) != ctx->step_labels)
     ctx->step_labels_last = false; // the map of an earlier call is not kept across a switch
@@ -1823,6 +1860,109 @@ int ssd_gpu_step_labels_device_ptr(ssd_gpu_ctx *ctx, const uint8_t **out)
   if(rc)
     return rc;
   *out = ctx->d_step_labels;
+  return SSD_OK;
+}
+
+int ssd_gpu_set_step_surfaces(ssd_gpu_ctx *ctx, int enable)
+{
+  if(!ctx)
+    return SSD_E_INVALID_ARG;
+  if(enable && !ctx->step_labels)
+    return fail(ctx, SSD_E_STATE, "ssd_gpu_set_step_surfaces: the pass reads the step labels, which are off (ssd_gpu_set_step_labels)");
+  const ssd_gpu_config &c = ctx->cfg;
+  // fixed-point coordinates below 2^32 (k_step_surface): every range shorter than 65536 m
+  if(enable && !(c.x_max - c.x_min < 65536.0 && c.y_max - c.y_min < 65536.0 && c.z_max - c.z_min < 65536.0))
+    return fail(ctx, SSD_E_RANGE, "ssd_gpu_set_step_surfaces: a measuring range of 65536 m or more (the moments are exact below it)");
+  CK(cudaSetDevice(ctx->device));
+  if((enable != 0) != ctx->surfaces)
+    ctx->surfaces_last = false; // the surfaces of an earlier call are not kept across a switch
+  if(!enable)
+  {
+    // the pointer and the flag are cleared whatever the free returns: a failed free must not leave a pointer to free again
+    const cudaError_t e = cudaFree(ctx->d_surf);
+    ctx->d_surf = nullptr;
+    ctx->surfaces = false;
+    if(e != cudaSuccess)
+      return fail(ctx, SSD_E_CUDA, std::string("ssd_gpu_set_step_surfaces: ") + cudaGetErrorString(e));
+    return SSD_OK;
+  }
+  if(!ctx->d_surf)
+  {
+    const cudaError_t e = cudaMalloc(&ctx->d_surf, sizeof(SurfaceDev) * SSD_GPU_MAX_STEPS * (size_t)ctx->max_frames);
+    if(e != cudaSuccess)
+    {
+      cudaGetLastError(); // clear the sticky allocation error: the context stays usable
+      ctx->d_surf = nullptr;
+      ctx->surfaces = false;
+      return fail(ctx, SSD_E_NOMEM, std::string("ssd_gpu_set_step_surfaces: ") + cudaGetErrorString(e));
+    }
+  }
+  ctx->surfaces = true;
+  return SSD_OK;
+}
+
+// 128-bit moments of one step (SurfaceDev) as signed 128-bit integers
+static __int128 u128_of(const unsigned long long m[2])
+{
+  return (__int128)(((unsigned __int128)m[1] << 64) | m[0]);
+}
+
+// The fields of include/ssd_gpu.h (ssd_gpu_step_surface) from the moments of one step and its record's ToExternalWorld.
+// Double arithmetic in the stated order; the host build passes -ffp-contract=off.
+static ssd_gpu_step_surface derive_surface(const SurfaceDev &m, const SurfaceXf &x, const ssd_gpu_config &c)
+{
+  ssd_gpu_step_surface o;
+  memset(&o, 0, sizeof(o));
+  if(m.n == 0)
+    return o;
+  const __int128 n = m.n, Sx = m.sx, Sy = m.sy, Sz = m.sz;
+  const __int128 Sxx = u128_of(m.m2[0]), Sxy = u128_of(m.m2[1]), Syy = u128_of(m.m2[2]), Sxz = u128_of(m.m2[3]), Syz = u128_of(m.m2[4]),
+                 Szz = u128_of(m.m2[5]);
+  const double cxx = (double)(n * Sxx - Sx * Sx), cxy = (double)(n * Sxy - Sx * Sy), cyy = (double)(n * Syy - Sy * Sy);
+  const double cxz = (double)(n * Sxz - Sx * Sz), cyz = (double)(n * Syz - Sy * Sz), czz = (double)(n * Szz - Sz * Sz);
+  const double det = cxx * cyy - cxy * cxy;
+  const double dn = (double)m.n;
+  o.n_points = m.n;
+  o.fit_valid = m.n >= 3 && det > 0;
+  double a = 0, b = 0;
+  if(o.fit_valid)
+  {
+    a = (cxz * cyy - cyz * cxy) / det;
+    b = (cyz * cxx - cxz * cxy) / det;
+    const double r = czz - a * cxz - b * cyz;
+    o.rms_dz = std::sqrt(r > 0 ? r : 0.0) / dn / 65536.0;
+    o.tilt_deg = std::atan(std::sqrt(a * a + b * b)) * (180.0 / M_PI);
+  }
+  const double xm = c.x_min + (double)m.sx / dn / 65536.0, ym = c.y_min + (double)m.sy / dn / 65536.0, zm = c.z_min + (double)m.sz / dn / 65536.0;
+  o.centroid[0] = (x.ext_a[0] * xm + x.ext_a[1] * ym) + x.ext_b[0];
+  o.centroid[1] = (x.ext_a[2] * xm + x.ext_a[3] * ym) + x.ext_b[1];
+  o.centroid[2] = x.ext_z + zm;
+  o.gradient[0] = x.ext_a[0] * a + x.ext_a[1] * b;
+  o.gradient[1] = x.ext_a[2] * a + x.ext_a[3] * b;
+  o.z_lo = x.ext_z + (c.z_min + (double)~m.zmin_inv / 65536.0);
+  o.z_hi = x.ext_z + (c.z_min + (double)m.zmax / 65536.0);
+  return o;
+}
+
+int ssd_gpu_get_step_surfaces(ssd_gpu_ctx *ctx, int frame, ssd_gpu_step_surface *out, int cap, int *n)
+{
+  const int rc = check_frame(ctx, frame);
+  if(rc)
+    return rc;
+  if(!ctx->surfaces || !ctx->surfaces_last)
+    return fail(ctx, SSD_E_STATE, "ssd_gpu_get_step_surfaces: not enabled for the last call (ssd_gpu_set_step_surfaces)");
+  const int r = frame_record(ctx, frame);
+  const int ns = ctx->h_out[r].info.n_steps;
+  if(n)
+    *n = ns;
+  const int k = out ? std::min(ns, cap) : 0;
+  if(k <= 0)
+    return SSD_OK;
+  CK(cudaSetDevice(ctx->device));
+  std::vector<SurfaceDev> m((size_t)k);
+  CK(cudaMemcpy(m.data(), ctx->d_surf + (size_t)r * SSD_GPU_MAX_STEPS, sizeof(SurfaceDev) * (size_t)k, cudaMemcpyDeviceToHost));
+  for(int s = 0; s < k; s++)
+    out[s] = derive_surface(m[s], ctx->surf_xf[r], ctx->cfg);
   return SSD_OK;
 }
 

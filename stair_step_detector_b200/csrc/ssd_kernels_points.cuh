@@ -1715,3 +1715,190 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_riser_reduce(const __grid_co
     atomicMax(&R.ymax, S.ymax[tid]);
   }
 }
+
+// ---------------------------------------------------------------------------------------------
+// k_step_surface: the exact integer moments of each step's points (include/ssd_gpu.h: ssd_gpu_set_step_surfaces). Optional
+// pass after the chain, launched only when step surfaces are on; it reads the step labels k_quad_reduce wrote and nothing the
+// chain reads afterwards. The words of the map that hold a step pixel (a byte other than SSD_STEP_LABEL_NONE) are compacted,
+// their points re-read and taken through the exact double-precision CameraToWorld. Fixed point X = (wx - x_min) * 65536 (Y, Z
+// likewise) is below 2^32 (ssd_gpu_set_step_surfaces refuses ranges of 65536 m or more), so every product is one u32 x u32 ->
+// u64 multiply and the second moments are summed in 128 bits. Per-lane running segment per step, shared-memory accumulators
+// per block, one set of global atomics per step and block; the record is the frame's (frame_slot: a group's members accumulate
+// into the group's). Integer sums: the result does not depend on the order of the points.
+// ---------------------------------------------------------------------------------------------
+// moments of one step; cleared to zero before the pass (zmin is kept as the largest ~Z, so zero is the identity of both extremes)
+struct SurfaceDev
+{
+  unsigned n, zmin_inv, zmax, pad;
+  unsigned long long sx, sy, sz;
+  unsigned long long m2[6][2]; // Sxx, Sxy, Syy, Sxz, Syz, Szz: {low, high} 64-bit halves
+};
+
+struct SurfaceShared
+{
+  SurfaceDev acc[SSD_GPU_MAX_STEPS];
+  unsigned lab[SSD_PT_WARPS][SSD_WT_PX / 4];
+  unsigned short act[SSD_PT_WARPS][SSD_WT_PX / 4];
+};
+
+struct SurfaceSeg
+{
+  unsigned s, n, zmin, zmax;
+  unsigned long long sx, sy, sz;
+  unsigned __int128 m2[6];
+};
+
+// a 128-bit add as two 64-bit atomics: the low half's carry is detected from the value it replaced, so the sum of the high
+// halves counts every wrap of the low half exactly once
+__device__ __forceinline__ void atomic_add_u128(unsigned long long *lohi, unsigned __int128 v)
+{
+  const unsigned long long lo = (unsigned long long)v, hi = (unsigned long long)(v >> 64);
+  const unsigned long long old = atomicAdd(lohi, lo);
+  const unsigned long long h = hi + (old + lo < old ? 1ull : 0ull);
+  if(h)
+    atomicAdd(lohi + 1, h);
+}
+
+__device__ __forceinline__ void surface_seg_clear(SurfaceSeg &g)
+{
+  g.n = 0;
+  g.zmin = 0xffffffffu;
+  g.zmax = 0;
+  g.sx = g.sy = g.sz = 0;
+#pragma unroll
+  for(int k = 0; k < 6; k++)
+    g.m2[k] = 0;
+}
+
+__device__ __forceinline__ void surface_flush(SurfaceShared &S, SurfaceSeg &g)
+{
+  if(g.n)
+  {
+    SurfaceDev &A = S.acc[g.s];
+    atomicAdd(&A.n, g.n);
+    atomicMax(&A.zmin_inv, ~g.zmin);
+    atomicMax(&A.zmax, g.zmax);
+    atomicAdd(&A.sx, g.sx);
+    atomicAdd(&A.sy, g.sy);
+    atomicAdd(&A.sz, g.sz);
+#pragma unroll
+    for(int k = 0; k < 6; k++)
+      atomic_add_u128(A.m2[k], g.m2[k]);
+  }
+  surface_seg_clear(g);
+}
+
+template<class SRC, class CAM = NoCam>
+__global__ void __launch_bounds__(SSD_PT_THREADS) k_step_surface(const __grid_constant__ DevParams p0, const SRC src0,
+                                                                 const unsigned char *__restrict__ steps, const FrameDev *__restrict__ frames,
+                                                                 SurfaceDev *__restrict__ surf, const CAM cam = CAM())
+{
+  __shared__ SurfaceShared S;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int frame = blockIdx.y;
+  const DevParams &p = frame_params(p0, cam, frame);
+  const auto &src = frame_src(src0, cam, p, frame);
+  const int slot = frame_slot(cam, frame);
+  if(frames[slot].quad_amask == 0u)
+    return; // no step: the frame's map is all SSD_STEP_LABEL_NONE
+  const size_t fbase = (size_t)frame * p.N;
+  const unsigned *st32 = reinterpret_cast<const unsigned *>(steps + fbase);
+  const int nquads = p.N >> 2;
+  int wt, wt_end, wt_stride;
+  warp_tile_range((p.N + SSD_WT_PX - 1) / SSD_WT_PX, warp, wt, wt_end, wt_stride);
+  {
+    unsigned long long *a = reinterpret_cast<unsigned long long *>(S.acc);
+    for(int i = tid; i < (int)(sizeof(S.acc) / 8); i += SSD_PT_THREADS)
+      a[i] = 0;
+  }
+  __syncthreads();
+  unsigned short *act = S.act[warp];
+  unsigned *labs = S.lab[warp];
+  const typename SrcTraits<SRC>::Frame FR = src_frame(src, p, fbase);
+  SurfaceSeg g;
+  g.s = 0;
+  surface_seg_clear(g);
+
+  for(; wt < wt_end; wt += wt_stride)
+  {
+    const unsigned wbase = (unsigned)wt * (SSD_WT_PX / 4);
+    // ---- phase A: words with a step pixel (a byte other than 255) ----
+    unsigned n = 0;
+#pragma unroll
+    for(int it = 0; it < SSD_WT_WORDS; it++)
+    {
+      const int q = wt * (SSD_WT_PX / 4) + it * 32 + lane;
+      const unsigned lw = q < nquads ? __ldg(st32 + q) : 0xffffffffu;
+      const unsigned x = ~lw;                                                       // non-zero byte <=> step pixel
+      const unsigned nz = ((x & 0x7f7f7f7fu) + 0x7f7f7f7fu) | x;                      // bit 7 of every non-zero byte
+      const unsigned am4 = (((nz >> 7) & 0x01010101u) * 0x10204080u) >> 28;
+      if(__any_sync(0xffffffffu, am4 != 0u))
+      {
+        if(am4)
+          labs[it * 32 + lane] = lw;
+        n = compact_append(act, n, am4, it, lane);
+      }
+    }
+    if(n == 0)
+      continue;
+    __syncwarp();
+    // ---- phase B: the step points of the compacted words ----
+    for(unsigned s0 = 0; s0 < n; s0 += 32)
+    {
+      const unsigned i0 = s0 + lane;
+      const unsigned e = i0 < n ? act[i0] : 0u;
+      if(e)
+      {
+        const unsigned lw = labs[e >> 4];
+        typename SrcTraits<SRC>::Word w;
+        word_load(FR, wbase + (e >> 4), w);
+        float vx[4], vy[4], vz[4];
+        word_unpack(FR, w, vx, vy, vz);
+#pragma unroll
+        for(int j = 0; j < 4; j++)
+          if((e >> j) & 1u)
+          {
+            double wx, wy, wz;
+            camera_to_world(p, vx[j], vy[j], vz[j], wx, wy, wz);
+            const unsigned X = (unsigned)(long long)((wx - p.x_min) * 65536.0), Y = (unsigned)(long long)((wy - p.y_min) * 65536.0),
+                           Z = (unsigned)(long long)((wz - p.z_min) * 65536.0);
+            const unsigned s = (lw >> (8 * j)) & 0xffu;
+            if(s != g.s)
+            {
+              surface_flush(S, g);
+              g.s = s;
+            }
+            g.n++;
+            g.zmin = min(g.zmin, Z);
+            g.zmax = max(g.zmax, Z);
+            g.sx += X;
+            g.sy += Y;
+            g.sz += Z;
+            g.m2[0] += (unsigned long long)X * X;
+            g.m2[1] += (unsigned long long)X * Y;
+            g.m2[2] += (unsigned long long)Y * Y;
+            g.m2[3] += (unsigned long long)X * Z;
+            g.m2[4] += (unsigned long long)Y * Z;
+            g.m2[5] += (unsigned long long)Z * Z;
+          }
+      }
+    }
+    __syncwarp();
+  }
+  surface_flush(S, g);
+  __syncthreads();
+  if(tid < SSD_GPU_MAX_STEPS && S.acc[tid].n)
+  {
+    const SurfaceDev &A = S.acc[tid];
+    SurfaceDev &R = surf[(size_t)slot * SSD_GPU_MAX_STEPS + tid];
+    atomicAdd(&R.n, A.n);
+    atomicMax(&R.zmin_inv, A.zmin_inv);
+    atomicMax(&R.zmax, A.zmax);
+    atomicAdd(&R.sx, A.sx);
+    atomicAdd(&R.sy, A.sy);
+    atomicAdd(&R.sz, A.sz);
+#pragma unroll
+    for(int k = 0; k < 6; k++)
+      atomic_add_u128(R.m2[k], ((unsigned __int128)A.m2[k][1] << 64) | A.m2[k][0]);
+  }
+}
