@@ -300,6 +300,33 @@ int ssd_gpu_process_depth_groups_host(ssd_gpu_ctx *ctx, const uint16_t *z16_host
 int ssd_gpu_process_depth_groups_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const int32_t *camera_of_frame, const int32_t *group_frames,
                                         int n_groups, int flags);
 
+/*
+ * ---- float depth frames: 32-bit depth images (ROS 32FC1, simulators, stereo matchers, depth networks) ----
+ * A float depth frame is width*height float samples, row-major, the layout of a z16 frame. A pixel is deprojected exactly as a
+ * z16 pixel, with the sample in place of (float)count:
+ *     z = depth * depth_unit,  then X = z * x, Y = z * y     (single-rounded f32 operations, no FMA; (x, y) from the pin-hole
+ *                                                              tables or the lens's ray table, as for z16)
+ * depth_unit is the same intrinsics field with the same check (> 0): 1.0f for depth in metres (exact), 0.001f for float
+ * millimetres. There are no special cases; what follows comes from the z > 0 test and the range filter:
+ *  - NaN, -inf, +-0 and negative samples are the invalid pixel (label SSD_LABEL_INVALID, not counted in n_nonzero);
+ *  - +inf, and a finite sample whose product with depth_unit overflows, give a vertex with z > 0 and a non-finite world
+ *    point: SSD_LABEL_OUT_OF_RANGE, counted in n_nonzero, as the same vertex given as vertex input would be;
+ *  - subnormal samples are kept (the library is built without flush-to-zero).
+ * So depth_f32[i] = (float)z16[i] with the same intrinsics gives, bit for bit, what the z16 call gives, and any float frame gives
+ * what the vertex call gives on the vertices deprojected on the host by the f32 operations above.
+ * Each entry point mirrors its z16 counterpart argument for argument, with every check, lens, option and getter of that call.
+ * The input must be 16-byte aligned (SSD_E_INVALID_ARG otherwise): the point kernels read 4 pixels per 16-byte load. Host input
+ * crosses PCIe at 4 bytes per pixel, through staging buffers of its own.
+ */
+int ssd_gpu_process_depth_f32_host(ssd_gpu_ctx *ctx, const float *depth_host, const ssd_gpu_intrinsics *intr, int n_frames);
+int ssd_gpu_process_depth_f32_device(ssd_gpu_ctx *ctx, const float *depth_dev, const ssd_gpu_intrinsics *intr, int n_frames);
+int ssd_gpu_process_depth_f32_cameras_host(ssd_gpu_ctx *ctx, const float *depth_host, const int32_t *camera_of_frame, int n_frames);
+int ssd_gpu_process_depth_f32_cameras_device(ssd_gpu_ctx *ctx, const float *depth_dev, const int32_t *camera_of_frame, int n_frames);
+int ssd_gpu_process_depth_f32_groups_host(ssd_gpu_ctx *ctx, const float *depth_host, const int32_t *camera_of_frame,
+                                          const int32_t *group_frames, int n_groups);
+int ssd_gpu_process_depth_f32_groups_device(ssd_gpu_ctx *ctx, const float *depth_dev, const int32_t *camera_of_frame,
+                                            const int32_t *group_frames, int n_groups, int flags);
+
 /* ---- results of the last process call ---- */
 /* Stairs of one frame: out[0..*n) ; replaces the value printed at pointcloud.cpp:624-625. */
 int ssd_gpu_get_steps(ssd_gpu_ctx *ctx, int frame, ssd_gpu_step *out, int cap, int *n, uint32_t *status);

@@ -256,6 +256,18 @@ class Detector:
     def process_depth_device(self, dev_ptr, intrinsics, n_frames):
         self._ck(self._l.ssd_gpu_process_depth_device(self._h, dev_ptr, C.byref(intrinsics), n_frames), "ssd_gpu_process_depth_device")
 
+    # ---- float depth frames: one float32 sample per pixel, deprojected as z = sample * depth_unit (include/ssd_gpu.h) ----
+    def process_depth_f32_host(self, depth, intrinsics):
+        """depth: (n_frames, H, W) float32 depth frames in host memory (e.g. ROS 32FC1 in metres with depth_unit = 1.0).
+        The buffer must be 16-byte aligned."""
+        depth = np.ascontiguousarray(depth, np.float32)
+        n = depth.size // self.n_points
+        self._ck(self._l.ssd_gpu_process_depth_f32_host(self._h, _ptr(depth), C.byref(intrinsics), n), "ssd_gpu_process_depth_f32_host")
+        return n
+
+    def process_depth_f32_device(self, dev_ptr, intrinsics, n_frames):
+        self._ck(self._l.ssd_gpu_process_depth_f32_device(self._h, dev_ptr, C.byref(intrinsics), n_frames), "ssd_gpu_process_depth_f32_device")
+
     def deproject_device(self, depth_dev, intrinsics, n_frames, xyz_dev):
         self._ck(self._l.ssd_gpu_deproject_device(self._h, depth_dev, C.byref(intrinsics), n_frames, xyz_dev), "ssd_gpu_deproject_device")
 
@@ -318,6 +330,19 @@ class Detector:
         cams = self._cams(camera_of_frame, n_frames)
         self._ck(self._l.ssd_gpu_process_depth_cameras_device(self._h, dev_ptr, _ptr(cams), n_frames), "ssd_gpu_process_depth_cameras_device")
 
+    def process_depth_f32_cameras_host(self, depth, camera_of_frame):
+        """depth as for process_depth_f32_host; each frame is deprojected with its camera's intrinsics and lens."""
+        depth = np.ascontiguousarray(depth, np.float32)
+        n = depth.size // self.n_points
+        cams = self._cams(camera_of_frame, n)
+        self._ck(self._l.ssd_gpu_process_depth_f32_cameras_host(self._h, _ptr(depth), _ptr(cams), n), "ssd_gpu_process_depth_f32_cameras_host")
+        return n
+
+    def process_depth_f32_cameras_device(self, dev_ptr, camera_of_frame, n_frames):
+        cams = self._cams(camera_of_frame, n_frames)
+        self._ck(self._l.ssd_gpu_process_depth_f32_cameras_device(self._h, dev_ptr, _ptr(cams), n_frames),
+                 "ssd_gpu_process_depth_f32_cameras_device")
+
     # ---- frame groups: one detection from the union of several frames' points (include/ssd_gpu.h) ----
     @staticmethod
     def _groups(group_frames, n_frames=None):
@@ -355,6 +380,22 @@ class Detector:
         cams = self._cams(camera_of_frame, int(g.sum()))
         self._ck(self._l.ssd_gpu_process_depth_groups_device(self._h, dev_ptr, _ptr(cams), _ptr(g), g.size, flags),
                  "ssd_gpu_process_depth_groups_device")
+
+    def process_depth_f32_groups_host(self, depth, camera_of_frame, group_frames):
+        """depth as for process_depth_f32_host; each frame is deprojected with its camera's intrinsics and lens."""
+        depth = np.ascontiguousarray(depth, np.float32)
+        n = depth.size // self.n_points
+        cams = self._cams(camera_of_frame, n)
+        g = self._groups(group_frames, n)
+        self._ck(self._l.ssd_gpu_process_depth_f32_groups_host(self._h, _ptr(depth), _ptr(cams), _ptr(g), g.size),
+                 "ssd_gpu_process_depth_f32_groups_host")
+        return n
+
+    def process_depth_f32_groups_device(self, dev_ptr, camera_of_frame, group_frames, flags=0):
+        g = self._groups(group_frames)
+        cams = self._cams(camera_of_frame, int(g.sum()))
+        self._ck(self._l.ssd_gpu_process_depth_f32_groups_device(self._h, dev_ptr, _ptr(cams), _ptr(g), g.size, flags),
+                 "ssd_gpu_process_depth_f32_groups_device")
 
     # ---- results ----
     def steps(self, frame):

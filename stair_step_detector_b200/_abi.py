@@ -154,6 +154,12 @@ PROTOTYPES = {
     "ssd_gpu_process_depth_groups_device": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int]),
     "ssd_gpu_process_depth_host": (C.c_int, [_vp, _vp, _P(Intrinsics), C.c_int]),
     "ssd_gpu_process_depth_device": (C.c_int, [_vp, _vp, _P(Intrinsics), C.c_int]),
+    "ssd_gpu_process_depth_f32_host": (C.c_int, [_vp, _vp, _P(Intrinsics), C.c_int]),
+    "ssd_gpu_process_depth_f32_device": (C.c_int, [_vp, _vp, _P(Intrinsics), C.c_int]),
+    "ssd_gpu_process_depth_f32_cameras_host": (C.c_int, [_vp, _vp, _vp, C.c_int]),
+    "ssd_gpu_process_depth_f32_cameras_device": (C.c_int, [_vp, _vp, _vp, C.c_int]),
+    "ssd_gpu_process_depth_f32_groups_host": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int]),
+    "ssd_gpu_process_depth_f32_groups_device": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int]),
     "ssd_gpu_deproject_device": (C.c_int, [_vp, _vp, _P(Intrinsics), C.c_int, _vp]),
     "ssd_gpu_get_steps": (C.c_int, [_vp, C.c_int, _P(Step), C.c_int, _P(C.c_int), _P(C.c_uint32)]),
     "ssd_gpu_set_overlay": (C.c_int, [_vp, _P(C.c_double), _P(Intrinsics)]),

@@ -117,8 +117,9 @@ std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, i
 {
   ensureContext(frames.width(), frames.height());
   applySettings();
-  // the lens of the plain call: the frame's for z16 frames, the overlay's for vertex frames (set only when it changes)
-  const ssd_gpu_distortion &lens = frames.z16 ? frames.distortion : _overlayDistortion;
+  // the lens of the plain call: the frame's for depth frames (z16 or float), the overlay's for vertex frames (set only when it
+  // changes)
+  const ssd_gpu_distortion &lens = frames.isDepth() ? frames.distortion : _overlayDistortion;
   if(memcmp(&lens, &_lensApplied, sizeof(lens)) != 0)
   {
     if(ssd_gpu_set_distortion(_ctx, &lens) != SSD_OK)
@@ -129,6 +130,9 @@ std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, i
   if(frames.z16)
     rc = frames.onDevice ? ssd_gpu_process_depth_device(_ctx, frames.z16, &frames.intrinsics, nFrames)
                          : ssd_gpu_process_depth_host(_ctx, frames.z16, &frames.intrinsics, nFrames);
+  else if(frames.depthF32)
+    rc = frames.onDevice ? ssd_gpu_process_depth_f32_device(_ctx, frames.depthF32, &frames.intrinsics, nFrames)
+                         : ssd_gpu_process_depth_f32_host(_ctx, frames.depthF32, &frames.intrinsics, nFrames);
   else
     rc = frames.onDevice ? ssd_gpu_process_device(_ctx, frames.vertices, nFrames) : ssd_gpu_process_host(_ctx, frames.vertices, nFrames);
   if(rc != SSD_OK)
@@ -172,6 +176,9 @@ std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, i
   if(frames.z16)
     rc = frames.onDevice ? ssd_gpu_process_depth_cameras_device(_ctx, frames.z16, cam, nFrames)
                          : ssd_gpu_process_depth_cameras_host(_ctx, frames.z16, cam, nFrames);
+  else if(frames.depthF32)
+    rc = frames.onDevice ? ssd_gpu_process_depth_f32_cameras_device(_ctx, frames.depthF32, cam, nFrames)
+                         : ssd_gpu_process_depth_f32_cameras_host(_ctx, frames.depthF32, cam, nFrames);
   else
     rc = frames.onDevice ? ssd_gpu_process_cameras_device(_ctx, frames.vertices, cam, nFrames)
                          : ssd_gpu_process_cameras_host(_ctx, frames.vertices, cam, nFrames);
@@ -198,6 +205,9 @@ std::vector<Stairs> Pointcloud::processGroups(const Camera::DepthFrame &frames, 
   if(frames.z16)
     rc = frames.onDevice ? ssd_gpu_process_depth_groups_device(_ctx, frames.z16, cam, grp, nGroups, 0)
                          : ssd_gpu_process_depth_groups_host(_ctx, frames.z16, cam, grp, nGroups);
+  else if(frames.depthF32)
+    rc = frames.onDevice ? ssd_gpu_process_depth_f32_groups_device(_ctx, frames.depthF32, cam, grp, nGroups, 0)
+                         : ssd_gpu_process_depth_f32_groups_host(_ctx, frames.depthF32, cam, grp, nGroups);
   else
     rc = frames.onDevice ? ssd_gpu_process_groups_device(_ctx, frames.vertices, cam, grp, nGroups, 0)
                          : ssd_gpu_process_groups_host(_ctx, frames.vertices, cam, grp, nGroups);

@@ -57,8 +57,8 @@ public:
   // (WorldToCamera, then DepthFrame::project with these depth-stream intrinsics). The quadrilaterals the reference
   // hands to drawQuadrilateral are then available per frame after process()/processBatch().
   void enableOverlay(const ssd_gpu_intrinsics &intrinsics) const;
-  // ... through a lens (ssd_gpu_set_distortion). The overlay of z16 frames uses the lens of the frame (DepthFrame::distortion),
-  // the overlay of vertex frames this one.
+  // ... through a lens (ssd_gpu_set_distortion). The overlay of depth frames (z16 or float) uses the lens of the frame
+  // (DepthFrame::distortion), the overlay of vertex frames this one.
   void enableOverlay(const ssd_gpu_intrinsics &intrinsics, const ssd_gpu_distortion &distortion) const;
   std::vector<Quadrilateralf_t> overlay(int frame = 0) const;
   // vertical faces (risers) from the remainder points -- the reference stops at "TODO use remainder to detect vertical faces"

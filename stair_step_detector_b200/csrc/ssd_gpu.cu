@@ -62,6 +62,7 @@ struct ssd_gpu_ctx
   unsigned *d_bev = nullptr; // 2 x chunk_frames * MAX_PLATEAUS * bm_words (per stream)
   float *d_stage[SSD_MAX_STREAMS]{};            // vertex staging of the host-input calls (host_chunk_frames)
   uint16_t *d_depth[SSD_MAX_STREAMS]{};         // z16 staging of the host depth-frame path
+  float *d_depth_f32[SSD_MAX_STREAMS]{};        // float-depth staging of the host float-depth path (its own: 4 B per pixel)
   float *d_xn = nullptr, *d_yn = nullptr;       // deprojection tables: (u - ppx) / fx per column, (v - ppy) / fy per row
   ssd_gpu_intrinsics intr{};                    // intrinsics the tables were built for
   bool risers = false;            // ssd_gpu_set_vertical_faces: k_riser_reduce after the chain
@@ -495,7 +496,7 @@ __global__ void k_single_camera_to_world(const __grid_constant__ DevParams p, co
   }
 }
 
-// Pass 1 (k_transform_bin): packed vertices through the kernel's bulk-copy staging, z16 frames (SrcDepth, SrcLens) from registers
+// Pass 1 (k_transform_bin): packed vertices through the kernel's bulk-copy staging, depth frames (SrcDepthT, SrcLensT) from registers
 template<bool FUSE, class CAM>
 static void launch_transform_bin(const dim3 &grid, cudaStream_t st, const DevParams &p, const SrcVertices &src, unsigned char *labels,
                                  FrameDev *frames, const CAM &cam)
@@ -510,7 +511,7 @@ static void launch_transform_bin(const dim3 &grid, cudaStream_t st, const DevPar
 }
 
 // The classic chain: k_transform_bin -> k_peaks -> k_label_bev -> k_outline -> k_frame_logic -> k_quad_reduce -> k_finalize
-// (+ k_riser_reduce), for one chunk of frames on stream s. SRC: where the points come from (SrcVertices, SrcDepth, SrcLens), its
+// (+ k_riser_reduce), for one chunk of frames on stream s. SRC: where the points come from (SrcVertices, SrcDepthT, SrcLensT), its
 // input pointer the chunk's. CAM = NoCam: every frame with the context's own camera; CamTable: each frame with its camera's
 // parameters (camera calls); GroupTable: as CamTable, with the frames of each group accumulated into one record (group calls).
 // OL: the outline work area of the frame size (OutlineSharedSmall, OutlineShared).
@@ -618,7 +619,7 @@ static SrcVertices chunk_src(SrcVertices s, const void *in)
 template<class SRC>
 static SRC chunk_src(SRC s, const void *in)
 {
-  s.z16 = static_cast<const uint16_t *>(in);
+  s.depth = static_cast<decltype(s.depth)>(in);
   return s;
 }
 static NoCam chunk_cam(NoCam c, int, int)
@@ -707,6 +708,7 @@ void ssd_gpu_destroy(ssd_gpu_ctx *ctx)
   {
     cudaFree(ctx->d_stage[i]);
     cudaFree(ctx->d_depth[i]);
+    cudaFree(ctx->d_depth_f32[i]);
     if(ctx->stream[i])
       cudaStreamDestroy(ctx->stream[i]);
     if(ctx->ev_in_ready[i])
@@ -957,19 +959,41 @@ static int ensure_deproject_tables(ssd_gpu_ctx *ctx, const ssd_gpu_intrinsics &i
   return SSD_OK;
 }
 
-// xyz != nullptr: packed vertices; else z16 depth frames + intrinsics (deprojected chunk by chunk into the vertex staging)
+} // extern "C": the templates of the depth sample type follow
+
+// The depth staging buffers of sample type T: each sample type has its own, so that a buffer is never read with another width.
+static uint16_t **depth_staging(ssd_gpu_ctx *ctx, const uint16_t *)
+{
+  return ctx->d_depth;
+}
+static float **depth_staging(ssd_gpu_ctx *ctx, const float *)
+{
+  return ctx->d_depth_f32;
+}
+// A call's depth pointer; its sample type T is named by the entry point (a vertex call passes none to deduce it from).
+template<class T>
+struct Samples
+{
+  typedef const T *ptr;
+};
+
+// xyz != nullptr: packed vertices; else depth frames of sample type T (z16 counts or float) + intrinsics, deprojected inside the
+// point kernels
 // cam_of_frame != nullptr: a camera call (validated by check_cameras; the depth tables are the camera table's, intr is unused)
 // group_frames != nullptr: a group call of n_groups groups (validated by check_groups; a camera call as well)
-static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16, const ssd_gpu_intrinsics *intr, bool host_input, int n_frames,
+template<class T>
+static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const T *depth, const ssd_gpu_intrinsics *intr, bool host_input, int n_frames,
                         int flags, const int32_t *cam_of_frame, const int32_t *group_frames, int n_groups)
 {
-  if(!ctx || (!xyz && !(z16 && (intr || cam_of_frame))) || n_frames <= 0)
+  if(!ctx || (!xyz && !(depth && (intr || cam_of_frame))) || n_frames <= 0)
     return fail(ctx, SSD_E_INVALID_ARG, "process: bad argument");
   if(n_frames > ctx->max_frames)
     return fail(ctx, SSD_E_RANGE, "process: n_frames exceeds max_frames of the context");
-  // the point kernels use 16-byte vector loads / bulk copies (vertices) and 8-byte loads (depth)
-  if((xyz && ((uintptr_t)xyz & 15u)) || (z16 && ((uintptr_t)z16 & 7u)))
-    return fail(ctx, SSD_E_INVALID_ARG, "process: the input buffer must be 16-byte aligned (vertices) / 8-byte aligned (depth)");
+  // the point kernels use 16-byte vector loads / bulk copies (vertices), one load per 4-pixel word of depth (8 bytes of z16,
+  // 16 bytes of float)
+  if((xyz && ((uintptr_t)xyz & 15u)) || (depth && ((uintptr_t)depth & (4 * sizeof(T) - 1))))
+    return fail(ctx, SSD_E_INVALID_ARG, sizeof(T) == 2 ? "process: the input buffer must be 16-byte aligned (vertices) / 8-byte aligned (depth)"
+                                                       : "process: float depth input must be 16-byte aligned");
   CK(cudaSetDevice(ctx->device));
   const DevParams &p = ctx->dp;
   const size_t frame_floats = (size_t)p.N * 3;
@@ -988,7 +1012,7 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
   const bool depth_input = xyz == nullptr;
   // a distorted lens: depth frames read their rays from ray tables (SrcLens), the overlay projects through the lens (LensCam)
   const bool plain_lens = !cam_of_frame && !ssd_lens_is_pinhole(&ctx->lens);
-  SrcLens sl{};
+  SrcLensT<T> sl{};
   bool use_lens = false;
   const ssd_gpu_distortion *ov_lens = nullptr;
   if(cam_of_frame)
@@ -1050,15 +1074,18 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
       {
         CK(cudaFree(ctx->d_stage[i]));
         CK(cudaFree(ctx->d_depth[i]));
+        CK(cudaFree(ctx->d_depth_f32[i]));
         ctx->d_stage[i] = nullptr;
         ctx->d_depth[i] = nullptr;
+        ctx->d_depth_f32[i] = nullptr;
       }
       ctx->stage_frames = max_nf;
     }
+    T **dstage = depth_staging(ctx, depth);
     for(int i = 0; i < ctx->n_streams; i++)
     {
-      if(depth_input && !ctx->d_depth[i])
-        CK(cudaMalloc(&ctx->d_depth[i], (size_t)ctx->stage_frames * p.N * sizeof(uint16_t)));
+      if(depth_input && !dstage[i])
+        CK(cudaMalloc(&dstage[i], (size_t)ctx->stage_frames * p.N * sizeof(T)));
       if(!depth_input && !ctx->d_stage[i])
         CK(cudaMalloc(&ctx->d_stage[i], (size_t)ctx->stage_frames * frame_floats * sizeof(float)));
     }
@@ -1170,7 +1197,7 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
     {
       const int f0 = chunks[chunk].f0, nf = chunks[chunk].nf;
       const int s = (flags & SSD_FLAG_SINGLE_STREAM) ? 0 : chunk % ctx->n_streams;
-      const void *in = depth_input ? (const void *)(z16 + (size_t)f0 * p.N) : (const void *)(xyz + (size_t)f0 * frame_floats);
+      const void *in = depth_input ? (const void *)(depth + (size_t)f0 * p.N) : (const void *)(xyz + (size_t)f0 * frame_floats);
       if(host_input)
       {
         // staging buffer s may be overwritten once the chunk that last used it has consumed it
@@ -1178,8 +1205,9 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
           CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_in_free[s], 0));
         if(depth_input)
         {
-          CK(cudaMemcpyAsync(ctx->d_depth[s], in, (size_t)nf * p.N * sizeof(uint16_t), cudaMemcpyHostToDevice, ctx->copy_stream));
-          in = ctx->d_depth[s];
+          T *dst = depth_staging(ctx, depth)[s];
+          CK(cudaMemcpyAsync(dst, in, (size_t)nf * p.N * sizeof(T), cudaMemcpyHostToDevice, ctx->copy_stream));
+          in = dst;
         }
         else
         {
@@ -1218,7 +1246,7 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
   {
     // depth frames are deprojected inside the point kernels with the pin-hole tables (a camera call's per camera)
     const unsigned long long wmagic = (((unsigned long long)1 << 40) + (unsigned long long)p.W - 1) / (unsigned long long)p.W;
-    rc = run_source(SrcDepth{ z16, ctx->d_xn, ctx->d_yn, intr ? intr->depth_unit : 0.f, wmagic });
+    rc = run_source(SrcDepthT<T>{ depth, ctx->d_xn, ctx->d_yn, intr ? intr->depth_unit : 0.f, wmagic });
   }
   if(rc)
     return rc;
@@ -1272,10 +1300,11 @@ static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16,
 // A failure inside the chain (launch error, bad user pointer, out of memory while growing a staging buffer) may leave streams
 // unsynchronised and BEV bitmaps half written: the bitmaps are "self-cleaning" only along a complete chain. Bring the context
 // back to a clean state so that the next call starts from zeroed bitmaps and no stale results can be read.
-static int process_common(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z16, const ssd_gpu_intrinsics *intr, bool host_input, int n_frames,
-                          int flags, const int32_t *cam_of_frame = nullptr, const int32_t *group_frames = nullptr, int n_groups = 0)
+template<class T = uint16_t>
+static int process_common(ssd_gpu_ctx *ctx, const float *xyz, typename Samples<T>::ptr depth, const ssd_gpu_intrinsics *intr, bool host_input,
+                          int n_frames, int flags, const int32_t *cam_of_frame = nullptr, const int32_t *group_frames = nullptr, int n_groups = 0)
 {
-  const int rc = process_impl(ctx, xyz, z16, intr, host_input, n_frames, flags, cam_of_frame, group_frames, n_groups);
+  const int rc = process_impl<T>(ctx, xyz, depth, intr, host_input, n_frames, flags, cam_of_frame, group_frames, n_groups);
   if(rc != SSD_OK && rc != SSD_E_INVALID_ARG && rc != SSD_E_RANGE && ctx)
   {
     const std::string keep = ctx->err;
@@ -1290,6 +1319,9 @@ static int process_common(ssd_gpu_ctx *ctx, const float *xyz, const uint16_t *z1
   }
   return rc;
 }
+
+extern "C"
+{
 
 int ssd_gpu_process_host(ssd_gpu_ctx *ctx, const float *xyz_host, int n_frames)
 {
@@ -1318,6 +1350,20 @@ int ssd_gpu_process_depth_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, cons
   if(!z16_dev || !intr)
     return fail(ctx, SSD_E_INVALID_ARG, "process_depth: bad argument");
   return process_common(ctx, nullptr, z16_dev, intr, false, n_frames, 0);
+}
+
+int ssd_gpu_process_depth_f32_host(ssd_gpu_ctx *ctx, const float *depth_host, const ssd_gpu_intrinsics *intr, int n_frames)
+{
+  if(!depth_host || !intr)
+    return fail(ctx, SSD_E_INVALID_ARG, "process_depth_f32: bad argument");
+  return process_common<float>(ctx, nullptr, depth_host, intr, true, n_frames, 0);
+}
+
+int ssd_gpu_process_depth_f32_device(ssd_gpu_ctx *ctx, const float *depth_dev, const ssd_gpu_intrinsics *intr, int n_frames)
+{
+  if(!depth_dev || !intr)
+    return fail(ctx, SSD_E_INVALID_ARG, "process_depth_f32: bad argument");
+  return process_common<float>(ctx, nullptr, depth_dev, intr, false, n_frames, 0);
 }
 
 // ---- per-frame cameras ----
@@ -1591,6 +1637,18 @@ int ssd_gpu_process_depth_cameras_device(ssd_gpu_ctx *ctx, const uint16_t *z16_d
   return rc ? rc : process_common(ctx, nullptr, z16_dev, nullptr, false, n_frames, 0, camera_of_frame);
 }
 
+int ssd_gpu_process_depth_f32_cameras_host(ssd_gpu_ctx *ctx, const float *depth_host, const int32_t *camera_of_frame, int n_frames)
+{
+  const int rc = check_cameras(ctx, depth_host, camera_of_frame, n_frames, true);
+  return rc ? rc : process_common<float>(ctx, nullptr, depth_host, nullptr, true, n_frames, 0, camera_of_frame);
+}
+
+int ssd_gpu_process_depth_f32_cameras_device(ssd_gpu_ctx *ctx, const float *depth_dev, const int32_t *camera_of_frame, int n_frames)
+{
+  const int rc = check_cameras(ctx, depth_dev, camera_of_frame, n_frames, true);
+  return rc ? rc : process_common<float>(ctx, nullptr, depth_dev, nullptr, false, n_frames, 0, camera_of_frame);
+}
+
 // Everything a group call can be refused for, before anything is launched (the previous results stay readable). *n_frames: the
 // call's frames.
 static int check_groups(ssd_gpu_ctx *ctx, const void *input, const int32_t *cam_of_frame, const int32_t *group_frames, int n_groups, bool depth,
@@ -1643,6 +1701,22 @@ int ssd_gpu_process_depth_groups_device(ssd_gpu_ctx *ctx, const uint16_t *z16_de
   int n = 0;
   const int rc = check_groups(ctx, z16_dev, camera_of_frame, group_frames, n_groups, true, &n);
   return rc ? rc : process_common(ctx, nullptr, z16_dev, nullptr, false, n, flags, camera_of_frame, group_frames, n_groups);
+}
+
+int ssd_gpu_process_depth_f32_groups_host(ssd_gpu_ctx *ctx, const float *depth_host, const int32_t *camera_of_frame, const int32_t *group_frames,
+                                          int n_groups)
+{
+  int n = 0;
+  const int rc = check_groups(ctx, depth_host, camera_of_frame, group_frames, n_groups, true, &n);
+  return rc ? rc : process_common<float>(ctx, nullptr, depth_host, nullptr, true, n, 0, camera_of_frame, group_frames, n_groups);
+}
+
+int ssd_gpu_process_depth_f32_groups_device(ssd_gpu_ctx *ctx, const float *depth_dev, const int32_t *camera_of_frame, const int32_t *group_frames,
+                                            int n_groups, int flags)
+{
+  int n = 0;
+  const int rc = check_groups(ctx, depth_dev, camera_of_frame, group_frames, n_groups, true, &n);
+  return rc ? rc : process_common<float>(ctx, nullptr, depth_dev, nullptr, false, n, flags, camera_of_frame, group_frames, n_groups);
 }
 
 int ssd_gpu_deproject_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const ssd_gpu_intrinsics *intr, int n_frames, float *xyz_dev)

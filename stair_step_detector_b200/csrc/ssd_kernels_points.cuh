@@ -47,7 +47,7 @@ __device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity)
 }
 
 // ---------------------------------------------------------------------------------------------
-// Where the point kernels read their vertices from. Two sources, chosen at launch (template parameter):
+// Where the point kernels read their vertices from. Two kinds of source, chosen at launch (template parameter):
 //   SrcVertices : the packed rs2::vertex array (12 B/point) -- what rs2::pointcloud::calculate returns
 //                 (pointcloud.cpp:138-147);
 //   SrcDepth    : the z16 depth frame itself (2 B/point) -- what Pointcloud::process receives (pointcloud.cpp:608).
@@ -55,6 +55,9 @@ __device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity)
 //                 rs2_deproject_pixel_to_point / camera.h:99-116) is evaluated in registers, with the single-rounded f32
 //                 operations of ssd_deproject_pixel (scene_model.h) / k_deproject: the vertices never exist in memory
 //                 and all three passes move 2 bytes per point instead of 12.
+// The depth sources (SrcDepthT, SrcLensT) are templated on the sample type T: uint16_t (z16 counts, SrcDepth / SrcLens) or
+// float (float depth frames, SrcDepthF32 / SrcLensF32, 4 B/point). A sample is converted to float and deprojected the same
+// way either way: z = (float)sample * unit.
 // A kernel derives a frame cursor once (src_frame), then loads 4-point words (word_load: where a kernel issues it ahead of use, the
 // registers of a word in flight are the raw loads) and unpacks them where they are consumed (word_unpack).
 // ---------------------------------------------------------------------------------------------
@@ -62,41 +65,82 @@ struct SrcVertices
 {
   const float *xyz; // n_frames x N x {x, y, z}
 };
-struct SrcDepth
+// The four samples of a 4-pixel word: one 8-byte load of z16 counts, one 16-byte load of float samples.
+template<class T>
+struct DepthWord;
+template<>
+struct DepthWord<uint16_t>
 {
-  const uint16_t *z16;         // n_frames x N
+  typedef uint2 type;
+};
+template<>
+struct DepthWord<float>
+{
+  typedef float4 type;
+};
+// sample j (0..3, a constant) of a word, as float
+__device__ __forceinline__ float word_sample(const uint2 &d, int j)
+{
+  const unsigned h = j < 2 ? d.x : d.y;
+  return (float)((j & 1) ? h >> 16 : h & 0xffffu);
+}
+__device__ __forceinline__ float word_sample(const float4 &d, int j)
+{
+  return j == 0 ? d.x : j == 1 ? d.y : j == 2 ? d.z : d.w;
+}
+// one sample by its pixel index (the compacted exact passes), converted to float where it is used
+__device__ __forceinline__ unsigned sample_load(const uint16_t *d, unsigned pt)
+{
+  return __ldg(reinterpret_cast<const unsigned short *>(d) + pt);
+}
+__device__ __forceinline__ float sample_load(const float *d, unsigned pt)
+{
+  return __ldg(d + pt);
+}
+template<class T>
+struct SrcDepthT
+{
+  const T *depth;              // n_frames x N samples
   const float *xn, *yn;        // (u - ppx) / fx per column, (v - ppy) / fy per row (k_deproject_tables)
   float unit;                  // metres per depth unit
   unsigned long long wmagic;   // ceil(2^40 / W): row of pixel i = (i * wmagic) >> 40, exact for i * W < 2^40
 };
-// SrcLens: z16 frames of a camera with a distorted lens (ssd_gpu_set_distortion). Its ray (x, y) depends on u and v, so it is
-// read per pixel from the lens's ray table (k_lens_rays): 2 B of depth + 8 B of ray per point, the table shared by every frame
-// of the lens and L2-resident at the usual frame sizes. Then X = z * x, Y = z * y as for SrcDepth.
-struct SrcLens
+// SrcLensT: depth frames of a camera with a distorted lens (ssd_gpu_set_distortion). Its ray (x, y) depends on u and v, so it is
+// read per pixel from the lens's ray table (k_lens_rays): 2 B (z16) or 4 B (float) of depth + 8 B of ray per point, the table
+// shared by every frame of the lens and L2-resident at the usual frame sizes. Then X = z * x, Y = z * y as for SrcDepthT.
+template<class T>
+struct SrcLensT
 {
-  const uint16_t *z16;              // n_frames x N
+  const T *depth;                   // n_frames x N samples
   const float2 *ray;                // N rays of the lens (plain calls)
   const float2 *const *cam_ray;     // camera calls: the ray table of each camera (a pin-hole camera's holds (xn[u], yn[v]))
   float unit;
 };
+typedef SrcDepthT<uint16_t> SrcDepth;
+typedef SrcLensT<uint16_t> SrcLens;
+typedef SrcDepthT<float> SrcDepthF32;
+typedef SrcLensT<float> SrcLensF32;
 struct FrameV
 {
   const float4 *f4;
 };
+template<class T>
 struct FrameL
 {
-  const uint2 *d2;    // four z16 pixels per element
-  const float4 *r4;   // two rays per element
+  const typename DepthWord<T>::type *d2; // four pixels per element
+  const float4 *r4;                      // two rays per element
   float unit;
 };
+template<class T>
 struct WordL
 {
-  uint2 d;
+  typename DepthWord<T>::type d;
   float4 r01, r23;
 };
+template<class T>
 struct FrameD
 {
-  const uint2 *d2; // four z16 pixels per element
+  const typename DepthWord<T>::type *d2; // four pixels per element
   const float *xn, *yn;
   float unit;
   unsigned long long wmagic;
@@ -106,9 +150,10 @@ struct WordV
 {
   float4 a, b, c;
 };
+template<class T>
 struct WordD
 {
-  uint2 d;
+  typename DepthWord<T>::type d;
   float4 x4;
   float y;
 };
@@ -120,51 +165,55 @@ struct SrcTraits<SrcVertices>
   typedef FrameV Frame;
   typedef WordV Word;
 };
-template<>
-struct SrcTraits<SrcDepth>
+template<class T>
+struct SrcTraits<SrcDepthT<T>>
 {
-  typedef FrameD Frame;
-  typedef WordD Word;
+  typedef FrameD<T> Frame;
+  typedef WordD<T> Word;
 };
-template<>
-struct SrcTraits<SrcLens>
+template<class T>
+struct SrcTraits<SrcLensT<T>>
 {
-  typedef FrameL Frame;
-  typedef WordL Word;
+  typedef FrameL<T> Frame;
+  typedef WordL<T> Word;
 };
-__device__ __forceinline__ FrameL src_frame(const SrcLens &s, const DevParams &, size_t fbase)
+template<class T>
+__device__ __forceinline__ FrameL<T> src_frame(const SrcLensT<T> &s, const DevParams &, size_t fbase)
 {
-  FrameL f;
-  f.d2 = reinterpret_cast<const uint2 *>(s.z16 + fbase);
+  FrameL<T> f;
+  f.d2 = reinterpret_cast<const typename DepthWord<T>::type *>(s.depth + fbase);
   f.r4 = reinterpret_cast<const float4 *>(s.ray);
   f.unit = s.unit;
   return f;
 }
-__device__ __forceinline__ SrcLens frame_src(const SrcLens &s, const CamTable &c, const DevParams &, int frame)
+template<class T>
+__device__ __forceinline__ SrcLensT<T> frame_src(const SrcLensT<T> &s, const CamTable &c, const DevParams &, int frame)
 {
   const int cam = frame_camera(c, frame);
-  SrcLens d = s;
+  SrcLensT<T> d = s;
   d.ray = s.cam_ray[cam];
   d.unit = __ldg(c.unit + cam);
   return d;
 }
-__device__ __forceinline__ void word_zero(WordL &r)
+template<class T>
+__device__ __forceinline__ void word_zero(WordL<T> &r)
 {
-  r.d = make_uint2(0u, 0u);
+  r.d = {};
   r.r01 = r.r23 = make_float4(0.f, 0.f, 0.f, 0.f);
 }
-__device__ __forceinline__ void word_load(const FrameL &f, unsigned w, WordL &r)
+template<class T>
+__device__ __forceinline__ void word_load(const FrameL<T> &f, unsigned w, WordL<T> &r)
 {
   r.d = __ldg(f.d2 + w);
   r.r01 = __ldg(f.r4 + (size_t)w * 2);
   r.r23 = __ldg(f.r4 + (size_t)w * 2 + 1);
 }
-__device__ __forceinline__ void word_unpack(const FrameL &f, const WordL &r, float vx[4], float vy[4], float vz[4])
+template<class T>
+__device__ __forceinline__ void word_unpack(const FrameL<T> &f, const WordL<T> &r, float vx[4], float vy[4], float vz[4])
 {
-  vz[0] = __fmul_rn((float)(r.d.x & 0xffffu), f.unit);
-  vz[1] = __fmul_rn((float)(r.d.x >> 16), f.unit);
-  vz[2] = __fmul_rn((float)(r.d.y & 0xffffu), f.unit);
-  vz[3] = __fmul_rn((float)(r.d.y >> 16), f.unit);
+#pragma unroll
+  for(int j = 0; j < 4; j++)
+    vz[j] = __fmul_rn(word_sample(r.d, j), f.unit);
   const float rx[4] = { r.r01.x, r.r01.z, r.r23.x, r.r23.z }, ry[4] = { r.r01.y, r.r01.w, r.r23.y, r.r23.w };
 #pragma unroll
   for(int j = 0; j < 4; j++)
@@ -173,14 +222,16 @@ __device__ __forceinline__ void word_unpack(const FrameL &f, const WordL &r, flo
     vy[j] = __fmul_rn(vz[j], ry[j]);
   }
 }
-__device__ __forceinline__ void word_prefetch_l2(const FrameL &f, unsigned w)
+template<class T>
+__device__ __forceinline__ void word_prefetch_l2(const FrameL<T> &f, unsigned w)
 {
   asm volatile("prefetch.global.L2 [%0];" ::"l"(f.d2 + w));
   asm volatile("prefetch.global.L2 [%0];" ::"l"(f.r4 + (size_t)w * 2)); // the word's 32 bytes of rays: one sector
 }
-__device__ __forceinline__ void point_load(const FrameL &f, unsigned pt, float &x, float &y, float &z)
+template<class T>
+__device__ __forceinline__ void point_load(const FrameL<T> &f, unsigned pt, float &x, float &y, float &z)
 {
-  const unsigned d = __ldg(reinterpret_cast<const unsigned short *>(f.d2) + pt);
+  const auto d = sample_load(reinterpret_cast<const T *>(f.d2), pt);
   const float2 r = __ldg(reinterpret_cast<const float2 *>(f.r4) + pt);
   z = __fmul_rn((float)d, f.unit);
   x = __fmul_rn(z, r.x);
@@ -192,10 +243,11 @@ __device__ __forceinline__ FrameV src_frame(const SrcVertices &s, const DevParam
   f.f4 = reinterpret_cast<const float4 *>(s.xyz + fbase * 3);
   return f;
 }
-__device__ __forceinline__ FrameD src_frame(const SrcDepth &s, const DevParams &p, size_t fbase)
+template<class T>
+__device__ __forceinline__ FrameD<T> src_frame(const SrcDepthT<T> &s, const DevParams &p, size_t fbase)
 {
-  FrameD f;
-  f.d2 = reinterpret_cast<const uint2 *>(s.z16 + fbase);
+  FrameD<T> f;
+  f.d2 = reinterpret_cast<const typename DepthWord<T>::type *>(s.depth + fbase);
   f.xn = s.xn;
   f.yn = s.yn;
   f.unit = s.unit;
@@ -213,10 +265,11 @@ __device__ __forceinline__ SrcVertices frame_src(const SrcVertices &s, const Cam
 {
   return s;
 }
-__device__ __forceinline__ SrcDepth frame_src(const SrcDepth &s, const CamTable &c, const DevParams &p, int frame)
+template<class T>
+__device__ __forceinline__ SrcDepthT<T> frame_src(const SrcDepthT<T> &s, const CamTable &c, const DevParams &p, int frame)
 {
   const int cam = frame_camera(c, frame);
-  SrcDepth d = s;
+  SrcDepthT<T> d = s;
   d.xn = c.xn + (size_t)cam * p.W;
   d.yn = c.yn + (size_t)cam * p.H;
   d.unit = __ldg(c.unit + cam);
@@ -231,9 +284,10 @@ __device__ __forceinline__ void word_zero(WordV &r)
 {
   r.a = r.b = r.c = make_float4(0.f, 0.f, 0.f, 0.f);
 }
-__device__ __forceinline__ void word_zero(WordD &r)
+template<class T>
+__device__ __forceinline__ void word_zero(WordD<T> &r)
 {
-  r.d = make_uint2(0u, 0u);
+  r.d = {};
   r.x4 = make_float4(0.f, 0.f, 0.f, 0.f);
   r.y = 0.f;
 }
@@ -245,7 +299,8 @@ __device__ __forceinline__ void word_load(const FrameV &f, unsigned w, WordV &r)
   r.b = __ldg(src + 1);
   r.c = __ldg(src + 2);
 }
-__device__ __forceinline__ void word_load(const FrameD &f, unsigned w, WordD &r)
+template<class T>
+__device__ __forceinline__ void word_load(const FrameD<T> &f, unsigned w, WordD<T> &r)
 {
   r.d = __ldg(f.d2 + w);
   const unsigned i0 = w * 4u;
@@ -260,12 +315,12 @@ __device__ __forceinline__ void word_unpack(const FrameV &, const WordV &r, floa
   vx[2] = r.b.z, vy[2] = r.b.w, vz[2] = r.c.x;
   vx[3] = r.c.y, vy[3] = r.c.z, vz[3] = r.c.w;
 }
-__device__ __forceinline__ void word_unpack(const FrameD &f, const WordD &r, float vx[4], float vy[4], float vz[4])
+template<class T>
+__device__ __forceinline__ void word_unpack(const FrameD<T> &f, const WordD<T> &r, float vx[4], float vy[4], float vz[4])
 {
-  vz[0] = __fmul_rn((float)(r.d.x & 0xffffu), f.unit);
-  vz[1] = __fmul_rn((float)(r.d.x >> 16), f.unit);
-  vz[2] = __fmul_rn((float)(r.d.y & 0xffffu), f.unit);
-  vz[3] = __fmul_rn((float)(r.d.y >> 16), f.unit);
+#pragma unroll
+  for(int j = 0; j < 4; j++)
+    vz[j] = __fmul_rn(word_sample(r.d, j), f.unit);
   const float xn[4] = { r.x4.x, r.x4.y, r.x4.z, r.x4.w };
 #pragma unroll
   for(int j = 0; j < 4; j++)
@@ -281,9 +336,10 @@ __device__ __forceinline__ void word_prefetch_l2(const FrameV &f, unsigned w)
   asm volatile("prefetch.global.L2 [%0];" ::"l"(src));     // both 32-byte sectors the 48 bytes can touch
   asm volatile("prefetch.global.L2 [%0];" ::"l"(src + 2));
 }
-__device__ __forceinline__ void word_prefetch_l2(const FrameD &f, unsigned w)
+template<class T>
+__device__ __forceinline__ void word_prefetch_l2(const FrameD<T> &f, unsigned w)
 {
-  asm volatile("prefetch.global.L2 [%0];" ::"l"(f.d2 + w));
+  asm volatile("prefetch.global.L2 [%0];" ::"l"(f.d2 + w)); // 8 or 16 bytes: within one sector
 }
 // one point by its index within the frame (the compacted exact passes)
 __device__ __forceinline__ void point_load(const FrameV &f, unsigned pt, float &x, float &y, float &z)
@@ -293,9 +349,10 @@ __device__ __forceinline__ void point_load(const FrameV &f, unsigned pt, float &
   y = __ldg(v + 1);
   z = __ldg(v + 2);
 }
-__device__ __forceinline__ void point_load(const FrameD &f, unsigned pt, float &x, float &y, float &z)
+template<class T>
+__device__ __forceinline__ void point_load(const FrameD<T> &f, unsigned pt, float &x, float &y, float &z)
 {
-  const unsigned d = __ldg(reinterpret_cast<const unsigned short *>(f.d2) + pt);
+  const auto d = sample_load(reinterpret_cast<const T *>(f.d2), pt);
   const unsigned v = (unsigned)(((unsigned long long)pt * f.wmagic) >> 40), u = pt - v * f.W;
   z = __fmul_rn((float)d, f.unit);
   x = __fmul_rn(z, __ldg(f.xn + u));
@@ -689,6 +746,7 @@ __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin(const __grid_c
 // lens: 10 bytes per point in, 2 of depth and 8 of L2-resident ray): 2 bytes per point come in, 1 goes out, the deprojected
 // vertices live in registers only. No staging: the loads are 8 bytes per lane (256 B per warp, coalesced) and all ITERS words
 // of a thread are requested before the first is consumed. Not HBM-bound (3 B/point with SrcDepth): issue-bound.
+// Float depth frames (SrcDepthF32, SrcLensF32) take the same kernel with 16-byte loads: 4 bytes per point come in.
 // ---------------------------------------------------------------------------------------------
 template<int ITERS, bool FUSE_PEAKS, class SRC, class CAM>
 __global__ void __launch_bounds__(SSD_PT_THREADS) k_transform_bin_z16(const __grid_constant__ DevParams p0, const SRC src0,
