@@ -233,46 +233,68 @@ class Detector:
             raise SsdError(f"{what} failed ({rc}): {self._l.ssd_gpu_last_error(self._h).decode()}")
 
     # ---- the hot path ----
+    _VERTICES, _Z16, _F32 = (np.float32, 3), (np.uint16, 1), (np.float32, 1)  # a host array's dtype and values per pixel
+
+    def _process(self, entry, data, kind=None, n_frames=None, intrinsics=None, camera_of_frame=None, group_frames=None, flags=None,
+                 what=None):
+        """One process call through the entry point named entry. data: a host array of the given kind (made contiguous, its frames
+        counted) or, with kind None, a pointer. camera_of_frame / group_frames are checked against the frame count. Returns it."""
+        if kind is not None:
+            data = np.ascontiguousarray(data, kind[0])
+            n_frames = data.size // (self.n_points * kind[1])
+        args = [_ptr(data) if kind is not None else data]
+        if intrinsics is not None:
+            args.append(C.byref(intrinsics))
+        g = None if group_frames is None else np.ascontiguousarray(group_frames, np.int32)
+        if n_frames is None:
+            n_frames = int(g.sum())
+        if camera_of_frame is not None:
+            cams = np.ascontiguousarray(camera_of_frame, np.int32)
+            if cams.size != n_frames:
+                raise ValueError(f"camera_of_frame has {cams.size} entries for {n_frames} frames")
+            args.append(_ptr(cams))
+        if g is None:
+            args.append(n_frames)
+        elif int(g.sum()) != n_frames:
+            raise ValueError(f"group_frames add up to {int(g.sum())} frames, the input holds {n_frames}")
+        else:
+            args += [_ptr(g), g.size]
+        if flags is not None:
+            args.append(flags)
+        self._ck(getattr(self._l, entry)(self._h, *args), what or entry)
+        return n_frames
+
     def process_host(self, xyz):
         """xyz: (n_frames, H, W, 3) or (n_frames, N, 3) float32 host array (pinned or pageable)."""
-        xyz = np.ascontiguousarray(xyz, np.float32)
-        n = xyz.size // (self.n_points * 3)
-        self._ck(self._l.ssd_gpu_process_host(self._h, _ptr(xyz), n), "ssd_gpu_process_host")
-        return n
+        return self._process("ssd_gpu_process_host", xyz, self._VERTICES)
 
     def process_host_ptr(self, ptr, n_frames):
-        self._ck(self._l.ssd_gpu_process_host(self._h, ptr, n_frames), "ssd_gpu_process_host")
+        self._process("ssd_gpu_process_host", ptr, n_frames=n_frames)
 
     def process_depth_host(self, depth, intrinsics):
         """depth: (n_frames, H, W) uint16 z16 depth frames in host memory -- what the reference's process() receives."""
-        depth = np.ascontiguousarray(depth, np.uint16)
-        n = depth.size // self.n_points
-        self._ck(self._l.ssd_gpu_process_depth_host(self._h, _ptr(depth), C.byref(intrinsics), n), "ssd_gpu_process_depth_host")
-        return n
+        return self._process("ssd_gpu_process_depth_host", depth, self._Z16, intrinsics=intrinsics)
 
     def process_depth_host_ptr(self, ptr, intrinsics, n_frames):
-        self._ck(self._l.ssd_gpu_process_depth_host(self._h, ptr, C.byref(intrinsics), n_frames), "ssd_gpu_process_depth_host")
+        self._process("ssd_gpu_process_depth_host", ptr, n_frames=n_frames, intrinsics=intrinsics)
 
     def process_depth_device(self, dev_ptr, intrinsics, n_frames):
-        self._ck(self._l.ssd_gpu_process_depth_device(self._h, dev_ptr, C.byref(intrinsics), n_frames), "ssd_gpu_process_depth_device")
+        self._process("ssd_gpu_process_depth_device", dev_ptr, n_frames=n_frames, intrinsics=intrinsics)
 
     # ---- float depth frames: one float32 sample per pixel, deprojected as z = sample * depth_unit (include/ssd_gpu.h) ----
     def process_depth_f32_host(self, depth, intrinsics):
         """depth: (n_frames, H, W) float32 depth frames in host memory (e.g. ROS 32FC1 in metres with depth_unit = 1.0).
         The buffer must be 16-byte aligned."""
-        depth = np.ascontiguousarray(depth, np.float32)
-        n = depth.size // self.n_points
-        self._ck(self._l.ssd_gpu_process_depth_f32_host(self._h, _ptr(depth), C.byref(intrinsics), n), "ssd_gpu_process_depth_f32_host")
-        return n
+        return self._process("ssd_gpu_process_depth_f32_host", depth, self._F32, intrinsics=intrinsics)
 
     def process_depth_f32_device(self, dev_ptr, intrinsics, n_frames):
-        self._ck(self._l.ssd_gpu_process_depth_f32_device(self._h, dev_ptr, C.byref(intrinsics), n_frames), "ssd_gpu_process_depth_f32_device")
+        self._process("ssd_gpu_process_depth_f32_device", dev_ptr, n_frames=n_frames, intrinsics=intrinsics)
 
     def deproject_device(self, depth_dev, intrinsics, n_frames, xyz_dev):
         self._ck(self._l.ssd_gpu_deproject_device(self._h, depth_dev, C.byref(intrinsics), n_frames, xyz_dev), "ssd_gpu_deproject_device")
 
     def process_device(self, dev_ptr, n_frames, flags=0):
-        self._ck(self._l.ssd_gpu_process_device_ex(self._h, dev_ptr, n_frames, flags), "ssd_gpu_process_device")
+        self._process("ssd_gpu_process_device_ex", dev_ptr, n_frames=n_frames, flags=flags, what="ssd_gpu_process_device")
 
     # ---- per-frame cameras ----
     def set_cameras(self, cameras, distortions=None):
@@ -299,103 +321,52 @@ class Detector:
     def n_cameras(self):
         return self._l.ssd_gpu_n_cameras(self._h)
 
-    @staticmethod
-    def _cams(camera_of_frame, n):
-        cams = np.ascontiguousarray(camera_of_frame, np.int32)
-        if cams.size != n:
-            raise ValueError(f"camera_of_frame has {cams.size} entries for {n} frames")
-        return cams
-
     def process_cameras_host(self, xyz, camera_of_frame):
         """xyz as for process_host; camera_of_frame: camera table index of each frame."""
-        xyz = np.ascontiguousarray(xyz, np.float32)
-        n = xyz.size // (self.n_points * 3)
-        cams = self._cams(camera_of_frame, n)
-        self._ck(self._l.ssd_gpu_process_cameras_host(self._h, _ptr(xyz), _ptr(cams), n), "ssd_gpu_process_cameras_host")
-        return n
+        return self._process("ssd_gpu_process_cameras_host", xyz, self._VERTICES, camera_of_frame=camera_of_frame)
 
     def process_cameras_device(self, dev_ptr, camera_of_frame, n_frames, flags=0):
-        cams = self._cams(camera_of_frame, n_frames)
-        self._ck(self._l.ssd_gpu_process_cameras_device_ex(self._h, dev_ptr, _ptr(cams), n_frames, flags), "ssd_gpu_process_cameras_device")
+        self._process("ssd_gpu_process_cameras_device_ex", dev_ptr, n_frames=n_frames, camera_of_frame=camera_of_frame, flags=flags,
+                      what="ssd_gpu_process_cameras_device")
 
     def process_depth_cameras_host(self, depth, camera_of_frame):
         """depth as for process_depth_host; each frame is deprojected with its camera's intrinsics."""
-        depth = np.ascontiguousarray(depth, np.uint16)
-        n = depth.size // self.n_points
-        cams = self._cams(camera_of_frame, n)
-        self._ck(self._l.ssd_gpu_process_depth_cameras_host(self._h, _ptr(depth), _ptr(cams), n), "ssd_gpu_process_depth_cameras_host")
-        return n
+        return self._process("ssd_gpu_process_depth_cameras_host", depth, self._Z16, camera_of_frame=camera_of_frame)
 
     def process_depth_cameras_device(self, dev_ptr, camera_of_frame, n_frames):
-        cams = self._cams(camera_of_frame, n_frames)
-        self._ck(self._l.ssd_gpu_process_depth_cameras_device(self._h, dev_ptr, _ptr(cams), n_frames), "ssd_gpu_process_depth_cameras_device")
+        self._process("ssd_gpu_process_depth_cameras_device", dev_ptr, n_frames=n_frames, camera_of_frame=camera_of_frame)
 
     def process_depth_f32_cameras_host(self, depth, camera_of_frame):
         """depth as for process_depth_f32_host; each frame is deprojected with its camera's intrinsics and lens."""
-        depth = np.ascontiguousarray(depth, np.float32)
-        n = depth.size // self.n_points
-        cams = self._cams(camera_of_frame, n)
-        self._ck(self._l.ssd_gpu_process_depth_f32_cameras_host(self._h, _ptr(depth), _ptr(cams), n), "ssd_gpu_process_depth_f32_cameras_host")
-        return n
+        return self._process("ssd_gpu_process_depth_f32_cameras_host", depth, self._F32, camera_of_frame=camera_of_frame)
 
     def process_depth_f32_cameras_device(self, dev_ptr, camera_of_frame, n_frames):
-        cams = self._cams(camera_of_frame, n_frames)
-        self._ck(self._l.ssd_gpu_process_depth_f32_cameras_device(self._h, dev_ptr, _ptr(cams), n_frames),
-                 "ssd_gpu_process_depth_f32_cameras_device")
+        self._process("ssd_gpu_process_depth_f32_cameras_device", dev_ptr, n_frames=n_frames, camera_of_frame=camera_of_frame)
 
     # ---- frame groups: one detection from the union of several frames' points (include/ssd_gpu.h) ----
-    @staticmethod
-    def _groups(group_frames, n_frames=None):
-        g = np.ascontiguousarray(group_frames, np.int32)
-        if n_frames is not None and int(g.sum()) != n_frames:
-            raise ValueError(f"group_frames add up to {int(g.sum())} frames, the input holds {n_frames}")
-        return g
-
     def process_groups_host(self, xyz, camera_of_frame, group_frames):
         """xyz as for process_host; camera_of_frame: camera table index of each frame; group_frames: members of each group
         (consecutive frames). Returns the number of frames."""
-        xyz = np.ascontiguousarray(xyz, np.float32)
-        n = xyz.size // (self.n_points * 3)
-        cams = self._cams(camera_of_frame, n)
-        g = self._groups(group_frames, n)
-        self._ck(self._l.ssd_gpu_process_groups_host(self._h, _ptr(xyz), _ptr(cams), _ptr(g), g.size), "ssd_gpu_process_groups_host")
-        return n
+        return self._process("ssd_gpu_process_groups_host", xyz, self._VERTICES, camera_of_frame=camera_of_frame, group_frames=group_frames)
 
     def process_groups_device(self, dev_ptr, camera_of_frame, group_frames, flags=0):
-        g = self._groups(group_frames)
-        cams = self._cams(camera_of_frame, int(g.sum()))
-        self._ck(self._l.ssd_gpu_process_groups_device(self._h, dev_ptr, _ptr(cams), _ptr(g), g.size, flags), "ssd_gpu_process_groups_device")
+        self._process("ssd_gpu_process_groups_device", dev_ptr, camera_of_frame=camera_of_frame, group_frames=group_frames, flags=flags)
 
     def process_depth_groups_host(self, depth, camera_of_frame, group_frames):
         """depth as for process_depth_host; each frame is deprojected with its camera's intrinsics and lens."""
-        depth = np.ascontiguousarray(depth, np.uint16)
-        n = depth.size // self.n_points
-        cams = self._cams(camera_of_frame, n)
-        g = self._groups(group_frames, n)
-        self._ck(self._l.ssd_gpu_process_depth_groups_host(self._h, _ptr(depth), _ptr(cams), _ptr(g), g.size), "ssd_gpu_process_depth_groups_host")
-        return n
+        return self._process("ssd_gpu_process_depth_groups_host", depth, self._Z16, camera_of_frame=camera_of_frame, group_frames=group_frames)
 
     def process_depth_groups_device(self, dev_ptr, camera_of_frame, group_frames, flags=0):
-        g = self._groups(group_frames)
-        cams = self._cams(camera_of_frame, int(g.sum()))
-        self._ck(self._l.ssd_gpu_process_depth_groups_device(self._h, dev_ptr, _ptr(cams), _ptr(g), g.size, flags),
-                 "ssd_gpu_process_depth_groups_device")
+        self._process("ssd_gpu_process_depth_groups_device", dev_ptr, camera_of_frame=camera_of_frame, group_frames=group_frames, flags=flags)
 
     def process_depth_f32_groups_host(self, depth, camera_of_frame, group_frames):
         """depth as for process_depth_f32_host; each frame is deprojected with its camera's intrinsics and lens."""
-        depth = np.ascontiguousarray(depth, np.float32)
-        n = depth.size // self.n_points
-        cams = self._cams(camera_of_frame, n)
-        g = self._groups(group_frames, n)
-        self._ck(self._l.ssd_gpu_process_depth_f32_groups_host(self._h, _ptr(depth), _ptr(cams), _ptr(g), g.size),
-                 "ssd_gpu_process_depth_f32_groups_host")
-        return n
+        return self._process("ssd_gpu_process_depth_f32_groups_host", depth, self._F32, camera_of_frame=camera_of_frame,
+                             group_frames=group_frames)
 
     def process_depth_f32_groups_device(self, dev_ptr, camera_of_frame, group_frames, flags=0):
-        g = self._groups(group_frames)
-        cams = self._cams(camera_of_frame, int(g.sum()))
-        self._ck(self._l.ssd_gpu_process_depth_f32_groups_device(self._h, dev_ptr, _ptr(cams), _ptr(g), g.size, flags),
-                 "ssd_gpu_process_depth_f32_groups_device")
+        self._process("ssd_gpu_process_depth_f32_groups_device", dev_ptr, camera_of_frame=camera_of_frame, group_frames=group_frames,
+                      flags=flags)
 
     # ---- results ----
     def steps(self, frame):

@@ -113,6 +113,30 @@ void Pointcloud::applySettings() const
   }
 }
 
+// The entry point for the frames' kind (z16, float or vertices) and memory (host or device): the plain call, the camera call when cam
+// is given, the group call of nGroups groups when grp is given as well.
+static int processFrames(ssd_gpu_ctx *c, const Camera::DepthFrame &f, int n, const int32_t *cam = nullptr, const int32_t *grp = nullptr, int ng = 0)
+{
+  const bool dev = f.onDevice;
+  if(grp && f.z16)
+    return dev ? ssd_gpu_process_depth_groups_device(c, f.z16, cam, grp, ng, 0) : ssd_gpu_process_depth_groups_host(c, f.z16, cam, grp, ng);
+  if(grp && f.depthF32)
+    return dev ? ssd_gpu_process_depth_f32_groups_device(c, f.depthF32, cam, grp, ng, 0) : ssd_gpu_process_depth_f32_groups_host(c, f.depthF32, cam, grp, ng);
+  if(grp)
+    return dev ? ssd_gpu_process_groups_device(c, f.vertices, cam, grp, ng, 0) : ssd_gpu_process_groups_host(c, f.vertices, cam, grp, ng);
+  if(cam && f.z16)
+    return dev ? ssd_gpu_process_depth_cameras_device(c, f.z16, cam, n) : ssd_gpu_process_depth_cameras_host(c, f.z16, cam, n);
+  if(cam && f.depthF32)
+    return dev ? ssd_gpu_process_depth_f32_cameras_device(c, f.depthF32, cam, n) : ssd_gpu_process_depth_f32_cameras_host(c, f.depthF32, cam, n);
+  if(cam)
+    return dev ? ssd_gpu_process_cameras_device(c, f.vertices, cam, n) : ssd_gpu_process_cameras_host(c, f.vertices, cam, n);
+  if(f.z16)
+    return dev ? ssd_gpu_process_depth_device(c, f.z16, &f.intrinsics, n) : ssd_gpu_process_depth_host(c, f.z16, &f.intrinsics, n);
+  if(f.depthF32)
+    return dev ? ssd_gpu_process_depth_f32_device(c, f.depthF32, &f.intrinsics, n) : ssd_gpu_process_depth_f32_host(c, f.depthF32, &f.intrinsics, n);
+  return dev ? ssd_gpu_process_device(c, f.vertices, n) : ssd_gpu_process_host(c, f.vertices, n);
+}
+
 std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, int nFrames, std::vector<unsigned> *status) const
 {
   ensureContext(frames.width(), frames.height());
@@ -126,16 +150,7 @@ std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, i
       throw std::runtime_error(std::string("ssd_gpu_set_distortion: ") + ssd_gpu_last_error(_ctx));
     _lensApplied = lens;
   }
-  int rc;
-  if(frames.z16)
-    rc = frames.onDevice ? ssd_gpu_process_depth_device(_ctx, frames.z16, &frames.intrinsics, nFrames)
-                         : ssd_gpu_process_depth_host(_ctx, frames.z16, &frames.intrinsics, nFrames);
-  else if(frames.depthF32)
-    rc = frames.onDevice ? ssd_gpu_process_depth_f32_device(_ctx, frames.depthF32, &frames.intrinsics, nFrames)
-                         : ssd_gpu_process_depth_f32_host(_ctx, frames.depthF32, &frames.intrinsics, nFrames);
-  else
-    rc = frames.onDevice ? ssd_gpu_process_device(_ctx, frames.vertices, nFrames) : ssd_gpu_process_host(_ctx, frames.vertices, nFrames);
-  if(rc != SSD_OK)
+  if(processFrames(_ctx, frames, nFrames) != SSD_OK)
     throw std::runtime_error(std::string("ssd_gpu_process: ") + ssd_gpu_last_error(_ctx));
   return collect(nFrames, status);
 }
@@ -171,18 +186,7 @@ std::vector<Stairs> Pointcloud::processBatch(const Camera::DepthFrame &frames, i
     throw std::invalid_argument("Pointcloud::processBatch: cameraOfFrame must hold one camera index per frame");
   ensureContext(frames.width(), frames.height());
   applySettings();
-  const int32_t *cam = cameraOfFrame.data();
-  int rc;
-  if(frames.z16)
-    rc = frames.onDevice ? ssd_gpu_process_depth_cameras_device(_ctx, frames.z16, cam, nFrames)
-                         : ssd_gpu_process_depth_cameras_host(_ctx, frames.z16, cam, nFrames);
-  else if(frames.depthF32)
-    rc = frames.onDevice ? ssd_gpu_process_depth_f32_cameras_device(_ctx, frames.depthF32, cam, nFrames)
-                         : ssd_gpu_process_depth_f32_cameras_host(_ctx, frames.depthF32, cam, nFrames);
-  else
-    rc = frames.onDevice ? ssd_gpu_process_cameras_device(_ctx, frames.vertices, cam, nFrames)
-                         : ssd_gpu_process_cameras_host(_ctx, frames.vertices, cam, nFrames);
-  if(rc != SSD_OK)
+  if(processFrames(_ctx, frames, nFrames, cameraOfFrame.data()) != SSD_OK)
     throw std::runtime_error(std::string("ssd_gpu_process_cameras: ") + ssd_gpu_last_error(_ctx));
   return collect(nFrames, status);
 }
@@ -199,19 +203,9 @@ std::vector<Stairs> Pointcloud::processGroups(const Camera::DepthFrame &frames, 
     throw std::invalid_argument("Pointcloud::processGroups: groupFrames must add up to nFrames");
   ensureContext(frames.width(), frames.height());
   applySettings();
-  const int32_t *cam = cameraOfFrame.data(), *grp = groupFrames.data();
+  const int32_t *grp = groupFrames.data();
   const int nGroups = static_cast<int>(groupFrames.size());
-  int rc;
-  if(frames.z16)
-    rc = frames.onDevice ? ssd_gpu_process_depth_groups_device(_ctx, frames.z16, cam, grp, nGroups, 0)
-                         : ssd_gpu_process_depth_groups_host(_ctx, frames.z16, cam, grp, nGroups);
-  else if(frames.depthF32)
-    rc = frames.onDevice ? ssd_gpu_process_depth_f32_groups_device(_ctx, frames.depthF32, cam, grp, nGroups, 0)
-                         : ssd_gpu_process_depth_f32_groups_host(_ctx, frames.depthF32, cam, grp, nGroups);
-  else
-    rc = frames.onDevice ? ssd_gpu_process_groups_device(_ctx, frames.vertices, cam, grp, nGroups, 0)
-                         : ssd_gpu_process_groups_host(_ctx, frames.vertices, cam, grp, nGroups);
-  if(rc != SSD_OK)
+  if(processFrames(_ctx, frames, nFrames, cameraOfFrame.data(), grp, nGroups) != SSD_OK)
     throw std::runtime_error(std::string("ssd_gpu_process_groups: ") + ssd_gpu_last_error(_ctx));
   // every member frame reads its group's result: keep the first member's
   const std::vector<Stairs> all = collect(nFrames, nullptr);

@@ -60,9 +60,8 @@ struct ssd_gpu_ctx
   ssd_gpu_overlay *d_ovl = nullptr, *h_ovl = nullptr; // max_frames * SSD_GPU_MAX_STEPS, allocated by ssd_gpu_set_overlay
   unsigned char *d_labels = nullptr; // max_frames * N
   unsigned *d_bev = nullptr; // 2 x chunk_frames * MAX_PLATEAUS * bm_words (per stream)
-  float *d_stage[SSD_MAX_STREAMS]{};            // vertex staging of the host-input calls (host_chunk_frames)
-  uint16_t *d_depth[SSD_MAX_STREAMS]{};         // z16 staging of the host depth-frame path
-  float *d_depth_f32[SSD_MAX_STREAMS]{};        // float-depth staging of the host float-depth path (its own: 4 B per pixel)
+  void *d_stage[SSD_MAX_STREAMS]{};             // staging of the host-input calls: a chunk of vertices, z16 or float frames
+  size_t stage_bytes = 0;                       // ... the bytes each holds: the largest chunk a call has needed
   float *d_xn = nullptr, *d_yn = nullptr;       // deprojection tables: (u - ppx) / fx per column, (v - ppy) / fy per row
   ssd_gpu_intrinsics intr{};                    // intrinsics the tables were built for
   bool risers = false;            // ssd_gpu_set_vertical_faces: k_riser_reduce after the chain
@@ -112,7 +111,6 @@ struct ssd_gpu_ctx
   std::vector<int> grp_of_frame;         // host copy of the last call's (empty after a call without groups)
   std::vector<int2> grp_members;
   std::vector<float> grp_epsc;
-  int stage_frames = 0;                  // frames the host-input staging buffers hold (host_chunk_frames, more for a larger group)
 };
 
 // the result record (FrameDev / FrameOut) of a frame of the last call: its group's in a group call
@@ -516,7 +514,7 @@ static void launch_transform_bin(const dim3 &grid, cudaStream_t st, const DevPar
 // parameters (camera calls); GroupTable: as CamTable, with the frames of each group accumulated into one record (group calls).
 // OL: the outline work area of the frame size (OutlineSharedSmall, OutlineShared).
 // Records (FrameDev, FrameOut, BEV slots): rec0 is the launch's first within the call, nr their number (frames, or groups).
-// ov_lens: the lenses the overlay projects through (LensCam), else nullptr.
+// ov_lens: the lenses the overlay projects through (k_finalize), else nullptr: the pin-hole.
 template<class OL, class SRC, class CAM>
 static int launch_classic(ssd_gpu_ctx *ctx, int s, const SRC &src, int frame0, int nf, int rec0, int nr, int *launches, cudaEvent_t *ev,
                           const CAM &cam, const ssd_gpu_distortion *ov_lens)
@@ -542,7 +540,7 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SRC &src, int frame0, i
   // small batches (the reference's real use is one frame per call): the last block of a frame in k_transform_bin evaluates the
   // peaks and the last block in k_outline the frame logic -- five launches instead of seven. Group calls take the seven
   // (their blocks do not count a frame's completion).
-  constexpr bool FUSABLE = !IsGroupCam<CAM>::value;
+  constexpr bool FUSABLE = !std::is_same<CAM, GroupTable>::value;
   const bool fused = FUSABLE && nf <= SSD_FUSE_MAX_FRAMES && !ev;
   STAGE_EV(0);
   if(!fused)
@@ -581,12 +579,8 @@ static int launch_classic(ssd_gpu_ctx *ctx, int s, const SRC &src, int frame0, i
     quad_reduce(StepLabelsOut<false>());
   STAGE_EV(6);
   // k_finalize runs SSD_OL_THREADS on either work area
-  if(ov_lens)
-    k_finalize<OL, LensCam<CAM>><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words, ctx->smem_cap_words,
-                                                                              ctx->ov, ovl, LensCam<CAM>{ cam, ov_lens });
-  else
-    k_finalize<OL, CAM><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words, ctx->smem_cap_words, ctx->ov,
-                                                                     ovl, cam);
+  k_finalize<OL, CAM><<<nr, SSD_OL_THREADS, ctx->ol_dyn_smem, st>>>(p, frames, ctx->d_out + rec0, bev, ctx->bm_words, ctx->smem_cap_words, ctx->ov,
+                                                                   ovl, ov_lens, cam);
   STAGE_EV(7);
 #undef STAGE_EV
   *launches += fused ? SSD_GPU_N_STAGES - 2 : SSD_GPU_N_STAGES;
@@ -639,20 +633,18 @@ static GroupTable chunk_cam(GroupTable g, int frame0, int rec0)
 }
 
 // The dynamic work area of the outline kernels a chain of camera type CAM launches with a dynamic band (launch_classic): the fused
-// k_outline (not in group calls) and k_finalize with and without the overlay's lens, on both work areas.
+// k_outline (not in group calls) and k_finalize, on both work areas.
 template<class CAM>
 static void allow_outline_smem(int dyn)
 {
   const auto allow = [dyn](auto kernel) { cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn); };
-  if constexpr(!IsGroupCam<CAM>::value)
+  if constexpr(!std::is_same<CAM, GroupTable>::value)
   {
     allow(k_outline<OutlineSharedSmall, true, CAM>);
     allow(k_outline<OutlineShared, true, CAM>);
   }
   allow(k_finalize<OutlineSharedSmall, CAM>);
   allow(k_finalize<OutlineShared, CAM>);
-  allow(k_finalize<OutlineSharedSmall, LensCam<CAM>>);
-  allow(k_finalize<OutlineShared, LensCam<CAM>>);
 }
 
 extern "C"
@@ -707,8 +699,6 @@ void ssd_gpu_destroy(ssd_gpu_ctx *ctx)
   for(int i = 0; i < SSD_MAX_STREAMS; i++)
   {
     cudaFree(ctx->d_stage[i]);
-    cudaFree(ctx->d_depth[i]);
-    cudaFree(ctx->d_depth_f32[i]);
     if(ctx->stream[i])
       cudaStreamDestroy(ctx->stream[i]);
     if(ctx->ev_in_ready[i])
@@ -782,7 +772,6 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
     if(const char *e = getenv("SSD_GPU_HOST_CHUNK_FRAMES"))
       hc = atoi(e);
     ctx->host_chunk_frames = std::max(1, std::min(hc, cf));
-    ctx->stage_frames = ctx->host_chunk_frames;
   }
 
   {
@@ -959,359 +948,391 @@ static int ensure_deproject_tables(ssd_gpu_ctx *ctx, const ssd_gpu_intrinsics &i
   return SSD_OK;
 }
 
-} // extern "C": the templates of the depth sample type follow
+} // extern "C": the call description and its driver follow
 
-// The depth staging buffers of sample type T: each sample type has its own, so that a buffer is never read with another width.
-static uint16_t **depth_staging(ssd_gpu_ctx *ctx, const uint16_t *)
+// One process call, as every entry point describes it
+enum CallMode
 {
-  return ctx->d_depth;
-}
-static float **depth_staging(ssd_gpu_ctx *ctx, const float *)
+  CALL_PLAIN,   // every frame with the context's own camera
+  CALL_CAMERAS, // each frame with the camera camera_of_frame names
+  CALL_GROUPS,  // as CALL_CAMERAS, the frames of each group detected as one point cloud
+};
+enum InputKind
 {
-  return ctx->d_depth_f32;
-}
-// A call's depth pointer; its sample type T is named by the entry point (a vertex call passes none to deduce it from).
-template<class T>
-struct Samples
+  IN_VERTICES, // packed {x, y, z} floats
+  IN_Z16,      // z16 depth counts, deprojected inside the point kernels
+  IN_F32,      // float depth samples, likewise
+};
+struct ProcessCall
 {
-  typedef const T *ptr;
+  CallMode mode;
+  InputKind kind;
+  const void *input; // n_frames x N pixels of the kind
+  bool host;         // input in host memory: staged through d_stage
+  int n_frames;      // group calls: set by check_call from group_frames
+  int flags;
+  const ssd_gpu_intrinsics *intr = nullptr; // plain depth calls
+  const int32_t *camera_of_frame = nullptr; // camera and group calls
+  const int32_t *group_frames = nullptr;    // group calls: frames of each of the n_groups groups
+  int n_groups = 0;
 };
 
-// xyz != nullptr: packed vertices; else depth frames of sample type T (z16 counts or float) + intrinsics, deprojected inside the
-// point kernels
-// cam_of_frame != nullptr: a camera call (validated by check_cameras; the depth tables are the camera table's, intr is unused)
-// group_frames != nullptr: a group call of n_groups groups (validated by check_groups; a camera call as well)
-template<class T>
-static int process_impl(ssd_gpu_ctx *ctx, const float *xyz, const T *depth, const ssd_gpu_intrinsics *intr, bool host_input, int n_frames,
-                        int flags, const int32_t *cam_of_frame, const int32_t *group_frames, int n_groups)
+// Everything a call can be refused for. Steps 1-7 change nothing; step 8 comes last because it builds the plain depth path's tables.
+// Only the RANGE / STATE checks sit between INVALID_ARG checks, so the code a call with several faults gets does not depend on which
+// INVALID_ARG fault is found first.
+static int check_call(ssd_gpu_ctx *ctx, ProcessCall &c)
 {
-  if(!ctx || (!xyz && !(depth && (intr || cam_of_frame))) || n_frames <= 0)
-    return fail(ctx, SSD_E_INVALID_ARG, "process: bad argument");
+  static const char *const family[] = { "process", "camera call", "group call" };
+  const std::string who = family[c.mode];
+  const bool depth = c.kind != IN_VERTICES;
+  // 1. null and count arguments
+  if(c.mode == CALL_PLAIN && depth && (!c.input || !c.intr))
+    return fail(ctx, SSD_E_INVALID_ARG, c.kind == IN_Z16 ? "process_depth: bad argument" : "process_depth_f32: bad argument");
+  if(!ctx || !c.input || (c.mode != CALL_PLAIN && !c.camera_of_frame) ||
+     (c.mode == CALL_GROUPS ? !c.group_frames || c.n_groups < 1 : c.n_frames <= 0))
+    return fail(ctx, SSD_E_INVALID_ARG, who + ": bad argument");
+  // 2. group sizes
+  long long n_frames = c.n_frames;
+  if(c.mode == CALL_GROUPS)
+  {
+    n_frames = 0;
+    for(int g = 0; g < c.n_groups; g++)
+    {
+      if(c.group_frames[g] < 1 || c.group_frames[g] > SSD_GPU_MAX_GROUP_FRAMES)
+        return fail(ctx, SSD_E_INVALID_ARG, "group call: group " + std::to_string(g) + " has " + std::to_string(c.group_frames[g]) +
+                                                " frames, outside [1, " + std::to_string(SSD_GPU_MAX_GROUP_FRAMES) + "]");
+      n_frames += c.group_frames[g];
+    }
+  }
+  // 3. the camera table
+  if(c.mode != CALL_PLAIN && ctx->n_cameras <= 0)
+    return fail(ctx, SSD_E_STATE, who + ": no camera table (ssd_gpu_set_cameras)");
+  // 4. frames
   if(n_frames > ctx->max_frames)
-    return fail(ctx, SSD_E_RANGE, "process: n_frames exceeds max_frames of the context");
-  // the point kernels use 16-byte vector loads / bulk copies (vertices), one load per 4-pixel word of depth (8 bytes of z16,
-  // 16 bytes of float)
-  if((xyz && ((uintptr_t)xyz & 15u)) || (depth && ((uintptr_t)depth & (4 * sizeof(T) - 1))))
-    return fail(ctx, SSD_E_INVALID_ARG, sizeof(T) == 2 ? "process: the input buffer must be 16-byte aligned (vertices) / 8-byte aligned (depth)"
-                                                       : "process: float depth input must be 16-byte aligned");
-  CK(cudaSetDevice(ctx->device));
-  const DevParams &p = ctx->dp;
-  const size_t frame_floats = (size_t)p.N * 3;
-  // host input: every byte crosses PCIe, the copy of chunk i+1 overlaps the kernels of chunk i and only the last
-  // chunk's kernels stay exposed -- small chunks. Device input: large chunks (the per-frame kernels need the parallelism).
-  int cf = host_input ? ctx->host_chunk_frames : ctx->chunk_frames;
-  // a device-resident batch that fits one chunk is still split over the streams, so that one half's latency-bound
-  // per-plateau kernels overlap the other half's point kernels (measured: 64 frames of 4096x3072 as 2 x 32: +5 %;
-  // below ~32 frames per chain the per-frame kernels lose more parallelism than the overlap returns)
-  if(!host_input && !(flags & SSD_FLAG_SINGLE_STREAM) && ctx->n_streams > 1 && n_frames <= cf && !ctx->no_split_small)
+    return fail(ctx, SSD_E_RANGE, c.mode == CALL_GROUPS ? "group call: the groups hold " + std::to_string(n_frames) +
+                                                            " frames, more than max_frames of the context"
+                                                      : "process: n_frames exceeds max_frames of the context");
+  c.n_frames = (int)n_frames;
+  // 5. the frame width of depth input: one load per 4-pixel word
+  if(depth && ctx->dp.W % 4 != 0)
+    return fail(ctx, SSD_E_INVALID_ARG, "depth input: the frame width must be a multiple of 4");
+  // 6. each frame's camera
+  for(int f = 0; f < c.n_frames && c.mode != CALL_PLAIN; f++)
   {
-    const int half = (n_frames + ctx->n_streams - 1) / ctx->n_streams;
-    if(half >= 32)
-      cf = half;
+    const int32_t cam = c.camera_of_frame[f];
+    if(cam < 0 || cam >= ctx->n_cameras)
+      return fail(ctx, SSD_E_RANGE, "camera call: frame " + std::to_string(f) + " names camera " + std::to_string(cam) + ", outside [0, " +
+                                      std::to_string(ctx->n_cameras) + ")");
+    if(depth && !ctx->cam_depth_ok[cam])
+      return fail(ctx, SSD_E_INVALID_ARG, "depth camera call: camera " + std::to_string(cam) + " has no depth intrinsics (fx, fy must be non-zero and "
+                                                                                              "depth_unit positive)");
   }
-  const bool depth_input = xyz == nullptr;
-  // a distorted lens: depth frames read their rays from ray tables (SrcLens), the overlay projects through the lens (LensCam)
-  const bool plain_lens = !cam_of_frame && !ssd_lens_is_pinhole(&ctx->lens);
-  SrcLensT<T> sl{};
-  bool use_lens = false;
-  const ssd_gpu_distortion *ov_lens = nullptr;
-  if(cam_of_frame)
+  // 7. alignment: the point kernels use 16-byte vector loads / bulk copies (vertices), one load per 4-pixel word of depth (8 bytes of
+  // z16, 16 bytes of float)
+  if((uintptr_t)c.input & (c.kind == IN_Z16 ? 7u : 15u))
+    return fail(ctx, SSD_E_INVALID_ARG, c.kind == IN_F32 ? "process: float depth input must be 16-byte aligned"
+                                                         : "process: the input buffer must be 16-byte aligned (vertices) / 8-byte aligned (depth)");
+  // 8. the plain depth path's intrinsics, and its deprojection and ray tables
+  if(c.mode == CALL_PLAIN && depth)
   {
-    for(int f = 0; f < n_frames && depth_input && ctx->cams_distorted && !use_lens; f++)
-      use_lens = ctx->cam_distorted[cam_of_frame[f]] != 0;
-    sl.cam_ray = ctx->d_cam_ray;
-    if(ctx->cams_distorted && ctx->ov.enabled)
-      ov_lens = ctx->d_cam_lens;
-  }
-  else if(plain_lens)
-  {
-    use_lens = depth_input;
-    if(ctx->ov.enabled)
-      ov_lens = ctx->d_lens;
-  }
-  if(depth_input && !cam_of_frame)
-  {
-    const int rc = ensure_deproject_tables(ctx, *intr);
-    if(rc)
-      return rc;
-    sl.ray = ctx->d_ray;
-    sl.unit = intr->depth_unit;
-  }
-  // chunks {first frame, frames, first record, records}: cf frames each, or in a group call whole groups up to cf frames (a group
-  // larger than cf is a chunk of its own)
-  struct Chunk
-  {
-    int f0, nf, r0, nr;
-  };
-  std::vector<Chunk> chunks;
-  int max_nf = 0;
-  if(group_frames)
-  {
-    for(int g = 0, f = 0; g < n_groups; f += group_frames[g], g++)
-    {
-      if(chunks.empty() || chunks.back().nf + group_frames[g] > cf)
-        chunks.push_back({ f, 0, g, 0 });
-      chunks.back().nf += group_frames[g];
-      chunks.back().nr++;
-      max_nf = std::max(max_nf, chunks.back().nf);
-    }
-  }
-  else
-    for(int f0 = 0; f0 < n_frames; f0 += cf)
-    {
-      const int nf = std::min(cf, n_frames - f0);
-      chunks.push_back({ f0, nf, f0, nf });
-      max_nf = std::max(max_nf, nf);
-    }
-  const int n_records = group_frames ? n_groups : n_frames;
-  // depth frames are deprojected inside the point kernels (SrcDepth): no vertex array is ever written.
-  if(host_input)
-  {
-    if(max_nf > ctx->stage_frames)
-    {
-      // a group larger than the host chunk: the staging buffers grow to hold it (no call is in flight between calls)
-      for(int i = 0; i < SSD_MAX_STREAMS; i++)
-      {
-        CK(cudaFree(ctx->d_stage[i]));
-        CK(cudaFree(ctx->d_depth[i]));
-        CK(cudaFree(ctx->d_depth_f32[i]));
-        ctx->d_stage[i] = nullptr;
-        ctx->d_depth[i] = nullptr;
-        ctx->d_depth_f32[i] = nullptr;
-      }
-      ctx->stage_frames = max_nf;
-    }
-    T **dstage = depth_staging(ctx, depth);
-    for(int i = 0; i < ctx->n_streams; i++)
-    {
-      if(depth_input && !dstage[i])
-        CK(cudaMalloc(&dstage[i], (size_t)ctx->stage_frames * p.N * sizeof(T)));
-      if(!depth_input && !ctx->d_stage[i])
-        CK(cudaMalloc(&ctx->d_stage[i], (size_t)ctx->stage_frames * frame_floats * sizeof(float)));
-    }
-  }
-
-  int launches = 0;
-  const bool stage_timing = (flags & SSD_FLAG_STAGE_TIMING) != 0;
-  const int n_chunks = (int)chunks.size();
-  if(stage_timing && ctx->stage_chunks < n_chunks)
-  {
-    const size_t want = (size_t)n_chunks * (SSD_GPU_N_STAGES + 1);
-    while(ctx->stage_ev.size() < want)
-    {
-      cudaEvent_t e;
-      CK(cudaEventCreate(&e));
-      ctx->stage_ev.push_back(e);
-    }
-    ctx->stage_chunks = n_chunks;
-  }
-  ctx->n_frames_last = n_frames;
-  ctx->flags_last = flags;
-  ctx->step_labels_last = ctx->step_labels;
-  ctx->surfaces_last = ctx->surfaces;
-  ctx->grp_of_frame.clear();
-  ctx->grp_members.clear();
-  ctx->grp_epsc.clear();
-  ctx->stats_eps0 = ctx->dp.E0s;
-  ctx->stats_eps1 = ctx->dp.E1s;
-  CamTable cams{};
-  if(cam_of_frame)
-  {
-    cams.params = ctx->d_cam_dp;
-    cams.ov = ctx->d_cam_ov;
-    cams.xn = ctx->d_cam_xn;
-    cams.yn = ctx->d_cam_yn;
-    cams.unit = ctx->d_cam_unit;
-    cams.cam = ctx->d_cam_of_frame;
-    ctx->stats_eps0 = ctx->stats_eps1 = 0;
-    for(int f = 0; f < n_frames; f++)
-    {
-      const DevParams &d = ctx->cam_dp[cam_of_frame[f]];
-      ctx->stats_eps0 = std::max(ctx->stats_eps0, (double)d.E0s);
-      ctx->stats_eps1 = std::max(ctx->stats_eps1, (double)d.E1s);
-    }
-  }
-  GroupTable grp{};
-  if(group_frames)
-  {
-    if(!ctx->d_grp_of_frame)
-    {
-      CK(cudaMalloc(&ctx->d_grp_of_frame, sizeof(int) * (size_t)ctx->max_frames));
-      CK(cudaMalloc(&ctx->d_grp_members, sizeof(int2) * (size_t)ctx->max_frames));
-      CK(cudaMalloc(&ctx->d_grp_epsc, sizeof(float) * (size_t)ctx->max_frames));
-    }
-    // the quadrilateral filters of a group decide the points of all its cameras: the largest of their bounds
-    for(int g = 0, f = 0; g < n_groups; f += group_frames[g], g++)
-    {
-      float e = 0.f;
-      for(int i = 0; i < group_frames[g]; i++)
-      {
-        ctx->grp_of_frame.push_back(g);
-        e = std::max(e, ctx->cam_dp[cam_of_frame[f + i]].epsc); // (an infinite bound stays infinite: every decision is exact)
-      }
-      ctx->grp_members.push_back(make_int2(f, group_frames[g]));
-      ctx->grp_epsc.push_back(e);
-    }
-    grp.cams = cams;
-    grp.group = ctx->d_grp_of_frame;
-    grp.members = ctx->d_grp_members;
-    grp.epsc = ctx->d_grp_epsc;
-  }
-  if(ctx->surfaces)
-  {
-    // each record's ToExternalWorld as k_finalize uses it: the context's, the frame's camera's, the group's first member's
-    ctx->surf_xf.resize((size_t)n_records);
-    for(int r = 0; r < n_records; r++)
-    {
-      const DevParams &d = !cam_of_frame ? ctx->dp : ctx->cam_dp[cam_of_frame[group_frames ? ctx->grp_members[r].x : r]];
-      SurfaceXf &x = ctx->surf_xf[r];
-      memcpy(x.ext_a, d.ext_a, sizeof(x.ext_a));
-      memcpy(x.ext_b, d.ext_b, sizeof(x.ext_b));
-      x.ext_z = d.ext_z;
-    }
-  }
-  // the whole call is ordered after ev_start on stream 0; stream 1 joins via events
-  CK(cudaEventRecord(ctx->ev_start, ctx->stream[0]));
-  for(int i = 1; i < ctx->n_streams; i++)
-    CK(cudaStreamWaitEvent(ctx->stream[i], ctx->ev_start, 0));
-  CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_start, 0));
-  if(host_input)
-    CK(cudaEventRecord(ctx->ev_h2d0, ctx->copy_stream));
-  // per-frame state: histogram must start at zero
-  CK(cudaMemsetAsync(ctx->d_frames, 0, sizeof(FrameDev) * (size_t)n_records, ctx->stream[0]));
-  if(cam_of_frame)
-    CK(cudaMemcpyAsync(ctx->d_cam_of_frame, cam_of_frame, sizeof(int32_t) * (size_t)n_frames, cudaMemcpyHostToDevice, ctx->stream[0]));
-  if(group_frames)
-  {
-    CK(cudaMemcpyAsync(ctx->d_grp_of_frame, ctx->grp_of_frame.data(), sizeof(int) * (size_t)n_frames, cudaMemcpyHostToDevice, ctx->stream[0]));
-    CK(cudaMemcpyAsync(ctx->d_grp_members, ctx->grp_members.data(), sizeof(int2) * (size_t)n_groups, cudaMemcpyHostToDevice, ctx->stream[0]));
-    CK(cudaMemcpyAsync(ctx->d_grp_epsc, ctx->grp_epsc.data(), sizeof(float) * (size_t)n_groups, cudaMemcpyHostToDevice, ctx->stream[0]));
-  }
-  CK(cudaEventRecord(ctx->ev_chunk_done[0], ctx->stream[0]));
-  for(int i = 1; i < ctx->n_streams; i++)
-    CK(cudaStreamWaitEvent(ctx->stream[i], ctx->ev_chunk_done[0], 0));
-
-  // the chunk loop for the call's one source and camera type
-  const auto run_chunks = [&](const auto &src, const auto &cam) -> int {
-    for(int chunk = 0; chunk < n_chunks; chunk++)
-    {
-      const int f0 = chunks[chunk].f0, nf = chunks[chunk].nf;
-      const int s = (flags & SSD_FLAG_SINGLE_STREAM) ? 0 : chunk % ctx->n_streams;
-      const void *in = depth_input ? (const void *)(depth + (size_t)f0 * p.N) : (const void *)(xyz + (size_t)f0 * frame_floats);
-      if(host_input)
-      {
-        // staging buffer s may be overwritten once the chunk that last used it has consumed it
-        if(chunk >= ((flags & SSD_FLAG_SINGLE_STREAM) ? 1 : ctx->n_streams))
-          CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_in_free[s], 0));
-        if(depth_input)
-        {
-          T *dst = depth_staging(ctx, depth)[s];
-          CK(cudaMemcpyAsync(dst, in, (size_t)nf * p.N * sizeof(T), cudaMemcpyHostToDevice, ctx->copy_stream));
-          in = dst;
-        }
-        else
-        {
-          CK(cudaMemcpyAsync(ctx->d_stage[s], in, (size_t)nf * frame_floats * sizeof(float), cudaMemcpyHostToDevice, ctx->copy_stream));
-          in = ctx->d_stage[s];
-        }
-        CK(cudaEventRecord(ctx->ev_in_ready[s], ctx->copy_stream));
-        CK(cudaStreamWaitEvent(ctx->stream[s], ctx->ev_in_ready[s], 0));
-      }
-      const auto csrc = chunk_src(src, in);
-      const auto ccam = chunk_cam(cam, f0, chunks[chunk].r0);
-      cudaEvent_t *ev = stage_timing ? &ctx->stage_ev[(size_t)chunk * (SSD_GPU_N_STAGES + 1)] : nullptr;
-      const int rc = ctx->outline_small
-                       ? launch_classic<OutlineSharedSmall>(ctx, s, csrc, f0, nf, chunks[chunk].r0, chunks[chunk].nr, &launches, ev, ccam, ov_lens)
-                       : launch_classic<OutlineShared>(ctx, s, csrc, f0, nf, chunks[chunk].r0, chunks[chunk].nr, &launches, ev, ccam, ov_lens);
-      if(rc)
-        return rc;
-      if(host_input)
-        CK(cudaEventRecord(ctx->ev_in_free[s], ctx->stream[s])); // all three passes have read the staging
-    }
-    return SSD_OK;
-  };
-  const auto run_source = [&](const auto &src) -> int {
-    if(group_frames)
-      return run_chunks(src, grp);
-    if(cam_of_frame)
-      return run_chunks(src, cams);
-    return run_chunks(src, NoCam());
-  };
-  int rc;
-  if(!depth_input)
-    rc = run_source(SrcVertices{ xyz });
-  else if(use_lens)
-    rc = run_source(sl);
-  else
-  {
-    // depth frames are deprojected inside the point kernels with the pin-hole tables (a camera call's per camera)
-    const unsigned long long wmagic = (((unsigned long long)1 << 40) + (unsigned long long)p.W - 1) / (unsigned long long)p.W;
-    rc = run_source(SrcDepthT<T>{ depth, ctx->d_xn, ctx->d_yn, intr ? intr->depth_unit : 0.f, wmagic });
-  }
-  if(rc)
-    return rc;
-  if(host_input)
-    CK(cudaEventRecord(ctx->ev_h2d1, ctx->copy_stream));
-  // join stream 1 into stream 0, then bring the compact results home
-  for(int i = 1; i < ctx->n_streams; i++)
-  {
-    CK(cudaEventRecord(ctx->ev_chunk_done[i], ctx->stream[i]));
-    CK(cudaStreamWaitEvent(ctx->stream[0], ctx->ev_chunk_done[i], 0));
-  }
-  CK(cudaMemcpyAsync(ctx->h_out, ctx->d_out, sizeof(FrameOut) * (size_t)n_records, cudaMemcpyDeviceToHost, ctx->stream[0]));
-  if(ctx->ov.enabled)
-    CK(cudaMemcpyAsync(ctx->h_ovl, ctx->d_ovl, sizeof(ssd_gpu_overlay) * SSD_GPU_MAX_STEPS * (size_t)n_frames, cudaMemcpyDeviceToHost, ctx->stream[0]));
-  CK(cudaEventRecord(ctx->ev_stop, ctx->stream[0]));
-  CK(cudaEventSynchronize(ctx->ev_stop));
-  CK(cudaGetLastError());
-  float ms = 0;
-  CK(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
-  ctx->timing.total_ms = ms;
-  ctx->timing.h2d_ms = 0;
-  if(host_input)
-  {
-    float h = 0;
-    CK(cudaEventElapsedTime(&h, ctx->ev_h2d0, ctx->ev_h2d1));
-    ctx->timing.h2d_ms = h;
-  }
-  ctx->timing.label_ms = 0;
-  ctx->timing.n_launches = launches;
-  for(int i = 0; i < SSD_GPU_N_STAGES; i++)
-  {
-    ctx->stage_ms[i] = 0;
-    ctx->stage_launches[i] = 0;
-  }
-  if(stage_timing)
-  {
-    for(int c = 0; c < n_chunks; c++)
-      for(int i = 0; i < SSD_GPU_N_STAGES; i++)
-      {
-        float t = 0;
-        const cudaEvent_t *ev = &ctx->stage_ev[(size_t)c * (SSD_GPU_N_STAGES + 1)];
-        CK(cudaEventElapsedTime(&t, ev[i], ev[i + 1]));
-        ctx->stage_ms[i] += t;
-        ctx->stage_launches[i]++;
-      }
-    ctx->timing.label_ms = ctx->stage_ms[0];
+    CK(cudaSetDevice(ctx->device));
+    return ensure_deproject_tables(ctx, *c.intr);
   }
   return SSD_OK;
 }
 
-// A failure inside the chain (launch error, bad user pointer, out of memory while growing a staging buffer) may leave streams
-// unsynchronised and BEV bitmaps half written: the bitmaps are "self-cleaning" only along a complete chain. Bring the context
-// back to a clean state so that the next call starts from zeroed bitmaps and no stale results can be read.
-template<class T = uint16_t>
-static int process_common(ssd_gpu_ctx *ctx, const float *xyz, typename Samples<T>::ptr depth, const ssd_gpu_intrinsics *intr, bool host_input,
-                          int n_frames, int flags, const int32_t *cam_of_frame = nullptr, const int32_t *group_frames = nullptr, int n_groups = 0)
+// Runs an accepted call: its frames in chunks through launch_classic, for the call's one source and camera type.
+static int process(ssd_gpu_ctx *ctx, ProcessCall c)
 {
-  const int rc = process_impl<T>(ctx, xyz, depth, intr, host_input, n_frames, flags, cam_of_frame, group_frames, n_groups);
-  if(rc != SSD_OK && rc != SSD_E_INVALID_ARG && rc != SSD_E_RANGE && ctx)
+  int rc = check_call(ctx, c);
+  if(rc == SSD_OK)
+    rc = [&]() -> int {
+      CK(cudaSetDevice(ctx->device));
+      const DevParams &p = ctx->dp;
+      const bool depth_input = c.kind != IN_VERTICES;
+      const size_t frame_bytes = (size_t)p.N * (c.kind == IN_VERTICES ? 12 : c.kind == IN_Z16 ? 2 : 4);
+      const int32_t *cam_of_frame = c.camera_of_frame, *group_frames = c.group_frames;
+      const int n_frames = c.n_frames, n_groups = c.n_groups, flags = c.flags;
+      // host input: every byte crosses PCIe, the copy of chunk i+1 overlaps the kernels of chunk i and only the last
+      // chunk's kernels stay exposed -- small chunks. Device input: large chunks (the per-frame kernels need the parallelism).
+      int cf = c.host ? ctx->host_chunk_frames : ctx->chunk_frames;
+      // a device-resident batch that fits one chunk is still split over the streams, so that one half's latency-bound
+      // per-plateau kernels overlap the other half's point kernels (measured: 64 frames of 4096x3072 as 2 x 32: +5 %;
+      // below ~32 frames per chain the per-frame kernels lose more parallelism than the overlap returns)
+      if(!c.host && !(flags & SSD_FLAG_SINGLE_STREAM) && ctx->n_streams > 1 && n_frames <= cf && !ctx->no_split_small)
+      {
+        const int half = (n_frames + ctx->n_streams - 1) / ctx->n_streams;
+        if(half >= 32)
+          cf = half;
+      }
+      // a distorted lens: depth frames read their rays from ray tables (SrcLens), the overlay projects through the lens
+      bool use_lens = false;
+      const ssd_gpu_distortion *ov_lens = nullptr;
+      if(cam_of_frame)
+      {
+        for(int f = 0; f < n_frames && depth_input && ctx->cams_distorted && !use_lens; f++)
+          use_lens = ctx->cam_distorted[cam_of_frame[f]] != 0;
+        if(ctx->cams_distorted && ctx->ov.enabled)
+          ov_lens = ctx->d_cam_lens;
+      }
+      else if(!ssd_lens_is_pinhole(&ctx->lens))
+      {
+        use_lens = depth_input;
+        if(ctx->ov.enabled)
+          ov_lens = ctx->d_lens;
+      }
+      // chunks {first frame, frames, first record, records}: cf frames each, or in a group call whole groups up to cf frames (a group
+      // larger than cf is a chunk of its own)
+      struct Chunk
+      {
+        int f0, nf, r0, nr;
+      };
+      std::vector<Chunk> chunks;
+      int max_nf = 0;
+      if(group_frames)
+      {
+        for(int g = 0, f = 0; g < n_groups; f += group_frames[g], g++)
+        {
+          if(chunks.empty() || chunks.back().nf + group_frames[g] > cf)
+            chunks.push_back({ f, 0, g, 0 });
+          chunks.back().nf += group_frames[g];
+          chunks.back().nr++;
+          max_nf = std::max(max_nf, chunks.back().nf);
+        }
+      }
+      else
+        for(int f0 = 0; f0 < n_frames; f0 += cf)
+        {
+          const int nf = std::min(cf, n_frames - f0);
+          chunks.push_back({ f0, nf, f0, nf });
+          max_nf = std::max(max_nf, nf);
+        }
+      const int n_records = group_frames ? n_groups : n_frames;
+      // host input: the staging buffers grow to the largest chunk any call has needed (no call is in flight between calls)
+      if(c.host && (size_t)max_nf * frame_bytes > ctx->stage_bytes)
+      {
+        ctx->stage_bytes = 0;
+        for(int i = 0; i < ctx->n_streams; i++)
+        {
+          CK(cudaFree(ctx->d_stage[i]));
+          ctx->d_stage[i] = nullptr;
+          CK(cudaMalloc(&ctx->d_stage[i], (size_t)max_nf * frame_bytes));
+        }
+        ctx->stage_bytes = (size_t)max_nf * frame_bytes;
+      }
+
+      int launches = 0;
+      const bool stage_timing = (flags & SSD_FLAG_STAGE_TIMING) != 0;
+      const int n_chunks = (int)chunks.size();
+      if(stage_timing && ctx->stage_chunks < n_chunks)
+      {
+        const size_t want = (size_t)n_chunks * (SSD_GPU_N_STAGES + 1);
+        while(ctx->stage_ev.size() < want)
+        {
+          cudaEvent_t e;
+          CK(cudaEventCreate(&e));
+          ctx->stage_ev.push_back(e);
+        }
+        ctx->stage_chunks = n_chunks;
+      }
+      ctx->n_frames_last = n_frames;
+      ctx->flags_last = flags;
+      ctx->step_labels_last = ctx->step_labels;
+      ctx->surfaces_last = ctx->surfaces;
+      ctx->grp_of_frame.clear();
+      ctx->grp_members.clear();
+      ctx->grp_epsc.clear();
+      ctx->stats_eps0 = ctx->dp.E0s;
+      ctx->stats_eps1 = ctx->dp.E1s;
+      CamTable cams{};
+      if(cam_of_frame)
+      {
+        cams.params = ctx->d_cam_dp;
+        cams.ov = ctx->d_cam_ov;
+        cams.xn = ctx->d_cam_xn;
+        cams.yn = ctx->d_cam_yn;
+        cams.unit = ctx->d_cam_unit;
+        cams.cam = ctx->d_cam_of_frame;
+        ctx->stats_eps0 = ctx->stats_eps1 = 0;
+        for(int f = 0; f < n_frames; f++)
+        {
+          const DevParams &d = ctx->cam_dp[cam_of_frame[f]];
+          ctx->stats_eps0 = std::max(ctx->stats_eps0, (double)d.E0s);
+          ctx->stats_eps1 = std::max(ctx->stats_eps1, (double)d.E1s);
+        }
+      }
+      GroupTable grp{};
+      if(group_frames)
+      {
+        if(!ctx->d_grp_of_frame)
+        {
+          CK(cudaMalloc(&ctx->d_grp_of_frame, sizeof(int) * (size_t)ctx->max_frames));
+          CK(cudaMalloc(&ctx->d_grp_members, sizeof(int2) * (size_t)ctx->max_frames));
+          CK(cudaMalloc(&ctx->d_grp_epsc, sizeof(float) * (size_t)ctx->max_frames));
+        }
+        // the quadrilateral filters of a group decide the points of all its cameras: the largest of their bounds
+        for(int g = 0, f = 0; g < n_groups; f += group_frames[g], g++)
+        {
+          float e = 0.f;
+          for(int i = 0; i < group_frames[g]; i++)
+          {
+            ctx->grp_of_frame.push_back(g);
+            e = std::max(e, ctx->cam_dp[cam_of_frame[f + i]].epsc); // (an infinite bound stays infinite: every decision is exact)
+          }
+          ctx->grp_members.push_back(make_int2(f, group_frames[g]));
+          ctx->grp_epsc.push_back(e);
+        }
+        grp.cams = cams;
+        grp.group = ctx->d_grp_of_frame;
+        grp.members = ctx->d_grp_members;
+        grp.epsc = ctx->d_grp_epsc;
+      }
+      if(ctx->surfaces)
+      {
+        // each record's ToExternalWorld as k_finalize uses it: the context's, the frame's camera's, the group's first member's
+        ctx->surf_xf.resize((size_t)n_records);
+        for(int r = 0; r < n_records; r++)
+        {
+          const DevParams &d = !cam_of_frame ? ctx->dp : ctx->cam_dp[cam_of_frame[group_frames ? ctx->grp_members[r].x : r]];
+          SurfaceXf &x = ctx->surf_xf[r];
+          memcpy(x.ext_a, d.ext_a, sizeof(x.ext_a));
+          memcpy(x.ext_b, d.ext_b, sizeof(x.ext_b));
+          x.ext_z = d.ext_z;
+        }
+      }
+      // the whole call is ordered after ev_start on stream 0; stream 1 joins via events
+      CK(cudaEventRecord(ctx->ev_start, ctx->stream[0]));
+      for(int i = 1; i < ctx->n_streams; i++)
+        CK(cudaStreamWaitEvent(ctx->stream[i], ctx->ev_start, 0));
+      CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_start, 0));
+      if(c.host)
+        CK(cudaEventRecord(ctx->ev_h2d0, ctx->copy_stream));
+      // per-frame state: histogram must start at zero
+      CK(cudaMemsetAsync(ctx->d_frames, 0, sizeof(FrameDev) * (size_t)n_records, ctx->stream[0]));
+      if(cam_of_frame)
+        CK(cudaMemcpyAsync(ctx->d_cam_of_frame, cam_of_frame, sizeof(int32_t) * (size_t)n_frames, cudaMemcpyHostToDevice, ctx->stream[0]));
+      if(group_frames)
+      {
+        CK(cudaMemcpyAsync(ctx->d_grp_of_frame, ctx->grp_of_frame.data(), sizeof(int) * (size_t)n_frames, cudaMemcpyHostToDevice, ctx->stream[0]));
+        CK(cudaMemcpyAsync(ctx->d_grp_members, ctx->grp_members.data(), sizeof(int2) * (size_t)n_groups, cudaMemcpyHostToDevice, ctx->stream[0]));
+        CK(cudaMemcpyAsync(ctx->d_grp_epsc, ctx->grp_epsc.data(), sizeof(float) * (size_t)n_groups, cudaMemcpyHostToDevice, ctx->stream[0]));
+      }
+      CK(cudaEventRecord(ctx->ev_chunk_done[0], ctx->stream[0]));
+      for(int i = 1; i < ctx->n_streams; i++)
+        CK(cudaStreamWaitEvent(ctx->stream[i], ctx->ev_chunk_done[0], 0));
+
+      // the chunk loop for the call's one source and camera type
+      const auto run_chunks = [&](const auto &src, const auto &cam) -> int {
+        for(int chunk = 0; chunk < n_chunks; chunk++)
+        {
+          const int f0 = chunks[chunk].f0, nf = chunks[chunk].nf;
+          const int s = (flags & SSD_FLAG_SINGLE_STREAM) ? 0 : chunk % ctx->n_streams;
+          const void *in = static_cast<const char *>(c.input) + (size_t)f0 * frame_bytes;
+          if(c.host)
+          {
+            // staging buffer s may be overwritten once the chunk that last used it has consumed it
+            if(chunk >= ((flags & SSD_FLAG_SINGLE_STREAM) ? 1 : ctx->n_streams))
+              CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_in_free[s], 0));
+            CK(cudaMemcpyAsync(ctx->d_stage[s], in, (size_t)nf * frame_bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
+            in = ctx->d_stage[s];
+            CK(cudaEventRecord(ctx->ev_in_ready[s], ctx->copy_stream));
+            CK(cudaStreamWaitEvent(ctx->stream[s], ctx->ev_in_ready[s], 0));
+          }
+          const auto csrc = chunk_src(src, in);
+          const auto ccam = chunk_cam(cam, f0, chunks[chunk].r0);
+          cudaEvent_t *ev = stage_timing ? &ctx->stage_ev[(size_t)chunk * (SSD_GPU_N_STAGES + 1)] : nullptr;
+          const int rc = ctx->outline_small
+                           ? launch_classic<OutlineSharedSmall>(ctx, s, csrc, f0, nf, chunks[chunk].r0, chunks[chunk].nr, &launches, ev, ccam, ov_lens)
+                           : launch_classic<OutlineShared>(ctx, s, csrc, f0, nf, chunks[chunk].r0, chunks[chunk].nr, &launches, ev, ccam, ov_lens);
+          if(rc)
+            return rc;
+          if(c.host)
+            CK(cudaEventRecord(ctx->ev_in_free[s], ctx->stream[s])); // all three passes have read the staging
+        }
+        return SSD_OK;
+      };
+      // The call's one source: vertices, or depth frames deprojected inside the point kernels, with the pin-hole tables (a camera
+      // call's per camera) or the rays of a distorted lens. Each chunk sets the input pointer.
+      const float unit = c.intr ? c.intr->depth_unit : 0.f;
+      const unsigned long long wmagic = (((unsigned long long)1 << 40) + (unsigned long long)p.W - 1) / (unsigned long long)p.W;
+      const auto run_depth = [&](auto sample, const auto &cam) -> int {
+        typedef decltype(sample) T;
+        if(use_lens)
+          return run_chunks(SrcLensT<T>{ nullptr, ctx->d_ray, ctx->d_cam_ray, unit }, cam);
+        return run_chunks(SrcDepthT<T>{ nullptr, ctx->d_xn, ctx->d_yn, unit, wmagic }, cam);
+      };
+      const auto run_source = [&](const auto &cam) -> int {
+        switch(c.kind)
+        {
+        case IN_VERTICES:
+          return run_chunks(SrcVertices{}, cam);
+        case IN_Z16:
+          return run_depth(uint16_t(), cam);
+        case IN_F32:
+          return run_depth(float(), cam);
+        }
+        return SSD_E_INVALID_ARG;
+      };
+      const int rs = group_frames ? run_source(grp) : cam_of_frame ? run_source(cams) : run_source(NoCam());
+      if(rs)
+        return rs;
+      if(c.host)
+        CK(cudaEventRecord(ctx->ev_h2d1, ctx->copy_stream));
+      // join stream 1 into stream 0, then bring the compact results home
+      for(int i = 1; i < ctx->n_streams; i++)
+      {
+        CK(cudaEventRecord(ctx->ev_chunk_done[i], ctx->stream[i]));
+        CK(cudaStreamWaitEvent(ctx->stream[0], ctx->ev_chunk_done[i], 0));
+      }
+      CK(cudaMemcpyAsync(ctx->h_out, ctx->d_out, sizeof(FrameOut) * (size_t)n_records, cudaMemcpyDeviceToHost, ctx->stream[0]));
+      if(ctx->ov.enabled)
+        CK(cudaMemcpyAsync(ctx->h_ovl, ctx->d_ovl, sizeof(ssd_gpu_overlay) * SSD_GPU_MAX_STEPS * (size_t)n_frames, cudaMemcpyDeviceToHost, ctx->stream[0]));
+      CK(cudaEventRecord(ctx->ev_stop, ctx->stream[0]));
+      CK(cudaEventSynchronize(ctx->ev_stop));
+      CK(cudaGetLastError());
+      float ms = 0;
+      CK(cudaEventElapsedTime(&ms, ctx->ev_start, ctx->ev_stop));
+      ctx->timing.total_ms = ms;
+      ctx->timing.h2d_ms = 0;
+      if(c.host)
+      {
+        float h = 0;
+        CK(cudaEventElapsedTime(&h, ctx->ev_h2d0, ctx->ev_h2d1));
+        ctx->timing.h2d_ms = h;
+      }
+      ctx->timing.label_ms = 0;
+      ctx->timing.n_launches = launches;
+      for(int i = 0; i < SSD_GPU_N_STAGES; i++)
+      {
+        ctx->stage_ms[i] = 0;
+        ctx->stage_launches[i] = 0;
+      }
+      if(stage_timing)
+      {
+        for(int ch = 0; ch < n_chunks; ch++)
+          for(int i = 0; i < SSD_GPU_N_STAGES; i++)
+          {
+            float t = 0;
+            const cudaEvent_t *ev = &ctx->stage_ev[(size_t)ch * (SSD_GPU_N_STAGES + 1)];
+            CK(cudaEventElapsedTime(&t, ev[i], ev[i + 1]));
+            ctx->stage_ms[i] += t;
+            ctx->stage_launches[i]++;
+          }
+        ctx->timing.label_ms = ctx->stage_ms[0];
+      }
+      return SSD_OK;
+    }();
+  // A refused call (INVALID_ARG, RANGE or STATE from check_call) has changed no result: the previous ones stay readable. Every other
+  // failure is a device error (SSD_E_CUDA) in step 8's table build or in the chain: a launch error, a bad user pointer, out of memory
+  // while growing a staging buffer. It may leave streams unsynchronised and BEV bitmaps half written (the bitmaps are
+  // "self-cleaning" only along a complete chain): bring the context back to a clean state so that the next call starts from zeroed
+  // bitmaps and no stale results can be read.
+  if(rc == SSD_E_CUDA)
   {
     const std::string keep = ctx->err;
     cudaDeviceSynchronize();
     cudaGetLastError();
-    if(ctx->d_bev)
-      cudaMemset(ctx->d_bev, 0, (size_t)ctx->n_streams * ctx->chunk_frames * SSD_GPU_MAX_PLATEAUS * ctx->bm_words * 4);
+    cudaMemset(ctx->d_bev, 0, (size_t)ctx->n_streams * ctx->chunk_frames * SSD_GPU_MAX_PLATEAUS * ctx->bm_words * 4);
     ctx->n_frames_last = 0;
     ctx->step_labels_last = false;
     ctx->surfaces_last = false;
@@ -1325,45 +1346,37 @@ extern "C"
 
 int ssd_gpu_process_host(ssd_gpu_ctx *ctx, const float *xyz_host, int n_frames)
 {
-  return process_common(ctx, xyz_host, nullptr, nullptr, true, n_frames, 0);
+  return process(ctx, { CALL_PLAIN, IN_VERTICES, xyz_host, true, n_frames, 0 });
 }
 
 int ssd_gpu_process_device(ssd_gpu_ctx *ctx, const float *xyz_dev, int n_frames)
 {
-  return process_common(ctx, xyz_dev, nullptr, nullptr, false, n_frames, 0);
+  return process(ctx, { CALL_PLAIN, IN_VERTICES, xyz_dev, false, n_frames, 0 });
 }
 
 int ssd_gpu_process_device_ex(ssd_gpu_ctx *ctx, const float *xyz_dev, int n_frames, int flags)
 {
-  return process_common(ctx, xyz_dev, nullptr, nullptr, false, n_frames, flags);
+  return process(ctx, { CALL_PLAIN, IN_VERTICES, xyz_dev, false, n_frames, flags });
 }
 
 int ssd_gpu_process_depth_host(ssd_gpu_ctx *ctx, const uint16_t *z16_host, const ssd_gpu_intrinsics *intr, int n_frames)
 {
-  if(!z16_host || !intr)
-    return fail(ctx, SSD_E_INVALID_ARG, "process_depth: bad argument");
-  return process_common(ctx, nullptr, z16_host, intr, true, n_frames, 0);
+  return process(ctx, { CALL_PLAIN, IN_Z16, z16_host, true, n_frames, 0, intr });
 }
 
 int ssd_gpu_process_depth_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const ssd_gpu_intrinsics *intr, int n_frames)
 {
-  if(!z16_dev || !intr)
-    return fail(ctx, SSD_E_INVALID_ARG, "process_depth: bad argument");
-  return process_common(ctx, nullptr, z16_dev, intr, false, n_frames, 0);
+  return process(ctx, { CALL_PLAIN, IN_Z16, z16_dev, false, n_frames, 0, intr });
 }
 
 int ssd_gpu_process_depth_f32_host(ssd_gpu_ctx *ctx, const float *depth_host, const ssd_gpu_intrinsics *intr, int n_frames)
 {
-  if(!depth_host || !intr)
-    return fail(ctx, SSD_E_INVALID_ARG, "process_depth_f32: bad argument");
-  return process_common<float>(ctx, nullptr, depth_host, intr, true, n_frames, 0);
+  return process(ctx, { CALL_PLAIN, IN_F32, depth_host, true, n_frames, 0, intr });
 }
 
 int ssd_gpu_process_depth_f32_device(ssd_gpu_ctx *ctx, const float *depth_dev, const ssd_gpu_intrinsics *intr, int n_frames)
 {
-  if(!depth_dev || !intr)
-    return fail(ctx, SSD_E_INVALID_ARG, "process_depth_f32: bad argument");
-  return process_common<float>(ctx, nullptr, depth_dev, intr, false, n_frames, 0);
+  return process(ctx, { CALL_PLAIN, IN_F32, depth_dev, false, n_frames, 0, intr });
 }
 
 // ---- per-frame cameras ----
@@ -1583,140 +1596,74 @@ int ssd_gpu_n_cameras(ssd_gpu_ctx *ctx)
   return ctx ? ctx->n_cameras : SSD_E_INVALID_ARG;
 }
 
-// Everything a camera call can be refused for, before anything is launched (the previous results stay readable).
-static int check_cameras(ssd_gpu_ctx *ctx, const void *input, const int32_t *cam_of_frame, int n_frames, bool depth)
-{
-  if(!ctx || !input || !cam_of_frame || n_frames <= 0)
-    return fail(ctx, SSD_E_INVALID_ARG, "camera call: bad argument");
-  if(ctx->n_cameras <= 0)
-    return fail(ctx, SSD_E_STATE, "camera call: no camera table (ssd_gpu_set_cameras)");
-  if(n_frames > ctx->max_frames)
-    return fail(ctx, SSD_E_RANGE, "process: n_frames exceeds max_frames of the context");
-  if(depth && ctx->dp.W % 4 != 0)
-    return fail(ctx, SSD_E_INVALID_ARG, "depth input: the frame width must be a multiple of 4");
-  for(int f = 0; f < n_frames; f++)
-  {
-    const int32_t c = cam_of_frame[f];
-    if(c < 0 || c >= ctx->n_cameras)
-      return fail(ctx, SSD_E_RANGE, "camera call: frame " + std::to_string(f) + " names camera " + std::to_string(c) + ", outside [0, " +
-                                      std::to_string(ctx->n_cameras) + ")");
-    if(depth && !ctx->cam_depth_ok[c])
-      return fail(ctx, SSD_E_INVALID_ARG, "depth camera call: camera " + std::to_string(c) + " has no depth intrinsics (fx, fy must be non-zero and "
-                                                                                            "depth_unit positive)");
-  }
-  return SSD_OK;
-}
-
 int ssd_gpu_process_cameras_host(ssd_gpu_ctx *ctx, const float *xyz_host, const int32_t *camera_of_frame, int n_frames)
 {
-  const int rc = check_cameras(ctx, xyz_host, camera_of_frame, n_frames, false);
-  return rc ? rc : process_common(ctx, xyz_host, nullptr, nullptr, true, n_frames, 0, camera_of_frame);
+  return process(ctx, { CALL_CAMERAS, IN_VERTICES, xyz_host, true, n_frames, 0, nullptr, camera_of_frame });
 }
 
 int ssd_gpu_process_cameras_device(ssd_gpu_ctx *ctx, const float *xyz_dev, const int32_t *camera_of_frame, int n_frames)
 {
-  const int rc = check_cameras(ctx, xyz_dev, camera_of_frame, n_frames, false);
-  return rc ? rc : process_common(ctx, xyz_dev, nullptr, nullptr, false, n_frames, 0, camera_of_frame);
+  return process(ctx, { CALL_CAMERAS, IN_VERTICES, xyz_dev, false, n_frames, 0, nullptr, camera_of_frame });
 }
 
 int ssd_gpu_process_cameras_device_ex(ssd_gpu_ctx *ctx, const float *xyz_dev, const int32_t *camera_of_frame, int n_frames, int flags)
 {
-  const int rc = check_cameras(ctx, xyz_dev, camera_of_frame, n_frames, false);
-  return rc ? rc : process_common(ctx, xyz_dev, nullptr, nullptr, false, n_frames, flags, camera_of_frame);
+  return process(ctx, { CALL_CAMERAS, IN_VERTICES, xyz_dev, false, n_frames, flags, nullptr, camera_of_frame });
 }
 
 int ssd_gpu_process_depth_cameras_host(ssd_gpu_ctx *ctx, const uint16_t *z16_host, const int32_t *camera_of_frame, int n_frames)
 {
-  const int rc = check_cameras(ctx, z16_host, camera_of_frame, n_frames, true);
-  return rc ? rc : process_common(ctx, nullptr, z16_host, nullptr, true, n_frames, 0, camera_of_frame);
+  return process(ctx, { CALL_CAMERAS, IN_Z16, z16_host, true, n_frames, 0, nullptr, camera_of_frame });
 }
 
 int ssd_gpu_process_depth_cameras_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const int32_t *camera_of_frame, int n_frames)
 {
-  const int rc = check_cameras(ctx, z16_dev, camera_of_frame, n_frames, true);
-  return rc ? rc : process_common(ctx, nullptr, z16_dev, nullptr, false, n_frames, 0, camera_of_frame);
+  return process(ctx, { CALL_CAMERAS, IN_Z16, z16_dev, false, n_frames, 0, nullptr, camera_of_frame });
 }
 
 int ssd_gpu_process_depth_f32_cameras_host(ssd_gpu_ctx *ctx, const float *depth_host, const int32_t *camera_of_frame, int n_frames)
 {
-  const int rc = check_cameras(ctx, depth_host, camera_of_frame, n_frames, true);
-  return rc ? rc : process_common<float>(ctx, nullptr, depth_host, nullptr, true, n_frames, 0, camera_of_frame);
+  return process(ctx, { CALL_CAMERAS, IN_F32, depth_host, true, n_frames, 0, nullptr, camera_of_frame });
 }
 
 int ssd_gpu_process_depth_f32_cameras_device(ssd_gpu_ctx *ctx, const float *depth_dev, const int32_t *camera_of_frame, int n_frames)
 {
-  const int rc = check_cameras(ctx, depth_dev, camera_of_frame, n_frames, true);
-  return rc ? rc : process_common<float>(ctx, nullptr, depth_dev, nullptr, false, n_frames, 0, camera_of_frame);
-}
-
-// Everything a group call can be refused for, before anything is launched (the previous results stay readable). *n_frames: the
-// call's frames.
-static int check_groups(ssd_gpu_ctx *ctx, const void *input, const int32_t *cam_of_frame, const int32_t *group_frames, int n_groups, bool depth,
-                        int *n_frames)
-{
-  if(!ctx || !input || !cam_of_frame || !group_frames || n_groups < 1)
-    return fail(ctx, SSD_E_INVALID_ARG, "group call: bad argument");
-  long long total = 0;
-  for(int g = 0; g < n_groups; g++)
-  {
-    if(group_frames[g] < 1 || group_frames[g] > SSD_GPU_MAX_GROUP_FRAMES)
-      return fail(ctx, SSD_E_INVALID_ARG, "group call: group " + std::to_string(g) + " has " + std::to_string(group_frames[g]) +
-                                              " frames, outside [1, " + std::to_string(SSD_GPU_MAX_GROUP_FRAMES) + "]");
-    total += group_frames[g];
-  }
-  if(ctx->n_cameras <= 0)
-    return fail(ctx, SSD_E_STATE, "group call: no camera table (ssd_gpu_set_cameras)");
-  if(total > ctx->max_frames)
-    return fail(ctx, SSD_E_RANGE, "group call: the groups hold " + std::to_string(total) + " frames, more than max_frames of the context");
-  *n_frames = (int)total;
-  return check_cameras(ctx, input, cam_of_frame, (int)total, depth);
+  return process(ctx, { CALL_CAMERAS, IN_F32, depth_dev, false, n_frames, 0, nullptr, camera_of_frame });
 }
 
 int ssd_gpu_process_groups_host(ssd_gpu_ctx *ctx, const float *xyz_host, const int32_t *camera_of_frame, const int32_t *group_frames, int n_groups)
 {
-  int n = 0;
-  const int rc = check_groups(ctx, xyz_host, camera_of_frame, group_frames, n_groups, false, &n);
-  return rc ? rc : process_common(ctx, xyz_host, nullptr, nullptr, true, n, 0, camera_of_frame, group_frames, n_groups);
+  return process(ctx, { CALL_GROUPS, IN_VERTICES, xyz_host, true, 0, 0, nullptr, camera_of_frame, group_frames, n_groups });
 }
 
 int ssd_gpu_process_groups_device(ssd_gpu_ctx *ctx, const float *xyz_dev, const int32_t *camera_of_frame, const int32_t *group_frames, int n_groups,
                                   int flags)
 {
-  int n = 0;
-  const int rc = check_groups(ctx, xyz_dev, camera_of_frame, group_frames, n_groups, false, &n);
-  return rc ? rc : process_common(ctx, xyz_dev, nullptr, nullptr, false, n, flags, camera_of_frame, group_frames, n_groups);
+  return process(ctx, { CALL_GROUPS, IN_VERTICES, xyz_dev, false, 0, flags, nullptr, camera_of_frame, group_frames, n_groups });
 }
 
 int ssd_gpu_process_depth_groups_host(ssd_gpu_ctx *ctx, const uint16_t *z16_host, const int32_t *camera_of_frame, const int32_t *group_frames,
                                       int n_groups)
 {
-  int n = 0;
-  const int rc = check_groups(ctx, z16_host, camera_of_frame, group_frames, n_groups, true, &n);
-  return rc ? rc : process_common(ctx, nullptr, z16_host, nullptr, true, n, 0, camera_of_frame, group_frames, n_groups);
+  return process(ctx, { CALL_GROUPS, IN_Z16, z16_host, true, 0, 0, nullptr, camera_of_frame, group_frames, n_groups });
 }
 
 int ssd_gpu_process_depth_groups_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const int32_t *camera_of_frame, const int32_t *group_frames,
                                         int n_groups, int flags)
 {
-  int n = 0;
-  const int rc = check_groups(ctx, z16_dev, camera_of_frame, group_frames, n_groups, true, &n);
-  return rc ? rc : process_common(ctx, nullptr, z16_dev, nullptr, false, n, flags, camera_of_frame, group_frames, n_groups);
+  return process(ctx, { CALL_GROUPS, IN_Z16, z16_dev, false, 0, flags, nullptr, camera_of_frame, group_frames, n_groups });
 }
 
 int ssd_gpu_process_depth_f32_groups_host(ssd_gpu_ctx *ctx, const float *depth_host, const int32_t *camera_of_frame, const int32_t *group_frames,
                                           int n_groups)
 {
-  int n = 0;
-  const int rc = check_groups(ctx, depth_host, camera_of_frame, group_frames, n_groups, true, &n);
-  return rc ? rc : process_common<float>(ctx, nullptr, depth_host, nullptr, true, n, 0, camera_of_frame, group_frames, n_groups);
+  return process(ctx, { CALL_GROUPS, IN_F32, depth_host, true, 0, 0, nullptr, camera_of_frame, group_frames, n_groups });
 }
 
 int ssd_gpu_process_depth_f32_groups_device(ssd_gpu_ctx *ctx, const float *depth_dev, const int32_t *camera_of_frame, const int32_t *group_frames,
                                             int n_groups, int flags)
 {
-  int n = 0;
-  const int rc = check_groups(ctx, depth_dev, camera_of_frame, group_frames, n_groups, true, &n);
-  return rc ? rc : process_common<float>(ctx, nullptr, depth_dev, nullptr, false, n, flags, camera_of_frame, group_frames, n_groups);
+  return process(ctx, { CALL_GROUPS, IN_F32, depth_dev, false, 0, flags, nullptr, camera_of_frame, group_frames, n_groups });
 }
 
 int ssd_gpu_deproject_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const ssd_gpu_intrinsics *intr, int n_frames, float *xyz_dev)

@@ -1371,18 +1371,28 @@ __global__ void __launch_bounds__(32) k_frame_logic(const __grid_constant__ DevP
   frame_logic_warp(p, frames[f], Sc, threadIdx.x);
 }
 
-// the lenses of a group call's overlay (LensCam<GroupTable>), or none (pin-hole)
-__device__ __forceinline__ const ssd_gpu_distortion *group_lens(const GroupTable &)
+// drawStairStep (pointcloud.cpp:588-597) of one step corner q: quadriWorld -> worldToCamera (b, a_inv) -> the lens, if any (nullptr:
+// the pin-hole) -> DepthFrame::project (intrinsics)
+__device__ __forceinline__ void overlay_corner(const double *q, const double *b, const OverlayDev &ov, const ssd_gpu_distortion *lens, float *px)
 {
-  return nullptr;
+  const double dx = q[0] - b[0], dy = q[1] - b[1], dz = q[2] - b[2];
+  const float X = (float)((ov.a_inv[0] * dx + ov.a_inv[1] * dy) + ov.a_inv[2] * dz);
+  const float Y = (float)((ov.a_inv[3] * dx + ov.a_inv[4] * dy) + ov.a_inv[5] * dz);
+  const float Z = (float)((ov.a_inv[6] * dx + ov.a_inv[7] * dy) + ov.a_inv[8] * dz);
+  float x = __fdiv_rn(X, Z), y = __fdiv_rn(Y, Z);
+  if(lens)
+  {
+    const ssd_gpu_distortion d = *lens;
+    float xd, yd;
+    ssd_lens_project(&d, x, y, &xd, &yd);
+    x = xd;
+    y = yd;
+  }
+  px[0] = __fadd_rn(__fmul_rn(x, ov.fx), ov.ppx);
+  px[1] = __fadd_rn(__fmul_rn(y, ov.fy), ov.ppy);
 }
-__device__ __forceinline__ const ssd_gpu_distortion *group_lens(const LensCam<GroupTable> &c)
-{
-  return c.lens;
-}
-// A group's steps into the overlay of every member frame, each through its own camera (b, a_inv, intrinsics, lens).
-template<class GCAM>
-__device__ __forceinline__ void group_overlay(const GroupTable &g, const GCAM &cam, int slot, const double (*sq)[4][3], int nSteps,
+// A group's steps into the overlay of every member frame, each through its own camera (b, a_inv, intrinsics, lens[camera]).
+__device__ __forceinline__ void group_overlay(const GroupTable &g, const ssd_gpu_distortion *lens, int slot, const double (*sq)[4][3], int nSteps,
                                               ssd_gpu_overlay *__restrict__ overlay)
 {
   const int2 m = group_members(g, slot);
@@ -1397,56 +1407,30 @@ __device__ __forceinline__ void group_overlay(const GroupTable &g, const GCAM &c
     ssd_gpu_overlay *Q = overlay + (size_t)frame * SSD_GPU_MAX_STEPS;
     for(int s = 0; s < nSteps; s++)
       for(int k = 0; k < 4; k++)
-      {
-        const double dx = sq[s][k][0] - b[0], dy = sq[s][k][1] - b[1], dz = sq[s][k][2] - b[2];
-        const float X = (float)((ov.a_inv[0] * dx + ov.a_inv[1] * dy) + ov.a_inv[2] * dz);
-        const float Y = (float)((ov.a_inv[3] * dx + ov.a_inv[4] * dy) + ov.a_inv[5] * dz);
-        const float Z = (float)((ov.a_inv[6] * dx + ov.a_inv[7] * dy) + ov.a_inv[8] * dz);
-        float x = __fdiv_rn(X, Z), y = __fdiv_rn(Y, Z);
-        if constexpr(!std::is_same<GCAM, GroupTable>::value)
-        {
-          const ssd_gpu_distortion d = group_lens(cam)[c];
-          float xd, yd;
-          ssd_lens_project(&d, x, y, &xd, &yd);
-          x = xd;
-          y = yd;
-        }
-        Q[s].px[k][0] = __fadd_rn(__fmul_rn(x, ov.fx), ov.ppx);
-        Q[s].px[k][1] = __fadd_rn(__fmul_rn(y, ov.fy), ov.ppy);
-      }
+        overlay_corner(sq[s][k], b, ov, lens ? lens + c : nullptr, Q[s].px[k]);
   }
 }
-template<class CAM>
-struct IsGroupCam : std::false_type
+__device__ __forceinline__ const ssd_gpu_distortion *frame_lens(const ssd_gpu_distortion *lens, const NoCam &, int)
 {
-};
-template<>
-struct IsGroupCam<GroupTable> : std::true_type
-{
-};
-template<>
-struct IsGroupCam<LensCam<GroupTable>> : std::true_type
-{
-};
-__device__ __forceinline__ const GroupTable &group_table(const GroupTable &c)
-{
-  return c;
+  return lens;
 }
-__device__ __forceinline__ const GroupTable &group_table(const LensCam<GroupTable> &c)
+__device__ __forceinline__ const ssd_gpu_distortion *frame_lens(const ssd_gpu_distortion *lens, const CamTable &c, int frame)
 {
-  return c.base;
+  return lens ? lens + frame_camera(c, frame) : nullptr;
 }
 
 // ---------------------------------------------------------------------------------------------
 // k_finalize: calcGround's front edge (pointcloud.cpp:531-547), calcStairStep (:549-558), the result
 // assembly of detectStairs with ToExternalWorld (:370-383, transformation.cpp:190-194).
-// grid = frames, one block per frame.
+// grid = frames, one block per frame. ov_lens: the lenses the overlay projects through (plain calls: [0], camera and group calls: per
+// camera), or nullptr: the pin-hole.
 // ---------------------------------------------------------------------------------------------
 template<class OutlineShared, class CAM = NoCam>
 __global__ void __launch_bounds__(SSD_OL_THREADS, SSD_OL_MINB) k_finalize(const __grid_constant__ DevParams p0, FrameDev *__restrict__ frames,
                                                               FrameOut *__restrict__ out, unsigned *__restrict__ bev, size_t bm_words,
                                                               size_t smem_cap_words, const __grid_constant__ OverlayDev ov0,
-                                                              ssd_gpu_overlay *__restrict__ overlay, const CAM cam = CAM())
+                                                              ssd_gpu_overlay *__restrict__ overlay, const ssd_gpu_distortion *ov_lens,
+                                                              const CAM cam = CAM())
 {
   extern __shared__ __align__(16) unsigned s_words[];
   __shared__ OutlineShared S;
@@ -1568,27 +1552,18 @@ __global__ void __launch_bounds__(SSD_OL_THREADS, SSD_OL_MINB) k_finalize(const 
     }
     O.steps[s].height = p.ext_z + sq[s][0][2];
   }
-  if constexpr(IsGroupCam<CAM>::value)
+  if constexpr(std::is_same<CAM, GroupTable>::value)
   {
     if(ov.enabled)
-      group_overlay(group_table(cam), cam, frame, sq, nSteps, overlay);
+      group_overlay(cam, ov_lens, frame, sq, nSteps, overlay);
   }
   else if(ov.enabled)
   {
-    // drawStairStep (pointcloud.cpp:588-597): quadriWorld -> worldToCamera -> DepthFrame::project
     ssd_gpu_overlay *Q = overlay + (size_t)frame * SSD_GPU_MAX_STEPS;
+    const ssd_gpu_distortion *lens = frame_lens(ov_lens, cam, frame);
     for(int s = 0; s < nSteps; s++)
       for(int c = 0; c < 4; c++)
-      {
-        const double dx = sq[s][c][0] - p.b[0], dy = sq[s][c][1] - p.b[1], dz = sq[s][c][2] - p.b[2];
-        const float X = (float)((ov.a_inv[0] * dx + ov.a_inv[1] * dy) + ov.a_inv[2] * dz);
-        const float Y = (float)((ov.a_inv[3] * dx + ov.a_inv[4] * dy) + ov.a_inv[5] * dz);
-        const float Z = (float)((ov.a_inv[6] * dx + ov.a_inv[7] * dy) + ov.a_inv[8] * dz);
-        float x, y;
-        overlay_lens(cam, frame, __fdiv_rn(X, Z), __fdiv_rn(Y, Z), x, y);
-        Q[s].px[c][0] = __fadd_rn(__fmul_rn(x, ov.fx), ov.ppx);
-        Q[s].px[c][1] = __fadd_rn(__fmul_rn(y, ov.fy), ov.ppy);
-      }
+        overlay_corner(sq[s][c], p.b, ov, lens, Q[s].px[c]);
   }
   F.n_steps = nSteps;
   F.status = status;

@@ -304,3 +304,28 @@ def compare_results(a, b, tol=1e-4, check_labels=True):
         if not np.allclose(s["quad"], t["quad"], rtol=0, atol=tol, equal_nan=True):
             bad.append(f"step {i}.quad differs by {np.abs(s['quad'] - t['quad']).max():.3g}")
     return bad
+
+
+# ---- the GPU results of a Detector, in the form of oracle_process's ----
+def gpu_result(det, frame):
+    """everything the last call produced for one frame (labels, histogram, plateaus, steps, result line)"""
+    info = det.frame_info(frame)
+    plats, _ = det.plateaus(frame)
+    steps = (A.Step * A.MAX_STEPS)()
+    n = C.c_int()
+    det._ck(det._l.ssd_gpu_get_steps(det._h, frame, steps, A.MAX_STEPS, C.byref(n), None), "get_steps")
+    hist = np.zeros(A.MAX_BINS, np.uint32)
+    hist[:info.n_bins] = det.histogram(frame)
+    return _collect(det.labels(frame), hist, info, plats, steps, det.line(frame))
+
+
+def exact(r):
+    """everything a frame produced, doubles as exact hex, labels as a digest, and the result line"""
+    return frame_record(r, 0xffffffff), r.line
+
+
+def to_device(det, a):
+    """a copy of host array a in device memory (free with det.free)"""
+    p = det.malloc(a.nbytes)
+    det.h2d(p, a)
+    return p

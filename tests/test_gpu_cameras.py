@@ -42,17 +42,6 @@ def test_scene_camera_record(S):
 
 
 # ---- helpers ----
-def gpu_result(det, f):
-    from test_gpu_parity import gpu_result as g
-    import stair_step_detector_b200 as S
-    return g(S, det, f)
-
-
-def exact(r):
-    """everything a frame produced, doubles as exact hex, labels as a digest, and the result line"""
-    return H.frame_record(r, 0xffffffff), r.line
-
-
 def camera_scenes(S, w, h):
     """the three synthetic camera mountings (also those of examples/detect_stairs_multicamera.cpp): default; higher, pitched,
     rolled and yawed with other intrinsics and an occluder; upside down with occluders and other intrinsics"""
@@ -83,12 +72,6 @@ def mixed_batch(S, w=1024, h=768, per_cam=3, seed=7):
     return cfg, cams, order, np.stack(depth), np.stack(xyz), xfs
 
 
-def to_device(det, a):
-    p = det.malloc(a.nbytes)
-    det.h2d(p, a)
-    return p
-
-
 # ---- 1. the stored reference runs, one call per size ----
 @gpu
 @pytest.mark.parametrize("key", ["frames_random_scenes/320x240", "frames_random_scenes/640x480", "frames_random_scenes/1024x768",
@@ -111,7 +94,7 @@ def test_camera_call_against_the_reference_runs(S, key):
         det.set_cameras([S.make_camera(xf) for _, xf, _ in inputs])
         det.process_cameras_host(xyz, np.arange(len(inputs)))
         for i in range(len(inputs)):
-            g = gpu_result(det, i)
+            g = H.gpu_result(det, i)
             assert not H.compare_with_record(want[i], g, tol=TOL), (i, H.compare_with_record(want[i], g, tol=TOL))
             assert (g.info["status"] & ~R.QUIRKS) == want[i]["info"]["status"], i
 
@@ -126,7 +109,7 @@ def test_mixed_cameras_equal_the_oracle(S, oracle):
     with S.Detector(cfg, cams[1].xf, max_frames=n) as det:
         det.set_cameras(cams)
         assert det.n_cameras == 3
-        d_xyz, d_z16 = to_device(det, xyz), to_device(det, depth)
+        d_xyz, d_z16 = H.to_device(det, xyz), H.to_device(det, depth)
         for kind in ("vertices/host", "vertices/device", "z16/host", "z16/device"):
             if kind == "vertices/host":
                 det.process_cameras_host(xyz, order)
@@ -138,11 +121,11 @@ def test_mixed_cameras_equal_the_oracle(S, oracle):
                 det.process_depth_cameras_device(d_z16, order, n)
             runs[kind] = []
             for f in range(n):
-                g = gpu_result(det, f)
+                g = H.gpu_result(det, f)
                 bad = H.compare_results(want[f], g, tol=TOL)
                 assert not bad, (kind, f, order[f], bad)
                 assert g.info["status"] == want[f].info["status"], (kind, f)
-                runs[kind].append(exact(g))
+                runs[kind].append(H.exact(g))
         det.free(d_xyz)
         det.free(d_z16)
     assert sum(len(w.steps) for w in want) >= 2 * n
@@ -161,14 +144,14 @@ def test_mixed_cameras_unfused_chain_equal_the_oracle(S, oracle):
     with S.Detector(cfg, cams[0].xf, max_frames=n) as det:
         assert det.chunk_frames >= n
         det.set_cameras(cams)
-        d_xyz, d_z16 = to_device(det, xyz), to_device(det, depth)
+        d_xyz, d_z16 = H.to_device(det, xyz), H.to_device(det, depth)
         for run in range(5):
             [lambda: det.process_cameras_host(xyz, order), lambda: det.process_cameras_device(d_xyz, order, n),
              lambda: det.process_cameras_device(d_xyz, order, n, A.FLAG_STAGE_TIMING | A.FLAG_SINGLE_STREAM),
              lambda: det.process_depth_cameras_host(depth, order), lambda: det.process_depth_cameras_device(d_z16, order, n)][run]()
             assert det.timing().n_launches == 7, run  # one chunk, the seven-launch chain
             for f in range(n):
-                g = gpu_result(det, f)
+                g = H.gpu_result(det, f)
                 assert not H.compare_results(want[f], g, tol=TOL), (run, f)
                 assert g.info["status"] == want[f].info["status"], (run, f)
         det.free(d_xyz)
@@ -183,7 +166,7 @@ def test_mixed_cameras_equal_per_camera_contexts(S):
     with S.Detector(cfg, cams[0].xf, max_frames=n) as det:
         det.set_cameras(cams)
         det.process_cameras_host(xyz, order)
-        got = [exact(gpu_result(det, f)) for f in range(n)]
+        got = [H.exact(H.gpu_result(det, f)) for f in range(n)]
         st = det.stats()
     fields = ("n_points", "n_exact_fallback", "n_quad_fast", "n_quad_exact", "n_bev_exact")
     total = dict.fromkeys(fields, 0)
@@ -193,7 +176,7 @@ def test_mixed_cameras_equal_per_camera_contexts(S):
         with S.Detector(cfg, cam.xf, max_frames=len(idx)) as one:
             one.process_host(xyz[idx])
             for j, f in enumerate(idx):
-                assert exact(gpu_result(one, j)) == got[f], (c, f)
+                assert H.exact(H.gpu_result(one, j)) == got[f], (c, f)
             s1 = one.stats()
             for k in fields:
                 total[k] += getattr(s1, k)
@@ -216,7 +199,7 @@ def test_one_camera_table_equals_the_plain_call(S):
     n = len(scenes)
 
     def everything(det):
-        return [(exact(gpu_result(det, f)), det.overlay(f).tobytes(), det.vertical_faces(f)) for f in range(n)]
+        return [(H.exact(H.gpu_result(det, f)), det.overlay(f).tobytes(), det.vertical_faces(f)) for f in range(n)]
 
     with S.Detector(cfg, xf, max_frames=n) as det:
         det.set_overlay(a_inv, intr)
@@ -244,13 +227,13 @@ def test_camera_calls_over_many_chunks(S, oracle, monkeypatch):
     want = [H.oracle_process(oracle, cfg, xfs[f], xyz[f]) for f in range(n)]
     with S.Detector(cfg, cams[2].xf, max_frames=n) as det:
         assert det.chunk_frames == 8 and n > 8
-        d_xyz, d_z16 = to_device(det, xyz), to_device(det, depth)
+        d_xyz, d_z16 = H.to_device(det, xyz), H.to_device(det, depth)
         det.set_cameras(cams)
         for run in range(4):
             [lambda: det.process_cameras_host(xyz, order), lambda: det.process_cameras_device(d_xyz, order, n),
              lambda: det.process_depth_cameras_host(depth, order), lambda: det.process_depth_cameras_device(d_z16, order, n)][run]()
             for f in range(n):
-                g = gpu_result(det, f)
+                g = H.gpu_result(det, f)
                 assert not H.compare_results(want[f], g, tol=TOL), (run, f)
                 assert g.info["status"] == want[f].info["status"], (run, f)
         det.free(d_xyz)
@@ -304,7 +287,7 @@ def test_per_frame_poses_at_scale(S, oracle):
             det.d2h(xyz, C.c_void_p(d_xyz.value + int(f) * N * 12))
             xf = S.scene_transform(scenes[f])
             o = H.oracle_process(oracle, cfg, xf, xyz)
-            g = gpu_result(det, int(f))
+            g = H.gpu_result(det, int(f))
             assert not H.compare_results(o, g, tol=TOL), f
             assert g.info["status"] == o.info["status"], f
         det.free(d_xyz)
@@ -320,7 +303,7 @@ def test_camera_call_rejections(S):
         with pytest.raises(S.SsdError, match=r"\(-5\).*no camera table"):
             det.process_cameras_host(xyz, order)
         det.process_host(xyz)
-        plain = [exact(gpu_result(det, f)) for f in range(n)]
+        plain = [H.exact(H.gpu_result(det, f)) for f in range(n)]
         with pytest.raises(S.SsdError, match=r"\(-5\)"):
             det.process_cameras_host(xyz, order)
         det.set_cameras(cams)
@@ -338,17 +321,17 @@ def test_camera_call_rejections(S):
         with pytest.raises(S.SsdError, match=r"\(-1\).*intrinsics"):
             det.process_depth_cameras_host(depth, o)
         # rejected calls left the plain call's results readable
-        assert [exact(gpu_result(det, f)) for f in range(n)] == plain
+        assert [H.exact(H.gpu_result(det, f)) for f in range(n)] == plain
         # camera 3 has the transform of camera 0 but no intrinsics: fine for vertex input
         det.process_cameras_host(xyz, o)
-        mixed = [exact(gpu_result(det, f)) for f in range(n)]
+        mixed = [H.exact(H.gpu_result(det, f)) for f in range(n)]
         # a plain call after a camera call uses the context's own transform
         det.process_host(xyz)
-        assert [exact(gpu_result(det, f)) for f in range(n)] == plain
+        assert [H.exact(H.gpu_result(det, f)) for f in range(n)] == plain
         # replacing the table takes effect: the reversed table with reversed indices is the same batch
         det.set_cameras(no_intr[::-1])
         det.process_cameras_host(xyz, 3 - o)
-        assert [exact(gpu_result(det, f)) for f in range(n)] == mixed
+        assert [H.exact(H.gpu_result(det, f)) for f in range(n)] == mixed
         with pytest.raises(S.SsdError, match=r"\(-1\)"):
             det.process_depth_cameras_host(depth, 3 - o)  # now camera 0 lacks the intrinsics
         det.set_cameras([])

@@ -13,7 +13,7 @@ import pytest
 
 import helpers as H
 from stair_step_detector_b200 import _abi as A
-from test_gpu_distortion import BC, IBC, NOISY, exact, gpu_result, lens_scene, np_deproject, to_device
+from test_gpu_distortion import BC, IBC, NOISY, lens_scene, np_deproject
 
 gpu = pytest.mark.gpu
 f32 = np.float32
@@ -52,7 +52,7 @@ def canon(x):
 
 def everything(S, det, n):
     """every result of the last call of det (all options on)"""
-    frames = [(exact(gpu_result(S, det, f)), det.overlay(f).tobytes(), canon(det.vertical_faces(f)), det.step_labels(f).tobytes(),
+    frames = [(H.exact(H.gpu_result(det, f)), det.overlay(f).tobytes(), canon(det.vertical_faces(f)), det.step_labels(f).tobytes(),
                canon(det.step_surfaces(f))) for f in range(n)]
     return frames, bytes(det.stats()), det.timing().n_launches
 
@@ -127,7 +127,7 @@ def test_float_of_z16_equals_z16(S, monkeypatch, size, n):
     assert sum(groups) == n and max(groups) > 2
     with S.Detector(cfg, xf, max_frames=n) as det:
         all_options(det, a_inv, intr)
-        d_z16, d_f, d_m = to_device(det, depth), to_device(det, as_float), to_device(det, metres)
+        d_z16, d_f, d_m = H.to_device(det, depth), H.to_device(det, as_float), H.to_device(det, metres)
         # each float call against the z16 call of the same input kind (host input runs in host chunks: other launch counts)
         plain = {"host": (lambda: det.process_depth_host(depth, intr),
                           {"": lambda: det.process_depth_f32_host(as_float, intr),
@@ -185,7 +185,7 @@ def test_float_of_z16_equals_z16_4096x3072(S):
         assert all(fr[0][0]["steps"] for fr in want[0])
         det.process_depth_f32_host(depth.astype(f32), intr)
         assert everything(S, det, n) == want
-        d_f = to_device(det, depth.astype(f32))
+        d_f = H.to_device(det, depth.astype(f32))
         det.process_depth_f32_device(d_f, intr, n)
         assert everything(S, det, n) == want
         det.free(d_f)
@@ -248,7 +248,7 @@ def test_float_frames_equal_vertex_input(S, size, lens):
                 assert sum(len(fr[0][0]["steps"]) for fr in want[0]) >= n
             intr = intr_with_unit(S, base, float(unit))
             det.set_cameras([camera_with_unit(S, base, float(unit))], [S.scene_distortion(base)])
-            d_f = to_device(det, frames)
+            d_f = H.to_device(det, frames)
             for kind, run in {"host": lambda: det.process_depth_f32_host(frames, intr),
                               "device": lambda: det.process_depth_f32_device(d_f, intr, n),
                               "camera host": lambda: det.process_depth_f32_cameras_host(frames, np.zeros(n, np.int32)),

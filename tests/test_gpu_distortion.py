@@ -210,21 +210,6 @@ def test_scene_distortion_is_real(S, name):
 
 
 # ---- GPU ----
-def gpu_result(S, det, f):
-    from test_gpu_parity import gpu_result as g
-    return g(S, det, f)
-
-
-def exact(r):
-    return H.frame_record(r, 0xffffffff), r.line
-
-
-def to_device(det, a):
-    p = det.malloc(a.nbytes)
-    det.h2d(p, a)
-    return p
-
-
 def lens_frames(S, w, h, lens, n, seed, cfg_kw=None, **kw):
     base = lens_scene(S, w, h, lens, **dict(NOISY, **kw))
     scenes = [S.randomize_scene(base, seed, i, 3, 8) for i in range(n)]
@@ -248,15 +233,15 @@ def test_lens_z16_equals_vertex_input(S, oracle, name, size):
     with S.Detector(cfg, xf, max_frames=n) as det:
         det.set_vertical_faces(True)
         det.process_host(xyz)
-        want = [exact(gpu_result(S, det, f)) for f in range(n)]
+        want = [H.exact(H.gpu_result(det, f)) for f in range(n)]
         want_r = [det.vertical_faces(f) for f in range(n)]
         for f in range(n):
             o = H.oracle_process(oracle, cfg, xf, xyz[f])
-            assert not H.compare_results(o, gpu_result(S, det, f), tol=TOL), f
+            assert not H.compare_results(o, H.gpu_result(det, f), tol=TOL), f
             assert want_r[f] == H.oracle_vertical_faces(oracle, cfg, xf, xyz[f])
         assert sum(len(H.oracle_process(oracle, cfg, xf, xyz[f]).steps) for f in range(n)) >= 2 * n
         det.set_distortion(dist)
-        d_z16 = to_device(det, depth)
+        d_z16 = H.to_device(det, depth)
         det.set_cameras([S.scene_camera(base)], [dist])
         runs = {"plain/host": lambda: det.process_depth_host(depth, intr),
                 "plain/device": lambda: det.process_depth_device(d_z16, intr, n),
@@ -265,7 +250,7 @@ def test_lens_z16_equals_vertex_input(S, oracle, name, size):
         for kind, run in runs.items():
             run()
             for f in range(n):
-                assert exact(gpu_result(S, det, f)) == want[f], (kind, f)
+                assert H.exact(H.gpu_result(det, f)) == want[f], (kind, f)
                 assert det.vertical_faces(f) == want_r[f], (kind, f)
         det.free(d_z16)
 
@@ -279,10 +264,10 @@ def test_lens_z16_4096x3072(S, name):
     xf = S.scene_transform(base)
     with S.Detector(cfg, xf, max_frames=n) as det:
         det.process_host(xyz)
-        want = [exact(gpu_result(S, det, f)) for f in range(n)]
+        want = [H.exact(H.gpu_result(det, f)) for f in range(n)]
         det.set_distortion(S.scene_distortion(base))
         det.process_depth_host(depth, S.scene_intrinsics(base))
-        assert [exact(gpu_result(S, det, f)) for f in range(n)] == want
+        assert [H.exact(H.gpu_result(det, f)) for f in range(n)] == want
         assert det.n_ray_tables == 1
 
 
@@ -297,7 +282,7 @@ def test_deproject_device(S, name):
     intr, dist = S.scene_intrinsics(base), S.scene_distortion(base)
     with S.Detector(cfg, xf, max_frames=n) as det:
         det.set_distortion(dist)
-        d_z16 = to_device(det, depth)
+        d_z16 = H.to_device(det, depth)
         d_xyz = det.malloc(xyz.nbytes)
         det.deproject_device(d_z16, intr, n, d_xyz)
         got = np.empty_like(xyz)
@@ -364,12 +349,12 @@ def test_mixed_lens_table_in_one_call(S):
         det.set_cameras(cams, dists)
         assert det.n_ray_tables == 3  # pin-hole (cameras 0, 4), BC (1, 3), IBC (2)
         det.process_depth_cameras_host(depth, order)
-        got = [exact(gpu_result(S, det, f)) for f in range(n)]
+        got = [H.exact(H.gpu_result(det, f)) for f in range(n)]
     for f, c in enumerate(order):
         with S.Detector(cfg, cams[c].xf, max_frames=1) as one:
             one.set_distortion(dists[c])
             one.process_depth_host(depth[f:f + 1], cams[c].intr)
-            assert exact(gpu_result(S, one, 0)) == got[f], f
+            assert H.exact(H.gpu_result(one, 0)) == got[f], f
             if c in (0, 4):
                 assert one.n_ray_tables == 0  # the plain pin-hole call: the existing kernels
 
@@ -385,15 +370,15 @@ def test_zero_coefficient_lens_runs_the_pinhole_kernels(S, model):
     zero = S.make_distortion(model)
     with S.Detector(cfg, xf, max_frames=n) as det:
         det.process_depth_host(depth, intr)
-        want = [exact(gpu_result(S, det, f)) for f in range(n)]
+        want = [H.exact(H.gpu_result(det, f)) for f in range(n)]
         launches = det.timing().n_launches
         det.set_distortion(zero)
         det.process_depth_host(depth, intr)
-        assert [exact(gpu_result(S, det, f)) for f in range(n)] == want
+        assert [H.exact(H.gpu_result(det, f)) for f in range(n)] == want
         assert det.n_ray_tables == 0 and det.timing().n_launches == launches  # no ray table exists: the z16 kernels ran
         det.set_cameras([S.scene_camera(base)], [zero])
         det.process_depth_cameras_host(depth, np.zeros(n, np.int32))
-        assert [exact(gpu_result(S, det, f)) for f in range(n)] == want
+        assert [H.exact(H.gpu_result(det, f)) for f in range(n)] == want
         assert det.n_ray_tables == 0
 
 
@@ -451,10 +436,10 @@ def test_errors_leave_results_and_table_in_place(S):
     with S.Detector(cfg, xf, max_frames=n) as det:
         det.set_cameras([S.scene_camera(base)], [dist])
         det.process_depth_cameras_host(depth, np.zeros(n, np.int32))
-        want = [exact(gpu_result(S, det, f)) for f in range(n)]
+        want = [H.exact(H.gpu_result(det, f)) for f in range(n)]
 
         def unchanged():
-            assert [exact(gpu_result(S, det, f)) for f in range(n)] == want
+            assert [H.exact(H.gpu_result(det, f)) for f in range(n)] == want
             assert det.n_cameras == 1 and det.n_ray_tables == 1
 
         for model in (1, 3, 5, 7):

@@ -61,13 +61,13 @@ def run_paths(S, cfg, xf, xyz):
     with S.Detector(cfg, xf, max_frames=1) as det:
         det.process_host(xyz[None])
         assert det.timing().n_launches == 5
-        res["fused"] = T.gpu_result(S, det, 0)
+        res["fused"] = H.gpu_result(det, 0)
         d = det.malloc(xyz.nbytes)
         try:
             det.h2d(d, xyz)
             det.process_device(d, 1, A.FLAG_STAGE_TIMING)
             assert det.timing().n_launches == 7
-            res["seven-launch"] = T.gpu_result(S, det, 0)
+            res["seven-launch"] = H.gpu_result(det, 0)
         finally:
             det.free(d)
     return res
@@ -169,8 +169,8 @@ def test_two_contexts_of_different_sizes_alternate(S, oracle):
             for _ in range(2):
                 small.process_host(small_xyz[None])
                 big.process_host(big_xyz[None])
-                assert not H.compare_results(H.oracle_process(oracle, big_cfg, big_xf, big_xyz), T.gpu_result(S, big, 0), tol=TOL)
-                assert not H.compare_results(H.oracle_process(oracle, small_cfg, small_xf, small_xyz), T.gpu_result(S, small, 0), tol=TOL)
+                assert not H.compare_results(H.oracle_process(oracle, big_cfg, big_xf, big_xyz), H.gpu_result(big, 0), tol=TOL)
+                assert not H.compare_results(H.oracle_process(oracle, small_cfg, small_xf, small_xyz), H.gpu_result(small, 0), tol=TOL)
 
 
 def test_misaligned_device_input_is_refused(S):

@@ -95,15 +95,6 @@ class Group:
 oracle_group = Group
 
 
-def gpu_result(S, det, f):
-    from test_gpu_parity import gpu_result as g
-    return g(S, det, f)
-
-
-def exact(r):
-    return H.frame_record(r, 0xffffffff), r.line
-
-
 def camera_scenes(S, w, h):
     from test_gpu_cameras import camera_scenes as cs
     return cs(S, w, h)
@@ -122,12 +113,6 @@ def frames_of(S, bases, cam_index, seed, lens_of=None):
         depth.append(d)
         xyz.append(S.deproject_host(sc, d))
     return np.stack(depth), np.stack(xyz)
-
-
-def to_device(det, a):
-    p = det.malloc(a.nbytes)
-    det.h2d(p, a)
-    return p
 
 
 def starts(sizes):
@@ -203,7 +188,7 @@ def test_oracle_group_histogram_and_label_classes(S, oracle):
 
 # ---- 1. groups of one frame equal the camera call ----
 def _everything(S, det, n):
-    return [(exact(gpu_result(S, det, f)), det.overlay(f).tobytes(), det.vertical_faces(f)) for f in range(n)]
+    return [(H.exact(H.gpu_result(det, f)), det.overlay(f).tobytes(), det.vertical_faces(f)) for f in range(n)]
 
 
 def _stats(det):
@@ -231,7 +216,7 @@ def test_groups_of_one_equal_the_camera_call(S, size):
             det.set_cameras(cams, dist)
             det.set_overlay(np.array(cams[0].a_inv[:]), cams[0].intr)
             det.set_vertical_faces(True)
-            d_xyz, d_z16 = to_device(det, xyz), to_device(det, depth)
+            d_xyz, d_z16 = H.to_device(det, xyz), H.to_device(det, depth)
             calls = [("vertices/host", lambda: det.process_cameras_host(xyz, idx), lambda: det.process_groups_host(xyz, idx, ones)),
                      ("vertices/device", lambda: det.process_cameras_device(d_xyz, idx, n), lambda: det.process_groups_device(d_xyz, idx, ones)),
                      ("vertices/device/timing", lambda: det.process_cameras_device(d_xyz, idx, n, A.FLAG_STAGE_TIMING),
@@ -254,7 +239,7 @@ def test_groups_of_one_equal_the_camera_call(S, size):
 # ---- 2. mixed groups against the oracle group ----
 def _check_group(S, det, cfg, f0, g, tag, risers=False):
     for m in range(len(g.rec.labels)):
-        r = gpu_result(S, det, f0 + m)
+        r = H.gpu_result(det, f0 + m)
         assert np.array_equal(r.labels, g.rec.labels[m]), (tag, m)
         bad = H.compare_results(g.rec, r, tol=TOL, check_labels=False)
         assert not bad, (tag, m, bad)
@@ -293,7 +278,7 @@ def test_mixed_groups_equal_the_oracle(S):
         det.set_cameras(cams)
         det.set_overlay(np.array(cams[0].a_inv[:]), cams[0].intr)
         det.set_vertical_faces(True)
-        d_z16 = to_device(det, depth)
+        d_z16 = H.to_device(det, depth)
         for kind in ("vertices/host", "z16/device"):
             if kind == "vertices/host":
                 det.process_groups_host(xyz, idx, sizes)
@@ -344,7 +329,7 @@ def test_chunking_does_not_matter(S, monkeypatch):
         det.set_vertical_faces(True)
         for s, k in zip(starts(sizes), sizes):
             det.process_groups_host(xyz[s:s + k], idx[s:s + k], [k])
-            alone.append([(exact(gpu_result(S, det, m)), det.vertical_faces(m)) for m in range(k)])
+            alone.append([(H.exact(H.gpu_result(det, m)), det.vertical_faces(m)) for m in range(k)])
     # chunks of 7 frames (device input) and 5 frames (host input): the old boundaries would split most groups
     monkeypatch.setenv("SSD_GPU_CHUNK_FRAMES", "7")
     monkeypatch.setenv("SSD_GPU_HOST_CHUNK_FRAMES", "5")
@@ -352,12 +337,12 @@ def test_chunking_does_not_matter(S, monkeypatch):
         assert det.chunk_frames == 7
         det.set_cameras(cams)
         det.set_vertical_faces(True)
-        d_xyz = to_device(det, xyz)
+        d_xyz = H.to_device(det, xyz)
         for run in range(3):
             [lambda: det.process_groups_host(xyz, idx, sizes), lambda: det.process_groups_device(d_xyz, idx, sizes),
              lambda: det.process_groups_device(d_xyz, idx, sizes, A.FLAG_SINGLE_STREAM | A.FLAG_STAGE_TIMING)][run]()
             for g, (s, k) in enumerate(zip(starts(sizes), sizes)):
-                got = [(exact(gpu_result(S, det, s + m)), det.vertical_faces(s + m)) for m in range(k)]
+                got = [(H.exact(H.gpu_result(det, s + m)), det.vertical_faces(s + m)) for m in range(k)]
                 assert got == alone[g], (run, g, k)
         det.free(d_xyz)
 
@@ -417,7 +402,7 @@ def test_group_call_rejections(S):
         assert L.ssd_gpu_process_groups_host(h_, ptr(xyz), ptr(idx), ptr(sizes), 2) == A.E_STATE
         det.set_cameras(cams[:2] + [A.Camera()])  # camera 2 has no depth intrinsics
         det.process_groups_host(xyz, idx, sizes)
-        want = [exact(gpu_result(S, det, f)) for f in range(4)]
+        want = [H.exact(H.gpu_result(det, f)) for f in range(4)]
         bad_idx = np.array([0, 1, 3, 0], np.int32)
         big = np.array([2, 3], np.int32)
         cases = [(L.ssd_gpu_process_groups_host, (ptr(xyz), ptr(bad_idx), ptr(sizes), 2), A.E_RANGE),
@@ -432,9 +417,9 @@ def test_group_call_rejections(S):
                  (L.ssd_gpu_process_groups_device, (xyz.ctypes.data + 4, ptr(idx), ptr(sizes), 2, 0), A.E_INVALID_ARG)]
         for i, (fn, args, rc) in enumerate(cases):
             assert fn(h_, *args) == rc, i
-            assert [exact(gpu_result(S, det, f)) for f in range(4)] == want, i
+            assert [H.exact(H.gpu_result(det, f)) for f in range(4)] == want, i
         det.process_groups_host(xyz, idx, sizes)
-        assert [exact(gpu_result(S, det, f)) for f in range(4)] == want
+        assert [H.exact(H.gpu_result(det, f)) for f in range(4)] == want
 
 
 # ---- 7. high resolution ----
@@ -451,7 +436,7 @@ def test_group_of_two_4096x3072_depth_frames(S):
     g = oracle_group(cfg, [c.xf for c in cams], xyz)
     with S.Detector(cfg, cams[0].xf, max_frames=2) as det:
         det.set_cameras(cams)
-        d_z16 = to_device(det, depth)
+        d_z16 = H.to_device(det, depth)
         det.process_depth_groups_device(d_z16, [0, 1], [2])
         _check_group(S, det, cfg, 0, g, "4096x3072")
         det.free(d_z16)
@@ -507,11 +492,11 @@ def test_group_filters_hold_for_every_member_camera(S):
     with S.Detector(cfg, xf_s, max_frames=2) as det:
         det.set_cameras([S.make_camera(xf_s), S.make_camera(xf_t)])
         for flags in (0, A.FLAG_STAGE_TIMING):
-            d = to_device(det, xyz)
+            d = H.to_device(det, xyz)
             det.process_groups_device(d, [0, 1], [2], flags)
             det.free(d)
             _check_group(S, det, cfg, 0, g, flags)
-            r = gpu_result(S, det, 1)
+            r = H.gpu_result(det, 1)
             for s in (1, 2, 3):
                 assert r.plateaus[s]["n_in_quad"] == g.rec.plateaus[s]["n_in_quad"], s
             assert det.stats().n_quad_exact >= len(pts) // 2, (det.stats().n_quad_exact, len(pts))

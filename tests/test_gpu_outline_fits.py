@@ -102,14 +102,13 @@ def test_chain_band_and_grid_stride(S, oracle, monkeypatch, w, h, n):
     xf = S.scene_transform(base)
     scenes = [S.randomize_scene(base, 77 + w, i, 3, 8) for i in range(n)]
     xyz = np.stack([S.deproject_host(sc, S.synth_depth_host(sc)) for sc in scenes])
-    from test_gpu_parity import gpu_result
 
     def run(smem, gridx, against_oracle=False):
         with _detector(S, monkeypatch, w, h, smem, gridx, max_frames=n, cfg=cfg, xf=xf) as det:
             det.process_host(xyz)
             fused = []
             for f in range(n):
-                g = gpu_result(S, det, f)
+                g = H.gpu_result(det, f)
                 fused.append((H.frame_record(g, 0xffffffff), g.line))
                 if against_oracle:
                     o = H.oracle_process(oracle, cfg, xf, xyz[f])
@@ -117,7 +116,7 @@ def test_chain_band_and_grid_stride(S, oracle, monkeypatch, w, h, n):
             p = det.malloc(xyz.nbytes)
             det.h2d(p, xyz)
             det.process_device(p, n, A.FLAG_STAGE_TIMING)
-            seven = [(H.frame_record(gpu_result(S, det, f), 0xffffffff), gpu_result(S, det, f).line) for f in range(n)]
+            seven = [(H.frame_record(H.gpu_result(det, f), 0xffffffff), H.gpu_result(det, f).line) for f in range(n)]
             assert seven == fused, (smem, gridx)
             return fused
 

@@ -15,17 +15,6 @@ TOL = 1e-4  # metres: 0.1 mm
 NOISY = dict(noise_sigma=0.0025, dropout=0.03, n_holes=3)
 
 
-def gpu_result(S, det, frame):
-    info = det.frame_info(frame)
-    plats, _ = det.plateaus(frame)
-    steps = (A.Step * A.MAX_STEPS)()
-    n = C.c_int()
-    det._ck(det._l.ssd_gpu_get_steps(det._h, frame, steps, A.MAX_STEPS, C.byref(n), None), "get_steps")
-    hist = np.zeros(A.MAX_BINS, np.uint32)
-    hist[:info.n_bins] = det.histogram(frame)
-    return H._collect(det.labels(frame), hist, info, plats, steps, det.line(frame))
-
-
 _REFS = {}
 
 
@@ -55,7 +44,7 @@ def run_frames(S, oracle, cfg, scenes, max_bad=0):
         det.process_host(xyz)
         out = []
         for f in range(len(scenes)):
-            g = gpu_result(S, det, f)
+            g = H.gpu_result(det, f)
             o = H.oracle_process(oracle, cfg, xf, xyz[f])
             bad = H.compare_results(o, g, tol=TOL)
             assert g.info["status"] == o.info["status"], (f, hex(g.info["status"]), hex(o.info["status"]))
@@ -89,7 +78,7 @@ def test_against_the_reference_runs(S, key):
     for i, (cfg, xf, xyz) in enumerate(inputs):
         with S.Detector(cfg, xf, max_frames=1) as det:
             det.process_host(xyz[None])
-            g = gpu_result(S, det, 0)
+            g = H.gpu_result(det, 0)
         assert not H.compare_with_record(want[i], g, tol=TOL), (i, H.compare_with_record(want[i], g, tol=TOL))
         assert (g.info["status"] & ~R.QUIRKS) == want[i]["info"]["status"], i
 
@@ -142,7 +131,7 @@ def test_empty_and_garbage_frames(S, oracle):
     with S.Detector(cfg, xf, max_frames=4) as det:
         det.process_host(frames)
         for f in range(4):
-            g = gpu_result(S, det, f)
+            g = H.gpu_result(det, f)
             o = H.oracle_process(oracle, cfg, xf, frames[f])
             assert not H.compare_results(o, g, tol=TOL), f
             assert g.info["status"] == o.info["status"]
@@ -179,7 +168,7 @@ def test_depth_frame_input(S, oracle, w, h):
         ref = [(det.labels(f), det.histogram(f), det.line(f), exact_steps(f)) for f in range(n)]
         for f in range(n):
             o = H.oracle_process(oracle, cfg, xf, xyz[f])
-            assert not H.compare_results(o, gpu_result(S, det, f), tol=TOL), f
+            assert not H.compare_results(o, H.gpu_result(det, f), tol=TOL), f
         for run in ("host", "device"):
             if run == "host":
                 det.process_depth_host(depth, k)
@@ -428,7 +417,7 @@ def test_device_input_and_determinism(S, oracle):
             for (h1, q1), (h2, q2) in zip(s, s2):
                 assert h1 == h2 and np.array_equal(q1, q2)
             assert np.array_equal(lab, det.labels(f))
-            g = gpu_result(S, det, f)
+            g = H.gpu_result(det, f)
             o = H.oracle_process(oracle, cfg, xf, xyz[f])
             assert not H.compare_results(o, g, tol=TOL), f
         det.free(d_xyz)
@@ -508,7 +497,7 @@ def test_batch_properties_at_scale(S, oracle, monkeypatch):
                     xyz = np.empty((N, 3), np.float32)
                     det.d2h(xyz, C.c_void_p(d_xyz.value + f * N * 12))
                     o = H.oracle_process(oracle, cfg, xf, xyz)
-                    assert not H.compare_results(o, gpu_result(S, det, f), tol=TOL), f
+                    assert not H.compare_results(o, H.gpu_result(det, f), tol=TOL), f
                 # a frame alone == the same frame inside the batch
                 det.process_device(C.c_void_p(d_xyz.value + 300 * N * 12), 1)
                 assert det.line(0) == ref_lines[300]

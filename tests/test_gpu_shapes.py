@@ -44,21 +44,6 @@ def size_case(S, key, n):
     return cfg, base, depth, xyz
 
 
-def gpu_result(S, det, f):
-    from test_gpu_parity import gpu_result as g
-    return g(S, det, f)
-
-
-def exact(r):
-    return H.frame_record(r, 0xffffffff), r.line
-
-
-def to_device(det, a):
-    p = det.malloc(a.nbytes)
-    det.h2d(p, a)
-    return p
-
-
 def test_size_class_boundaries_are_where_the_sizes_claim():
     """the sizes sit where their comments put them: partial last BEV word, the k_outline size-class boundary. This restates
     ssd_gpu.cu's outline_small condition to document the choice of sizes; which class the library picks is not observable
@@ -97,7 +82,7 @@ def test_sizes_every_input_kind(S, oracle, key):
         det.set_vertical_faces(True)
 
         def everything():
-            return [(exact(gpu_result(S, det, f)), det.overlay(f).tobytes(), det.vertical_faces(f)) for f in range(n)]
+            return [(H.exact(H.gpu_result(det, f)), det.overlay(f).tobytes(), det.vertical_faces(f)) for f in range(n)]
 
         det.process_host(xyz)
         fused = det.timing().n_launches  # five, plus the overlay's k_finalize
@@ -105,7 +90,7 @@ def test_sizes_every_input_kind(S, oracle, key):
         n_steps = 0
         for f in range(n):
             o = H.oracle_process(oracle, cfg, xf, xyz[f])
-            g = gpu_result(S, det, f)
+            g = H.gpu_result(det, f)
             assert not H.compare_results(o, g, tol=TOL), (f, H.compare_results(o, g, tol=TOL))
             assert g.info["status"] == o.info["status"], f
             ov = H.oracle_overlay(oracle, xf, a_inv, intr)
@@ -117,7 +102,7 @@ def test_sizes_every_input_kind(S, oracle, key):
             n_steps += o.info["n_steps"]
         if steps:
             assert n_steps >= 3 * n
-        d_xyz = to_device(det, xyz)
+        d_xyz = H.to_device(det, xyz)
         det.process_device(d_xyz, n, A.FLAG_STAGE_TIMING)
         assert det.timing().n_launches == fused + 2  # k_peaks and k_frame_logic as launches of their own
         assert everything() == want, "seven-launch chain"
@@ -129,10 +114,10 @@ def test_sizes_every_input_kind(S, oracle, key):
         det.process_cameras_device(d_xyz, cof, n)
         for f in range(n):
             if cof[f]:
-                assert exact(gpu_result(S, det, f)) == want[f][0], ("camera table, own camera", f)
+                assert H.exact(H.gpu_result(det, f)) == want[f][0], ("camera table, own camera", f)
             else:
                 o = H.oracle_process(oracle, cfg, other, xyz[f])
-                g = gpu_result(S, det, f)
+                g = H.gpu_result(det, f)
                 assert not H.compare_results(o, g, tol=TOL) and g.info["status"] == o.info["status"], ("camera table, camera 0", f)
         det.free(d_xyz)
         if w % 4:
@@ -140,7 +125,7 @@ def test_sizes_every_input_kind(S, oracle, key):
                 with pytest.raises(S.SsdError, match=r"\(-1\).*multiple of 4"):
                     call()
             return
-        d_z16 = to_device(det, depth)
+        d_z16 = H.to_device(det, depth)
         for kind, run in (("z16 host", lambda: det.process_depth_host(depth, intr)),
                           ("z16 device", lambda: det.process_depth_device(d_z16, intr, n)),
                           ("z16 camera table", lambda: det.process_depth_cameras_device(d_z16, np.ones(n, np.int32), n))):
@@ -166,12 +151,12 @@ def test_sizes_lens_frame(S, oracle, key):
     with S.Detector(cfg, xf, max_frames=1) as det:
         det.set_vertical_faces(True)
         det.process_host(xyz)
-        want = (exact(gpu_result(S, det, 0)), det.vertical_faces(0))
+        want = (H.exact(H.gpu_result(det, 0)), det.vertical_faces(0))
         o = H.oracle_process(oracle, cfg, xf, xyz[0])
-        assert not H.compare_results(o, gpu_result(S, det, 0), tol=TOL)
+        assert not H.compare_results(o, H.gpu_result(det, 0), tol=TOL)
         det.set_distortion(S.scene_distortion(base))
         det.process_depth_host(depth, S.scene_intrinsics(base))
-        assert (exact(gpu_result(S, det, 0)), det.vertical_faces(0)) == want
+        assert (H.exact(H.gpu_result(det, 0)), det.vertical_faces(0)) == want
 
 
 # ---- configurations (640x480) ----
@@ -237,16 +222,16 @@ def test_configurations(S, oracle, key):
     with S.Detector(cfg, xf, max_frames=n) as det:
         det.set_vertical_faces(True)
         det.process_host(xyz)
-        want = [(exact(gpu_result(S, det, f)), det.vertical_faces(f)) for f in range(n)]
+        want = [(H.exact(H.gpu_result(det, f)), det.vertical_faces(f)) for f in range(n)]
         for f in range(n):
             o = H.oracle_process(oracle, cfg, xf, xyz[f])
-            g = gpu_result(S, det, f)
+            g = H.gpu_result(det, f)
             assert not H.compare_results(o, g, tol=TOL), (f, H.compare_results(o, g, tol=TOL))
             assert g.info["status"] == o.info["status"], f
             assert want[f][1] == H.oracle_vertical_faces(oracle, cfg, xf, xyz[f].reshape(-1, 3)), f
-        d_z16 = to_device(det, depth)
+        d_z16 = H.to_device(det, depth)
         for kind, run in (("z16 host", lambda: det.process_depth_host(depth, intr)),
                           ("z16 device", lambda: det.process_depth_device(d_z16, intr, n))):
             run()
-            assert [(exact(gpu_result(S, det, f)), det.vertical_faces(f)) for f in range(n)] == want, kind
+            assert [(H.exact(H.gpu_result(det, f)), det.vertical_faces(f)) for f in range(n)] == want, kind
         det.free(d_z16)

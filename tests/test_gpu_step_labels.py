@@ -126,17 +126,6 @@ def test_reference_map_counts_on_the_reference_runs(S, oracle, key):
 
 
 # ---- on the GPU ----
-def gpu_result(S, det, f):
-    from test_gpu_parity import gpu_result as g
-    return g(S, det, f)
-
-
-def to_device(det, a):
-    p = det.malloc(a.nbytes)
-    det.h2d(p, a)
-    return p
-
-
 def assert_maps(det, want, what, f0=0):
     for f, m in enumerate(want):
         got = det.step_labels(f0 + f)
@@ -170,14 +159,14 @@ def test_random_scenes_fused_and_seven_launch(S, oracle, w, h):
             assert_maps(det, want[:1], "vertices/host one frame (fused)")
             det.process_host(xyz)
             assert_maps(det, want, ("vertices/host", n))
-            d = to_device(det, xyz)
+            d = H.to_device(det, xyz)
             det.process_device(d, n, A.FLAG_STAGE_TIMING)
             assert det.timing().n_launches == 7 * det.stage_times()["transform_bin"][1]
             assert_maps(det, want, "vertices/device seven-launch")
             det.free(d)
             det.process_depth_host(depth, intr)
             assert_maps(det, want, "z16/host")
-            d = to_device(det, depth)
+            d = H.to_device(det, depth)
             det.process_depth_device(d, intr, n)
             assert_maps(det, want, "z16/device")
             det.free(d)
@@ -195,7 +184,7 @@ def test_hires_frame(S, oracle):
         det.set_step_labels(True)
         det.process_host(xyz[None])
         assert_maps(det, [want], "4096x3072 fused")
-        d = to_device(det, np.ascontiguousarray(xyz[None]))
+        d = H.to_device(det, np.ascontiguousarray(xyz[None]))
         det.process_device(d, 1, A.FLAG_STAGE_TIMING)
         assert_maps(det, [want], "4096x3072 seven-launch")
         det.free(d)
@@ -215,7 +204,7 @@ def test_brown_conrady_lenses(S, oracle, name):
         det.set_step_labels(True)
         det.process_depth_host(depth, S.scene_intrinsics(base))
         assert_maps(det, want, (name, "z16/host"))
-        d = to_device(det, depth)
+        d = H.to_device(det, depth)
         det.process_depth_device(d, S.scene_intrinsics(base), 5)
         assert_maps(det, want, (name, "z16/device"))
         det.free(d)
@@ -266,7 +255,7 @@ def test_groups_of_1_3_and_8(S):
         det.set_step_labels(True)
         det.process_groups_host(xyz, idx, sizes)
         assert_maps(det, want, "groups vertices/host")
-        d = to_device(det, depth)
+        d = H.to_device(det, depth)
         det.process_depth_groups_device(d, idx, sizes)
         assert_maps(det, want, "groups z16/device")
         det.free(d)
@@ -285,7 +274,7 @@ def test_quadrilateral_threshold_constructions(S, oracle):
             det.process_host(f[None])
             assert det.stats().n_quad_exact > 0, name
             assert_maps(det, [want], (name, "fused"))
-            d = to_device(det, np.ascontiguousarray(f[None]))
+            d = H.to_device(det, np.ascontiguousarray(f[None]))
             det.process_device(d, 1, A.FLAG_STAGE_TIMING)
             assert det.stats().n_quad_exact > 0, name
             assert_maps(det, [want], (name, "seven-launch"))
@@ -299,7 +288,7 @@ def _edge_map(S, oracle, cfg, xf, xyz, bit):
         det.set_step_labels(True)
         det.process_host(xyz[None])
         assert_maps(det, [want], ("fused", bit))
-        d = to_device(det, np.ascontiguousarray(xyz[None]))
+        d = H.to_device(det, np.ascontiguousarray(xyz[None]))
         det.process_device(d, 1, A.FLAG_STAGE_TIMING)
         assert_maps(det, [want], ("seven-launch", bit))
         det.free(d)
@@ -401,7 +390,7 @@ def test_invariants_at_scale(S, oracle):
 def _everything(S, det, n):
     out = []
     for f in range(n):
-        r = gpu_result(S, det, f)
+        r = H.gpu_result(det, f)
         out.append((H.frame_record(r, 0xffffffff), r.line, H.digest(r.labels), det.overlay(f).tobytes(), det.vertical_faces(f)))
     return out
 

@@ -139,11 +139,6 @@ def test_quad_construct(S, oracle, name):
 
 
 # ---- on the GPU ----
-def gpu_result(S, det, f):
-    from test_gpu_parity import gpu_result as g
-    return g(S, det, f)
-
-
 def check_against_oracle(o, g, what):
     bad = H.compare_results(o, g, tol=TOL)
     assert not bad, (what, bad)
@@ -167,7 +162,7 @@ def test_thresholds_fused_and_seven_launch(S, oracle, name, construct):
     with S.Detector(cfg, xf, max_frames=1) as det:
         det.process_host(f[None])
         assert det.timing().n_launches == 5
-        g = gpu_result(S, det, 0)
+        g = H.gpu_result(det, 0)
         check_against_oracle(o, g, "fused")
         st = det.stats()
         assert floor_counter(construct, st) >= len(pts) // 2, (floor_counter(construct, st), len(pts))
@@ -176,7 +171,7 @@ def test_thresholds_fused_and_seven_launch(S, oracle, name, construct):
         det.h2d(d, f)
         det.process_device(d, 1, A.FLAG_STAGE_TIMING)
         assert det.timing().n_launches == 7
-        assert H.frame_record(gpu_result(S, det, 0), 0xffffffff) == want, "seven-launch"
+        assert H.frame_record(H.gpu_result(det, 0), 0xffffffff) == want, "seven-launch"
         assert floor_counter(construct, det.stats()) >= len(pts) // 2, "seven-launch"
         det.free(d)
     if construct == "bins_range":
@@ -207,7 +202,7 @@ def test_thresholds_camera_table(S, oracle, construct):
         det.process_cameras_host(frames[order], order)
         st = det.stats()
         for i, c in enumerate(order):
-            check_against_oracle(H.oracle_process(oracle, cfg, cases[c][1], frames[c]), gpu_result(S, det, i), (construct, names[c]))
+            check_against_oracle(H.oracle_process(oracle, cfg, cases[c][1], frames[c]), H.gpu_result(det, i), (construct, names[c]))
         assert floor_counter(construct, st) >= sum(len(c[3]) for c in cases) // 2
 
 
@@ -259,7 +254,7 @@ def test_depth_rectangles_on_bin_boundaries(S, oracle):
         assert o.info["n_in_range"] > 100000
         with S.Detector(cfg, xf, max_frames=1) as det:
             det.process_host(xyz[None])
-            g = gpu_result(S, det, 0)
+            g = H.gpu_result(det, 0)
             check_against_oracle(o, g, ("vertex", lens))
             assert det.stats().n_exact_fallback >= o.info["n_in_range"] // 2
             want = H.frame_record(g, 0xffffffff)
@@ -272,6 +267,6 @@ def test_depth_rectangles_on_bin_boundaries(S, oracle):
                               ("z16 device", lambda: det.process_depth_device(d, intr, 1)),
                               ("z16 camera table", lambda: det.process_depth_cameras_host(depth[None], np.zeros(1, np.int32)))):
                 run()
-                assert H.frame_record(gpu_result(S, det, 0), 0xffffffff) == want, (kind, lens)
+                assert H.frame_record(H.gpu_result(det, 0), 0xffffffff) == want, (kind, lens)
                 assert det.stats().n_exact_fallback >= o.info["n_in_range"] // 2, (kind, lens)
             det.free(d)

@@ -291,14 +291,14 @@ def test_random_scenes_fused_and_seven_launch(S, oracle, w, h):
             assert_surfaces(det, want[:1], "vertices/host one frame (fused)")
             det.process_host(xyz)
             assert_surfaces(det, want, ("vertices/host", n))
-            d = L.to_device(det, xyz)
+            d = H.to_device(det, xyz)
             det.process_device(d, n, A.FLAG_STAGE_TIMING)
             assert det.timing().n_launches == 8 * det.stage_times()["transform_bin"][1]
             assert_surfaces(det, want, "vertices/device seven-launch")
             det.free(d)
             det.process_depth_host(depth, intr)
             assert_surfaces(det, want, "z16/host")
-            d = L.to_device(det, depth)
+            d = H.to_device(det, depth)
             det.process_depth_device(d, intr, n)
             assert_surfaces(det, want, "z16/device")
             det.free(d)
@@ -348,7 +348,7 @@ def test_hires_frame(S, oracle):
         det.set_step_surfaces(True)
         det.process_host(xyz[None])
         assert_surfaces(det, want, "4096x3072 fused")
-        d = L.to_device(det, np.ascontiguousarray(xyz[None]))
+        d = H.to_device(det, np.ascontiguousarray(xyz[None]))
         det.process_device(d, 1, A.FLAG_STAGE_TIMING)
         assert_surfaces(det, want, "4096x3072 seven-launch")
         det.free(d)
@@ -369,7 +369,7 @@ def test_brown_conrady_lenses(S, oracle, name):
         det.set_step_surfaces(True)
         det.process_depth_host(depth, S.scene_intrinsics(base))
         assert_surfaces(det, want, (name, "z16/host"))
-        d = L.to_device(det, depth)
+        d = H.to_device(det, depth)
         det.process_depth_device(d, S.scene_intrinsics(base), 5)
         assert_surfaces(det, want, (name, "z16/device"))
         det.free(d)
@@ -419,7 +419,7 @@ def test_groups_of_1_3_and_8(S, oracle):
         det.set_step_surfaces(True)
         det.process_groups_host(xyz, idx, sizes)
         assert_surfaces(det, want, "groups vertices/host")
-        d = L.to_device(det, depth)
+        d = H.to_device(det, depth)
         det.process_depth_groups_device(d, idx, sizes)
         assert_surfaces(det, want, "groups z16/device")
         det.free(d)
@@ -433,7 +433,7 @@ def _edge(S, oracle, cfg, xf, xyz, bit):
         det.set_step_surfaces(True)
         det.process_host(xyz[None])
         assert_surfaces(det, [want], ("fused", bit))
-        d = L.to_device(det, np.ascontiguousarray(xyz[None]))
+        d = H.to_device(det, np.ascontiguousarray(xyz[None]))
         det.process_device(d, 1, A.FLAG_STAGE_TIMING)
         assert_surfaces(det, [want], ("seven-launch", bit))
         det.free(d)
@@ -469,7 +469,7 @@ def test_edge_statuses(S, oracle):
 def _everything(S, det, n):
     out = []
     for f in range(n):
-        r = L.gpu_result(S, det, f)
+        r = H.gpu_result(det, f)
         out.append((H.frame_record(r, 0xffffffff), r.line, H.digest(r.labels), H.digest(det.step_labels(f)), det.overlay(f).tobytes(),
                     det.vertical_faces(f)))
     return out
@@ -513,7 +513,7 @@ def test_launch_counts(S):
     xf = S.scene_transform(base)
     xyz = np.stack([S.deproject_host(base, S.synth_depth_host(base))] * 40)
     with S.Detector(cfg, xf, max_frames=40) as det:
-        d = L.to_device(det, xyz)
+        d = H.to_device(det, xyz)
         det.set_step_labels(True)
         for on in (False, True):
             det.set_step_surfaces(on)
