@@ -64,7 +64,7 @@ extern "C" {
  */
 typedef struct ssd_gpu_config
 {
-  int32_t width, height;          /* streams.depth width x height; also the BEV image size (pointcloud.cpp:71) */
+  int32_t width, height;          /* streams.depth width x height: the FRAME size (ssd_gpu_create_bev: the BEV size is separate) */
   double x_min, x_max;            /* measuringRange.x  (-0.6, 0.6) */
   double y_min, y_max;            /* measuringRange.y  ( 0.1, 1.3) */
   double z_min, z_max;            /* measuringRange.z  (-0.1, 1.1) */
@@ -146,11 +146,39 @@ int ssd_gpu_device_count(void);
 /* Replaces Pointcloud::Pointcloud(const Window&, const GeometricTransformation&) (pointcloud.cpp:602-606):
  * binds the constant transform and configuration, allocates device buffers for up to max_frames frames. */
 int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int device, int max_frames, ssd_gpu_ctx **out);
+/*
+ * A context has two sizes. The FRAME size, cfg->width x cfg->height, is the pixel grid of the input, of the segment labels and
+ * step labels, and of the depth deprojection. The BEV size, bev_width x bev_height, is the bird's-eye image the detector works
+ * in. The reference ties both to Configuration.streams.depth (pointcloud.cpp:71-76); ssd_gpu_create keeps that coupling and is
+ * ssd_gpu_create_bev(cfg, cfg->width, cfg->height, ...). A BEV size of its own keeps one detector tuning (the outline constants
+ * are in BEV pixels) for frames of any resolution, and any point grid (a LiDAR range image, an unorganised M x 1 cloud).
+ * Everything the reference computes in image pixels uses the BEV size:
+ *   x_to_image = bev_width / (x_max - x_min), y_to_image = bev_height / (y_max - y_min),
+ *   min_img_y_extent = (int)(min_step_depth * bev_height / (y_max - y_min)),
+ *   the column scans, front-edge columns and vertical probes of the outline, the SSD_STATUS_BEV_OOB test, and the images the
+ *   single-stage entry points take (ssd_gpu_detect_outline, ssd_gpu_detect_front_edge).
+ * What a frame produces: the reference chain run on that frame's points, in pixel order, with the configuration whose image is
+ * the BEV size. Equivalently: pack the frame's points in pixel order into k = ceil(N_frame / N_bev) frames of BEV size, the rest
+ * filled with invalid points (0,0,0); one frame (k = 1) goes through the plain call, more through one group. The labels of the
+ * frame are the first N_frame labels of that packing; n_nonzero and n_in_range are the frame's own. min_peak_points stays
+ * absolute (pointcloud.cpp:251). Camera tables, lenses, groups, overlay, risers, step labels and step surfaces all apply; every
+ * camera of a context shares its frame size and its BEV size.
+ * Limits (each a refusal that creates nothing):
+ *   bev_width, bev_height <= 0: SSD_E_INVALID_ARG;
+ *   BEV: bev_width / 25 + 4 <= 384 scans, bev_width / 50 + 6 <= 192 line points, bev_height / 10 + 2 <= 512 vertical probes
+ *     (bev_width <= 9349, bev_height <= 5109), else SSD_E_RANGE;
+ *   frame: N = width * height with N % 16 == 0 (SSD_E_INVALID_ARG) and N <= 9348 * 5108 (SSD_E_RANGE), the largest frame with
+ *     the BEV of its own size: it keeps the 32-bit point counters of frame groups exact.
+ * Depth input also needs width % 4 == 0 and N * width < 2^40 (the exact row division of the point kernels); a depth call on a
+ * frame that breaks either returns SSD_E_INVALID_ARG and leaves the previous results readable.
+ */
+int ssd_gpu_create_bev(const ssd_gpu_config *cfg, int32_t bev_width, int32_t bev_height, const ssd_gpu_transform *xf, int device,
+                       int max_frames, ssd_gpu_ctx **out);
 void ssd_gpu_destroy(ssd_gpu_ctx *ctx);
 const char *ssd_gpu_last_error(const ssd_gpu_ctx *ctx); /* ctx may be NULL: last create() error */
 
 /* ---- the hot path: replaces Pointcloud::process (pointcloud.cpp:608-626), batched ---- */
-/* xyz: n_frames * width*height packed {float x,y,z} vertices (rs2::vertex layout, qvmTraits.h:70-90),
+/* xyz: n_frames * width*height (the frame size) packed {float x,y,z} vertices (rs2::vertex layout, qvmTraits.h:70-90),
  * row-major pixel order, invalid pixel = (0,0,0). Results stay in the ctx until the next call. */
 int ssd_gpu_process_host(ssd_gpu_ctx *ctx, const float *xyz_host, int n_frames);
 int ssd_gpu_process_device(ssd_gpu_ctx *ctx, const float *xyz_dev, int n_frames);
@@ -161,7 +189,7 @@ int ssd_gpu_process_device(ssd_gpu_ctx *ctx, const float *xyz_dev, int n_frames)
  * DepthFrame::deproject (camera.h:99-116) unless a lens is set (ssd_gpu_set_distortion, below):
  *     z = depth * depth_unit,  x = z * ((u - ppx) / fx),  y = z * ((v - ppy) / fy),   depth 0 -> invalid vertex (0,0,0)
  * single-rounded f32 operations in exactly this order. 2 bytes per pixel cross PCIe / HBM instead of 12.
- * depth: n_frames * width*height uint16, row-major.
+ * depth: n_frames * width*height (the frame size) uint16, row-major.
  */
 typedef struct ssd_gpu_intrinsics
 {
@@ -171,7 +199,7 @@ typedef struct ssd_gpu_intrinsics
 } ssd_gpu_intrinsics;
 int ssd_gpu_process_depth_host(ssd_gpu_ctx *ctx, const uint16_t *z16_host, const ssd_gpu_intrinsics *intr, int n_frames);
 int ssd_gpu_process_depth_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const ssd_gpu_intrinsics *intr, int n_frames);
-/* Deprojection alone: n_frames depth frames (device) -> packed vertices (device), for parity checks. */
+/* Deprojection alone: n_frames depth frames (device) -> packed vertices (device), for parity checks; frame size. */
 int ssd_gpu_deproject_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const ssd_gpu_intrinsics *intr, int n_frames, float *xyz_dev);
 
 /* Record CUDA events around every kernel of the chain (on the launching streams); read with ssd_gpu_get_stage_times. */
@@ -405,9 +433,9 @@ int ssd_gpu_get_vertical_faces(ssd_gpu_ctx *ctx, int frame, ssd_gpu_riser *out, 
  */
 #define SSD_STEP_LABEL_NONE 255u
 int ssd_gpu_set_step_labels(ssd_gpu_ctx *ctx, int enable);
-/* device -> host copy of frame's width*height step labels */
+/* device -> host copy of frame's width*height step labels (the frame size) */
 int ssd_gpu_get_step_labels(ssd_gpu_ctx *ctx, int frame, uint8_t *out_host);
-/* Device pointer to the step labels of the last call (n_frames * width*height bytes). */
+/* Device pointer to the step labels of the last call (n_frames * width*height bytes, the frame size). */
 int ssd_gpu_step_labels_device_ptr(ssd_gpu_ctx *ctx, const uint8_t **out);
 /*
  * Step surfaces: what the point set behind each step's height looks like -- a level tread, a ramp, a tread with something on
@@ -458,7 +486,7 @@ typedef struct ssd_gpu_step_surface
 int ssd_gpu_set_step_surfaces(ssd_gpu_ctx *ctx, int enable);
 /* out[0..min(*n, cap)): *n = n_steps of the frame, in the order of ssd_gpu_get_steps. */
 int ssd_gpu_get_step_surfaces(ssd_gpu_ctx *ctx, int frame, ssd_gpu_step_surface *out, int cap, int *n);
-/* Per-pixel segment labels (device -> host copy of width*height bytes). */
+/* Per-pixel segment labels (device -> host copy of width*height bytes, the frame size). */
 int ssd_gpu_get_labels(ssd_gpu_ctx *ctx, int frame, uint8_t *out_host);
 /* Height histogram, HeightsHistogram::calcHist (pointcloud.cpp:194-204). */
 int ssd_gpu_get_histogram(ssd_gpu_ctx *ctx, int frame, uint32_t *out, int cap, int *n_bins);
@@ -484,7 +512,7 @@ int ssd_gpu_get_stage_times(ssd_gpu_ctx *ctx, float ms[SSD_GPU_N_STAGES], int la
 const char *ssd_gpu_stage_name(int stage);
 /* Frames per launch chain (chunk) chosen for this context. */
 int ssd_gpu_chunk_frames(ssd_gpu_ctx *ctx);
-/* Device pointer to the label array of the last call (n_frames * width*height bytes). */
+/* Device pointer to the label array of the last call (n_frames * width*height bytes, the frame size). */
 int ssd_gpu_labels_device_ptr(ssd_gpu_ctx *ctx, const uint8_t **out);
 
 /* Stairs::serialize (stairs.cpp:55-70): writes the NUL-terminated line into buf; returns the length
@@ -492,11 +520,11 @@ int ssd_gpu_labels_device_ptr(ssd_gpu_ctx *ctx, const uint8_t **out);
 int ssd_stairs_serialize(const ssd_gpu_step *steps, int n, char *buf, size_t cap);
 
 /* ---- single-stage entry points (same kernels, one image / one quadrilateral) ---- */
-/* Segmentation::detectOutline (segmentation.cpp:919-971): image is width*height u8 (non-zero = set).
+/* Segmentation::detectOutline (segmentation.cpp:919-971): image is a BEV image, bev_width*bev_height u8 (non-zero = set).
  * quad_px: 4 x (x,y) image points, valid: isConvex. */
 int ssd_gpu_detect_outline(ssd_gpu_ctx *ctx, const uint8_t *image_host, int min_img_y_extent, double xy_ratio,
                            double quad_px[8], int *valid);
-/* Segmentation::detectFrontEdge (segmentation.cpp:879-917). */
+/* Segmentation::detectFrontEdge (segmentation.cpp:879-917); image as for ssd_gpu_detect_outline. */
 int ssd_gpu_detect_front_edge(ssd_gpu_ctx *ctx, const uint8_t *image_host, double left_px[2], double right_px[2], int *valid);
 /* QuadrilateralTest ctor + isPointWithin (quadrilateralTest.cpp:275-451) over n host points (x,y pairs).
  * *ctor_status = 0 ok, 1 the reference ctor would throw (then inside[] is all 0). */

@@ -205,12 +205,18 @@ class Detector:
     """One GPU context: the constant transform + configuration bound to device buffers
     (replaces Pointcloud's constructor, reference pointcloud.cpp:602-606)."""
 
-    def __init__(self, cfg, xf, device=0, max_frames=1):
+    def __init__(self, cfg, xf, device=0, max_frames=1, bev=None):
+        """bev: (width, height) of the bird's-eye image the detector works in (ssd_gpu_create_bev); None: the frame size
+        cfg.width x cfg.height, as the reference. Input frames, labels and step labels keep the frame size."""
         self._l = lib()
         self.cfg, self.xf, self.device, self.max_frames = cfg, xf, device, max_frames
         self.n_points = cfg.width * cfg.height
+        self.bev = (cfg.width, cfg.height) if bev is None else (int(bev[0]), int(bev[1]))
         h = C.c_void_p()
-        rc = self._l.ssd_gpu_create(C.byref(cfg), C.byref(xf), device, max_frames, C.byref(h))
+        if bev is None:
+            rc = self._l.ssd_gpu_create(C.byref(cfg), C.byref(xf), device, max_frames, C.byref(h))
+        else:
+            rc = self._l.ssd_gpu_create_bev(C.byref(cfg), self.bev[0], self.bev[1], C.byref(xf), device, max_frames, C.byref(h))
         if rc:
             raise SsdError(f"ssd_gpu_create failed ({rc}): {self._l.ssd_gpu_last_error(None).decode()}")
         self._h = h

@@ -133,6 +133,7 @@ PROTOTYPES = {
     "ssd_gpu_abi_version": (C.c_int, []),
     "ssd_gpu_device_count": (C.c_int, []),
     "ssd_gpu_create": (C.c_int, [_P(Config), _P(Transform), C.c_int, C.c_int, _P(_vp)]),
+    "ssd_gpu_create_bev": (C.c_int, [_P(Config), C.c_int32, C.c_int32, _P(Transform), C.c_int, C.c_int, _P(_vp)]),
     "ssd_gpu_destroy": (None, [_vp]),
     "ssd_gpu_last_error": (C.c_char_p, [_vp]),
     "ssd_gpu_process_host": (C.c_int, [_vp, _vp, C.c_int]),

@@ -36,6 +36,13 @@ struct Configuration
   double minHeightAboveGround = 0.05;
   double minStepDepth = 0.1; // minimum extent in forward (y) direction
   unsigned minPeakPoints = 2000; // absolute histogram floor (reference pointcloud.cpp:251)
+  // size of the bird's-eye image the detector works in (ssd_gpu_create_bev); {0, 0} means the depth stream's size, the reference's
+  // coupling (Projection2D, pointcloud.cpp:71-76). The outline constants are in BEV pixels: a fixed BEV keeps one detector tuning
+  // for depth frames of any resolution. Both sizes are set, or neither: Pointcloud refuses anything else (std::invalid_argument).
+  struct BinaryImage
+  {
+    int width = 0, height = 0;
+  } binaryImage;
 
   Configuration() = default;
   Configuration(int depthWidth, int depthHeight)
@@ -43,6 +50,10 @@ struct Configuration
     streams.depth.width = streams.infrared.width = depthWidth;
     streams.depth.height = streams.infrared.height = depthHeight;
   }
+
+  bool ownBinaryImage() const { return binaryImage.width != 0 || binaryImage.height != 0; }
+  int bevWidth() const { return ownBinaryImage() ? binaryImage.width : streams.depth.width; }
+  int bevHeight() const { return ownBinaryImage() ? binaryImage.height : streams.depth.height; }
 
   ssd_gpu_config abi() const
   {

@@ -34,9 +34,11 @@ void Pointcloud::ensureContext(int width, int height) const
     _config = Configuration(width, height); // the reference takes the size from its compile-time Configuration
   else if(_config.streams.depth.width != width || _config.streams.depth.height != height)
     throw std::invalid_argument("Pointcloud: frame size differs from the configured depth stream");
+  if(_config.ownBinaryImage() && !(_config.binaryImage.width > 0 && _config.binaryImage.height > 0))
+    throw std::invalid_argument("Pointcloud: Configuration::binaryImage needs a positive width and height, or both 0 (the depth stream's size)");
   const ssd_gpu_config cfg = _config.abi();
   const ssd_gpu_transform xf = _transformation.abi();
-  if(ssd_gpu_create(&cfg, &xf, _device, _maxFrames, &_ctx) != SSD_OK)
+  if(ssd_gpu_create_bev(&cfg, _config.bevWidth(), _config.bevHeight(), &xf, _device, _maxFrames, &_ctx) != SSD_OK)
     throw std::runtime_error(std::string("ssd_gpu_create: ") + ssd_gpu_last_error(nullptr)); // no CPU fallback
 }
 

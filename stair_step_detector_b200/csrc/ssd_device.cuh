@@ -19,15 +19,15 @@
 // Constant per-context parameters, passed to every kernel by value (__grid_constant__).
 struct DevParams
 {
-  int W, H, N;             // image size, points per frame
+  int W, H, N;             // BEV image size; points per frame (FW * FH)
   int wpr;                 // 32-bit words per BEV bitmap row
   int n_bins;              // HeightsHistogram size (pointcloud.cpp:196)
   int min_height;          // ProcessingConfiguration::minHeight (pointcloud.cpp:102)
   int min_img_y_extent;    // (pointcloud.cpp:103)
   unsigned min_peak_points;
   int bev_slots;           // BEV bitmaps per frame
-  int tiles_per_frame;
-  int pad0, pad1;
+  int tiles_per_frame;     // of the frame's N points
+  int FW, FH;              // frame size: pixel grid of the input, the labels and the depth deprojection
   double a[9], b[3];       // CameraToWorld
   double ext_a[4], ext_b[2], ext_z;
   double x_min, x_max, y_min, y_max, z_min, z_max;

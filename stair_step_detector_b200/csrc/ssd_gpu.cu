@@ -78,7 +78,7 @@ struct ssd_gpu_ctx
   ssd_gpu_timing timing{};
   std::string err;
   // single-stage scratch
-  unsigned char *d_img = nullptr;
+  unsigned char *d_img = nullptr; // a BEV image (W x H of the BEV)
   // optional per-kernel events (SSD_FLAG_STAGE_TIMING): (SSD_GPU_N_STAGES + 1) per chunk
   std::vector<cudaEvent_t> stage_ev;
   int stage_chunks = 0;
@@ -143,28 +143,37 @@ static int fail(ssd_gpu_ctx *ctx, int code, const std::string &msg)
   return code;
 }
 
-// ProcessingConfiguration / Projection2D (pointcloud.cpp:60-106)
-static int derive_params(const ssd_gpu_config &c, const ssd_gpu_transform &t, DevParams &d)
+// The largest frame: N <= 9348 * 5108 points (the largest frame of a context whose BEV is its frame size), which keeps the
+// 32-bit point counters of a frame group exact (DESIGN.md, frame groups)
+#define SSD_MAX_FRAME_POINTS (9348LL * 5108LL)
+
+// ProcessingConfiguration / Projection2D (pointcloud.cpp:60-106) for frames of c.width x c.height pixels and a BEV image of bw x bh
+// pixels: the frame fields (N, FW, FH, tiles_per_frame) address the input, every image-pixel field is the BEV's
+static int derive_params(const ssd_gpu_config &c, int bw, int bh, const ssd_gpu_transform &t, DevParams &d)
 {
   memset(&d, 0, sizeof(d));
-  if(c.width <= 0 || c.height <= 0 || !(c.x_max > c.x_min) || !(c.y_max > c.y_min) || !(c.z_max > c.z_min) || !(c.height_interval > 0))
+  if(c.width <= 0 || c.height <= 0 || bw <= 0 || bh <= 0 || !(c.x_max > c.x_min) || !(c.y_max > c.y_min) || !(c.z_max > c.z_min) ||
+     !(c.height_interval > 0))
     return SSD_E_INVALID_ARG;
-  d.W = c.width;
-  d.H = c.height;
-  d.N = c.width * c.height;
-  d.wpr = (c.width + 31) / 32;
+  const long long n_frame = (long long)c.width * c.height;
+  d.W = bw;
+  d.H = bh;
+  d.N = (int)std::min<long long>(n_frame, INT32_MAX); // (refused below when it exceeds SSD_MAX_FRAME_POINTS)
+  d.FW = c.width;
+  d.FH = c.height;
+  d.wpr = (int)(((long long)bw + 31) / 32); // (64-bit: a BEV past the limits is refused below, after these are derived)
   d.hir = 1.0 / c.height_interval;
   d.min_height = (uint16_t)((c.min_height_above_ground - c.z_min) * d.hir);
-  d.min_img_y_extent = (int)(c.min_step_depth * c.height / (c.y_max - c.y_min));
-  d.x_to_image = c.width / (c.x_max - c.x_min);
-  d.y_to_image = c.height / (c.y_max - c.y_min);
+  d.min_img_y_extent = (int)(c.min_step_depth * bh / (c.y_max - c.y_min));
+  d.x_to_image = bw / (c.x_max - c.x_min);
+  d.y_to_image = bh / (c.y_max - c.y_min);
   d.x_to_world = 1 / d.x_to_image;
   d.y_to_world = 1 / d.y_to_image;
   d.xy_ratio = d.x_to_image / d.y_to_image;
   d.n_bins = (int)((size_t)((c.z_max - c.z_min) * d.hir) + 1);
   d.min_peak_points = c.min_peak_points;
   d.bev_slots = SSD_GPU_MAX_PLATEAUS;
-  d.tiles_per_frame = (d.N + SSD_TILE_POINTS - 1) / SSD_TILE_POINTS;
+  d.tiles_per_frame = (int)(((long long)d.N + SSD_TILE_POINTS - 1) / SSD_TILE_POINTS);
   memcpy(d.a, t.a, sizeof(d.a));
   memcpy(d.b, t.b, sizeof(d.b));
   memcpy(d.ext_a, t.ext_a, sizeof(d.ext_a));
@@ -284,12 +293,12 @@ static int derive_params(const ssd_gpu_config &c, const ssd_gpu_transform &t, De
     {
       // ground BEV columns W/2 - 2 + 50 j + {0..4}: f32 pre-filter with a conservative margin (pixel error of the f32
       // world x: epsc * sx, plus the rounding of the filter's own arithmetic)
-      const double gd = ((double)d.epsc * sx * 1.0001 + 8.0 * c.width / 16777216.0 + 1e-3) / 50.0;
+      const double gd = ((double)d.epsc * sx * 1.0001 + 8.0 * bw / 16777216.0 + 1e-3) / 50.0;
       d.gcol_a = (float)(sx / 50.0);
-      d.gcol_b = (float)((-c.x_min * sx - (c.width / 2 - 2)) / 50.0);
+      d.gcol_b = (float)((-c.x_min * sx - (bw / 2 - 2)) / 50.0);
       d.gcol_lo = (float)(0.1 + gd);
       d.gcol_hi = (float)(1.0 - gd);
-      d.gcol_tmax = (float)((c.width - 2 - (c.width / 2 - 2)) / 50.0 - gd);
+      d.gcol_tmax = (float)((bw - 2 - (bw / 2 - 2)) / 50.0 - gd);
     }
     for(int j = 0; j < 3; j++)
     {
@@ -303,9 +312,12 @@ static int derive_params(const ssd_gpu_config &c, const ssd_gpu_transform &t, De
   }
   if(d.n_bins < 3 || d.n_bins > SSD_GPU_MAX_BINS)
     return SSD_E_RANGE;
-  if(d.N % 16 != 0)
+  if(n_frame % 16 != 0)
     return SSD_E_INVALID_ARG; // vertices are loaded four at a time (three 16-byte loads), labels sixteen at a time
-  if(c.width / 25 + 4 > SSD_MAX_SCANS || c.width / 50 + 6 > SSD_MAX_LINE_PTS || c.height / 10 + 2 > SSD_MAX_VPTS)
+  // the BEV: column scans, front-edge line points and vertical probes of the outline (ssd_kernels_outline.cuh)
+  if(bw / 25 + 4 > SSD_MAX_SCANS || bw / 50 + 6 > SSD_MAX_LINE_PTS || bh / 10 + 2 > SSD_MAX_VPTS)
+    return SSD_E_RANGE;
+  if(n_frame > SSD_MAX_FRAME_POINTS)
     return SSD_E_RANGE;
   return SSD_OK;
 }
@@ -720,6 +732,14 @@ void ssd_gpu_destroy(ssd_gpu_ctx *ctx)
 
 int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int device, int max_frames, ssd_gpu_ctx **out)
 {
+  if(!cfg)
+    return fail(nullptr, SSD_E_INVALID_ARG, "ssd_gpu_create: bad argument");
+  return ssd_gpu_create_bev(cfg, cfg->width, cfg->height, xf, device, max_frames, out);
+}
+
+int ssd_gpu_create_bev(const ssd_gpu_config *cfg, int32_t bev_width, int32_t bev_height, const ssd_gpu_transform *xf, int device, int max_frames,
+                       ssd_gpu_ctx **out)
+{
   if(!cfg || !xf || !out || max_frames <= 0)
     return fail(nullptr, SSD_E_INVALID_ARG, "ssd_gpu_create: bad argument");
   *out = nullptr;
@@ -729,9 +749,10 @@ int ssd_gpu_create(const ssd_gpu_config *cfg, const ssd_gpu_transform *xf, int d
   if(device < 0 || device >= ndev)
     return fail(nullptr, SSD_E_INVALID_ARG, "ssd_gpu_create: bad device index");
   DevParams dp;
-  const int rc = derive_params(*cfg, *xf, dp);
+  const int rc = derive_params(*cfg, bev_width, bev_height, *xf, dp);
   if(rc)
-    return fail(nullptr, rc, "ssd_gpu_create: configuration out of range (3 <= height bins <= 253, width*height % 16 == 0, width <= 4700, height <= 5100)");
+    return fail(nullptr, rc, "ssd_gpu_create: configuration out of range (3 <= height bins <= 253, frame width*height % 16 == 0 and at most "
+                             "9348*5108, BEV width <= 9349, BEV height <= 5109)");
 
   ssd_gpu_ctx *ctx = new ssd_gpu_ctx();
   ctx->device = device;
@@ -882,7 +903,7 @@ static int build_ray_table(ssd_gpu_ctx *ctx, const ssd_gpu_intrinsics &in, const
   cudaError_t e = cudaMemsetAsync(d_bad, 0, sizeof(unsigned), st);
   if(e == cudaSuccess)
   {
-    k_lens_rays<<<(int)std::min<size_t>(((size_t)p.N + 255) / 256, 4096), 256, 0, st>>>(p.W, p.H, in, d, ray, d_bad);
+    k_lens_rays<<<(int)std::min<size_t>(((size_t)p.N + 255) / 256, 4096), 256, 0, st>>>(p.FW, p.FH, in, d, ray, d_bad);
     e = cudaGetLastError();
   }
   if(e == cudaSuccess)
@@ -915,18 +936,18 @@ static int ensure_deproject_tables(ssd_gpu_ctx *ctx, const ssd_gpu_intrinsics &i
   const DevParams &p = ctx->dp;
   if(!(in.fx != 0.f) || !(in.fy != 0.f) || !(in.depth_unit > 0.f))
     return fail(ctx, SSD_E_INVALID_ARG, "depth input: fx, fy must be non-zero and depth_unit positive");
-  if(p.W % 4 != 0)
+  if(p.FW % 4 != 0)
     return fail(ctx, SSD_E_INVALID_ARG, "depth input: the frame width must be a multiple of 4");
   if(!ctx->d_xn)
   {
-    CK(cudaMalloc(&ctx->d_xn, sizeof(float) * (size_t)p.W));
-    CK(cudaMalloc(&ctx->d_yn, sizeof(float) * (size_t)p.H));
+    CK(cudaMalloc(&ctx->d_xn, sizeof(float) * (size_t)p.FW));
+    CK(cudaMalloc(&ctx->d_yn, sizeof(float) * (size_t)p.FH));
     memset(&ctx->intr, 0, sizeof(ctx->intr));
   }
   if(memcmp(&ctx->intr, &in, sizeof(float) * 5) != 0)
   {
-    const int n = std::max(p.W, p.H);
-    k_deproject_tables<<<(n + 255) / 256, 256, 0, ctx->stream[0]>>>(p.W, p.H, in, ctx->d_xn, ctx->d_yn);
+    const int n = std::max(p.FW, p.FH);
+    k_deproject_tables<<<(n + 255) / 256, 256, 0, ctx->stream[0]>>>(p.FW, p.FH, in, ctx->d_xn, ctx->d_yn);
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(ctx->stream[0])); // every stream reads the tables
     ctx->intr = in;
@@ -1013,9 +1034,12 @@ static int check_call(ssd_gpu_ctx *ctx, ProcessCall &c)
                                                             " frames, more than max_frames of the context"
                                                       : "process: n_frames exceeds max_frames of the context");
   c.n_frames = (int)n_frames;
-  // 5. the frame width of depth input: one load per 4-pixel word
-  if(depth && ctx->dp.W % 4 != 0)
+  // 5. the frame width of depth input: one load per 4-pixel word; the point kernels divide a pixel index by the width with a 40-bit
+  // reciprocal (wmagic), exact for every index of the frame when N * W < 2^40
+  if(depth && ctx->dp.FW % 4 != 0)
     return fail(ctx, SSD_E_INVALID_ARG, "depth input: the frame width must be a multiple of 4");
+  if(depth && (unsigned long long)ctx->dp.N * (unsigned long long)ctx->dp.FW >= (1ull << 40))
+    return fail(ctx, SSD_E_INVALID_ARG, "depth input: the frame's points times its width must stay below 2^40 (row division)");
   // 6. each frame's camera
   for(int f = 0; f < c.n_frames && c.mode != CALL_PLAIN; f++)
   {
@@ -1254,7 +1278,7 @@ static int process(ssd_gpu_ctx *ctx, ProcessCall c)
       // The call's one source: vertices, or depth frames deprojected inside the point kernels, with the pin-hole tables (a camera
       // call's per camera) or the rays of a distorted lens. Each chunk sets the input pointer.
       const float unit = c.intr ? c.intr->depth_unit : 0.f;
-      const unsigned long long wmagic = (((unsigned long long)1 << 40) + (unsigned long long)p.W - 1) / (unsigned long long)p.W;
+      const unsigned long long wmagic = (((unsigned long long)1 << 40) + (unsigned long long)p.FW - 1) / (unsigned long long)p.FW;
       const auto run_depth = [&](auto sample, const auto &cam) -> int {
         typedef decltype(sample) T;
         if(use_lens)
@@ -1477,7 +1501,7 @@ int ssd_gpu_set_cameras_ex(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, const s
   std::vector<unsigned char> depth_ok((size_t)n_cameras);
   for(int c = 0; c < n_cameras; c++)
   {
-    if(derive_params(ctx->cfg, cams[c].xf, dp[c]))
+    if(derive_params(ctx->cfg, ctx->dp.W, ctx->dp.H, cams[c].xf, dp[c]))
       return fail(ctx, SSD_E_INVALID_ARG, "ssd_gpu_set_cameras: camera " + std::to_string(c) + ": transform out of range");
     const ssd_gpu_intrinsics &in = cams[c].intr;
     OverlayDev &o = ov[c];
@@ -1518,8 +1542,8 @@ int ssd_gpu_set_cameras_ex(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, const s
   CK(cudaMalloc(&ctx->d_cam_dp, sizeof(DevParams) * (size_t)n_cameras));
   CK(cudaMalloc(&ctx->d_cam_ov, sizeof(OverlayDev) * (size_t)n_cameras));
   CK(cudaMalloc(&ctx->d_cam_unit, sizeof(float) * (size_t)n_cameras));
-  CK(cudaMalloc(&ctx->d_cam_xn, sizeof(float) * (size_t)n_cameras * p.W));
-  CK(cudaMalloc(&ctx->d_cam_yn, sizeof(float) * (size_t)n_cameras * p.H));
+  CK(cudaMalloc(&ctx->d_cam_xn, sizeof(float) * (size_t)n_cameras * p.FW));
+  CK(cudaMalloc(&ctx->d_cam_yn, sizeof(float) * (size_t)n_cameras * p.FH));
   CK(cudaMalloc(&d_in, sizeof(ssd_gpu_camera) * (size_t)n_cameras));
   CK(cudaMalloc(&ctx->d_cam_lens, sizeof(ssd_gpu_distortion) * (size_t)n_cameras));
   CK(cudaMalloc(&ctx->d_cam_ray, sizeof(float2 *) * (size_t)n_cameras));
@@ -1538,8 +1562,8 @@ int ssd_gpu_set_cameras_ex(ssd_gpu_ctx *ctx, const ssd_gpu_camera *cams, const s
   if(e == cudaSuccess)
   {
     // (cameras without depth intrinsics get meaningless tables: depth calls never use them)
-    const int n = std::max(p.W, p.H);
-    k_deproject_tables_cams<<<dim3((n + 255) / 256, std::min(n_cameras, 65535)), 256, 0, st>>>(p.W, p.H, d_in, n_cameras, ctx->d_cam_xn, ctx->d_cam_yn);
+    const int n = std::max(p.FW, p.FH);
+    k_deproject_tables_cams<<<dim3((n + 255) / 256, std::min(n_cameras, 65535)), 256, 0, st>>>(p.FW, p.FH, d_in, n_cameras, ctx->d_cam_xn, ctx->d_cam_yn);
     e = cudaGetLastError();
   }
   if(e == cudaSuccess)
@@ -1685,7 +1709,7 @@ int ssd_gpu_deproject_device(ssd_gpu_ctx *ctx, const uint16_t *z16_dev, const ss
                                                                                   xyz_dev + (size_t)f0 * p.N * 3);
       continue;
     }
-    k_deproject<<<dim3((p.N / 4 + 255) / 256, nf), 256, 0, ctx->stream[0]>>>(p.W, p.N, intr->depth_unit, ctx->d_xn, ctx->d_yn, z16_dev + (size_t)f0 * p.N,
+    k_deproject<<<dim3((p.N / 4 + 255) / 256, nf), 256, 0, ctx->stream[0]>>>(p.FW, p.N, intr->depth_unit, ctx->d_xn, ctx->d_yn, z16_dev + (size_t)f0 * p.N,
                                                                             xyz_dev + (size_t)f0 * p.N * 3);
   }
   CK(cudaGetLastError());
@@ -2121,10 +2145,11 @@ int ssd_gpu_labels_device_ptr(ssd_gpu_ctx *ctx, const uint8_t **out)
 static int upload_image(ssd_gpu_ctx *ctx, const uint8_t *image_host)
 {
   const DevParams &p = ctx->dp;
+  const size_t bev_pixels = (size_t)p.W * p.H;
   CK(cudaSetDevice(ctx->device));
   if(!ctx->d_img)
-    CK(cudaMalloc(&ctx->d_img, (size_t)p.N));
-  CK(cudaMemcpyAsync(ctx->d_img, image_host, (size_t)p.N, cudaMemcpyHostToDevice, ctx->stream[0]));
+    CK(cudaMalloc(&ctx->d_img, bev_pixels));
+  CK(cudaMemcpyAsync(ctx->d_img, image_host, bev_pixels, cudaMemcpyHostToDevice, ctx->stream[0]));
   const int words = p.H * p.wpr;
   k_pack_bitmap<<<(words + 255) / 256, 256, 0, ctx->stream[0]>>>(p, ctx->d_img, ctx->d_bev);
   CK(cudaGetLastError());

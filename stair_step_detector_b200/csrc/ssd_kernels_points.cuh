@@ -252,7 +252,7 @@ __device__ __forceinline__ FrameD<T> src_frame(const SrcDepthT<T> &s, const DevP
   f.yn = s.yn;
   f.unit = s.unit;
   f.wmagic = s.wmagic;
-  f.W = (unsigned)p.W;
+  f.W = (unsigned)p.FW;
   return f;
 }
 // The source of one frame: in camera mode a depth frame is deprojected with its own camera's tables and depth unit.
@@ -270,8 +270,8 @@ __device__ __forceinline__ SrcDepthT<T> frame_src(const SrcDepthT<T> &s, const C
 {
   const int cam = frame_camera(c, frame);
   SrcDepthT<T> d = s;
-  d.xn = c.xn + (size_t)cam * p.W;
-  d.yn = c.yn + (size_t)cam * p.H;
+  d.xn = c.xn + (size_t)cam * p.FW;
+  d.yn = c.yn + (size_t)cam * p.FH;
   d.unit = __ldg(c.unit + cam);
   return d;
 }
